@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the MC variational-BNN hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--engine tc|simt]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--engine tc|simt] [--dump-outputs DIR]
 
 Headline workload (config.workload): the LRT experiment's Inception BNN (experiment=ncmapss_lrt,
 q_scale 1.351e-3, prior 0.138793) predicting B=10 000 synthetic N-CMAPSS windows [30x18] with S=100
@@ -17,6 +17,9 @@ over the ranks + moment merge), "deep_ensemble" (five members as one launch) and
 (configs[4] at its stated scale: 1M windows, 5 members + LRT BNN at S=1000, members / samples sharded
 over the ranks, NCCL moment merges inside the timed region).  One process per GPU; windows are sharded across ranks, no data-path collective in the
 headline (weak scaling).  Only the JSON line is written to stdout.
+--dump-outputs DIR: after the timed headline steps, the (pred, std, ep_var, al_var) vectors of the last one are
+written as DIR/<name>.npy (float32, 4 x 40 KB per rank; `_rank<r>` suffix when several ranks run).  Inputs, weights
+and noise are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -30,6 +33,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 NET = "inception"
@@ -124,6 +128,14 @@ def timed_steps(fn, steps, warmup, flush_buf, dist):
         dist.barrier()
     torch.cuda.synchronize()
     return sum(a.elapsed_time(b) for a, b in evs) / 1e3
+
+
+def dump_outputs(out_dir, arrays, rank, world):
+    """Each [B] result tensor as out_dir/<name>.npy in float32 (<name>_rank<r>.npy when several ranks run)."""
+    os.makedirs(out_dir, exist_ok=True)
+    suffix = f"_rank{rank}" if world > 1 else ""
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}{suffix}.npy"), a.detach().float().cpu().numpy())
 
 
 def max_over_ranks(t, dist, device):
@@ -230,7 +242,12 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-train", action="store_true")
     ap.add_argument("--no-full", action="store_true", help="skip the 1M-window configs[4] pass (about 5 s at one GPU)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed headline step's results as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the CUDA path's results; the reference arm computes a bounded sample")
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
     local = int(os.environ.get("LOCAL_RANK", 0))
@@ -287,6 +304,8 @@ def main():
         eng.tc_timing(False)
     launches = lib.brl_launch_count() - l0
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dict(zip(("pred", "std", "ep_var", "al_var"), outs["m"])), rank, world)
     launches_timed = launches * args.steps // (args.steps + args.warmup)  # warm-up steps launch the same kernels
     t = max_over_ranks(t_local, dist, device)
     units_per_step = B_PRED * S_PRED

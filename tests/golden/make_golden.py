@@ -1,15 +1,18 @@
-"""Generate tests/golden/*.npz from the reference's OWN code (run in the dev container only).
+"""Generate tests/golden/*.npz from the reference's OWN code.
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py <path of the reference's `bayesrul` package directory>
 
-Imports (read-only) /root/reference/bayesrul/models/nets/{inception,conv,linear}.py (with a stub
+Imports (read-only) <bayesrul>/models/nets/{inception,conv,linear}.py (with a stub
 `torchinfo`), models/deepens.py and utils/miscellaneous.py, runs them on seeded inputs and stores
-inputs + outputs.  Nothing from /root/reference is copied into the repo; the fixtures are the
-reference's numerical behaviour.  TyXe / Pyro are not importable, so for the LRT / Flipout / weight
--sampling fixtures the reference nets are executed with `torch.nn.functional.{conv1d,conv2d,linear}`
-patched by the published per-call rule (SURVEY Appendix A.3/A.4) -- this pins the *composition*
-(which call sees which tensor, in which order) on the reference's module code, while the per-call
-rule itself stays "parity unpinned".
+inputs + outputs.  Nothing from the reference is copied into the repo; the fixtures are the
+reference's numerical behaviour.  The parameter-sized inputs (theta, ws_eps) and the LRT noise are
+stored as a SHA-256 of their values and sigma as its constant, which keeps every fixture small:
+tests/helpers.load_golden regenerates them from the same seeds and checks each against its digest.
+TyXe / Pyro are not importable, so for the LRT / Flipout / weight-sampling fixtures the reference
+nets are executed with `torch.nn.functional.{conv1d,conv2d,linear}` patched by the published
+per-call rule (SURVEY Appendix A.3/A.4) -- this pins the *composition* (which call sees which
+tensor, in which order) on the reference's module code, while the per-call rule itself stays
+"parity unpinned".
 """
 import importlib.util
 import os
@@ -21,8 +24,12 @@ import torch
 import torch.nn as nn
 import torch.nn.functional as F
 
-REF = "/root/reference/bayesrul"
+if len(sys.argv) != 2:
+    sys.exit(__doc__)
+REF = sys.argv[1]
 OUT = os.path.dirname(os.path.abspath(__file__))
+sys.path.insert(0, os.path.dirname(os.path.dirname(OUT)))
+from tests.helpers import golden_digest  # noqa: E402
 
 
 def _load(name, path):
@@ -116,7 +123,7 @@ def main():
         names = [n for n, _ in m.named_parameters()]
         shapes = [tuple(p.shape) for _, p in m.named_parameters()]
         x = torch.randn(B, 30, 18, generator=g)
-        fx = {"theta": theta.numpy(), "x": x.numpy(), "names": np.array(names),
+        fx = {"theta_sha256": np.array(golden_digest(theta)), "x": x.numpy(), "names": np.array(names),
               "shapes": np.array([str(s) for s in shapes])}
         with torch.no_grad():
             fx["out_det"] = m(x).numpy()
@@ -148,8 +155,9 @@ def main():
         loc, scale = out[:, :, 0], out[:, :, 1]
         ep_var = loc.var(0)
         al_var = (scale**2).mean(0)
-        fx.update(sigma=sigma.numpy(), ws_eps=eps.numpy(), out_ws=out.numpy(), ep_var=ep_var.numpy(),
-                  al_var=al_var.numpy(), std=al_var.add(ep_var).sqrt().numpy(), pred=loc.mean(0).numpy())
+        fx.update(sigma_value=sigma[0].numpy(), ws_eps_sha256=np.array(golden_digest(eps)), out_ws=out.numpy(),
+                  ep_var=ep_var.numpy(), al_var=al_var.numpy(), std=al_var.add(ep_var).sqrt().numpy(),
+                  pred=loc.mean(0).numpy())
 
         # ---- LRT (A5): per-call rule of SURVEY A.3 patched into the reference forward
         off, lay_w = 0, []
@@ -169,8 +177,8 @@ def main():
 
         with torch.no_grad(), Patched(lrt_rule):
             fx["out_lrt"] = m(x).numpy()
-        for i, e in enumerate(lrt_eps):
-            fx[f"lrt_eps_call{i}"] = e.numpy()
+        fx["lrt_eps_shapes"] = np.array([str(tuple(e.shape)) for e in lrt_eps])
+        fx["lrt_eps_sha256"] = np.array([golden_digest(e) for e in lrt_eps])
 
         # ---- Flipout (A6): per-call rule of SURVEY A.4
         w_s = theta + sigma * eps[0]

@@ -7,6 +7,10 @@ import sys
 import types
 from contextlib import redirect_stdout
 
+import numpy as np
+import pytest
+import torch
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -39,6 +43,27 @@ def test_reference_arm_line(monkeypatch):
     with redirect_stdout(buf):
         bench.run_reference(args, rank=1, world=2)
     assert buf.getvalue() == ""
+
+
+def test_dump_outputs_files(tmp_path):
+    bench = _bench()
+    m = (torch.arange(4.0), torch.ones(4), torch.zeros(4), torch.full((4,), 2.0))
+    bench.dump_outputs(str(tmp_path / "one"), dict(zip(("pred", "std", "ep_var", "al_var"), m)), rank=0, world=1)
+    assert sorted(os.listdir(tmp_path / "one")) == ["al_var.npy", "ep_var.npy", "pred.npy", "std.npy"]
+    got = np.load(tmp_path / "one" / "pred.npy")
+    assert got.dtype == np.float32 and got.tolist() == [0.0, 1.0, 2.0, 3.0]
+    bench.dump_outputs(str(tmp_path / "two"), {"pred": m[0]}, rank=1, world=2)
+    assert os.listdir(tmp_path / "two") == ["pred_rank1.npy"]
+
+
+def test_bad_arguments_stop_before_any_gpu_work(monkeypatch, capsys):
+    bench = _bench()
+    for argv in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "out"]):
+        monkeypatch.setattr(sys, "argv", ["bench.py", *argv])
+        with pytest.raises(SystemExit) as e:
+            bench.main()
+        assert e.value.code == 2
+    assert capsys.readouterr().out == ""
 
 
 def test_both_arms_share_the_workload_config():

@@ -7,7 +7,7 @@ import pytest
 import torch
 
 from oracle import bnn_oracle as O
-from tests.helpers import assert_close, injected_to_engine, synth
+from tests.helpers import assert_close, injected_to_engine, synth, load_golden as _fx
 
 pytestmark = pytest.mark.gpu
 NETS = ["inception", "conv", "linear"]
@@ -19,11 +19,6 @@ DEV = "cuda:0"
 def engines():
     from bayesrul_b200 import Engine
     return {n: Engine(n, DEV) for n in NETS}
-
-
-def _fx(golden_dir, net):
-    z = np.load(os.path.join(golden_dir, f"{net}.npz"))
-    return {k: z[k] for k in z.files}
 
 
 def _t(a):

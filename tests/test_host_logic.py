@@ -5,12 +5,14 @@ import numpy as np
 import pytest
 import torch
 
+from tests.helpers import load_golden
+
 
 @pytest.mark.parametrize("kind", ["inception", "conv", "linear"])
 def test_state_dict_keys_match_reference(golden_dir, kind):
     from bayesrul_b200.compat import Conv, Inception, Linear
     cls = {"inception": Inception, "conv": Conv, "linear": Linear}[kind]
-    z = np.load(os.path.join(golden_dir, f"{kind}.npz"))
+    z = load_golden(golden_dir, kind)
     net = cls(30, 18)
     assert list(net.state_dict().keys()) == list(z["names"])
     assert [str(tuple(v.shape)) for v in net.state_dict().values()] == list(z["shapes"])

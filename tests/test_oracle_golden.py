@@ -9,14 +9,10 @@ import torch
 import torch.nn.functional as F
 
 from oracle import bnn_oracle as O
+from tests.helpers import load_golden as _load
 
 NETS = ["inception", "conv", "linear"]
 DROP_ORDER = {"inception": [0, 1, 2, 3, 4, 6, 8, 9, 10], "conv": [0, 1, 2], "linear": [0, 1, 2, 3]}
-
-
-def _load(golden_dir, net):
-    z = np.load(os.path.join(golden_dir, f"{net}.npz"))
-    return {k: z[k] for k in z.files}
 
 
 @pytest.mark.parametrize("net", NETS)
