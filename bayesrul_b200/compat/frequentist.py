@@ -41,7 +41,8 @@ class HNN(_Base):
         self.net.apply(weights_init)
         self._engine_kind = engine
         # kernels of HNN.step: "auto" = the level-fused tcgen05 kernels for the Inception net (fp16 / bf16 operands: loss 5e-3,
-        # gradient cosine > 0.999 of the fp32 oracle), the fp32 FFMA kernels for the other nets; "simt" forces the fp32 parity back-end
+        # gradient cosine > 0.999 of the fp32 oracle), the fp32 FFMA kernels for the other nets; "fused" also runs the level-fused
+        # kernels on the Linear net (same bound); "simt" forces the fp32 parity back-end
         self._train_backend = train_backend
         self._it = 0
         if device is not None:

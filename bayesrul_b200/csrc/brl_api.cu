@@ -137,6 +137,9 @@ struct ActBufs {
   // level-fused tcgen05 training kernels (Inception conv stack, brl_tc_train.cu): images of one particle lane
   TtLane tt{};
   bool has_tt = false;
+  // level-fused tcgen05 training kernels of the Linear net (brl_tc_train_linear.cuh): carved last, only where they fit
+  TlLane tl{};
+  bool has_tl = false;
 };
 constexpr int GRAPH_MAX_PARTICLES = 8;
 
@@ -183,6 +186,17 @@ static void carve_train(const NetSpec& n, Carve& c, long long B, ActBufs& ab) {
     if (base) tt_carve(base, B, ab.tt);
     ab.has_tt = base != nullptr;
   }
+}
+
+// images of the Linear net's fused training kernels, behind everything else of the workspace: a workspace sized for the
+// per-layer kernels alone keeps its layout, and a step whose workspace has no room for them runs the per-layer kernels
+static void carve_tl(const NetSpec& n, Carve& c, long long B, ActBufs& ab) {
+  if (n.id != BRL_NET_LINEAR) return;
+  const size_t bytes = ((size_t)tl_lane_bytes(B) + 255) & ~(size_t)255;
+  if (c.base && (!c.ok || c.used + bytes > c.cap)) return;
+  unsigned char* base = c.take<unsigned char>((long long)bytes);
+  if (base) tl_carve(base, B, ab.tl);
+  ab.has_tl = base != nullptr;
 }
 
 // device {seed, sample0, window0} of the step being captured (nullptr outside a capture): every Philox stream built by
@@ -752,10 +766,14 @@ int64_t brl_workspace_bytes(const brl_ctx* ctx, int64_t B, int64_t S, int train,
   if (engine == BRL_ENGINE_TC_FP16) c.used += tc_workspace_bytes(ctx->tc, B, S);
   else carve_forward(n, c, B, S, ab);
   if (train == 1) carve_train(n, c, B, ab);
+  ActBufs ab1;
   if (train == 1 && S >= 2) {  // second lane of brl_elbo_step: two particles side by side
-    ActBufs ab1;
     carve_forward(n, c, B, 1, ab1);
     carve_train(n, c, B, ab1);
+  }
+  if (train == 1) {  // fused Linear-net images of the lanes (brl_elbo_step / brl_hnn_step carve them last)
+    carve_tl(n, c, B, ab);
+    if (S >= 2) carve_tl(n, c, B, ab1);
   }
   if (train == 2)  // brl_forward in BRL_MODE_FLIPOUT with native signs: [S,B,Cin] + [S,B,Cout] per layer
     for (const LayerSpec& L : n.layers) { c.take<float>(S * B * L.cin); c.take<float>(S * B * L.cout); }
@@ -1133,13 +1151,16 @@ static int elbo_body(brl_ctx* ctx, const ActBufs* const* lanes, int n_lanes, con
       const bool use_tt = ctx->gemm_backend == BRL_GEMM_TC_FUSED && n.id == BRL_NET_INCEPTION && ab.has_tt &&
                           (mode == BRL_MODE_LRT || mode == BRL_MODE_FLIPOUT || mode == BRL_MODE_WS) &&
                           2 * B * 64 <= SPLITK_SCRATCH_FLOATS;  // fc partial sums live in the split-K scratch (B <= 4736), else per-layer
+      // the Linear net's four hidden layers on the tensor pipe, the head in the same tail kernel (width 32)
+      const bool use_tl = ctx->gemm_backend == BRL_GEMM_TC_FUSED && n.id == BRL_NET_LINEAR && ab.has_tl &&
+                          (mode == BRL_MODE_LRT || mode == BRL_MODE_FLIPOUT || mode == BRL_MODE_WS);
       if (compute_grads) {  // a dozen memsets: on a side stream underneath the forward pass, joined before the NLL
         cudaStream_t zs = ctx->multi_stream ? ln.zero : ls;
         if (zs != ls) {
           BRL_CUDA(cudaEventRecord(ln.ev_zero, ls));
           BRL_CUDA(cudaStreamWaitEvent(zs, ln.ev_zero, 0));
         }
-        if (!use_tt) {  // the fused back-end keeps its gradients in bf16 images that are written, not accumulated
+        if (!use_tt && !use_tl) {  // the fused back-end keeps its gradients in bf16 images that are written, not accumulated
           int rc = zero_grads(n, ab, B, zs);
           if (rc) return rc;
         }
@@ -1165,6 +1186,18 @@ static int elbo_body(brl_ctx* ctx, const ActBufs* const* lanes, int n_lanes, con
         const TtSide tsd{ln.side[0], ln.ev_fork, ln.ev_join[0]};
         tt_forward(ab.tt, ts, ls, tsd);
         tt_fc_forward(ab.tt, ts, ab.part[0], ls);
+      } else if (use_tl) {
+        ts.x = x; ts.B = B; ts.mode = mode; ts.mu = mode == BRL_MODE_WS ? ab.wsamp : mu; ts.sigma = sigma; ts.wsamp = ab.wsamp;
+        for (int ly = 0; ly < 4; ++ly) {
+          ts.eps[ly] = nref(&nz, nz.lrt_eps[ly], KIND_LRT_EPS, (unsigned)ly);
+          ts.keep[ly] = 1.0f;
+          ts.sgn_out[ly] = sout_[ly];
+          ts.w_off[ly] = n.layers[ly].w_off; ts.b_off[ly] = n.layers[ly].b_off;
+        }
+        for (int ly = 0; ly < 5; ++ly) ts.sgn_in[ly] = sin_[ly];
+        ts.w_off_fc = n.layers[3].w_off; ts.b_off_fc = n.layers[3].b_off;
+        ts.g0 = ab.g0; ts.g1 = ab.g1;
+        tl_forward(ab.tl, ts, ls, TtSide{ln.side[0], ln.ev_fork, ln.ev_join[0]});
       } else {
         run_forward(ctx, ab, fa, ls, l);
       }
@@ -1179,6 +1212,15 @@ static int elbo_body(brl_ctx* ctx, const ActBufs* const* lanes, int n_lanes, con
         tl.sout_fc = sout_[fc_layer]; tl.sin_head = sin_[hd_layer]; tl.sout_head = sout_[hd_layer];
         tl.hw_off = n.layers[hd_layer].w_off; tl.hb_off = n.layers[hd_layer].b_off;
         tt_tail(ts, tl, ls);
+      } else if (use_tl) {
+        TtTail tl{};
+        tl.part = ab.tl.part; tl.width = 32; tl.y = y; tl.gscale = (float)(c_nll / particles); tl.compute_grads = compute_grads;
+        tl.acc = ab0.acc; tl.out = outp; tl.dpre = ab.dpre[3]; tl.dsec = ab.dsec[3];
+        tl.eps_fc = nref(&nz, nz.lrt_eps[3], KIND_LRT_EPS, 3u);
+        tl.eps_head = nref(&nz, nz.lrt_eps[4], KIND_LRT_EPS, 4u);
+        tl.sout_fc = sout_[3]; tl.sin_head = sin_[4]; tl.sout_head = sout_[4];
+        tl.hw_off = n.layers[4].w_off; tl.hb_off = n.layers[4].b_off;
+        tt_tail(ts, tl, ls);
       } else {
         launch_nll_elbo(outp, y, B, (float)(c_nll / particles), ab0.acc, compute_grads ? ab.grad[n.out_buf] : nullptr, ls);
       }
@@ -1189,6 +1231,8 @@ static int elbo_body(brl_ctx* ctx, const ActBufs* const* lanes, int n_lanes, con
           const TtSide tsd{ln.side[0], ln.ev_fork, ln.ev_join[0]};
           tt_fc_backward(ab.tt, ts, ab.dpre[fc_op], ab.dsec[fc_op], ls, tsd);
           tt_backward(ab.tt, ts, ls, tsd);
+        } else if (use_tl) {
+          tl_backward(ab.tl, ts, ab.dpre.data(), ab.dsec.data(), ls, TtSide{ln.side[0], ln.ev_fork, ln.ev_join[0]});
         } else {
           run_backward(ctx, ab, ba, ls, l);
         }
@@ -1257,6 +1301,11 @@ int brl_elbo_step(brl_ctx* ctx, const float* x, const float* y, int64_t B, const
     carve_forward(n, c, B, 1, ab1);
     carve_train(n, c, B, ab1);
     if (c.ok) n_lanes = 2;
+  }
+  carve_tl(n, c, B, ab);
+  if (n_lanes == 2) {
+    carve_tl(n, c, B, ab1);
+    if (!ab1.has_tl) ab.has_tl = false;  // both particle lanes run the same back-end
   }
   const ActBufs* lanes[2] = {&ab, &ab1};
   // ---- graph replay (native Philox noise): eager on first sight of a configuration, captured on the second, replayed after
@@ -1379,6 +1428,33 @@ static int hnn_body(brl_ctx* ctx, const ActBufs& ab, const float* x, const float
     BRL_CUDA(cudaGetLastError());
     return BRL_OK;
   }
+  if (ctx->gemm_backend == BRL_GEMM_TC_FUSED && n.id == BRL_NET_LINEAR && ab.has_tl) {
+    // the Linear net's fused kernels, one contraction with the deterministic weights; keep decisions in the epilogues
+    const brl_ctx::Lane& ln = ctx->lanes[0];
+    auto keep_of = [&](int ly) { return (p_dropout > 0.f && n.layers[ly].drop_factor > 0.f) ? 1.0f - p_dropout * n.layers[ly].drop_factor : 1.0f; };
+    TtStep ts{};
+    ts.x = x; ts.B = B; ts.mode = BRL_MODE_DET; ts.mu = theta;
+    for (int ly = 0; ly < 4; ++ly) {
+      ts.drop[ly] = nref(&nz, nz.drop_mask[ly], KIND_DROPOUT, (unsigned)ly);
+      ts.keep[ly] = keep_of(ly);
+      ts.w_off[ly] = n.layers[ly].w_off; ts.b_off[ly] = n.layers[ly].b_off;
+    }
+    ts.w_off_fc = n.layers[3].w_off; ts.b_off_fc = n.layers[3].b_off;
+    ts.g0 = grad_theta; ts.g1 = nullptr;
+    const TtSide tsd{ln.side[0], ln.ev_fork, ln.ev_join[0]};
+    BRL_CUDA(cudaMemsetAsync(scalars, 0, 2 * sizeof(double), st));
+    if (compute_grads) BRL_CUDA(cudaMemsetAsync(grad_theta, 0, sizeof(float) * n.P, st));
+    tl_forward(ab.tl, ts, st, tsd);
+    TtTail tl{};
+    tl.part = ab.tl.part; tl.width = 32; tl.y = y; tl.gscale = 0.f; tl.compute_grads = compute_grads; tl.acc = scalars; tl.out = out;
+    tl.dpre = ab.dpre[3]; tl.dsec = ab.dsec[3];
+    tl.hw_off = n.layers[4].w_off; tl.hb_off = n.layers[4].b_off;
+    tl.loss_kind = 1; tl.keep_fc = keep_of(3); tl.drop_fc = nref(&nz, nz.drop_mask[3], KIND_DROPOUT, 3u);
+    tt_tail(ts, tl, st);
+    if (compute_grads) tl_backward(ab.tl, ts, ab.dpre.data(), ab.dsec.data(), st, tsd);
+    BRL_CUDA(cudaGetLastError());
+    return BRL_OK;
+  }
   FwdArgs fa{x, B, 1, BRL_MODE_DET, theta, nullptr, nullptr, p_dropout, &nz, nullptr, nullptr, out, false};
   run_forward(ctx, ab, fa, st);
   BRL_CUDA(cudaMemsetAsync(scalars, 0, 2 * sizeof(double), st));
@@ -1410,6 +1486,7 @@ int brl_hnn_step(brl_ctx* ctx, const float* x, const float* y, int64_t B, const 
   carve_forward(n, c, B, 1, ab);
   carve_train(n, c, B, ab);
   if (!c.ok) return fail(BRL_ERR_WORKSPACE, "brl_hnn_step: workspace too small");
+  carve_tl(n, c, B, ab);
   // ---- graph replay, same scheme as brl_elbo_step (native dropout masks or no dropout): eager, capture, replay
   brl_ctx::StepGraph* sg = nullptr;
   bool caller_captures = false;

@@ -1069,6 +1069,7 @@ __global__ void __launch_bounds__(256, 1) tt_fc_dw_kernel(const TtFcBwdArgs a) {
 // gradients) -> activation backward of the fc layer (the compact dpre / dsec tensors of tt_fc_backward).  It replaces eight
 // per-layer launches (split-K epilogue, head GEMM, NLL, two activation-backward, head dX / dW) of 3 - 11 us each; the arithmetic
 // is that of brl_gemm_epi.cuh / nll_elbo_kernel / bwd_act_kernel, one warp per window, lane = hidden units {lane, lane + 32}.
+// HW = width of the hidden layer in front of the head: 64 (Inception fc layer), 32 (Linear layer 3, lane = hidden unit lane).
 // ------------------------------------------------------------------------------------------------
 __device__ __forceinline__ double tt_block_sum(double v) {  // valid in thread 0
   __shared__ double red[32];
@@ -1086,50 +1087,51 @@ __device__ __forceinline__ double tt_block_sum(double v) {  // valid in thread 0
 }
 struct TtTailArgs {
   int B, mode, compute_grads;
-  const float* part;           // [2][B][64] fc partial sums (mean path, second path)
+  const float* part;           // [2][B][HW] fc partial sums (mean path, second path)
   const float *fc_b0, *fc_b1;  // LRT: mu_b, sigma_b of the fc layer; Flipout: fc_b0 = sampled bias
-  const float *hw0, *hw1;      // head weights [2][64]: LRT mu, sigma; Flipout mu, sampled W
+  const float *hw0, *hw1;      // head weights [2][HW]: LRT mu, sigma; Flipout mu, sampled W
   const float *hb0, *hb1;      // head bias [2]:      LRT mu_b, sigma_b; Flipout hb0 = sampled bias
   NoiseRef eps_fc, eps_head;   // LRT
-  const float *sout_fc, *sin_head, *sout_head;  // Flipout [B,64], [B,64], [B,2]
+  const float *sout_fc, *sin_head, *sout_head;  // Flipout [B,HW], [B,HW], [B,2]
   const float* y;
   float gscale;
   double* acc;                 // [0] += nll, [1] += squared error
   float* out;                  // [B,2]
-  float *dpre, *dsec;          // [B,64] compact gradients of the fc layer's pre-activation / second path
+  float *dpre, *dsec;          // [B,HW] compact gradients of the fc layer's pre-activation / second path
   float *g0, *g1;              // flat gradient accumulators (head layer: atomics)
   long long hw_off, hb_off;
   // PLAIN mode (one contraction: HNN / MC-dropout step, weight-sampling ELBO): fc_b0 / hw0 / hb0 are the weights in use
   int loss_kind;               // 0: ELBO likelihood (second softplus, sums in acc); 1: F.gaussian_nll_loss (frequentist.py:39-48, means in acc)
   float keep_fc;               // keep probability of the dropout site behind the fc layer (1 = none)
-  NoiseRef drop_fc;            // its masks: injected [B, 64] or Philox
+  NoiseRef drop_fc;            // its masks: injected [B, HW] or Philox
 };
-template <int MODE>
+template <int MODE, int HW>
 __global__ void __launch_bounds__(256) tt_tail_kernel(const TtTailArgs a) {
-  __shared__ float sg[2][2][64 + 1];  // [path][output][hidden unit | bias] head weight-gradient partials of the CTA
+  __shared__ float sg[2][2][HW + 1];  // [path][output][hidden unit | bias] head weight-gradient partials of the CTA
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  for (int i = tid; i < 2 * 2 * 65; i += 256) (&sg[0][0][0])[i] = 0.f;
+  for (int i = tid; i < 2 * 2 * (HW + 1); i += 256) (&sg[0][0][0])[i] = 0.f;
   __syncthreads();
-  float w0[2][2], w1[2][2];  // head weights of this lane's two hidden units: [output][unit]
+  constexpr int U = HW / 32;  // hidden units per lane
+  float w0[2][U], w1[2][U];  // head weights of this lane's hidden units: [output][unit]
 #pragma unroll
   for (int o = 0; o < 2; ++o)
 #pragma unroll
-    for (int u = 0; u < 2; ++u) {
+    for (int u = 0; u < U; ++u) {
       const int k = lane + 32 * u;
-      const float m = a.hw0[o * 64 + k], v = MODE == TT_PLAIN ? 0.f : a.hw1[o * 64 + k];
+      const float m = a.hw0[o * HW + k], v = MODE == TT_PLAIN ? 0.f : a.hw1[o * HW + k];
       w0[o][u] = m;
       w1[o][u] = MODE == BRL_MODE_LRT ? v * v : v - m;
     }
-  float gw0[2][2] = {{0.f, 0.f}, {0.f, 0.f}}, gw1[2][2] = {{0.f, 0.f}, {0.f, 0.f}}, gb0[2] = {0.f, 0.f}, gb1[2] = {0.f, 0.f};
+  float gw0[2][U] = {}, gw1[2][U] = {}, gb0[2] = {0.f, 0.f}, gb1[2] = {0.f, 0.f};
   double nll = 0.0, se = 0.0;
   const int nwarps = gridDim.x * 8;
   for (int m = blockIdx.x * 8 + warp; m < a.B; m += nwarps) {
     // ---- fc epilogue
-    float h[2], sd[2], ef[2], sgn_in[2];
+    float h[U], sd[U], ef[U], sgn_in[U];
 #pragma unroll
-    for (int u = 0; u < 2; ++u) {
+    for (int u = 0; u < U; ++u) {
       const int k = lane + 32 * u;
-      const float a0 = a.part[(long long)m * 64 + k], a1 = MODE == TT_PLAIN ? 0.f : a.part[((long long)a.B + m) * 64 + k];
+      const float a0 = a.part[(long long)m * HW + k], a1 = MODE == TT_PLAIN ? 0.f : a.part[((long long)a.B + m) * HW + k];
       float pre;
       if (MODE == TT_PLAIN) {
         pre = a0 + a.fc_b0[k];
@@ -1139,33 +1141,33 @@ __global__ void __launch_bounds__(256) tt_tail_kernel(const TtTailArgs a) {
         float var = fmaf(sb, sb, a1);
         if (var < 0.f) var += fabsf(var) + 1e-6f;
         sd[u] = sqrtf(var);
-        ef[u] = gnoise_normal(a.eps_fc, 0, m, a.B, 64, k);
+        ef[u] = gnoise_normal(a.eps_fc, 0, m, a.B, HW, k);
         pre = fmaf(sd[u], ef[u], a0 + a.fc_b0[k]);
         sgn_in[u] = 0.f;
       } else {
-        ef[u] = a.sout_fc[(long long)m * 64 + k];
+        ef[u] = a.sout_fc[(long long)m * HW + k];
         pre = a0 + a1 * ef[u] + a.fc_b0[k];
         sd[u] = 0.f;
-        sgn_in[u] = a.sin_head[(long long)m * 64 + k];
+        sgn_in[u] = a.sin_head[(long long)m * HW + k];
       }
       h[u] = fmaxf(pre, 0.f);
       if (MODE == TT_PLAIN && a.keep_fc < 1.0f) {  // dropout behind the fc layer's ReLU (inception.py:204-206)
         bool kp;
-        if (a.drop_fc.ptr) kp = a.drop_fc.ptr[(long long)m * 64 + k] != 0.f;
+        if (a.drop_fc.ptr) kp = a.drop_fc.ptr[(long long)m * HW + k] != 0.f;
         else {
           const NoiseKey dk = noise_key(a.drop_fc);
-          kp = philox_keep(dk.seed, a.drop_fc.kind, a.drop_fc.site, dk.sample0, dk.window0 + m, 64, 0, k, a.keep_fc);
+          kp = philox_keep(dk.seed, a.drop_fc.kind, a.drop_fc.site, dk.sample0, dk.window0 + m, HW, 0, k, a.keep_fc);
         }
         h[u] = kp ? h[u] / a.keep_fc : 0.f;
       }
     }
-    // ---- head: two outputs x two paths, reduced over the 64 hidden units
+    // ---- head: two outputs x two paths, reduced over the HW hidden units
     float p0[2], p1[2];
 #pragma unroll
     for (int o = 0; o < 2; ++o) {
       float s0 = 0.f, s1 = 0.f;
 #pragma unroll
-      for (int u = 0; u < 2; ++u) {
+      for (int u = 0; u < U; ++u) {
         s0 = fmaf(h[u], w0[o][u], s0);
         if (MODE != TT_PLAIN) s1 = fmaf(MODE == BRL_MODE_LRT ? h[u] * h[u] : h[u] * sgn_in[u], w1[o][u], s1);
       }
@@ -1228,7 +1230,7 @@ __global__ void __launch_bounds__(256) tt_tail_kernel(const TtTailArgs a) {
       gb1[o] += MODE == BRL_MODE_LRT ? d1[o] : d[o];
     }
 #pragma unroll
-    for (int u = 0; u < 2; ++u) {
+    for (int u = 0; u < U; ++u) {
       const int k = lane + 32 * u;
       const float x1 = MODE == BRL_MODE_LRT ? h[u] * h[u] : h[u] * sgn_in[u];
       float dh0 = 0.f, dh1 = 0.f;
@@ -1242,8 +1244,8 @@ __global__ void __launch_bounds__(256) tt_tail_kernel(const TtTailArgs a) {
       const float dh = MODE == TT_PLAIN ? dh0 : MODE == BRL_MODE_LRT ? fmaf(2.0f * h[u], dh1, dh0) : fmaf(sgn_in[u], dh1, dh0);
       // ---- activation backward of the fc layer (with dropout the stored activation is a * m / keep: it gates, 1 / keep scales)
       const float dp = h[u] > 0.f ? (MODE == TT_PLAIN ? dh / a.keep_fc : dh) : 0.f;
-      a.dpre[(long long)m * 64 + k] = dp;
-      if (MODE != TT_PLAIN) a.dsec[(long long)m * 64 + k] = MODE == BRL_MODE_LRT ? (sd[u] > 0.f ? dp * ef[u] / (2.0f * sd[u]) : 0.f) : dp * ef[u];
+      a.dpre[(long long)m * HW + k] = dp;
+      if (MODE != TT_PLAIN) a.dsec[(long long)m * HW + k] = MODE == BRL_MODE_LRT ? (sd[u] > 0.f ? dp * ef[u] / (2.0f * sd[u]) : 0.f) : dp * ef[u];
     }
   }
   // ---- reductions: likelihood sums (lane 0 of every warp holds its windows'), head weight gradients
@@ -1258,20 +1260,20 @@ __global__ void __launch_bounds__(256) tt_tail_kernel(const TtTailArgs a) {
 #pragma unroll
   for (int o = 0; o < 2; ++o) {
 #pragma unroll
-    for (int u = 0; u < 2; ++u) {
+    for (int u = 0; u < U; ++u) {
       atomicAdd(&sg[0][o][lane + 32 * u], gw0[o][u]);
       atomicAdd(&sg[1][o][lane + 32 * u], gw1[o][u]);
     }
     if (lane == 0) {  // d[o] is warp-uniform: one lane carries the bias gradient
-      atomicAdd(&sg[0][o][64], gb0[o]);
-      atomicAdd(&sg[1][o][64], gb1[o]);
+      atomicAdd(&sg[0][o][HW], gb0[o]);
+      atomicAdd(&sg[1][o][HW], gb1[o]);
     }
   }
   __syncthreads();
-  for (int i = tid; i < (MODE == TT_PLAIN ? 1 : 2) * 2 * 65; i += 256) {
-    const int path = i / 130, r = i - path * 130, o = r / 65, k = r - o * 65;
+  for (int i = tid; i < (MODE == TT_PLAIN ? 1 : 2) * 2 * (HW + 1); i += 256) {
+    const int path = i / (2 * (HW + 1)), r = i - path * 2 * (HW + 1), o = r / (HW + 1), k = r - o * (HW + 1);
     float* g = path ? a.g1 : a.g0;
-    atomicAdd(g + (k < 64 ? a.hw_off + o * 64 + k : a.hb_off + o), sg[path][o][k]);
+    atomicAdd(g + (k < HW ? a.hw_off + o * HW + k : a.hb_off + o), sg[path][o][k]);
   }
 }
 
@@ -1341,6 +1343,8 @@ int* tt_status_word() {
   return g_tt_status[d];
 }
 inline size_t al256(size_t v) { return (v + 255) & ~(size_t)255; }
+
+#include "brl_tc_train_linear.cuh"
 
 }  // namespace
 
@@ -1485,9 +1489,15 @@ void tt_tail(const TtStep& s, const TtTail& t, cudaStream_t st) {
   a.g0 = s.g0; a.g1 = s.g1; a.hw_off = t.hw_off; a.hb_off = t.hb_off;
   const int grid = (int)std::min<long long>((s.B + 7) / 8, 148);
   ++g_launch_count;
-  if (lrt) tt_tail_kernel<BRL_MODE_LRT><<<grid, 256, 0, st>>>(a);
-  else if (plain) tt_tail_kernel<TT_PLAIN><<<grid, 256, 0, st>>>(a);
-  else tt_tail_kernel<BRL_MODE_FLIPOUT><<<grid, 256, 0, st>>>(a);
+  if (t.width == 32) {
+    if (lrt) tt_tail_kernel<BRL_MODE_LRT, 32><<<grid, 256, 0, st>>>(a);
+    else if (plain) tt_tail_kernel<TT_PLAIN, 32><<<grid, 256, 0, st>>>(a);
+    else tt_tail_kernel<BRL_MODE_FLIPOUT, 32><<<grid, 256, 0, st>>>(a);
+  } else {
+    if (lrt) tt_tail_kernel<BRL_MODE_LRT, 64><<<grid, 256, 0, st>>>(a);
+    else if (plain) tt_tail_kernel<TT_PLAIN, 64><<<grid, 256, 0, st>>>(a);
+    else tt_tail_kernel<BRL_MODE_FLIPOUT, 64><<<grid, 256, 0, st>>>(a);
+  }
 }
 
 void tt_fc_backward(const TtLane& ln, const TtStep& s, const float* dpre, const float* dsec, cudaStream_t st, const TtSide& sd) {
@@ -1558,6 +1568,111 @@ void tt_backward(const TtLane& ln, const TtStep& s, cudaStream_t st, const TtSid
   ++g_launch_count;
   tt_reduce_kernel<<<dim3((tot + 255) / 256, RED_SPLIT), 256, 0, st>>>(ra);
   cudaStreamWaitEvent(st, sd.join, 0);  // the fc weight gradient (tt_fc_backward) is part of what the caller finalises next
+}
+
+// ---- Linear net (brl_tc_train_linear.cuh) --------------------------------------------------------------------------------
+size_t tl_lane_bytes(long long B) {
+  const size_t nmt = (size_t)((B + 127) / 128);
+  size_t b = 256;
+  for (int l = 0; l < 4; ++l) b += 4 * al256(nmt * tl_kc(l) * TL_CH) + al256(4 * (size_t)tl_wimg(l));
+  for (int l = 0; l < 3; ++l) b += al256((size_t)B * tl_n(l) * sizeof(float));
+  return b + al256(2 * (size_t)B * 32 * sizeof(float));
+}
+void tl_carve(unsigned char* base, long long B, TlLane& ln) {
+  const size_t nmt = (size_t)((B + 127) / 128);
+  unsigned char* p = reinterpret_cast<unsigned char*>(al256(reinterpret_cast<size_t>(base)));
+  auto take = [&](size_t bytes) { unsigned char* r = p; p += al256(bytes); return r; };
+  for (int l = 0; l < 4; ++l) {
+    for (int k = 0; k < 4; ++k) ln.act[l][k] = take(nmt * tl_kc(l) * TL_CH);
+    ln.w[l] = take(4 * (size_t)tl_wimg(l));
+  }
+  for (int l = 0; l < 3; ++l) ln.rbuf[l] = reinterpret_cast<float*>(take((size_t)B * tl_n(l) * sizeof(float)));
+  ln.part = reinterpret_cast<float*>(take(2 * (size_t)B * 32 * sizeof(float)));
+}
+
+static void tl_configure() {
+  static bool done_dev[TT_MAX_DEV] = {};
+  bool& done = done_dev[tt_device()];
+  if (done) return;
+  cudaFuncSetAttribute(tl_fwd_kernel<BRL_MODE_LRT>, cudaFuncAttributeMaxDynamicSharedMemorySize, TLF_SMEM);
+  cudaFuncSetAttribute(tl_fwd_kernel<BRL_MODE_FLIPOUT>, cudaFuncAttributeMaxDynamicSharedMemorySize, TLF_SMEM);
+  cudaFuncSetAttribute(tl_fwd_kernel<TT_PLAIN>, cudaFuncAttributeMaxDynamicSharedMemorySize, TLF_SMEM);
+  cudaFuncSetAttribute(tl_dx_kernel<BRL_MODE_LRT>, cudaFuncAttributeMaxDynamicSharedMemorySize, TLX_SMEM);
+  cudaFuncSetAttribute(tl_dx_kernel<BRL_MODE_FLIPOUT>, cudaFuncAttributeMaxDynamicSharedMemorySize, TLX_SMEM);
+  cudaFuncSetAttribute(tl_dx_kernel<TT_PLAIN>, cudaFuncAttributeMaxDynamicSharedMemorySize, TLX_SMEM);
+  cudaFuncSetAttribute(tl_dw_kernel<BRL_MODE_LRT>, cudaFuncAttributeMaxDynamicSharedMemorySize, TLW_SMEM);
+  cudaFuncSetAttribute(tl_dw_kernel<BRL_MODE_FLIPOUT>, cudaFuncAttributeMaxDynamicSharedMemorySize, TLW_SMEM);
+  cudaFuncSetAttribute(tl_dw_kernel<TT_PLAIN>, cudaFuncAttributeMaxDynamicSharedMemorySize, TLW_SMEM);
+  done = true;
+}
+
+void tl_forward(const TlLane& ln, const TtStep& s, cudaStream_t st, const TtSide& sd) {
+  tl_configure();
+  const int B = (int)s.B, nmt = (B + 127) / 128;
+  const bool lrt = s.mode == BRL_MODE_LRT, flip = s.mode == BRL_MODE_FLIPOUT;
+  cudaEventRecord(sd.fork, st);  // the parameters (and a weight draw) are complete on `st` here
+  cudaStreamWaitEvent(sd.side, sd.fork, 0);
+  TlPackWArgs pw{};
+  pw.mode = s.mode; pw.mu = s.mu; pw.second = lrt ? s.sigma : flip ? s.wsamp : s.mu;
+  for (int l = 0; l < 4; ++l) { pw.w_off[l] = s.w_off[l]; pw.w[l] = ln.w[l]; }
+  tl_pack_w_kernel<<<(TL_PACK_END + 255) / 256, 256, 0, sd.side>>>(pw);
+  cudaEventRecord(sd.join, sd.side);
+  TlPackXArgs px{};
+  px.x = s.x; px.sgn_in = s.sgn_in[0]; px.B = B; px.mode = s.mode;
+  for (int k = 0; k < 4; ++k) px.img[k] = ln.act[0][k];
+  tl_packx_kernel<<<(unsigned)(((long long)nmt * 72 * 128 + 255) / 256), 256, 0, st>>>(px);
+  cudaStreamWaitEvent(st, sd.join, 0);  // weight images ready
+  g_launch_count += 6;
+  for (int l = 0; l < 4; ++l) {
+    TlFwdArgs fa{};
+    fa.a0 = ln.act[l][0]; fa.a1 = ln.act[l][2];
+    fa.w0 = ln.w[l]; fa.w1 = ln.w[l] + (flip ? 3 : 2) * (size_t)tl_wimg(l);
+    fa.B = B; fa.N = tl_n(l); fa.KC = tl_kc(l); fa.last = l == 3;
+    fa.b0 = (flip ? s.wsamp : s.mu) + s.b_off[l]; fa.b1 = lrt ? s.sigma + s.b_off[l] : nullptr;
+    fa.eps = s.eps[l]; fa.drop = s.drop[l]; fa.keep = s.keep[l];
+    fa.sout = s.sgn_out[l]; fa.sin_next = s.sgn_in[l + 1];
+    if (l < 3)
+      for (int k = 0; k < 4; ++k) fa.out[k] = ln.act[l + 1][k];
+    fa.rbuf = l < 3 ? ln.rbuf[l] : nullptr; fa.part = ln.part; fa.status = tt_status_word();
+    const dim3 grid(nmt, tl_n(l) / TL_NS);
+    if (lrt) tl_fwd_kernel<BRL_MODE_LRT><<<grid, 128, TLF_SMEM, st>>>(fa);
+    else if (flip) tl_fwd_kernel<BRL_MODE_FLIPOUT><<<grid, 128, TLF_SMEM, st>>>(fa);
+    else tl_fwd_kernel<TT_PLAIN><<<grid, 128, TLF_SMEM, st>>>(fa);
+  }
+}
+
+void tl_backward(const TlLane& ln, const TtStep& s, float* const* dpre, float* const* dsec, cudaStream_t st, const TtSide& sd) {
+  tl_configure();
+  const int B = (int)s.B, nmt = (B + 127) / 128;
+  const bool lrt = s.mode == BRL_MODE_LRT, flip = s.mode == BRL_MODE_FLIPOUT;
+  for (int l = 3; l >= 0; --l) {
+    // weight gradient of layer l: needs nothing downstream of it until the finalisation, so it runs on the side stream
+    cudaEventRecord(sd.fork, st);
+    cudaStreamWaitEvent(sd.side, sd.fork, 0);
+    TlDwArgs wa{};
+    wa.a0 = ln.act[l][1]; wa.a1 = ln.act[l][lrt ? 2 : 3]; wa.g0 = dpre[l]; wa.g1 = dsec[l];
+    wa.B = B; wa.N = tl_n(l); wa.KC = tl_kc(l); wa.cin = tl_cin(l); wa.nsl = std::min(TL_WS, tl_n(l));
+    wa.gw0 = s.g0; wa.gw1 = s.g1; wa.w_off = s.w_off[l]; wa.b_off = s.b_off[l]; wa.status = tt_status_word();
+    const dim3 wgrid((tl_kc(l) + 15) / 16, tl_n(l) / wa.nsl);
+    if (lrt) tl_dw_kernel<BRL_MODE_LRT><<<wgrid, 256, TLW_SMEM, sd.side>>>(wa);
+    else if (flip) tl_dw_kernel<BRL_MODE_FLIPOUT><<<wgrid, 256, TLW_SMEM, sd.side>>>(wa);
+    else tl_dw_kernel<TT_PLAIN><<<wgrid, 256, TLW_SMEM, sd.side>>>(wa);
+    ++g_launch_count;
+    if (l == 0) break;  // layer 0's input is x: no input gradient
+    TlDxArgs xa{};
+    xa.g0 = dpre[l]; xa.g1 = dsec[l];
+    xa.w0 = ln.w[l] + tl_wimg(l); xa.w1 = ln.w[l] + 2 * (size_t)tl_wimg(l); xa.act = ln.act[l][0];
+    xa.B = B; xa.Nl = tl_n(l); xa.KCl = tl_kc(l);
+    xa.sin_ = s.sgn_in[l]; xa.rb = ln.rbuf[l - 1]; xa.sout = s.sgn_out[l - 1]; xa.keep = s.keep[l - 1];
+    xa.d0 = dpre[l - 1]; xa.d1 = dsec[l - 1]; xa.status = tt_status_word();
+    const dim3 xgrid(nmt, tl_cin(l) / TL_XS);
+    if (lrt) tl_dx_kernel<BRL_MODE_LRT><<<xgrid, 256, TLX_SMEM, st>>>(xa);
+    else if (flip) tl_dx_kernel<BRL_MODE_FLIPOUT><<<xgrid, 256, TLX_SMEM, st>>>(xa);
+    else tl_dx_kernel<TT_PLAIN><<<xgrid, 256, TLX_SMEM, st>>>(xa);
+    ++g_launch_count;
+  }
+  cudaEventRecord(sd.join, sd.side);
+  cudaStreamWaitEvent(st, sd.join, 0);  // the weight gradients are part of what the caller finalises next
 }
 
 }  // namespace brl

@@ -78,6 +78,7 @@ struct TtTail {
   int loss_kind = 0;         // single-contraction modes: 0 ELBO likelihood, 1 F.gaussian_nll_loss (HNN step)
   float keep_fc = 1.0f;      // dropout site behind the fc layer
   NoiseRef drop_fc{};
+  int width = 64;            // hidden units in front of the head: 64 (Inception fc layer), 32 (Linear layer 3)
 };
 void tt_tail(const TtStep& s, const TtTail& t, cudaStream_t st);
 // backward: feature-gradient image -> g0 / g1 of the ten conv layers (accumulated: the buffers must be zeroed); 4 launches
@@ -86,5 +87,24 @@ void tt_backward(const TtLane& ln, const TtStep& s, cudaStream_t st, const TtSid
 // backward level launches (nullptr = off)
 void tt_trace(long long* device_buf);
 int tt_status();  // 0 ok; else the code of the first bounded mbarrier wait that timed out (synchronises)
+
+// ---- Linear net (brl_tc_train_linear.cuh): the four hidden layers on the tensor pipe, the head in tt_tail (width 32).
+// A TtStep describes the step with the hidden layers at indices 0..3 (eps, sgn_in / sgn_out, drop / keep, w_off / b_off; sgn_in[4]
+// = the head's s_in) and w_off_fc / b_off_fc = layer 3, the layer whose epilogue the tail runs.
+struct TlLane {
+  unsigned char* act[4][4];  // input images of hidden layer l, [M-tile][K/8 chunks][128 windows][16 B]: fp16 a | bf16 a |
+                             // bf16 a^2 (LRT) or fp16 a * s_in (Flipout) | bf16 a * s_in (Flipout)
+  unsigned char* w[4];       // weight images of hidden layer l, [N/32 slices][K/8][32][16 B]: fp16 mu | bf16 mu |
+                             // bf16 sigma^2 or (W - mu) | fp16 (W - mu)
+  float* rbuf[3];            // LRT: eps / (2 sd) of hidden layers 0..2 [B, N]
+  float* part;               // layer 3's sums for the tail [2][B][32]
+};
+size_t tl_lane_bytes(long long B);
+void tl_carve(unsigned char* base, long long B, TlLane& ln);
+// window / weight packing + the four forward launches (layer 3 leaves its sums in ln.part for tt_tail with width 32)
+void tl_forward(const TlLane& ln, const TtStep& s, cudaStream_t st, const TtSide& sd);
+// dpre / dsec[l]: compact [B, N_l] gradients of hidden layer l ([3] written by tt_tail); writes [0..2] and g0 / g1 of the four
+// hidden layers (plain stores)
+void tl_backward(const TlLane& ln, const TtStep& s, float* const* dpre, float* const* dsec, cudaStream_t st, const TtSide& sd);
 
 }  // namespace brl

@@ -62,8 +62,11 @@ extern "C" {
                               * run the ten conv layers and the fc layer as LEVEL-FUSED tcgen05 kernels (one CTA
                               * per layer per 4-window tile; operands are bulk-copied activation / weight images, taps are
                               * descriptor shifts, the backward contractions read the same images through MN-major descriptors;
-                              * fp16 / bf16 operands, fp32 accumulation: outputs 1e-2, loss 5e-3, gradient cosine > 0.999);
-                              * the fc layer, the head and every other net / mode keep the fp32 FFMA kernels */
+                              * fp16 / bf16 operands, fp32 accumulation: outputs 1e-2, loss 5e-3, gradient cosine > 0.999).
+                              * Linear: the same two steps run the four hidden layers as tcgen05 GEMMs over 128-window tiles
+                              * (same operand precision and bound) when the workspace holds their images
+                              * (brl_workspace_bytes(B, S, 1) includes them), else the per-layer kernels.
+                              * Every other net keeps the fp32 FFMA kernels */
 
 #define BRL_MAX_LAYERS 16
 
