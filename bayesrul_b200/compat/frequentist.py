@@ -42,7 +42,7 @@ class HNN(_Base):
         self._engine_kind = engine
         # kernels of HNN.step: "auto" = the level-fused tcgen05 kernels for the Inception net (fp16 / bf16 operands: loss 5e-3,
         # gradient cosine > 0.999 of the fp32 oracle), the fp32 FFMA kernels for the other nets; "fused" also runs the level-fused
-        # kernels on the Linear net (same bound); "simt" forces the fp32 parity back-end
+        # kernels on the Linear and Conv-D3 nets (same bound); "simt" forces the fp32 parity back-end
         self._train_backend = train_backend
         self._it = 0
         if device is not None:

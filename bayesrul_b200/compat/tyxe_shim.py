@@ -122,8 +122,8 @@ class VariationalBNN:
         self.engine_kind = engine
         # kernels of the ELBO step: "auto" = the level-fused tcgen05 kernels where they exist (Inception: LRT, Flipout and the
         # weight-sampling ELBO; fp16 / bf16 operands, loss 5e-3, gradient cosine > 0.999), else the fp32 FFMA kernels; "simt" = always the fp32 parity
-        # back-end (rtol 1e-3 against the oracle); "fused" / "tc" force a back-end ("fused" also covers the Linear net, with the
-        # same bound; on the Conv-D3 net it runs the fp32 FFMA kernels)
+        # back-end (rtol 1e-3 against the oracle); "fused" / "tc" force a back-end ("fused" also covers the Linear and Conv-D3
+        # nets, with the same bound)
         self.train_backend = train_backend
         self.seed = int(torch.initial_seed() % (2**62))
         self._step = 0

@@ -140,6 +140,9 @@ struct ActBufs {
   // level-fused tcgen05 training kernels of the Linear net (brl_tc_train_linear.cuh): carved last, only where they fit
   TlLane tl{};
   bool has_tl = false;
+  // level-fused tcgen05 training kernels of the Conv-D3 net (brl_tc_train_convd3.cuh): carved last, only where they fit
+  Tc3Lane tc3{};
+  bool has_tc3 = false;
 };
 constexpr int GRAPH_MAX_PARTICLES = 8;
 
@@ -188,15 +191,17 @@ static void carve_train(const NetSpec& n, Carve& c, long long B, ActBufs& ab) {
   }
 }
 
-// images of the Linear net's fused training kernels, behind everything else of the workspace: a workspace sized for the
+// images of the Linear / Conv-D3 nets' fused training kernels, behind everything else of the workspace: a workspace sized for the
 // per-layer kernels alone keeps its layout, and a step whose workspace has no room for them runs the per-layer kernels
 static void carve_tl(const NetSpec& n, Carve& c, long long B, ActBufs& ab) {
-  if (n.id != BRL_NET_LINEAR) return;
-  const size_t bytes = ((size_t)tl_lane_bytes(B) + 255) & ~(size_t)255;
+  if (n.id != BRL_NET_LINEAR && n.id != BRL_NET_CONV) return;
+  const bool lin = n.id == BRL_NET_LINEAR;
+  const size_t bytes = ((size_t)(lin ? tl_lane_bytes(B) : tc3_lane_bytes(B)) + 255) & ~(size_t)255;
   if (c.base && (!c.ok || c.used + bytes > c.cap)) return;
   unsigned char* base = c.take<unsigned char>((long long)bytes);
-  if (base) tl_carve(base, B, ab.tl);
-  ab.has_tl = base != nullptr;
+  if (base && lin) tl_carve(base, B, ab.tl);
+  if (base && !lin) tc3_carve(base, B, ab.tc3);
+  (lin ? ab.has_tl : ab.has_tc3) = base != nullptr;
 }
 
 // device {seed, sample0, window0} of the step being captured (nullptr outside a capture): every Philox stream built by
@@ -771,7 +776,7 @@ int64_t brl_workspace_bytes(const brl_ctx* ctx, int64_t B, int64_t S, int train,
     carve_forward(n, c, B, 1, ab1);
     carve_train(n, c, B, ab1);
   }
-  if (train == 1) {  // fused Linear-net images of the lanes (brl_elbo_step / brl_hnn_step carve them last)
+  if (train == 1) {  // fused Linear / Conv-D3 images of the lanes (brl_elbo_step / brl_hnn_step carve them last)
     carve_tl(n, c, B, ab);
     if (S >= 2) carve_tl(n, c, B, ab1);
   }
@@ -1154,13 +1159,16 @@ static int elbo_body(brl_ctx* ctx, const ActBufs* const* lanes, int n_lanes, con
       // the Linear net's four hidden layers on the tensor pipe, the head in the same tail kernel (width 32)
       const bool use_tl = ctx->gemm_backend == BRL_GEMM_TC_FUSED && n.id == BRL_NET_LINEAR && ab.has_tl &&
                           (mode == BRL_MODE_LRT || mode == BRL_MODE_FLIPOUT || mode == BRL_MODE_WS);
+      // the Conv-D3 net's three convs on the tensor pipe, the head in the same tail kernel (width 320)
+      const bool use_tc3 = ctx->gemm_backend == BRL_GEMM_TC_FUSED && n.id == BRL_NET_CONV && ab.has_tc3 &&
+                           (mode == BRL_MODE_LRT || mode == BRL_MODE_FLIPOUT || mode == BRL_MODE_WS);
       if (compute_grads) {  // a dozen memsets: on a side stream underneath the forward pass, joined before the NLL
         cudaStream_t zs = ctx->multi_stream ? ln.zero : ls;
         if (zs != ls) {
           BRL_CUDA(cudaEventRecord(ln.ev_zero, ls));
           BRL_CUDA(cudaStreamWaitEvent(zs, ln.ev_zero, 0));
         }
-        if (!use_tt && !use_tl) {  // the fused back-end keeps its gradients in bf16 images that are written, not accumulated
+        if (!use_tt && !use_tl && !use_tc3) {  // the fused back-end keeps its gradients in bf16 images that are written, not accumulated
           int rc = zero_grads(n, ab, B, zs);
           if (rc) return rc;
         }
@@ -1198,6 +1206,17 @@ static int elbo_body(brl_ctx* ctx, const ActBufs* const* lanes, int n_lanes, con
         ts.w_off_fc = n.layers[3].w_off; ts.b_off_fc = n.layers[3].b_off;
         ts.g0 = ab.g0; ts.g1 = ab.g1;
         tl_forward(ab.tl, ts, ls, TtSide{ln.side[0], ln.ev_fork, ln.ev_join[0]});
+      } else if (use_tc3) {
+        ts.x = x; ts.B = B; ts.mode = mode; ts.mu = mode == BRL_MODE_WS ? ab.wsamp : mu; ts.sigma = sigma; ts.wsamp = ab.wsamp;
+        for (int ly = 0; ly < 3; ++ly) {
+          ts.eps[ly] = nref(&nz, nz.lrt_eps[ly], KIND_LRT_EPS, (unsigned)ly);
+          ts.keep[ly] = 1.0f;
+          ts.sgn_out[ly] = sout_[ly];
+          ts.w_off[ly] = n.layers[ly].w_off; ts.b_off[ly] = n.layers[ly].b_off;
+        }
+        for (int ly = 0; ly < 4; ++ly) ts.sgn_in[ly] = sin_[ly];
+        ts.g0 = ab.g0; ts.g1 = ab.g1;
+        tc3_forward(ab.tc3, ts, ls, TtSide{ln.side[0], ln.ev_fork, ln.ev_join[0]});
       } else {
         run_forward(ctx, ab, fa, ls, l);
       }
@@ -1221,6 +1240,14 @@ static int elbo_body(brl_ctx* ctx, const ActBufs* const* lanes, int n_lanes, con
         tl.sout_fc = sout_[3]; tl.sin_head = sin_[4]; tl.sout_head = sout_[4];
         tl.hw_off = n.layers[4].w_off; tl.hb_off = n.layers[4].b_off;
         tt_tail(ts, tl, ls);
+      } else if (use_tc3) {
+        TtTail tl{};
+        tl.part = ab.tc3.feat; tl.width = 320; tl.y = y; tl.gscale = (float)(c_nll / particles); tl.compute_grads = compute_grads;
+        tl.acc = ab0.acc; tl.out = outp; tl.dpre = ab.tc3.dfeat;
+        tl.eps_head = nref(&nz, nz.lrt_eps[3], KIND_LRT_EPS, 3u);
+        tl.sin_head = sin_[3]; tl.sout_head = sout_[3];
+        tl.hw_off = n.layers[3].w_off; tl.hb_off = n.layers[3].b_off;
+        tt_tail(ts, tl, ls);
       } else {
         launch_nll_elbo(outp, y, B, (float)(c_nll / particles), ab0.acc, compute_grads ? ab.grad[n.out_buf] : nullptr, ls);
       }
@@ -1233,6 +1260,8 @@ static int elbo_body(brl_ctx* ctx, const ActBufs* const* lanes, int n_lanes, con
           tt_backward(ab.tt, ts, ls, tsd);
         } else if (use_tl) {
           tl_backward(ab.tl, ts, ab.dpre.data(), ab.dsec.data(), ls, TtSide{ln.side[0], ln.ev_fork, ln.ev_join[0]});
+        } else if (use_tc3) {
+          tc3_backward(ab.tc3, ts, ls, TtSide{ln.side[0], ln.ev_fork, ln.ev_join[0]});
         } else {
           run_backward(ctx, ab, ba, ls, l);
         }
@@ -1306,6 +1335,7 @@ int brl_elbo_step(brl_ctx* ctx, const float* x, const float* y, int64_t B, const
   if (n_lanes == 2) {
     carve_tl(n, c, B, ab1);
     if (!ab1.has_tl) ab.has_tl = false;  // both particle lanes run the same back-end
+    if (!ab1.has_tc3) ab.has_tc3 = false;
   }
   const ActBufs* lanes[2] = {&ab, &ab1};
   // ---- graph replay (native Philox noise): eager on first sight of a configuration, captured on the second, replayed after
@@ -1452,6 +1482,32 @@ static int hnn_body(brl_ctx* ctx, const ActBufs& ab, const float* x, const float
     tl.loss_kind = 1; tl.keep_fc = keep_of(3); tl.drop_fc = nref(&nz, nz.drop_mask[3], KIND_DROPOUT, 3u);
     tt_tail(ts, tl, st);
     if (compute_grads) tl_backward(ab.tl, ts, ab.dpre.data(), ab.dsec.data(), st, tsd);
+    BRL_CUDA(cudaGetLastError());
+    return BRL_OK;
+  }
+  if (ctx->gemm_backend == BRL_GEMM_TC_FUSED && n.id == BRL_NET_CONV && ab.has_tc3) {
+    // the Conv-D3 net's fused kernels, one contraction with the deterministic weights; keep decisions in the conv epilogues
+    const brl_ctx::Lane& ln = ctx->lanes[0];
+    auto keep_of = [&](int ly) { return (p_dropout > 0.f && n.layers[ly].drop_factor > 0.f) ? 1.0f - p_dropout * n.layers[ly].drop_factor : 1.0f; };
+    TtStep ts{};
+    ts.x = x; ts.B = B; ts.mode = BRL_MODE_DET; ts.mu = theta;
+    for (int ly = 0; ly < 3; ++ly) {
+      ts.drop[ly] = nref(&nz, nz.drop_mask[ly], KIND_DROPOUT, (unsigned)ly);
+      ts.keep[ly] = keep_of(ly);
+      ts.w_off[ly] = n.layers[ly].w_off; ts.b_off[ly] = n.layers[ly].b_off;
+    }
+    ts.g0 = grad_theta; ts.g1 = nullptr;
+    const TtSide tsd{ln.side[0], ln.ev_fork, ln.ev_join[0]};
+    BRL_CUDA(cudaMemsetAsync(scalars, 0, 2 * sizeof(double), st));
+    if (compute_grads) BRL_CUDA(cudaMemsetAsync(grad_theta, 0, sizeof(float) * n.P, st));
+    tc3_forward(ab.tc3, ts, st, tsd);
+    TtTail tl{};
+    tl.part = ab.tc3.feat; tl.width = 320; tl.y = y; tl.gscale = 0.f; tl.compute_grads = compute_grads; tl.acc = scalars; tl.out = out;
+    tl.dpre = ab.tc3.dfeat;
+    tl.hw_off = n.layers[3].w_off; tl.hb_off = n.layers[3].b_off;
+    tl.loss_kind = 1;
+    tt_tail(ts, tl, st);
+    if (compute_grads) tc3_backward(ab.tc3, ts, st, tsd);
     BRL_CUDA(cudaGetLastError());
     return BRL_OK;
   }

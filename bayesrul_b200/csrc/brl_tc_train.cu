@@ -1069,7 +1069,9 @@ __global__ void __launch_bounds__(256, 1) tt_fc_dw_kernel(const TtFcBwdArgs a) {
 // gradients) -> activation backward of the fc layer (the compact dpre / dsec tensors of tt_fc_backward).  It replaces eight
 // per-layer launches (split-K epilogue, head GEMM, NLL, two activation-backward, head dX / dW) of 3 - 11 us each; the arithmetic
 // is that of brl_gemm_epi.cuh / nll_elbo_kernel / bwd_act_kernel, one warp per window, lane = hidden units {lane, lane + 32}.
-// HW = width of the hidden layer in front of the head: 64 (Inception fc layer), 32 (Linear layer 3, lane = hidden unit lane).
+// HW = width of the hidden layer in front of the head: 64 (Inception fc layer), 32 (Linear layer 3, lane = hidden unit lane),
+// 320 (Conv-D3: `part` holds the pooled, activated conv3 features [B, 320] as they are -- no fc epilogue -- and `dpre` receives
+// their gradient).
 // ------------------------------------------------------------------------------------------------
 __device__ __forceinline__ double tt_block_sum(double v) {  // valid in thread 0
   __shared__ double red[32];
@@ -1112,6 +1114,7 @@ __global__ void __launch_bounds__(256) tt_tail_kernel(const TtTailArgs a) {
   for (int i = tid; i < 2 * 2 * (HW + 1); i += 256) (&sg[0][0][0])[i] = 0.f;
   __syncthreads();
   constexpr int U = HW / 32;  // hidden units per lane
+  constexpr bool FEAT = HW == 320;
   float w0[2][U], w1[2][U];  // head weights of this lane's hidden units: [output][unit]
 #pragma unroll
   for (int o = 0; o < 2; ++o)
@@ -1131,6 +1134,12 @@ __global__ void __launch_bounds__(256) tt_tail_kernel(const TtTailArgs a) {
 #pragma unroll
     for (int u = 0; u < U; ++u) {
       const int k = lane + 32 * u;
+      if (FEAT) {
+        h[u] = a.part[(long long)m * HW + k];
+        sd[u] = ef[u] = 0.f;
+        sgn_in[u] = MODE == BRL_MODE_FLIPOUT ? a.sin_head[(long long)m * HW + k] : 0.f;
+        continue;
+      }
       const float a0 = a.part[(long long)m * HW + k], a1 = MODE == TT_PLAIN ? 0.f : a.part[((long long)a.B + m) * HW + k];
       float pre;
       if (MODE == TT_PLAIN) {
@@ -1242,6 +1251,10 @@ __global__ void __launch_bounds__(256) tt_tail_kernel(const TtTailArgs a) {
         dh1 = fmaf(d1[o], w1[o][u], dh1);
       }
       const float dh = MODE == TT_PLAIN ? dh0 : MODE == BRL_MODE_LRT ? fmaf(2.0f * h[u], dh1, dh0) : fmaf(sgn_in[u], dh1, dh0);
+      if (FEAT) {
+        a.dpre[(long long)m * HW + k] = dh;
+        continue;
+      }
       // ---- activation backward of the fc layer (with dropout the stored activation is a * m / keep: it gates, 1 / keep scales)
       const float dp = h[u] > 0.f ? (MODE == TT_PLAIN ? dh / a.keep_fc : dh) : 0.f;
       a.dpre[(long long)m * HW + k] = dp;
@@ -1345,6 +1358,7 @@ int* tt_status_word() {
 inline size_t al256(size_t v) { return (v + 255) & ~(size_t)255; }
 
 #include "brl_tc_train_linear.cuh"
+#include "brl_tc_train_convd3.cuh"
 
 }  // namespace
 
@@ -1489,7 +1503,11 @@ void tt_tail(const TtStep& s, const TtTail& t, cudaStream_t st) {
   a.g0 = s.g0; a.g1 = s.g1; a.hw_off = t.hw_off; a.hb_off = t.hb_off;
   const int grid = (int)std::min<long long>((s.B + 7) / 8, 148);
   ++g_launch_count;
-  if (t.width == 32) {
+  if (t.width == 320) {
+    if (lrt) tt_tail_kernel<BRL_MODE_LRT, 320><<<grid, 256, 0, st>>>(a);
+    else if (plain) tt_tail_kernel<TT_PLAIN, 320><<<grid, 256, 0, st>>>(a);
+    else tt_tail_kernel<BRL_MODE_FLIPOUT, 320><<<grid, 256, 0, st>>>(a);
+  } else if (t.width == 32) {
     if (lrt) tt_tail_kernel<BRL_MODE_LRT, 32><<<grid, 256, 0, st>>>(a);
     else if (plain) tt_tail_kernel<TT_PLAIN, 32><<<grid, 256, 0, st>>>(a);
     else tt_tail_kernel<BRL_MODE_FLIPOUT, 32><<<grid, 256, 0, st>>>(a);
@@ -1651,7 +1669,7 @@ void tl_backward(const TlLane& ln, const TtStep& s, float* const* dpre, float* c
     cudaStreamWaitEvent(sd.side, sd.fork, 0);
     TlDwArgs wa{};
     wa.a0 = ln.act[l][1]; wa.a1 = ln.act[l][lrt ? 2 : 3]; wa.g0 = dpre[l]; wa.g1 = dsec[l];
-    wa.B = B; wa.N = tl_n(l); wa.KC = tl_kc(l); wa.cin = tl_cin(l); wa.nsl = std::min(TL_WS, tl_n(l));
+    wa.B = B; wa.N = tl_n(l); wa.KC = tl_kc(l); wa.cin = tl_cin(l); wa.nsl = std::min(TL_WS, tl_n(l)); wa.mt_per = nmt;
     wa.gw0 = s.g0; wa.gw1 = s.g1; wa.w_off = s.w_off[l]; wa.b_off = s.b_off[l]; wa.status = tt_status_word();
     const dim3 wgrid((tl_kc(l) + 15) / 16, tl_n(l) / wa.nsl);
     if (lrt) tl_dw_kernel<BRL_MODE_LRT><<<wgrid, 256, TLW_SMEM, sd.side>>>(wa);
@@ -1670,6 +1688,127 @@ void tl_backward(const TlLane& ln, const TtStep& s, float* const* dpre, float* c
     else if (flip) tl_dx_kernel<BRL_MODE_FLIPOUT><<<xgrid, 256, TLX_SMEM, st>>>(xa);
     else tl_dx_kernel<TT_PLAIN><<<xgrid, 256, TLX_SMEM, st>>>(xa);
     ++g_launch_count;
+  }
+  cudaEventRecord(sd.join, sd.side);
+  cudaStreamWaitEvent(st, sd.join, 0);  // the weight gradients are part of what the caller finalises next
+}
+
+// ---- Conv-D3 net (brl_tc_train_convd3.cuh) -------------------------------------------------------------------------------
+size_t tc3_lane_bytes(long long B) {
+  size_t b = 256;
+  for (int l = 0; l < 3; ++l) {
+    const size_t M = (size_t)B * tc3_p(l), nmt = (M + 127) / 128;
+    b += 4 * al256(nmt * tc3_kc(l) * TL_CH) + al256(4 * (size_t)tc3_wimg(l)) + 4 * al256(M * tc3_n(l) * sizeof(float));
+  }
+  return b + 2 * al256((size_t)B * 25 * 320 * sizeof(float)) + 2 * al256((size_t)B * 320 * sizeof(float));
+}
+void tc3_carve(unsigned char* base, long long B, Tc3Lane& ln) {
+  unsigned char* p = reinterpret_cast<unsigned char*>(al256(reinterpret_cast<size_t>(base)));
+  auto take = [&](size_t bytes) { unsigned char* r = p; p += al256(bytes); return r; };
+  auto takef = [&](size_t n) { return reinterpret_cast<float*>(take(n * sizeof(float))); };
+  for (int l = 0; l < 3; ++l) {
+    const size_t M = (size_t)B * tc3_p(l), nmt = (M + 127) / 128;
+    for (int k = 0; k < 4; ++k) ln.img[l][k] = take(nmt * tc3_kc(l) * TL_CH);
+    ln.w[l] = take(4 * (size_t)tc3_wimg(l));
+    ln.act[l] = takef(M * tc3_n(l));
+    ln.rbuf[l] = takef(M * tc3_n(l));
+    ln.g[l][0] = takef(M * tc3_n(l));
+    ln.g[l][1] = takef(M * tc3_n(l));
+  }
+  ln.col[0] = takef((size_t)B * 25 * 320);
+  ln.col[1] = takef((size_t)B * 25 * 320);
+  ln.feat = takef((size_t)B * 320);
+  ln.dfeat = takef((size_t)B * 320);
+}
+
+static void tc3_configure() {
+  static bool done_dev[TT_MAX_DEV] = {};
+  bool& done = done_dev[tt_device()];
+  if (done) return;
+  tl_configure();  // tl_dx_kernel / tl_dw_kernel
+  cudaFuncSetAttribute(tc3_fwd_kernel<BRL_MODE_LRT>, cudaFuncAttributeMaxDynamicSharedMemorySize, TLF_SMEM);
+  cudaFuncSetAttribute(tc3_fwd_kernel<BRL_MODE_FLIPOUT>, cudaFuncAttributeMaxDynamicSharedMemorySize, TLF_SMEM);
+  cudaFuncSetAttribute(tc3_fwd_kernel<TT_PLAIN>, cudaFuncAttributeMaxDynamicSharedMemorySize, TLF_SMEM);
+  done = true;
+}
+
+void tc3_forward(const Tc3Lane& ln, const TtStep& s, cudaStream_t st, const TtSide& sd) {
+  tc3_configure();
+  const int B = (int)s.B;
+  const bool lrt = s.mode == BRL_MODE_LRT, flip = s.mode == BRL_MODE_FLIPOUT;
+  cudaEventRecord(sd.fork, st);  // the parameters (and a weight draw) are complete on `st` here
+  cudaStreamWaitEvent(sd.side, sd.fork, 0);
+  Tc3PackWArgs pw{};
+  pw.mode = s.mode; pw.mu = s.mu; pw.second = lrt ? s.sigma : flip ? s.wsamp : s.mu;
+  for (int l = 0; l < 3; ++l) { pw.w_off[l] = s.w_off[l]; pw.w[l] = ln.w[l]; }
+  tc3_pack_w_kernel<<<(TC3_PACK_END + 255) / 256, 256, 0, sd.side>>>(pw);
+  cudaEventRecord(sd.join, sd.side);
+  g_launch_count += 8;
+  for (int l = 0; l < 3; ++l) {
+    const int M = B * tc3_p(l), nmt = (M + 127) / 128;
+    Tc3Im2colArgs ia{};
+    ia.l = l; ia.B = B; ia.mode = s.mode; ia.src = l == 0 ? s.x : ln.act[l - 1]; ia.sgn_in = s.sgn_in[l];
+    for (int k = 0; k < 4; ++k) ia.img[k] = ln.img[l][k];
+    tc3_im2col_kernel<<<(unsigned)(((long long)nmt * tc3_kc(l) * 128 + 255) / 256), 256, 0, st>>>(ia);
+    if (l == 0) cudaStreamWaitEvent(st, sd.join, 0);  // weight images ready
+    Tc3FwdArgs fa{};
+    fa.a0 = ln.img[l][0]; fa.a1 = ln.img[l][2];
+    fa.w0 = ln.w[l]; fa.w1 = ln.w[l] + (flip ? 3 : 2) * (size_t)tc3_wimg(l);
+    fa.B = B; fa.N = tc3_n(l); fa.P = tc3_p(l); fa.KC = tc3_kc(l);
+    fa.b0 = (flip ? s.wsamp : s.mu) + s.b_off[l]; fa.b1 = lrt ? s.sigma + s.b_off[l] : nullptr;
+    fa.eps = s.eps[l]; fa.drop = s.drop[l]; fa.keep = s.keep[l]; fa.sout = s.sgn_out[l];
+    fa.act = ln.act[l]; fa.rbuf = ln.rbuf[l]; fa.status = tt_status_word();
+    const dim3 grid(nmt, tc3_nimg(l) / TL_NS);
+    if (lrt) tc3_fwd_kernel<BRL_MODE_LRT><<<grid, 128, TLF_SMEM, st>>>(fa);
+    else if (flip) tc3_fwd_kernel<BRL_MODE_FLIPOUT><<<grid, 128, TLF_SMEM, st>>>(fa);
+    else tc3_fwd_kernel<TT_PLAIN><<<grid, 128, TLF_SMEM, st>>>(fa);
+  }
+  tc3_pool_kernel<<<(B * 320 + 255) / 256, 256, 0, st>>>(ln.act[2], ln.feat, B);
+}
+
+void tc3_backward(const Tc3Lane& ln, const TtStep& s, cudaStream_t st, const TtSide& sd) {
+  tc3_configure();
+  const int B = (int)s.B;
+  const bool lrt = s.mode == BRL_MODE_LRT, flip = s.mode == BRL_MODE_FLIPOUT;
+  auto act_bwd = [&](int l, const float* src0, const float* src1) {
+    Tc3ActBwdArgs aa{};
+    aa.l = l; aa.B = B; aa.mode = lrt ? BRL_MODE_LRT : flip ? BRL_MODE_FLIPOUT : TT_PLAIN; aa.keep = s.keep[l];
+    aa.src0 = src0; aa.src1 = src1; aa.act = ln.act[l]; aa.rb = ln.rbuf[l]; aa.sout = s.sgn_out[l]; aa.sin_next = s.sgn_in[l + 1];
+    aa.d0 = ln.g[l][0]; aa.d1 = ln.g[l][1];
+    const long long n = (long long)B * tc3_p(l) * tc3_n(l);
+    tc3_bwd_act_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(aa);
+    ++g_launch_count;
+  };
+  act_bwd(2, ln.dfeat, nullptr);
+  for (int l = 2; l >= 0; --l) {
+    const int M = B * tc3_p(l), nmt = (M + 127) / 128;
+    // weight gradient of conv l: needs nothing downstream of it until the finalisation, so it runs on the side stream; its M-tiles
+    // are split so that the launch covers the GPU (conv1: 520 M-tiles at B = 256)
+    cudaEventRecord(sd.fork, st);
+    cudaStreamWaitEvent(sd.side, sd.fork, 0);
+    TlDwArgs wa{};
+    wa.a0 = ln.img[l][1]; wa.a1 = ln.img[l][lrt ? 2 : 3]; wa.g0 = ln.g[l][0]; wa.g1 = ln.g[l][1];
+    wa.B = M; wa.N = tc3_n(l); wa.KC = tc3_kc(l); wa.cin = tc3_k(l); wa.nsl = tc3_n(l);
+    const int kt = (tc3_kc(l) + 15) / 16, split = std::max(1, std::min(nmt, 148 / kt));
+    wa.mt_per = (nmt + split - 1) / split; wa.atomic = 1;
+    wa.gw0 = s.g0; wa.gw1 = s.g1; wa.w_off = s.w_off[l]; wa.b_off = s.b_off[l]; wa.status = tt_status_word();
+    const dim3 wgrid(kt, 1, (nmt + wa.mt_per - 1) / wa.mt_per);
+    if (lrt) tl_dw_kernel<BRL_MODE_LRT><<<wgrid, 256, TLW_SMEM, sd.side>>>(wa);
+    else if (flip) tl_dw_kernel<BRL_MODE_FLIPOUT><<<wgrid, 256, TLW_SMEM, sd.side>>>(wa);
+    else tl_dw_kernel<TT_PLAIN><<<wgrid, 256, TLW_SMEM, sd.side>>>(wa);
+    ++g_launch_count;
+    if (l == 0) break;  // conv1's input is x: no input gradient
+    TlDxArgs xa{};
+    xa.g0 = ln.g[l][0]; xa.g1 = ln.g[l][1];
+    xa.w0 = ln.w[l] + tc3_wimg(l); xa.w1 = ln.w[l] + 2 * (size_t)tc3_wimg(l);
+    xa.B = M; xa.Nl = tc3_n(l); xa.KCl = tc3_kc(l); xa.keep = 1.0f; xa.raw = 1;
+    xa.d0 = ln.col[0]; xa.d1 = ln.col[1]; xa.status = tt_status_word();
+    const dim3 xgrid(nmt, tc3_kc(l) * 8 / TL_XS);
+    if (lrt) tl_dx_kernel<BRL_MODE_LRT><<<xgrid, 256, TLX_SMEM, st>>>(xa);
+    else if (flip) tl_dx_kernel<BRL_MODE_FLIPOUT><<<xgrid, 256, TLX_SMEM, st>>>(xa);
+    else tl_dx_kernel<TT_PLAIN><<<xgrid, 256, TLX_SMEM, st>>>(xa);
+    ++g_launch_count;
+    act_bwd(l - 1, ln.col[0], ln.col[1]);
   }
   cudaEventRecord(sd.join, sd.side);
   cudaStreamWaitEvent(st, sd.join, 0);  // the weight gradients are part of what the caller finalises next

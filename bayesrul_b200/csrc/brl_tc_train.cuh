@@ -78,7 +78,8 @@ struct TtTail {
   int loss_kind = 0;         // single-contraction modes: 0 ELBO likelihood, 1 F.gaussian_nll_loss (HNN step)
   float keep_fc = 1.0f;      // dropout site behind the fc layer
   NoiseRef drop_fc{};
-  int width = 64;            // hidden units in front of the head: 64 (Inception fc layer), 32 (Linear layer 3)
+  int width = 64;            // hidden units in front of the head: 64 (Inception fc layer), 32 (Linear layer 3), 320 (Conv-D3: the
+                             // pooled conv3 features, given in `part` as [B, 320]; their gradient goes to `dpre`)
 };
 void tt_tail(const TtStep& s, const TtTail& t, cudaStream_t st);
 // backward: feature-gradient image -> g0 / g1 of the ten conv layers (accumulated: the buffers must be zeroed); 4 launches
@@ -106,5 +107,26 @@ void tl_forward(const TlLane& ln, const TtStep& s, cudaStream_t st, const TtSide
 // dpre / dsec[l]: compact [B, N_l] gradients of hidden layer l ([3] written by tt_tail); writes [0..2] and g0 / g1 of the four
 // hidden layers (plain stores)
 void tl_backward(const TlLane& ln, const TtStep& s, float* const* dpre, float* const* dsec, cudaStream_t st, const TtSide& sd);
+
+// ---- Conv-D3 net (brl_tc_train_convd3.cuh): the three convs on the tensor pipe as GEMMs over (window, position) rows, the head in
+// tt_tail (width 320: features in `feat`, their gradient to `dfeat`).  A TtStep describes the step with the convs at indices 0..2
+// (eps, sgn_in / sgn_out, drop / keep, w_off / b_off) and sgn_in[3] = the head's s_in.
+struct Tc3Lane {
+  unsigned char* img[3][4];  // im2col images of conv l's input, [M-tile][K/8 chunks][128 rows][16 B]: fp16 a | bf16 a |
+                             // bf16 a^2 (LRT) or fp16 a * s_in (Flipout) | bf16 a * s_in (Flipout)
+  unsigned char* w[3];       // weight images of conv l, [N/32 slices][K/8][32][16 B] (four roles as TlLane::w)
+  float* act[3];             // conv l's activation after ReLU / dropout [B * P, N]
+  float* rbuf[3];            // LRT: eps / (2 sd) [B * P, N]
+  float* g[3][2];            // gradients w.r.t. conv l's pre-activation / second path [B * P, N]
+  float* col[2];             // column gradients of conv3 / conv2 (input-gradient GEMMs, mean / second path) [B * 25, 320]
+  float* feat;               // pooled conv3 features [B, 320] (tt_tail's `part`)
+  float* dfeat;              // their gradient (tt_tail's `dpre`)
+};
+size_t tc3_lane_bytes(long long B);
+void tc3_carve(unsigned char* base, long long B, Tc3Lane& ln);
+// weight packing + 3 x (im2col, forward) + the pool into ln.feat
+void tc3_forward(const Tc3Lane& ln, const TtStep& s, cudaStream_t st, const TtSide& sd);
+// from ln.dfeat (written by tt_tail): g0 / g1 of the three convs (accumulated: the buffers must be zeroed)
+void tc3_backward(const Tc3Lane& ln, const TtStep& s, cudaStream_t st, const TtSide& sd);
 
 }  // namespace brl

@@ -112,11 +112,14 @@ struct TlFwdArgs {
   float* part;                   // last: [2][B][N]
   int* status;
 };
+// the K loop shared by the forward kernels (tl_fwd_kernel, tc3_fwd_kernel): sets up the CTA's barriers and 64 TMEM columns, thread 0
+// streams the slabs of M-tile `mt` / 32-column weight slice `ns` through the ring and issues the MMAs (mean path at column 0, the
+// second path at column TL_NS); every thread returns the TMEM base once the accumulators are complete
 template <int MODE>
-__global__ void __launch_bounds__(128, 1) tl_fwd_kernel(const TlFwdArgs a) {
-  extern __shared__ __align__(128) unsigned char smem[];
+__device__ __forceinline__ uint32_t tl_fwd_mainloop(unsigned char* smem, const unsigned char* a0, const unsigned char* a1,
+                                                    const unsigned char* w0, const unsigned char* w1, int KC, int mt, int ns, int* status) {
   constexpr bool DUAL = MODE != TT_PLAIN;
-  const int mt = blockIdx.x, ns = blockIdx.y, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  const int tid = threadIdx.x, warp = tid >> 5;
   const uint32_t sbase = smem_u32(smem), bfull = sbase + TLF_BAR, bempty = bfull + 8 * TL_STAGES, bdone = bempty + 8 * TL_STAGES;
   uint32_t* tslot = reinterpret_cast<uint32_t*>(smem + TLF_BAR + 64);
   if (tid == 0) {
@@ -130,25 +133,25 @@ __global__ void __launch_bounds__(128, 1) tl_fwd_kernel(const TlFwdArgs a) {
   tc_fence_after();
   const uint32_t tmem = *tslot;
   if (tid == 0) {  // producer and MMA issuer: slab `it` is loaded while slab `it - 2` is multiplied
-    const int nslab = a.KC / TL_KS;
-    const long long ao = (long long)mt * a.KC * TL_CH, wo = (long long)ns * a.KC * 512;
+    const int nslab = KC / TL_KS;
+    const long long ao = (long long)mt * KC * TL_CH, wo = (long long)ns * KC * 512;
     for (int it = 0; it < nslab + TL_STAGES - 1; ++it) {
       if (it < nslab) {
         const int s = it % TL_STAGES;
-        if (it >= TL_STAGES) mbar_wait(bempty + 8 * s, (it / TL_STAGES - 1) & 1, a.status, 60);
+        if (it >= TL_STAGES) mbar_wait(bempty + 8 * s, (it / TL_STAGES - 1) & 1, status, 60);
         const uint32_t st = sbase + s * TLF_STG, bar = bfull + 8 * s;
         mbar_expect_tx(bar, (DUAL ? 2 : 1) * (TL_KS * TL_CH + TL_KS * 512));
-        bulk_g2s(st, a.a0 + ao + (long long)it * TL_KS * TL_CH, TL_KS * TL_CH, bar);
-        bulk_g2s(st + 2 * TL_KS * TL_CH, a.w0 + wo + it * TL_KS * 512, TL_KS * 512, bar);
+        bulk_g2s(st, a0 + ao + (long long)it * TL_KS * TL_CH, TL_KS * TL_CH, bar);
+        bulk_g2s(st + 2 * TL_KS * TL_CH, w0 + wo + it * TL_KS * 512, TL_KS * 512, bar);
         if (DUAL) {
-          bulk_g2s(st + TL_KS * TL_CH, a.a1 + ao + (long long)it * TL_KS * TL_CH, TL_KS * TL_CH, bar);
-          bulk_g2s(st + 2 * TL_KS * TL_CH + TL_KS * 512, a.w1 + wo + it * TL_KS * 512, TL_KS * 512, bar);
+          bulk_g2s(st + TL_KS * TL_CH, a1 + ao + (long long)it * TL_KS * TL_CH, TL_KS * TL_CH, bar);
+          bulk_g2s(st + 2 * TL_KS * TL_CH + TL_KS * 512, w1 + wo + it * TL_KS * 512, TL_KS * 512, bar);
         }
       }
       const int j = it - (TL_STAGES - 1);
       if (j >= 0) {
         const int s = j % TL_STAGES;
-        mbar_wait(bfull + 8 * s, (j / TL_STAGES) & 1, a.status, 61);
+        mbar_wait(bfull + 8 * s, (j / TL_STAGES) & 1, status, 61);
         tc_fence_after();
         const uint32_t st = sbase + s * TLF_STG;
         for (int ks = 0; ks < TL_KS / 2; ++ks) {
@@ -165,8 +168,17 @@ __global__ void __launch_bounds__(128, 1) tl_fwd_kernel(const TlFwdArgs a) {
     }
     umma_commit(bdone);
   }
-  mbar_wait(bdone, 0, a.status, 62);
+  mbar_wait(bdone, 0, status, 62);
   tc_fence_after();
+  return tmem;
+}
+
+template <int MODE>
+__global__ void __launch_bounds__(128, 1) tl_fwd_kernel(const TlFwdArgs a) {
+  extern __shared__ __align__(128) unsigned char smem[];
+  constexpr bool DUAL = MODE != TT_PLAIN;
+  const int mt = blockIdx.x, ns = blockIdx.y, warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const uint32_t tmem = tl_fwd_mainloop<MODE>(smem, a.a0, a.a1, a.w0, a.w1, a.KC, mt, ns, a.status);
   // ---- epilogue: thread = window row (TMEM lane), eight columns at a time
   const int row = warp * 32 + lane, m = mt * 128 + row, N = a.N;
   const bool live = m < a.B;
@@ -299,6 +311,7 @@ struct TlDxArgs {
   const float* sout;             // Flipout: layer l - 1's s_out
   float keep;                    // dropout site behind layer l - 1 (plain mode)
   float *d0, *d1;                // layer l - 1's compact gradients [B, KCl * 8]
+  int raw;                       // 1: d0 / d1 receive the two GEMM results as they are (Conv-D3: col2im follows), no activation backward
   int* status;
 };
 template <int MODE>
@@ -360,6 +373,15 @@ __global__ void __launch_bounds__(256, 1) tl_dx_kernel(const TlDxArgs a) {
     tmem_ld_wait();
     if (m >= a.B) continue;
     const int k0 = xs * TL_XS + g * 8;
+    if (a.raw) {
+      const long long r0 = (long long)m * cin + k0;
+#pragma unroll
+      for (int j = 0; j < 8; ++j) {
+        a.d0[r0 + j] = v0[j];
+        if (DUAL) a.d1[r0 + j] = v1[j];
+      }
+      continue;
+    }
     unpack_h8(*reinterpret_cast<const uint4*>(a.act + (((long long)mt * a.KCl + (k0 >> 3)) * 128 + row) * 16), av);
     const long long e0 = (long long)m * cin + k0;
 #pragma unroll
@@ -380,8 +402,9 @@ __global__ void __launch_bounds__(256, 1) tl_dx_kernel(const TlDxArgs a) {
 }
 
 // ------------------------------------------------------------------------------------------------
-// weight gradient of hidden layer l: one CTA = 128 input features x (up to) 64 output columns, K = all windows (M-tile loop);
-// results as plain stores.  The CTAs of feature tile 0 also write the bias sums.
+// weight gradient of hidden layer l: one CTA = 128 input features x (up to) 64 output columns, K = the M-tiles
+// [blockIdx.z * mt_per, + mt_per); results as plain stores (one CTA per output: Linear) or atomics into the zeroed accumulators
+// (the M-tiles split over gridDim.z CTAs: Conv-D3).  The CTAs of feature tile 0 also write the bias sums.
 // ------------------------------------------------------------------------------------------------
 constexpr int TLW_A0 = 0, TLW_A1 = 16 * TL_CH, TLW_G0 = 32 * TL_CH, TLW_G1 = 40 * TL_CH, TLW_SUM = 48 * TL_CH,
               TLW_BAR = TLW_SUM + 512, TLW_SMEM = TLW_BAR + 64;
@@ -389,6 +412,7 @@ struct TlDwArgs {
   const unsigned char *a0, *a1;  // bf16 input images of layer l: a; a^2 (LRT) or a * s_in (Flipout)
   const float *g0, *g1;          // compact gradients [B, N]
   int B, N, KC, cin, nsl;
+  int mt_per, atomic;
   float *gw0, *gw1;
   long long w_off, b_off;
   int* status;
@@ -413,14 +437,14 @@ __global__ void __launch_bounds__(256, 1) tl_dw_kernel(const TlDwArgs a) {
   tc_fence_after();
   const uint32_t tmem = *tslot;
   // the last feature tile of layer 0 holds 8 chunks: features beyond them are accumulator rows nobody reads
-  const int nch = min(16, a.KC - kt * 16), nmt = (a.B + 127) / 128;
+  const int nch = min(16, a.KC - kt * 16), mt0 = blockIdx.z * a.mt_per, mt1 = min((a.B + 127) / 128, mt0 + a.mt_per);
   float bs0[4][8], bs1[4][8];
 #pragma unroll
   for (int t = 0; t < 4; ++t)
 #pragma unroll
     for (int j = 0; j < 8; ++j) bs0[t][j] = bs1[t][j] = 0.f;
   uint32_t ph = 0;
-  for (int mt = 0; mt < nmt; ++mt) {
+  for (int mt = mt0; mt < mt1; ++mt) {
     if (tid == 0) {
       const long long ao = ((long long)mt * a.KC + kt * 16) * TL_CH;
       mbar_expect_tx(bar_ld, (DUAL ? 2 : 1) * nch * TL_CH);
@@ -437,7 +461,7 @@ __global__ void __launch_bounds__(256, 1) tl_dw_kernel(const TlDwArgs a) {
       tc_fence_after();
       if (elect_one()) {
         for (int k = 0; k < 8; ++k) {  // 16 windows per k-step; both operands MN-major
-          const uint32_t acc = (mt | k) != 0;
+          const uint32_t acc = (mt != mt0) | (k != 0);
           umma(tmem, umma_desc(sbase + TLW_A0 + k * 256, 128, TL_CH), umma_desc(sbase + TLW_G0 + k * 256, 128, TL_CH),
                tt_idesc(a.nsl, 1, 1, 1), acc);
           if (DUAL)
@@ -465,8 +489,13 @@ __global__ void __launch_bounds__(256, 1) tl_dw_kernel(const TlDwArgs a) {
 #pragma unroll
       for (int j = 0; j < 8; ++j) {
         const long long wi = a.w_off + (long long)(n0 + g * 8 + j) * a.cin + k;
-        a.gw0[wi] = v0[j];
-        if (DUAL) a.gw1[wi] = v1[j];
+        if (a.atomic) {
+          atomicAdd(a.gw0 + wi, v0[j]);
+          if (DUAL) atomicAdd(a.gw1 + wi, v1[j]);
+        } else {
+          a.gw0[wi] = v0[j];
+          if (DUAL) a.gw1[wi] = v1[j];
+        }
       }
   }
   if (kt == 0) {  // bias: column sums of the staged gradients (a warp's items share their chunk: t-th chunk = (tid >> 7) + 2 t)
@@ -482,8 +511,14 @@ __global__ void __launch_bounds__(256, 1) tl_dw_kernel(const TlDwArgs a) {
     }
     __syncthreads();
     if (tid < a.nsl) {
-      a.gw0[a.b_off + n0 + tid] = sums[tid];
-      if (DUAL) a.gw1[a.b_off + n0 + tid] = MODE == BRL_MODE_LRT ? sums[64 + tid] : sums[tid];  // Flipout: the sampled bias
+      const float s1 = MODE == BRL_MODE_LRT ? sums[64 + tid] : sums[tid];  // Flipout: the sampled bias
+      if (a.atomic) {
+        atomicAdd(a.gw0 + a.b_off + n0 + tid, sums[tid]);
+        if (DUAL) atomicAdd(a.gw1 + a.b_off + n0 + tid, s1);
+      } else {
+        a.gw0[a.b_off + n0 + tid] = sums[tid];
+        if (DUAL) a.gw1[a.b_off + n0 + tid] = s1;
+      }
     }
   }
   tc_fence_before();

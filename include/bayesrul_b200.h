@@ -63,10 +63,10 @@ extern "C" {
                               * per layer per 4-window tile; operands are bulk-copied activation / weight images, taps are
                               * descriptor shifts, the backward contractions read the same images through MN-major descriptors;
                               * fp16 / bf16 operands, fp32 accumulation: outputs 1e-2, loss 5e-3, gradient cosine > 0.999).
-                              * Linear: the same two steps run the four hidden layers as tcgen05 GEMMs over 128-window tiles
-                              * (same operand precision and bound) when the workspace holds their images
-                              * (brl_workspace_bytes(B, S, 1) includes them), else the per-layer kernels.
-                              * Every other net keeps the fp32 FFMA kernels */
+                              * Linear: the same two steps run the four hidden layers as tcgen05 GEMMs over 128-window tiles;
+                              * Conv-D3: they run the three convs as tcgen05 GEMMs over (window, output position) rows of
+                              * im2col images.  Both with the same operand precision and bound, when the workspace holds their
+                              * images (brl_workspace_bytes(B, S, 1) includes them), else the per-layer kernels */
 
 #define BRL_MAX_LAYERS 16
 

@@ -3,7 +3,7 @@
     python tools/probe_train_fused.py [B] [net]
 
 net = inception (default): ELBO step (LRT 1 particle, Flipout 2 particles) at B (default 256) on simt / fused.
-net = linear: at B = 64 / 256 / 1024 (or the given B) the ELBO step (LRT 1 particle, Flipout 2 particles, weight sampling
+net = linear / conv: at B = 64 / 256 / 1024 (or the given B) the ELBO step (LRT 1 particle, Flipout 2 particles, weight sampling
 with the radial guide) + clipped_adam_vi and hnn_step at p = 0.3 + clipped_adam, on simt / tc / fused; CUDA events around
 200 steps after warm-up, median of 3 alternated repeats; the device name and power limit; at each size the fused-vs-fp32 loss
 ratio and gradient cosine of the first step."""
@@ -52,15 +52,15 @@ def inception():
     eng.set_gemm_backend("simt")
 
 
-def linear():
+def small_net(name):
     try:
         q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
                            capture_output=True, text=True).stdout.strip()
     except OSError:
         q = "nvidia-smi unavailable"
     print(f"device: {torch.cuda.get_device_name(dev)} | {q}")
-    eng = Engine("linear", dev)
-    mu0 = init_flat_params("linear", 12345).to(dev)
+    eng = Engine(name, dev)
+    mu0 = init_flat_params(name, 12345).to(dev)
     cases = (("lrt", 1, "normal", 1.351e-3, 0.138793), ("flipout", 2, "normal", 2.14e-4, 0.198768), ("ws", 1, "radial", 1.351e-3, 0.138793),
              ("hnn", 1, None, 0.0, 0.0))
     for B in ([B_arg] if B_arg else [64, 256, 1024]):
@@ -108,4 +108,4 @@ def linear():
     eng.set_gemm_backend("simt")
 
 
-linear() if net == "linear" else inception()
+small_net(net) if net in ("linear", "conv") else inception()
