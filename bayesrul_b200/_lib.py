@@ -71,6 +71,7 @@ SIGNATURES = {
     "brl_elbo_step": (_i, [_vp, _vp, _vp, _i64, _vp, _vp, _i, _i, _i, _f, _f, _i64, _np, _i, _vp, _vp, _vp, _vp, _vp,
                            _vp, _sz, _vp]),
     "brl_hnn_step": (_i, [_vp, _vp, _vp, _i64, _vp, _f, _np, _i, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "brl_hnn_step_ensemble": (_i, [_vp, _vp, _vp, _i64, _i64, _vp, _f, _np, _i, _vp, _vp, _vp, _vp, _sz, _vp]),
     "brl_mixture_moments": (_i, [_vp, _vp, _i64, _i64, _vp, _vp, _vp]),
     "brl_step_metrics": (_i, [_vp, _vp, _vp, _i64, _vp, _vp, _sz, _vp]),
     "brl_clipped_adam_vi_scaled": (_i, [_vp] * 9 + [_i64, _i64] + [_f] * 8 + [_vp]),

@@ -90,13 +90,13 @@ struct brl_ctx {
   // stream) over staging buffers in the caller's workspace; later calls replay it.
   struct StepKey {
     long long B, dataset_size;
-    int mode, guide, particles, compute_grads, backend, has_log_sigma;
+    int mode, guide, particles, compute_grads, backend, has_log_sigma, members;
     float prior_loc, prior_scale;
     const void *mu, *sigma, *ws;
     size_t ws_bytes;
     bool operator==(const StepKey& o) const {
       return B == o.B && dataset_size == o.dataset_size && mode == o.mode && guide == o.guide && particles == o.particles &&
-             compute_grads == o.compute_grads && backend == o.backend && has_log_sigma == o.has_log_sigma &&
+             compute_grads == o.compute_grads && backend == o.backend && has_log_sigma == o.has_log_sigma && members == o.members &&
              prior_loc == o.prior_loc && prior_scale == o.prior_scale && mu == o.mu && sigma == o.sigma && ws == o.ws &&
              ws_bytes == o.ws_bytes;
     }
@@ -137,6 +137,8 @@ struct ActBufs {
   // level-fused tcgen05 training kernels (Inception conv stack, brl_tc_train.cu): images of one particle lane
   TtLane tt{};
   bool has_tt = false;
+  int tt_members = 1;         // brl_hnn_step_ensemble: members whose lanes sit back to back from `tt`, tt_stride bytes apart
+  long long tt_stride = 0;
   // level-fused tcgen05 training kernels of the Linear net (brl_tc_train_linear.cuh): carved last, only where they fit
   TlLane tl{};
   bool has_tl = false;
@@ -202,6 +204,30 @@ static void carve_tl(const NetSpec& n, Carve& c, long long B, ActBufs& ab) {
   if (base && lin) tl_carve(base, B, ab.tl);
   if (base && !lin) tc3_carve(base, B, ab.tc3);
   (lin ? ab.has_tl : ab.has_tc3) = base != nullptr;
+}
+
+// brl_hnn_step_ensemble on the fused Inception kernels: the other M - 1 members' lanes right behind lane 0 (carve_train carves it
+// last), the members' fc-layer sums and gradients, and graph staging for M members.  A workspace without room for all of it keeps
+// the layout of the single-member step, whose body then runs once per member.
+static void carve_members(const NetSpec& n, Carve& c, long long B, long long M, ActBufs& ab) {
+  if (M < 2 || n.id != BRL_NET_INCEPTION || 2 * B * 64 > SPLITK_SCRATCH_FLOATS) return;
+  Carve t = c;
+  t.take<unsigned char>((M - 1) * (long long)tt_lane_bytes(B));  // tt_lane_bytes is a multiple of the carve alignment
+  float* part = t.take<float>(M * 2 * B * 64);
+  float* dpre = t.take<float>(M * B * 64);
+  float* sx = t.take<float>(M * B * 540);
+  float* sy = t.take<float>(M * B);
+  float* sout = t.take<float>(M * B * 2);
+  float* sg = t.take<float>(M * n.P);
+  double* ss = t.take<double>(2 * M);
+  if (c.base && (!t.ok || !ab.has_tt)) return;
+  c = t;
+  if (!c.base) return;
+  ab.tt_members = (int)M;
+  ab.tt_stride = (long long)tt_lane_bytes(B);
+  ab.part[0] = part;  // hnn_body's fc split-K sums, [M][2][B][64]
+  ab.dpre[n.ops.size() - 2] = dpre;
+  ab.st_x = sx; ab.st_y = sy; ab.st_out = sout; ab.st_gmu = sg; ab.st_scal = ss;
 }
 
 // device {seed, sample0, window0} of the step being captured (nullptr outside a capture): every Philox stream built by
@@ -764,6 +790,13 @@ int64_t brl_workspace_bytes(const brl_ctx* ctx, int64_t B, int64_t S, int train,
   const NetSpec& n = *ctx->net;
   Carve c(nullptr, 0);
   ActBufs ab;
+  if (train == 3) {  // brl_hnn_step_ensemble over S members: the layout of hnn_step
+    carve_forward(n, c, B, 1, ab);
+    carve_train(n, c, B, ab);
+    carve_tl(n, c, B, ab);
+    carve_members(n, c, B, S, ab);
+    return (int64_t)c.used + 4096;
+  }
   c.take<float>(4 * B);          // moment state
   c.take<float>(S * n.P);        // weight samples
   c.take<float>(S * 2 * (long long)n.layers.size());
@@ -1421,13 +1454,22 @@ int brl_elbo_step(brl_ctx* ctx, const float* x, const float* y, int64_t B, const
                    scalars, grad_mu, grad_sigma, grad_log_sigma, out, st);
 }
 
-// the launches of one heteroscedastic-NN step (every pointer final); captured as is by the graph path of brl_hnn_step
-static int hnn_body(brl_ctx* ctx, const ActBufs& ab, const float* x, const float* y, int64_t B, const float* theta, float p_dropout,
-                    const brl_noise* noise, int compute_grads, double* scalars, float* grad_theta, float* out, cudaStream_t st) {
+// M members of an HNN step in ONE chain of launches: the level-fused Inception kernels with the workspace's lanes for M members
+static bool hnn_batched(const brl_ctx* ctx, const ActBufs& ab, long long M, long long B) {
+  return ctx->gemm_backend == BRL_GEMM_TC_FUSED && ctx->net->id == BRL_NET_INCEPTION && ab.has_tt && ab.tt_members >= M &&
+         2 * B * 64 <= SPLITK_SCRATCH_FLOATS;
+}
+
+// the launches of one heteroscedastic-NN step of M members (every pointer final; M > 1 only where hnn_batched holds); captured
+// as is by the graph path of hnn_step
+static int hnn_body(brl_ctx* ctx, const ActBufs& ab, const float* x, const float* y, int64_t M, int64_t B, const float* theta,
+                    float p_dropout, const brl_noise* noise, int compute_grads, double* scalars, float* grad_theta, float* out,
+                    cudaStream_t st) {
   const NetSpec& n = *ctx->net;
   brl_noise nz = noise_at_sample(n, noise, 0, B);
-  if (ctx->gemm_backend == BRL_GEMM_TC_FUSED && n.id == BRL_NET_INCEPTION && ab.has_tt && 2 * B * 64 <= SPLITK_SCRATCH_FLOATS) {
-    // level-fused tcgen05 kernels, one contraction with the deterministic weights; dropout masks in the epilogues
+  if (hnn_batched(ctx, ab, M, B)) {
+    // level-fused tcgen05 kernels, one contraction with the deterministic weights; dropout masks in the epilogues; member m on
+    // blockIdx.z with its own lane, parameters, gradients and MC-sample index sample0 + m
     const brl_ctx::Lane& ln = ctx->lanes[0];
     const int fc_op = (int)n.ops.size() - 2, fc_layer = n.ops[fc_op].layer, hd_layer = n.ops[fc_op + 1].layer;
     auto keep_of = [&](int ly) { return (p_dropout > 0.f && n.layers[ly].drop_factor > 0.f) ? 1.0f - p_dropout * n.layers[ly].drop_factor : 1.0f; };
@@ -1440,9 +1482,10 @@ static int hnn_body(brl_ctx* ctx, const ActBufs& ab, const float* x, const float
     }
     ts.w_off_fc = n.layers[fc_layer].w_off; ts.b_off_fc = n.layers[fc_layer].b_off;
     ts.g0 = grad_theta; ts.g1 = nullptr;
+    ts.members = (int)M; ts.P = n.P; ts.lane_stride = ab.tt_stride;
     const TtSide tsd{ln.side[0], ln.ev_fork, ln.ev_join[0]};
-    BRL_CUDA(cudaMemsetAsync(scalars, 0, 2 * sizeof(double), st));
-    if (compute_grads) BRL_CUDA(cudaMemsetAsync(grad_theta, 0, sizeof(float) * n.P, st));
+    BRL_CUDA(cudaMemsetAsync(scalars, 0, 2 * M * sizeof(double), st));
+    if (compute_grads) BRL_CUDA(cudaMemsetAsync(grad_theta, 0, sizeof(float) * M * n.P, st));
     tt_forward(ab.tt, ts, st, tsd);
     tt_fc_forward(ab.tt, ts, ab.part[0], st);
     TtTail tl{};
@@ -1458,6 +1501,7 @@ static int hnn_body(brl_ctx* ctx, const ActBufs& ab, const float* x, const float
     BRL_CUDA(cudaGetLastError());
     return BRL_OK;
   }
+  if (M != 1) return fail(BRL_ERR_INVALID, "bayesrul_b200: hnn_body: members need the batched path");
   if (ctx->gemm_backend == BRL_GEMM_TC_FUSED && n.id == BRL_NET_LINEAR && ab.has_tl) {
     // the Linear net's fused kernels, one contraction with the deterministic weights; keep decisions in the epilogues
     const brl_ctx::Lane& ln = ctx->lanes[0];
@@ -1528,21 +1572,31 @@ static int hnn_body(brl_ctx* ctx, const ActBufs& ab, const float* x, const float
   return BRL_OK;
 }
 
-int brl_hnn_step(brl_ctx* ctx, const float* x, const float* y, int64_t B, const float* theta, float p_dropout,
-                 const brl_noise* noise, int compute_grads, double* scalars, float* grad_theta, float* out,
-                 void* workspace, size_t workspace_bytes, void* stream) {
-  BRL_REQUIRE(ctx && x && y && theta && scalars && out && workspace, "brl_hnn_step: NULL argument");
-  DeviceGuard dg(ctx->device);
-  BRL_REQUIRE(B > 0 && p_dropout >= 0.f && p_dropout < 1.f, "brl_hnn_step: bad B or p_dropout");
-  BRL_REQUIRE(!compute_grads || grad_theta, "brl_hnn_step: grad_theta is NULL");
-  cudaStream_t st = (cudaStream_t)stream;
+// brl_hnn_step (M = 1) and brl_hnn_step_ensemble: M members in one chain of launches where hnn_batched holds, else one member
+// after another on the single-member step
+static int hnn_step(brl_ctx* ctx, const float* x, const float* y, int64_t M, int64_t B, const float* theta, float p_dropout,
+                    const brl_noise* noise, int compute_grads, double* scalars, float* grad_theta, float* out,
+                    void* workspace, size_t workspace_bytes, cudaStream_t st) {
   const NetSpec& n = *ctx->net;
   Carve c(workspace, workspace_bytes);
   ActBufs ab;
   carve_forward(n, c, B, 1, ab);
   carve_train(n, c, B, ab);
-  if (!c.ok) return fail(BRL_ERR_WORKSPACE, "brl_hnn_step: workspace too small");
+  if (!c.ok) return fail(BRL_ERR_WORKSPACE, M == 1 ? "brl_hnn_step: workspace too small" : "brl_hnn_step_ensemble: workspace too small");
   carve_tl(n, c, B, ab);
+  carve_members(n, c, B, M, ab);
+  if (M > 1 && !hnn_batched(ctx, ab, M, B)) {
+    brl_noise base;
+    memset(&base, 0, sizeof(base));
+    if (noise) base = *noise;
+    for (int64_t m = 0; m < M; ++m) {
+      const brl_noise nm = noise_at_sample(n, &base, m, B);  // MC-sample index sample0 + m, injected masks of member m
+      const int rc = hnn_step(ctx, x + m * B * 540, y + m * B, 1, B, theta + m * n.P, p_dropout, &nm, compute_grads, scalars + 2 * m,
+                              compute_grads ? grad_theta + m * n.P : nullptr, out + m * B * 2, workspace, workspace_bytes, st);
+      if (rc != BRL_OK) return rc;
+    }
+    return BRL_OK;
+  }
   // ---- graph replay, same scheme as brl_elbo_step (native dropout masks or no dropout): eager, capture, replay
   brl_ctx::StepGraph* sg = nullptr;
   bool caller_captures = false;
@@ -1555,6 +1609,7 @@ int brl_hnn_step(brl_ctx* ctx, const float* x, const float* y, int64_t B, const 
     brl_ctx::StepKey key;
     memset(&key, 0, sizeof(key));
     key.B = B; key.mode = -1 /* HNN */; key.particles = 1; key.compute_grads = compute_grads; key.backend = ctx->gemm_backend;
+    key.members = (int)M;
     key.prior_loc = p_dropout; key.mu = theta; key.ws = workspace; key.ws_bytes = workspace_bytes;
     for (auto it = ctx->graphs.begin(); it != ctx->graphs.end(); ++it)
       if (it->key == key) { ctx->graphs.splice(ctx->graphs.begin(), ctx->graphs, it); sg = &ctx->graphs.front(); break; }
@@ -1575,7 +1630,7 @@ int brl_hnn_step(brl_ctx* ctx, const float* x, const float* y, int64_t B, const 
         const long long l0 = launch_count();
         brl_noise zero;
         memset(&zero, 0, sizeof(zero));
-        const int rc = hnn_body(ctx, ab, ab.st_x, ab.st_y, B, theta, p_dropout, &zero, compute_grads, ab.st_scal,
+        const int rc = hnn_body(ctx, ab, ab.st_x, ab.st_y, M, B, theta, p_dropout, &zero, compute_grads, ab.st_scal,
                                 compute_grads ? ab.st_gmu : nullptr, ab.st_out, ctx->cap);
         g_dyn = nullptr;
         sg->launches = (int)(launch_count() - l0);
@@ -1595,8 +1650,8 @@ int brl_hnn_step(brl_ctx* ctx, const float* x, const float* y, int64_t B, const 
   if (sg && sg->exec) {
     count_launch(sg->launches);
     CopyJobs in{};
-    in.dst[0] = ab.st_x; in.src[0] = x; in.n[0] = B * 540;
-    in.dst[1] = ab.st_y; in.src[1] = y; in.n[1] = B;
+    in.dst[0] = ab.st_x; in.src[0] = x; in.n[0] = M * B * 540;
+    in.dst[1] = ab.st_y; in.src[1] = y; in.n[1] = M * B;
     in.njobs = 2;
     in.dyn = ab.dyn;
     in.seed = noise ? noise->seed : 0ull;
@@ -1605,15 +1660,37 @@ int brl_hnn_step(brl_ctx* ctx, const float* x, const float* y, int64_t B, const 
     launch_copy_jobs(in, st);
     BRL_CUDA(cudaGraphLaunch(sg->exec, st));
     CopyJobs o{};
-    o.dst[0] = reinterpret_cast<float*>(scalars); o.src[0] = reinterpret_cast<const float*>(ab.st_scal); o.n[0] = 4;
-    o.dst[1] = out; o.src[1] = ab.st_out; o.n[1] = B * 2;
+    o.dst[0] = reinterpret_cast<float*>(scalars); o.src[0] = reinterpret_cast<const float*>(ab.st_scal); o.n[0] = 4 * M;
+    o.dst[1] = out; o.src[1] = ab.st_out; o.n[1] = M * B * 2;
     o.njobs = 2;
-    if (compute_grads) { o.dst[2] = grad_theta; o.src[2] = ab.st_gmu; o.n[2] = n.P; o.njobs = 3; }
+    if (compute_grads) { o.dst[2] = grad_theta; o.src[2] = ab.st_gmu; o.n[2] = M * n.P; o.njobs = 3; }
     launch_copy_jobs(o, st);
     BRL_CUDA(cudaGetLastError());
     return BRL_OK;
   }
-  return hnn_body(ctx, ab, x, y, B, theta, p_dropout, noise, compute_grads, scalars, grad_theta, out, st);
+  return hnn_body(ctx, ab, x, y, M, B, theta, p_dropout, noise, compute_grads, scalars, grad_theta, out, st);
+}
+
+int brl_hnn_step(brl_ctx* ctx, const float* x, const float* y, int64_t B, const float* theta, float p_dropout,
+                 const brl_noise* noise, int compute_grads, double* scalars, float* grad_theta, float* out,
+                 void* workspace, size_t workspace_bytes, void* stream) {
+  BRL_REQUIRE(ctx && x && y && theta && scalars && out && workspace, "brl_hnn_step: NULL argument");
+  DeviceGuard dg(ctx->device);
+  BRL_REQUIRE(B > 0 && p_dropout >= 0.f && p_dropout < 1.f, "brl_hnn_step: bad B or p_dropout");
+  BRL_REQUIRE(!compute_grads || grad_theta, "brl_hnn_step: grad_theta is NULL");
+  return hnn_step(ctx, x, y, 1, B, theta, p_dropout, noise, compute_grads, scalars, grad_theta, out, workspace, workspace_bytes,
+                  (cudaStream_t)stream);
+}
+
+int brl_hnn_step_ensemble(brl_ctx* ctx, const float* x, const float* y, int64_t M, int64_t B, const float* theta, float p_dropout,
+                          const brl_noise* noise, int compute_grads, double* scalars, float* grad_theta, float* out,
+                          void* workspace, size_t workspace_bytes, void* stream) {
+  BRL_REQUIRE(ctx && x && y && theta && scalars && out && workspace, "brl_hnn_step_ensemble: NULL argument");
+  DeviceGuard dg(ctx->device);
+  BRL_REQUIRE(M > 0 && M < (1 << 16) && B > 0 && p_dropout >= 0.f && p_dropout < 1.f, "brl_hnn_step_ensemble: bad M, B or p_dropout");
+  BRL_REQUIRE(!compute_grads || grad_theta, "brl_hnn_step_ensemble: grad_theta is NULL");
+  return hnn_step(ctx, x, y, M, B, theta, p_dropout, noise, compute_grads, scalars, grad_theta, out, workspace, workspace_bytes,
+                  (cudaStream_t)stream);
 }
 
 int brl_mixture_moments(const float* mu_m, const float* sigma_m, int64_t M, int64_t nn, float* mu, float* sigma, void* stream) {

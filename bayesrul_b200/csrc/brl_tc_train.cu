@@ -186,13 +186,34 @@ __device__ __forceinline__ float warp_sum(float v) {
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
   return v;
 }
+// ensemble member blockIdx.z (TtStep::members): its lane images sit `stride` bytes after the previous member's
+__device__ __forceinline__ TtLane member_lane(TtLane ln, long long stride) {
+  const long long o = stride * blockIdx.z;
+  auto sh = [o](auto* p) { return p ? reinterpret_cast<decltype(p)>(reinterpret_cast<unsigned char*>(p) + o) : p; };
+  ln.ximg = sh(ln.ximg); ln.m1 = sh(ln.m1); ln.t2 = sh(ln.t2); ln.t3 = sh(ln.t3);
+  for (int k = 0; k < 6; ++k) ln.g[k] = sh(ln.g[k]);
+  ln.rbuf = sh(ln.rbuf); ln.blob = sh(ln.blob); ln.part = sh(ln.part);
+  ln.fimg = sh(ln.fimg); ln.fbimg = sh(ln.fbimg); ln.f2img = sh(ln.f2img); ln.f2bimg = sh(ln.f2bimg); ln.gfimg = sh(ln.gfimg);
+  ln.fcblob = sh(ln.fcblob);
+  return ln;
+}
+// the member's dropout stream: injected masks [members, B, per_window], Philox keys with MC-sample index sample0 + member
+__device__ __forceinline__ NoiseRef member_noise(NoiseRef nz, long long per_window, int B) {
+  if (nz.ptr) nz.ptr += (long long)blockIdx.z * B * per_window;
+  else nz.sample0 += blockIdx.z;
+  return nz;
+}
+template <typename T>
+__device__ __forceinline__ T* member_ptr(T* p, long long stride) { return p ? p + stride * blockIdx.z : p; }
 
 // ------------------------------------------------------------------------------------------------
 // window images: fp32 windows -> fp16 chunk images X and XP = MaxPool1d(3,1,1)(X) (-inf padding), pad rows zero
 // ------------------------------------------------------------------------------------------------
-__global__ void tt_packx_kernel(const float* __restrict__ x, unsigned char* __restrict__ ximg, int B, int ntile) {
+__global__ void tt_packx_kernel(const float* __restrict__ x, unsigned char* __restrict__ ximg, int B, int ntile, long long lane_stride) {
   const long long u = blockIdx.x * (long long)blockDim.x + threadIdx.x;
   if (u >= (long long)ntile * 3 * ROWS) return;
+  x += (long long)blockIdx.z * B * 540;
+  ximg += lane_stride * blockIdx.z;
   const int tile = (int)(u / (3 * ROWS)), v = (int)(u % (3 * ROWS)), c = v / ROWS, rr = v % ROWS;
   const RowInfo ri = row_info(rr, tile, B);
   float f[8], pm[8];
@@ -226,9 +247,13 @@ struct TtPackArgs {
   int mode;
   const float *mu, *second;  // second: sigma (LRT) or the weight draw (Flipout)
   unsigned char* blob;
+  long long P, lane_stride;  // ensemble members (blockIdx.z): parameter / lane strides
 };
 __global__ void tt_pack_kernel(const TtPackArgs a) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  const float* mu = a.mu + a.P * blockIdx.z;
+  const float* second = a.second + a.P * blockIdx.z;
+  unsigned char* blob = a.blob + a.lane_stride * blockIdx.z;
   if (i < a.start[TT_LAYERS]) {
     int li = 0;
     while (i >= a.start[li + 1]) ++li;
@@ -241,15 +266,15 @@ __global__ void tt_pack_kernel(const TtPackArgs a) {
     float m = 0.f, s = 0.f;
     if (n < l.N && cr >= 0) {
       const long long wi = l.w_off + ((long long)n * l.cin + cr) * l.T + tap;
-      m = a.mu[wi];
-      const float v = a.second[wi];
+      m = mu[wi];
+      const float v = second[wi];
       s = a.mode == BRL_MODE_LRT ? v * v : a.mode == BRL_MODE_FLIPOUT ? v - m : 0.f;
     }
     const int o = tap * l.tap_bytes + (k >> 3) * (l.NP * 16) + n * 16 + (k & 7) * 2;
-    *reinterpret_cast<__half*>(a.blob + l.w0h + o) = __float2half_rn(m);
-    *reinterpret_cast<__nv_bfloat16*>(a.blob + l.w0b + o) = __float2bfloat16_rn(m);
-    *reinterpret_cast<__nv_bfloat16*>(a.blob + l.w1b + o) = __float2bfloat16_rn(s);
-    *reinterpret_cast<__half*>(a.blob + l.w1h + o) = __float2half_rn(s);
+    *reinterpret_cast<__half*>(blob + l.w0h + o) = __float2half_rn(m);
+    *reinterpret_cast<__nv_bfloat16*>(blob + l.w0b + o) = __float2bfloat16_rn(m);
+    *reinterpret_cast<__nv_bfloat16*>(blob + l.w1b + o) = __float2bfloat16_rn(s);
+    *reinterpret_cast<__half*>(blob + l.w1h + o) = __float2half_rn(s);
     return;
   }
   const int b = i - a.start[TT_LAYERS];
@@ -258,11 +283,11 @@ __global__ void tt_pack_kernel(const TtPackArgs a) {
     const int n = b & 63;
     float b0 = 0.f, b1 = 0.f;
     if (n < l.N) {
-      if (a.mode == BRL_MODE_LRT) { b0 = a.mu[l.b_off + n]; const float sb = a.second[l.b_off + n]; b1 = sb * sb; }
-      else if (a.mode == BRL_MODE_FLIPOUT) b0 = a.second[l.b_off + n];  // Flipout adds the SAMPLED bias (SURVEY A.4)
-      else b0 = a.mu[l.b_off + n];
+      if (a.mode == BRL_MODE_LRT) { b0 = mu[l.b_off + n]; const float sb = second[l.b_off + n]; b1 = sb * sb; }
+      else if (a.mode == BRL_MODE_FLIPOUT) b0 = second[l.b_off + n];  // Flipout adds the SAMPLED bias (SURVEY A.4)
+      else b0 = mu[l.b_off + n];
     }
-    float* bias = reinterpret_cast<float*>(a.blob + l.bias);
+    float* bias = reinterpret_cast<float*>(blob + l.bias);
     bias[n] = b0;
     bias[64 + n] = b1;
   }
@@ -284,6 +309,7 @@ struct TtFwdArgs {
   const float* sgn_fc_in;  // Flipout: s_in of the fc layer [B, 2400] (the feature producers build its perturbation operand)
   NoiseRef drop[4];        // PLAIN mode: dropout site behind the layer (injected masks [B, N, 30] or Philox)
   float keep[4];           // its keep probability (1 = no dropout site / dropout off)
+  long long lane_stride;   // ensemble members (blockIdx.z, PLAIN mode): bytes between their lanes
   int* status;
   long long* trace;  // debug: clock64 stamps of CTA (0, y), [4 layers][16] (nullptr = off)
 };
@@ -343,7 +369,8 @@ __global__ void __launch_bounds__(NT, 1) tt_fwd_kernel(const TtFwdArgs a) {
   extern __shared__ __align__(128) unsigned char smem[];
   const TtLayer& L = a.lay[blockIdx.y];
   const int tile = blockIdx.x, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  long long* tr = (a.trace && blockIdx.x == 0 && tid == 0) ? a.trace + blockIdx.y * 16 : nullptr;
+  long long* tr = (a.trace && blockIdx.x == 0 && blockIdx.z == 0 && tid == 0) ? a.trace + blockIdx.y * 16 : nullptr;
+  const TtLane ln = MODE == TT_PLAIN ? member_lane(a.ln, a.lane_stride) : a.ln;
   if (tr) tr[0] = clock64();
   const uint32_t sbase = smem_u32(smem);
   const uint32_t bar_ld = sbase + F_BAR, bar_mma = bar_ld + 8;
@@ -365,10 +392,10 @@ __global__ void __launch_bounds__(NT, 1) tt_fwd_kernel(const TtFwdArgs a) {
   const int img_bytes = L.T * L.tap_bytes;
   if (tid == 0) {
     mbar_expect_tx(bar_ld, ncopy * CS + (MODE == TT_PLAIN ? 1 : 2) * img_bytes + 512);
-    bulk_copy_chunked(sbase + (L.in == IN_M1P ? F_A2 : F_A), input_image(a.ln, L.in, tile), ncopy * CS, bar_ld);
-    bulk_copy_chunked(sbase + F_W0, a.ln.blob + L.w0h, img_bytes, bar_ld);
-    if (MODE != TT_PLAIN) bulk_copy_chunked(sbase + F_W1, a.ln.blob + (MODE == BRL_MODE_FLIPOUT ? L.w1h : L.w1b), img_bytes, bar_ld);
-    bulk_g2s(sbase + F_BIAS, a.ln.blob + L.bias, 512, bar_ld);
+    bulk_copy_chunked(sbase + (L.in == IN_M1P ? F_A2 : F_A), input_image(ln, L.in, tile), ncopy * CS, bar_ld);
+    bulk_copy_chunked(sbase + F_W0, ln.blob + L.w0h, img_bytes, bar_ld);
+    if (MODE != TT_PLAIN) bulk_copy_chunked(sbase + F_W1, ln.blob + (MODE == BRL_MODE_FLIPOUT ? L.w1h : L.w1b), img_bytes, bar_ld);
+    bulk_g2s(sbase + F_BIAS, ln.blob + L.bias, 512, bar_ld);
   }
   if (tr) tr[1] = clock64();
   mbar_wait(bar_ld, 0, a.status, 40);
@@ -411,10 +438,11 @@ __global__ void __launch_bounds__(NT, 1) tt_fwd_kernel(const TtFwdArgs a) {
   const NoiseRef& nz = a.eps[blockIdx.y];
   const NoiseKey nk = noise_key(nz);
   const float* sout = a.sgn_out[blockIdx.y];
-  float* rb = a.ln.rbuf ? a.ln.rbuf + (long long)tile * RBUF_PER_TILE + L.roff_per_tile : nullptr;
-  unsigned char* oimg = L.out == OUT_M1 ? a.ln.m1 + (long long)tile * 16 * CS
-                        : L.out == OUT_T2 ? a.ln.t2 + (long long)tile * 8 * CS
-                        : L.out == OUT_T3 ? a.ln.t3 + (long long)tile * 8 * CS : nullptr;
+  const NoiseRef dz = MODE == TT_PLAIN ? member_noise(a.drop[blockIdx.y], (long long)L.N * 30, a.B) : a.drop[blockIdx.y];
+  float* rb = ln.rbuf ? ln.rbuf + (long long)tile * RBUF_PER_TILE + L.roff_per_tile : nullptr;
+  unsigned char* oimg = L.out == OUT_M1 ? ln.m1 + (long long)tile * 16 * CS
+                        : L.out == OUT_T2 ? ln.t2 + (long long)tile * 8 * CS
+                        : L.out == OUT_T3 ? ln.t3 + (long long)tile * 8 * CS : nullptr;
   // LRT eps of the warp's window (one warp = the 30 steps of one window x 8 channels = elements [240 g, 240 g + 240) of the
   // layer's stream, i.e. exactly Philox blocks [60 g, 60 g + 60)): every lane draws two blocks = eight normals into a per-warp
   // scratch (the operand regions are dead once the MMAs have completed) instead of one block per element
@@ -426,8 +454,7 @@ __global__ void __launch_bounds__(NT, 1) tt_fwd_kernel(const TtFwdArgs a) {
     KeepBits kb = {};
     const float keep = MODE == TT_PLAIN ? a.keep[blockIdx.y] : 1.0f;
     const uint32_t e0 = (uint32_t)ri.t * (uint32_t)((L.N + 15) & ~15) + (uint32_t)(g * 8);  // dropout element order: position-major
-    if (MODE == TT_PLAIN && keep < 1.0f && !a.drop[blockIdx.y].ptr) {  // 8 of the 16 keep decisions of one Philox block
-      const NoiseRef& dz = a.drop[blockIdx.y];
+    if (MODE == TT_PLAIN && keep < 1.0f && !dz.ptr) {  // 8 of the 16 keep decisions of one Philox block
       const NoiseKey dk = noise_key(dz);
       kb = keep_bits(philox_block_mask(dk.seed, dz.kind, dz.site, dk.sample0, dk.window0 + ri.gw, e0 >> 4), keep_threshold(keep));
     }
@@ -462,7 +489,6 @@ __global__ void __launch_bounds__(NT, 1) tt_fwd_kernel(const TtFwdArgs a) {
       }
       o[j] = on ? fmaxf(pre, 0.f) : 0.f;
       if (MODE == TT_PLAIN && keep < 1.0f && on) {  // dropout site behind the ReLU (inception.py:48-52,119-123)
-        const NoiseRef& dz = a.drop[blockIdx.y];
         const bool kp = dz.ptr ? dz.ptr[((long long)ri.gw * L.N + n) * 30 + ri.t] != 0.f : keep_at(kb, (e0 & 15u) + j);
         o[j] = kp ? o[j] / keep : 0.f;
       }
@@ -479,13 +505,13 @@ __global__ void __launch_bounds__(NT, 1) tt_fwd_kernel(const TtFwdArgs a) {
       for (int j = 0; j < 8; ++j)
         f2[j] = MODE == BRL_MODE_LRT ? fr[j] * fr[j]
                 : MODE == BRL_MODE_FLIPOUT ? fr[j] * __ldg(a.sgn_fc_in + (long long)ri.gw * 2400 + (c0 + j) * 30 + ri.t) : 0.f;
-      *reinterpret_cast<uint4*>(a.ln.fimg + fa) = fh;
-      *reinterpret_cast<uint4*>(a.ln.fbimg + fa) = pack_b8(fr);
+      *reinterpret_cast<uint4*>(ln.fimg + fa) = fh;
+      *reinterpret_cast<uint4*>(ln.fbimg + fa) = pack_b8(fr);
       if (MODE == BRL_MODE_LRT) {
-        *reinterpret_cast<uint4*>(a.ln.f2img + fa) = pack_b8(f2);
+        *reinterpret_cast<uint4*>(ln.f2img + fa) = pack_b8(f2);
       } else if (MODE == BRL_MODE_FLIPOUT) {  // the perturbation GEMM runs fp16 x fp16 in the forward pass (f * s_in is exact in fp16), bf16 in the backward pass
-        *reinterpret_cast<uint4*>(a.ln.f2img + fa) = pack_h8(f2);
-        *reinterpret_cast<uint4*>(a.ln.f2bimg + fa) = pack_b8(f2);
+        *reinterpret_cast<uint4*>(ln.f2img + fa) = pack_h8(f2);
+        *reinterpret_cast<uint4*>(ln.f2bimg + fa) = pack_b8(f2);
       }
     }
   }
@@ -515,6 +541,7 @@ struct TtBwdArgs {
   const float* sgn_out[4];
   float *g0, *g1;
   float keep[4];  // PLAIN mode: keep probability of the dropout site behind each layer (1 = none)
+  long long lane_stride;  // ensemble members (blockIdx.z, PLAIN mode): bytes between their lanes
   int part_floats;
   int* status;
   long long* trace;
@@ -522,7 +549,7 @@ struct TtBwdArgs {
 
 // gradient w.r.t. the layer OUTPUT (post-activation), 8 channels [n0, n0 + 8) of tile row `row`, and the ReLU gate
 template <int MODE>
-__device__ __forceinline__ void output_grad(const TtBwdArgs& a, const TtLayer& L, int tile, int row, const RowInfo& ri, int n0,
+__device__ __forceinline__ void output_grad(const TtLane& ln, const TtLayer& L, int tile, int row, const RowInfo& ri, int n0,
                                             float (&d)[8]) {
 #pragma unroll
   for (int j = 0; j < 8; ++j) d[j] = 0.f;
@@ -530,8 +557,8 @@ __device__ __forceinline__ void output_grad(const TtBwdArgs& a, const TtLayer& L
   if (L.out == OUT_FEAT) {
     const long long fa = feat_addr(ri.gw, ri.t, L.out_c0 + n0);
     float f[8], gr[8];
-    unpack_h8(*reinterpret_cast<const uint4*>(a.ln.fimg + fa), f);
-    unpack_b8(*reinterpret_cast<const uint4*>(a.ln.gfimg + fa), gr);
+    unpack_h8(*reinterpret_cast<const uint4*>(ln.fimg + fa), f);
+    unpack_b8(*reinterpret_cast<const uint4*>(ln.gfimg + fa), gr);
 #pragma unroll
     for (int j = 0; j < 8; ++j) d[j] = f[j] > 0.f ? gr[j] : 0.f;
     return;
@@ -540,8 +567,8 @@ __device__ __forceinline__ void output_grad(const TtBwdArgs& a, const TtLayer& L
   float act[8], g[8];
   if (L.out != OUT_M1) {
     const int c = n0 >> 3;
-    const unsigned char* ai = (L.out == OUT_T2 ? a.ln.t2 : a.ln.t3) + ((long long)tile * 8 + c) * CS + ro;
-    const unsigned char* gi = a.ln.g[L.out == OUT_T2 ? 4 : 5] + ((long long)tile * 8 + c) * CS + ro;
+    const unsigned char* ai = (L.out == OUT_T2 ? ln.t2 : ln.t3) + ((long long)tile * 8 + c) * CS + ro;
+    const unsigned char* gi = ln.g[L.out == OUT_T2 ? 4 : 5] + ((long long)tile * 8 + c) * CS + ro;
     unpack_h8(*reinterpret_cast<const uint4*>(ai), act);
     unpack_b8(*reinterpret_cast<const uint4*>(gi), g);
 #pragma unroll
@@ -552,12 +579,12 @@ __device__ __forceinline__ void output_grad(const TtBwdArgs& a, const TtLayer& L
   const long long co = ((long long)tile * 16 + L.out_c0 + (n0 >> 3)) * CS + ro;
   float m[5][8], gp[3][8];
 #pragma unroll
-  for (int q = 0; q < 5; ++q) unpack_h8(*reinterpret_cast<const uint4*>(a.ln.m1 + co + (q - 2) * 16), m[q]);
+  for (int q = 0; q < 5; ++q) unpack_h8(*reinterpret_cast<const uint4*>(ln.m1 + co + (q - 2) * 16), m[q]);
 #pragma unroll
-  for (int q = 0; q < 3; ++q) unpack_b8(*reinterpret_cast<const uint4*>(a.ln.g[3] + co + (q - 1) * 16), gp[q]);
+  for (int q = 0; q < 3; ++q) unpack_b8(*reinterpret_cast<const uint4*>(ln.g[3] + co + (q - 1) * 16), gp[q]);
 #pragma unroll
   for (int k = 0; k < 3; ++k) {
-    unpack_b8(*reinterpret_cast<const uint4*>(a.ln.g[k] + co), g);
+    unpack_b8(*reinterpret_cast<const uint4*>(ln.g[k] + co), g);
 #pragma unroll
     for (int j = 0; j < 8; ++j) d[j] += g[j];
   }
@@ -590,7 +617,8 @@ __global__ void __launch_bounds__(NT, 1) tt_bwd_kernel(const TtBwdArgs a) {
   extern __shared__ __align__(128) unsigned char smem[];
   const TtLayer& L = a.lay[blockIdx.y];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  long long* tr = (a.trace && blockIdx.x == 0 && tid == 0) ? a.trace + blockIdx.y * 16 : nullptr;
+  long long* tr = (a.trace && blockIdx.x == 0 && blockIdx.z == 0 && tid == 0) ? a.trace + blockIdx.y * 16 : nullptr;
+  const TtLane ln = MODE == TT_PLAIN ? member_lane(a.ln, a.lane_stride) : a.ln;
   if (tr) tr[0] = clock64();
   const uint32_t sbase = smem_u32(smem);
   const uint32_t bar_ld = sbase + B_BAR, bar_mma = bar_ld + 8;
@@ -629,21 +657,21 @@ __global__ void __launch_bounds__(NT, 1) tt_bwd_kernel(const TtBwdArgs a) {
     if (tid == 0) {
       const bool first = tile == tile0;
       mbar_expect_tx(bar_ld, ncopy * CS + (first ? (MODE == TT_PLAIN ? 1 : 2) * img_bytes : 0));
-      bulk_copy_chunked(sbase + (L.in == IN_M1P ? B_AB : B_AH), input_image(a.ln, L.in, tile), ncopy * CS, bar_ld);
+      bulk_copy_chunked(sbase + (L.in == IN_M1P ? B_AB : B_AH), input_image(ln, L.in, tile), ncopy * CS, bar_ld);
       if (first) {
-        bulk_copy_chunked(sbase + B_W0, a.ln.blob + L.w0b, img_bytes, bar_ld);
-        if (MODE != TT_PLAIN) bulk_copy_chunked(sbase + B_W1, a.ln.blob + L.w1b, img_bytes, bar_ld);
+        bulk_copy_chunked(sbase + B_W0, ln.blob + L.w0b, img_bytes, bar_ld);
+        if (MODE != TT_PLAIN) bulk_copy_chunked(sbase + B_W1, ln.blob + L.w1b, img_bytes, bar_ld);
       }
     }
     // ---- gradient operands (global reads only): G0 = d/d(pre-activation), G1 = d/d(variance) or d/d(perturbation);
     //      thread = row x chunk quarter
     const int row = (warp & 3) * 32 + lane, cq = warp >> 2;
     const RowInfo ri = row_info(ROW0 + row, tile, a.B);
-    const float* rb = a.ln.rbuf + (long long)tile * RBUF_PER_TILE + L.roff_per_tile;
+    const float* rb = ln.rbuf + (long long)tile * RBUF_PER_TILE + L.roff_per_tile;
     const float* sout = a.sgn_out[blockIdx.y];
     for (int c = cq; c < L.NP / 8; c += 4) {
       float d[8], d1[8];
-      output_grad<MODE>(a, L, tile, row, ri, c * 8, d);
+      output_grad<MODE>(ln, L, tile, row, ri, c * 8, d);
       if (MODE == TT_PLAIN && a.keep[blockIdx.y] < 1.0f) {  // dropout behind the ReLU: the stored activation a * m / keep gates, 1 / keep scales
         const float ik = 1.0f / a.keep[blockIdx.y];
 #pragma unroll
@@ -708,7 +736,7 @@ __global__ void __launch_bounds__(NT, 1) tt_bwd_kernel(const TtBwdArgs a) {
     ph ^= 1;
     if (tr && tile == tile0) tr[4] = clock64();
     if (has_dx) {  // ---- input gradient of this tile -> bf16 image (thread = row x column quarter)
-      unsigned char* gi = a.ln.g[L.gdst] + (long long)tile * L.KC * CS;
+      unsigned char* gi = member_ptr(a.ln.g[L.gdst], a.lane_stride) + (long long)tile * L.KC * CS;  // (ln.g[L.gdst]: a local-memory copy)
       const uint32_t la = tmem + ((uint32_t)((warp & 3) * 32) << 16);
       const float* sin_ = a.sgn_in[blockIdx.y];
       for (int g = cq; g < dxw / 8; g += 4) {
@@ -746,7 +774,7 @@ __global__ void __launch_bounds__(NT, 1) tt_bwd_kernel(const TtBwdArgs a) {
   if (tile0 < tile1) {
     const int ch = (warp & 3) * 32 + lane, cq = warp >> 2;
     const int CH = L.KC * 8;
-    float* part = a.ln.part + (long long)blockIdx.x * a.part_floats + L.poff;
+    float* part = ln.part + (long long)blockIdx.x * a.part_floats + L.poff;
     const uint32_t la = tmem + ((uint32_t)((warp & 3) * 32) << 16);
     const int ng = L.NP / 8;
     for (int it = cq; it < L.T * ng; it += 4) {
@@ -787,15 +815,16 @@ struct TtFcPackArgs {
   const float *mu, *second;
   long long w_off;
   unsigned char* blob;  // w0h | w0b | w1b | w1h, FC_WIMG bytes each
+  long long P, lane_stride;  // ensemble members (blockIdx.z): parameter / lane strides
 };
 __global__ void tt_pack_fc_kernel(const TtFcPackArgs a) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= 64 * 2400) return;
   const int n = i / 2400, kp = i - n * 2400, t = kp / 80, c = kp - t * 80;
   const long long wi = a.w_off + (long long)n * 2400 + c * 30 + t;
-  const float m = a.mu[wi], v = a.second[wi];
+  const float m = a.mu[wi + a.P * blockIdx.z], v = a.second[wi + a.P * blockIdx.z];
   const float s = a.mode == BRL_MODE_LRT ? v * v : a.mode == BRL_MODE_FLIPOUT ? v - m : 0.f;
-  const int o = (kp >> 3) * 1024 + n * 16 + (kp & 7) * 2;
+  const long long o = a.lane_stride * blockIdx.z + (kp >> 3) * 1024 + n * 16 + (kp & 7) * 2;
   *reinterpret_cast<__half*>(a.blob + o) = __float2half_rn(m);
   *reinterpret_cast<__nv_bfloat16*>(a.blob + FC_WIMG + o) = __float2bfloat16_rn(m);
   *reinterpret_cast<__nv_bfloat16*>(a.blob + 2 * FC_WIMG + o) = __float2bfloat16_rn(s);
@@ -808,6 +837,7 @@ struct TtFcFwdArgs {
   TtLane ln;
   int B, mode;
   float* part;  // [2][B][64] fp32, zeroed: mean-path and second-path sums (brl_gemm.cu split-K scratch layout)
+  long long lane_stride, part_stride;  // ensemble members (blockIdx.z): bytes between their lanes, floats between their `part`
   int* status;
 };
 __global__ void __launch_bounds__(256, 1) tt_fc_fwd_kernel(const TtFcFwdArgs a) {
@@ -815,6 +845,8 @@ __global__ void __launch_bounds__(256, 1) tt_fc_fwd_kernel(const TtFcFwdArgs a) 
   const int mt = blockIdx.x, ks = blockIdx.y, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const uint32_t sbase = smem_u32(smem), bar_ld = sbase + FF_BAR, bar_mma = bar_ld + 8;
   uint32_t* tslot = reinterpret_cast<uint32_t*>(smem + FF_BAR + 16);
+  const TtLane ln = member_lane(a.ln, a.lane_stride);
+  float* part = a.part + a.part_stride * blockIdx.z;
   if (tid == 0) {
     mbar_init(bar_ld, 1);
     mbar_init(bar_mma, 1);
@@ -829,10 +861,10 @@ __global__ void __launch_bounds__(256, 1) tt_fc_fwd_kernel(const TtFcFwdArgs a) 
     const long long ao = ((long long)mt * FC_KC + ks * FC_KCS) * FC_CHUNK;
     const bool dual = a.mode == BRL_MODE_LRT || a.mode == BRL_MODE_FLIPOUT;
     mbar_expect_tx(bar_ld, (dual ? 2 : 1) * (FC_KCS * FC_CHUNK + FC_KCS * 1024));
-    bulk_copy_chunked(sbase + FF_A, a.ln.fimg + ao, FC_KCS * FC_CHUNK, bar_ld);
-    bulk_copy_chunked(sbase + FF_W0, a.ln.fcblob + (long long)ks * FC_KCS * 1024, FC_KCS * 1024, bar_ld);
-    if (dual) bulk_copy_chunked(sbase + FF_A2, a.ln.f2img + ao, FC_KCS * FC_CHUNK, bar_ld);
-    if (dual) bulk_copy_chunked(sbase + FF_W1, a.ln.fcblob + (a.mode == BRL_MODE_LRT ? 2 : 3) * (long long)FC_WIMG + (long long)ks * FC_KCS * 1024, FC_KCS * 1024, bar_ld);
+    bulk_copy_chunked(sbase + FF_A, ln.fimg + ao, FC_KCS * FC_CHUNK, bar_ld);
+    bulk_copy_chunked(sbase + FF_W0, ln.fcblob + (long long)ks * FC_KCS * 1024, FC_KCS * 1024, bar_ld);
+    if (dual) bulk_copy_chunked(sbase + FF_A2, ln.f2img + ao, FC_KCS * FC_CHUNK, bar_ld);
+    if (dual) bulk_copy_chunked(sbase + FF_W1, ln.fcblob + (a.mode == BRL_MODE_LRT ? 2 : 3) * (long long)FC_WIMG + (long long)ks * FC_KCS * 1024, FC_KCS * 1024, bar_ld);
   }
   mbar_wait(bar_ld, 0, a.status, 44);
   if (warp == 0) {
@@ -861,7 +893,7 @@ __global__ void __launch_bounds__(256, 1) tt_fc_fwd_kernel(const TtFcFwdArgs a) 
     if (dual) tmem_ld16(la + 64 + half * 32 + g * 16, v1);
     tmem_ld_wait();
     if (m < a.B) {
-      float* p0 = a.part + (long long)m * 64 + half * 32 + g * 16;
+      float* p0 = part + (long long)m * 64 + half * 32 + g * 16;
 #pragma unroll
       for (int j = 0; j < 16; ++j) {
         atomicAdd(p0 + j, v0[j]);
@@ -899,12 +931,23 @@ struct TtFcBwdArgs {
   const float* sgn_in;       // Flipout [B, 2400]
   float *g0, *g1;
   long long w_off, b_off;
+  long long P, lane_stride;  // ensemble members (blockIdx.z): parameter / lane strides; dpre / dsec [members][B][64]
   int* status;
 };
+// the arguments as ensemble member blockIdx.z sees them
+__device__ __forceinline__ TtFcBwdArgs member_fc(TtFcBwdArgs a) {
+  a.ln = member_lane(a.ln, a.lane_stride);
+  a.dpre = member_ptr(a.dpre, 64ll * a.B);
+  a.dsec = member_ptr(a.dsec, 64ll * a.B);
+  a.g0 = member_ptr(a.g0, a.P);
+  a.g1 = member_ptr(a.g1, a.P);
+  return a;
+}
 // d/d(features)[m, k'] = dpre[m, :] * W0[:, k'] + {2 f, s_in}[m, k'] * (dsec[m, :] * W1[:, k'])  -> bf16 image for the level kernels
 template <int MODE>
-__global__ void __launch_bounds__(256, 1) tt_fc_dx_kernel(const TtFcBwdArgs a) {
+__global__ void __launch_bounds__(256, 1) tt_fc_dx_kernel(const TtFcBwdArgs a_) {
   extern __shared__ __align__(128) unsigned char smem[];
+  const TtFcBwdArgs a = MODE == TT_PLAIN ? member_fc(a_) : a_;
   const int mt = blockIdx.x, ns = blockIdx.y, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const uint32_t sbase = smem_u32(smem), bar_ld = sbase + FX_BAR, bar_mma = bar_ld + 8;
   uint32_t* tslot = reinterpret_cast<uint32_t*>(smem + FX_BAR + 16);
@@ -975,8 +1018,9 @@ constexpr int FW_A = 0, FW_A2 = 16 * FC_CHUNK, FW_G0 = 32 * FC_CHUNK, FW_G1 = 40
 constexpr int FW_SMEM = FW_BAR + 64;
 // weight gradient: D[k', n] = sum_m F[m, k'] * dpre[m, n] (and the second path), M = 128 features per CTA, K = all windows
 template <int MODE>
-__global__ void __launch_bounds__(256, 1) tt_fc_dw_kernel(const TtFcBwdArgs a) {
+__global__ void __launch_bounds__(256, 1) tt_fc_dw_kernel(const TtFcBwdArgs a_) {
   extern __shared__ __align__(128) unsigned char smem[];
+  const TtFcBwdArgs a = MODE == TT_PLAIN ? member_fc(a_) : a_;
   const int kt = blockIdx.x, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const uint32_t sbase = smem_u32(smem), bar_ld = sbase + FW_BAR, bar_mma = bar_ld + 8;
   uint32_t* tslot = reinterpret_cast<uint32_t*>(smem + FW_BAR + 16);
@@ -1106,9 +1150,26 @@ struct TtTailArgs {
   int loss_kind;               // 0: ELBO likelihood (second softplus, sums in acc); 1: F.gaussian_nll_loss (frequentist.py:39-48, means in acc)
   float keep_fc;               // keep probability of the dropout site behind the fc layer (1 = none)
   NoiseRef drop_fc;            // its masks: injected [B, HW] or Philox
+  long long P, part_stride;    // ensemble members (blockIdx.z): floats between their parameters / gradients and their `part`
 };
+// the arguments as ensemble member blockIdx.z sees them (y, out, dpre, dsec: [members][B][...]; acc: [members][2])
+template <int HW>
+__device__ __forceinline__ TtTailArgs member_tail(TtTailArgs a) {
+  a.part = member_ptr(a.part, a.part_stride);
+  a.fc_b0 = member_ptr(a.fc_b0, a.P); a.fc_b1 = member_ptr(a.fc_b1, a.P);
+  a.hw0 = member_ptr(a.hw0, a.P); a.hw1 = member_ptr(a.hw1, a.P);
+  a.hb0 = member_ptr(a.hb0, a.P); a.hb1 = member_ptr(a.hb1, a.P);
+  a.y = member_ptr(a.y, (long long)a.B);
+  a.acc = member_ptr(a.acc, 2ll);
+  a.out = member_ptr(a.out, 2ll * a.B);
+  a.dpre = member_ptr(a.dpre, (long long)HW * a.B); a.dsec = member_ptr(a.dsec, (long long)HW * a.B);
+  a.g0 = member_ptr(a.g0, a.P); a.g1 = member_ptr(a.g1, a.P);
+  a.drop_fc = member_noise(a.drop_fc, HW, a.B);
+  return a;
+}
 template <int MODE, int HW>
-__global__ void __launch_bounds__(256) tt_tail_kernel(const TtTailArgs a) {
+__global__ void __launch_bounds__(256) tt_tail_kernel(const TtTailArgs a_) {
+  const TtTailArgs a = MODE == TT_PLAIN ? member_tail<HW>(a_) : a_;
   __shared__ float sg[2][2][HW + 1];  // [path][output][hidden unit | bias] head weight-gradient partials of the CTA
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   for (int i = tid; i < 2 * 2 * (HW + 1); i += 256) (&sg[0][0][0])[i] = 0.f;
@@ -1298,6 +1359,7 @@ struct TtReduceArgs {
   int part_floats, mode;
   const float* part;
   float *g0, *g1;
+  long long P, lane_stride;  // ensemble members (blockIdx.z): parameter / lane strides
 };
 constexpr int RED_SPLIT = 8;  // group ranges per output: blockIdx.y; each thread keeps <= 2 x 8 independent loads in flight
 __global__ void tt_reduce_kernel(const TtReduceArgs a) {
@@ -1311,7 +1373,9 @@ __global__ void tt_reduce_kernel(const TtReduceArgs a) {
   const int per = (a.ngroups[li] + RED_SPLIT - 1) / RED_SPLIT;
   const int g_lo = blockIdx.y * per, g_hi = min(a.ngroups[li], g_lo + per);
   if (g_lo >= g_hi) return;
-  const float* p = a.part + l.poff;
+  const float* p = reinterpret_cast<const float*>(reinterpret_cast<const unsigned char*>(a.part) + a.lane_stride * blockIdx.z) + l.poff;
+  float* g0 = a.g0 + a.P * blockIdx.z;
+  float* g1 = member_ptr(a.g1, a.P);
   const bool dual = a.mode == BRL_MODE_LRT || a.mode == BRL_MODE_FLIPOUT;
   float s0 = 0.f, s1 = 0.f;
   if (j < nw) {
@@ -1324,8 +1388,8 @@ __global__ void tt_reduce_kernel(const TtReduceArgs a) {
     }
     const int nt_ = j / CH, n = nt_ / l.T, tap = nt_ - n * l.T;
     const long long wi = l.w_off + ((long long)n * l.cin + cr) * l.T + tap;
-    atomicAdd(a.g0 + wi, s0);
-    if (dual) atomicAdd(a.g1 + wi, s1);
+    atomicAdd(g0 + wi, s0);
+    if (dual) atomicAdd(g1 + wi, s1);
   } else {
     const int n = j - nw;
 #pragma unroll 8
@@ -1333,8 +1397,8 @@ __global__ void tt_reduce_kernel(const TtReduceArgs a) {
       s0 += p[(long long)gidx * a.part_floats + 2ll * nw + n];
       if (dual) s1 += p[(long long)gidx * a.part_floats + 2ll * nw + 64 + n];
     }
-    atomicAdd(a.g0 + l.b_off + n, s0);
-    if (dual) atomicAdd(a.g1 + l.b_off + n, a.mode == BRL_MODE_LRT ? s1 : s0);  // Flipout: the sampled bias (brl_api.cu: gb2)
+    atomicAdd(g0 + l.b_off + n, s0);
+    if (dual) atomicAdd(g1 + l.b_off + n, a.mode == BRL_MODE_LRT ? s1 : s0);  // Flipout: the sampled bias (brl_api.cu: gb2)
   }
 }
 
@@ -1432,23 +1496,26 @@ void tt_forward(const TtLane& ln, const TtStep& s, cudaStream_t st, const TtSide
   const Table& tb = table();
   cudaEventRecord(sd.fork, st);  // the parameters (and a Flipout weight draw) are complete on `st` here
   cudaStreamWaitEvent(sd.side, sd.fork, 0);
-  tt_packx_kernel<<<(unsigned)(((long long)nt * 3 * ROWS + 255) / 256), 256, 0, st>>>(s.x, ln.ximg, (int)s.B, nt);
+  const unsigned M = (unsigned)s.members;
+  tt_packx_kernel<<<dim3((unsigned)(((long long)nt * 3 * ROWS + 255) / 256), 1, M), 256, 0, st>>>(s.x, ln.ximg, (int)s.B, nt, s.lane_stride);
   TtPackArgs pa;
   for (int i = 0; i < TT_LAYERS; ++i) { pa.L[i] = layer_of(s, i); pa.start[i] = tb.pack_start[i]; }
   pa.start[TT_LAYERS] = tb.pack_start[TT_LAYERS];
   pa.mode = s.mode; pa.mu = s.mu; pa.second = s.mode == BRL_MODE_LRT ? s.sigma : s.mode == BRL_MODE_FLIPOUT ? s.wsamp : s.mu; pa.blob = ln.blob;
-  tt_pack_kernel<<<(tb.pack_start[TT_LAYERS] + TT_LAYERS * 64 + 255) / 256, 256, 0, sd.side>>>(pa);
+  pa.P = s.P; pa.lane_stride = s.lane_stride;
+  tt_pack_kernel<<<dim3((tb.pack_start[TT_LAYERS] + TT_LAYERS * 64 + 255) / 256, 1, M), 256, 0, sd.side>>>(pa);
   TtFcPackArgs fp;
   fp.mode = s.mode; fp.mu = s.mu; fp.second = pa.second; fp.w_off = s.w_off_fc; fp.blob = ln.fcblob;
-  tt_pack_fc_kernel<<<(64 * 2400 + 255) / 256, 256, 0, sd.side>>>(fp);
+  fp.P = s.P; fp.lane_stride = s.lane_stride;
+  tt_pack_fc_kernel<<<dim3((64 * 2400 + 255) / 256, 1, M), 256, 0, sd.side>>>(fp);
   cudaEventRecord(sd.join, sd.side);
   g_launch_count += 3;
   if (s.B % 128 != 0) {  // windows beyond B of the last 128-window M-tile are K rows of the fc weight-gradient GEMM: they must be zero
-    const size_t last = (size_t)(s.B / 128) * FC_MT_BYTES;
-    cudaMemsetAsync(ln.fbimg + last, 0, FC_MT_BYTES, st);
-    cudaMemsetAsync(ln.f2img + last, 0, FC_MT_BYTES, st);
-    cudaMemsetAsync(ln.f2bimg + last, 0, FC_MT_BYTES, st);
-    cudaMemsetAsync(ln.fimg + last, 0, FC_MT_BYTES, st);
+    const size_t last = (size_t)(s.B / 128) * FC_MT_BYTES, pitch = M > 1 ? (size_t)s.lane_stride : FC_MT_BYTES;  // every member's
+    cudaMemset2DAsync(ln.fbimg + last, pitch, 0, FC_MT_BYTES, M, st);
+    cudaMemset2DAsync(ln.f2img + last, pitch, 0, FC_MT_BYTES, M, st);
+    cudaMemset2DAsync(ln.f2bimg + last, pitch, 0, FC_MT_BYTES, M, st);
+    cudaMemset2DAsync(ln.fimg + last, pitch, 0, FC_MT_BYTES, M, st);
   }
   cudaStreamWaitEvent(st, sd.join, 0);  // weight images ready
   static const int levels[3][4] = {{0, 1, 2, 3}, {5, 7, 4, 9}, {6, 8, -1, -1}};
@@ -1456,7 +1523,7 @@ void tt_forward(const TtLane& ln, const TtStep& s, cudaStream_t st, const TtSide
     TtFwdArgs fa{};
     fa.ln = ln;
     if (s.mode != BRL_MODE_LRT) fa.ln.rbuf = nullptr;
-    fa.B = (int)s.B; fa.ntile = nt; fa.sgn_fc_in = s.sgn_fc_in; fa.status = tt_status_word();
+    fa.B = (int)s.B; fa.ntile = nt; fa.sgn_fc_in = s.sgn_fc_in; fa.lane_stride = s.lane_stride; fa.status = tt_status_word();
     fa.trace = g_tt_trace ? g_tt_trace + lv * 64 : nullptr;
     int nl = 0;
     for (int k = 0; k < 4; ++k) {
@@ -1474,18 +1541,19 @@ void tt_forward(const TtLane& ln, const TtStep& s, cudaStream_t st, const TtSide
     ++g_launch_count;
     if (s.mode == BRL_MODE_LRT) tt_fwd_kernel<BRL_MODE_LRT><<<dim3(nt, nl), NT, F_SMEM, st>>>(fa);
     else if (s.mode == BRL_MODE_FLIPOUT) tt_fwd_kernel<BRL_MODE_FLIPOUT><<<dim3(nt, nl), NT, F_SMEM, st>>>(fa);
-    else tt_fwd_kernel<TT_PLAIN><<<dim3(nt, nl), NT, F_SMEM, st>>>(fa);
+    else tt_fwd_kernel<TT_PLAIN><<<dim3(nt, nl, M), NT, F_SMEM, st>>>(fa);
   }
 }
 
 void tt_fc_forward(const TtLane& ln, const TtStep& s, float* part, cudaStream_t st) {
   tt_configure();
   const int nmt = (int)((s.B + 127) / 128);
-  cudaMemsetAsync(part, 0, sizeof(float) * 2 * (size_t)s.B * 64, st);
+  cudaMemsetAsync(part, 0, sizeof(float) * 2 * (size_t)s.B * 64 * s.members, st);  // [members][2][B][64]
   TtFcFwdArgs fa{};
   fa.ln = ln; fa.B = (int)s.B; fa.mode = s.mode; fa.part = part; fa.status = tt_status_word();
+  fa.lane_stride = s.lane_stride; fa.part_stride = 2 * s.B * 64;
   ++g_launch_count;
-  tt_fc_fwd_kernel<<<dim3(nmt, FC_KS), 256, FF_SMEM, st>>>(fa);
+  tt_fc_fwd_kernel<<<dim3(nmt, FC_KS, s.members), 256, FF_SMEM, st>>>(fa);
 }
 
 void tt_tail(const TtStep& s, const TtTail& t, cudaStream_t st) {
@@ -1501,7 +1569,8 @@ void tt_tail(const TtStep& s, const TtTail& t, cudaStream_t st) {
   a.sout_fc = t.sout_fc; a.sin_head = t.sin_head; a.sout_head = t.sout_head;
   a.y = t.y; a.gscale = t.gscale; a.acc = t.acc; a.out = t.out; a.dpre = t.dpre; a.dsec = t.dsec;
   a.g0 = s.g0; a.g1 = s.g1; a.hw_off = t.hw_off; a.hb_off = t.hb_off;
-  const int grid = (int)std::min<long long>((s.B + 7) / 8, 148);
+  a.P = s.P; a.part_stride = 2 * s.B * t.width;
+  const dim3 grid((unsigned)std::min<long long>((s.B + 7) / 8, 148), 1, (unsigned)s.members);
   ++g_launch_count;
   if (t.width == 320) {
     if (lrt) tt_tail_kernel<BRL_MODE_LRT, 320><<<grid, 256, 0, st>>>(a);
@@ -1523,6 +1592,7 @@ void tt_fc_backward(const TtLane& ln, const TtStep& s, const float* dpre, const 
   TtFcBwdArgs ba{};
   ba.ln = ln; ba.B = (int)s.B; ba.nmt = (int)((s.B + 127) / 128); ba.mode = s.mode; ba.dpre = dpre; ba.dsec = dsec;
   ba.sgn_in = s.sgn_fc_in; ba.g0 = s.g0; ba.g1 = s.g1; ba.w_off = s.w_off_fc; ba.b_off = s.b_off_fc; ba.status = tt_status_word();
+  ba.P = s.P; ba.lane_stride = s.lane_stride;
   g_launch_count += 2;
   // the weight gradient needs nothing downstream of it until the finalisation: it leaves the critical chain for the side stream
   // (joined at the end of tt_backward)
@@ -1532,8 +1602,8 @@ void tt_fc_backward(const TtLane& ln, const TtStep& s, const float* dpre, const 
     tt_fc_dx_kernel<BRL_MODE_LRT><<<dim3(ba.nmt, FC_NS), 256, FX_SMEM, st>>>(ba);
     tt_fc_dw_kernel<BRL_MODE_LRT><<<(FC_KC + 15) / 16, 256, FW_SMEM, sd.side>>>(ba);
   } else if (s.mode != BRL_MODE_FLIPOUT) {
-    tt_fc_dx_kernel<TT_PLAIN><<<dim3(ba.nmt, FC_NS), 256, FX_SMEM, st>>>(ba);
-    tt_fc_dw_kernel<TT_PLAIN><<<(FC_KC + 15) / 16, 256, FW_SMEM, sd.side>>>(ba);
+    tt_fc_dx_kernel<TT_PLAIN><<<dim3(ba.nmt, FC_NS, s.members), 256, FX_SMEM, st>>>(ba);
+    tt_fc_dw_kernel<TT_PLAIN><<<dim3((FC_KC + 15) / 16, 1, s.members), 256, FW_SMEM, sd.side>>>(ba);
   } else {
     tt_fc_dx_kernel<BRL_MODE_FLIPOUT><<<dim3(ba.nmt, FC_NS), 256, FX_SMEM, st>>>(ba);
     tt_fc_dw_kernel<BRL_MODE_FLIPOUT><<<(FC_KC + 15) / 16, 256, FW_SMEM, sd.side>>>(ba);
@@ -1553,7 +1623,7 @@ void tt_backward(const TtLane& ln, const TtStep& s, cudaStream_t st, const TtSid
     TtBwdArgs ba{};
     ba.ln = ln;
     ba.part_floats = tb.part_floats;
-    ba.B = (int)s.B; ba.ntile = nt; ba.g0 = s.g0; ba.g1 = s.g1; ba.status = tt_status_word();
+    ba.B = (int)s.B; ba.ntile = nt; ba.g0 = s.g0; ba.g1 = s.g1; ba.lane_stride = s.lane_stride; ba.status = tt_status_word();
     ba.trace = g_tt_trace ? g_tt_trace + (3 + lv) * 64 : nullptr;
     int nl = 0;
     for (int k = 0; k < 4; ++k) {
@@ -1566,14 +1636,14 @@ void tt_backward(const TtLane& ln, const TtStep& s, cudaStream_t st, const TtSid
       ++nl;
     }
     ba.nl = nl;
-    ba.tiles_per_cta = std::max(1, (nt * nl + 147) / 148);
+    ba.tiles_per_cta = std::max(1, (nt * nl * s.members + 147) / 148);  // about one wave of 148 CTAs over all members
     const int ngroups = (nt + ba.tiles_per_cta - 1) / ba.tiles_per_cta;
     for (int k = 0; k < 4; ++k)
       if (levels[lv][k] >= 0) ra.ngroups[levels[lv][k]] = ngroups;
     ++g_launch_count;
     if (s.mode == BRL_MODE_LRT) tt_bwd_kernel<BRL_MODE_LRT><<<dim3(ngroups, nl), NT, B_SMEM, st>>>(ba);
     else if (s.mode == BRL_MODE_FLIPOUT) tt_bwd_kernel<BRL_MODE_FLIPOUT><<<dim3(ngroups, nl), NT, B_SMEM, st>>>(ba);
-    else tt_bwd_kernel<TT_PLAIN><<<dim3(ngroups, nl), NT, B_SMEM, st>>>(ba);
+    else tt_bwd_kernel<TT_PLAIN><<<dim3(ngroups, nl, s.members), NT, B_SMEM, st>>>(ba);
   }
   int tot = 0;
   for (int i = 0; i < TT_LAYERS; ++i) {
@@ -1583,8 +1653,9 @@ void tt_backward(const TtLane& ln, const TtStep& s, cudaStream_t st, const TtSid
   }
   ra.start[TT_LAYERS] = tot;
   ra.part_floats = tb.part_floats; ra.mode = s.mode; ra.part = ln.part; ra.g0 = s.g0; ra.g1 = s.g1;
+  ra.P = s.P; ra.lane_stride = s.lane_stride;
   ++g_launch_count;
-  tt_reduce_kernel<<<dim3((tot + 255) / 256, RED_SPLIT), 256, 0, st>>>(ra);
+  tt_reduce_kernel<<<dim3((tot + 255) / 256, RED_SPLIT, s.members), 256, 0, st>>>(ra);
   cudaStreamWaitEvent(st, sd.join, 0);  // the fc weight gradient (tt_fc_backward) is part of what the caller finalises next
 }
 

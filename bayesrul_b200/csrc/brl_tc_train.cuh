@@ -29,7 +29,7 @@ struct TtLane {
   unsigned char* gfimg;  // bf16 gradient w.r.t. the features (written by the fc input-gradient kernel)
   unsigned char* fcblob; // fc weight images [300][64][8]: fp16 mu | bf16 mu | bf16 sigma^2 or (W - mu) | fp16 of the same
 };
-size_t tt_lane_bytes(long long B);
+size_t tt_lane_bytes(long long B);  // a multiple of 256: lanes carved back to back are tt_lane_bytes(B) apart
 void tt_carve(unsigned char* base, long long B, TtLane& ln);
 
 struct TtStep {
@@ -50,6 +50,12 @@ struct TtStep {
   float* g0;             // flat gradient accumulators [P] (brl_kernels.cuh: Finalize): mean path / variance or perturbation path
   float* g1;
   long long w_off[TT_LAYERS], b_off[TT_LAYERS];
+  // Inception, BRL_MODE_DET: `members` independent nets (a deep ensemble) in the same launches, member m on blockIdx.z.  Member m
+  // reads x + m B 540, mu + m P, its lane images at lane + m lane_stride bytes, and writes g0 + m P; its dropout streams are the
+  // injected masks + m B out_elems or Philox with MC-sample index sample0 + m.  The tail's y / out / acc / part / dpre follow.
+  int members = 1;
+  long long P = 0;            // floats between members' parameters / gradients
+  long long lane_stride = 0;  // bytes between members' TtLane images (tt_carve of M lanes back to back)
 };
 // forward of the ten conv layers: x -> feature images (+ the activation / eps images the backward pass re-reads); 6 launches
 // side stream + two events of the calling lane: independent kernels of a step (weight packing next to the window packing, the fc

@@ -352,6 +352,41 @@ class Engine:
                                          ws.numel(), self._stream()))
         return dict(scalars=scalars, grad=grad, out=out)
 
+    def hnn_step_ensemble(self, x, y, theta, p_dropout: float = 0.0, noise: Optional[Noise] = None, compute_grads: bool = True,
+                          out_grad: Optional[torch.Tensor] = None):
+        """hnn_step of the M members of a deep ensemble (models/deepens.py) in one call: x [M,B,30,18], y [M,B], theta [M,P].
+        Member m is hnn_step(x[m], y[m], theta[m], p_dropout, noise with sample0 + m); injected masks are [M,B,out_elems].
+        Returns dict(scalars [M,2] (device, float64: loss, mse), grad [M,P], out [M,B,2]).  torch.optim.Adam or clipped_adam
+        over the [M,P] parameter tensor are elementwise: M independent optimisers."""
+        x = _chk(x, self.device, "x")
+        if x.dim() != 4 or x.shape[2] != WIN_LENGTH or x.shape[3] != N_FEATURES:
+            raise RuntimeError(f"bayesrul_b200: x must be [M,B,{WIN_LENGTH},{N_FEATURES}], got {tuple(x.shape)}")
+        M, B = x.shape[0], x.shape[1]
+        if M == 0 or B == 0:
+            raise RuntimeError("bayesrul_b200: empty ensemble or batch")
+        y = _chk(y, self.device, "y")
+        if tuple(y.shape) != (M, B):
+            raise RuntimeError(f"bayesrul_b200: y must have shape {(M, B)}, got {tuple(y.shape)}")
+        theta = self._theta(theta, "theta", (M,))
+        scalars = torch.empty(M, 2, dtype=torch.float64, device=self.device)
+        out = torch.empty(M, B, 2, device=self.device)
+        grad = None
+        if compute_grads:  # out_grad: a caller-owned buffer of >= M P floats
+            if out_grad is not None:
+                grad = _chk(out_grad, self.device, "out_grad")
+                if grad.numel() < M * self.P:
+                    raise RuntimeError(f"bayesrul_b200: out_grad needs at least {M * self.P} floats")
+                grad = grad.view(-1)[: M * self.P].view(M, self.P)
+            else:
+                grad = torch.empty(M, self.P, device=self.device)
+        ws = self._ws_for(B, M, 3, "simt")
+        nz, keep = self._noise(noise)
+        _lib.check(self.lib.brl_hnn_step_ensemble(self.ctx, x.data_ptr(), y.data_ptr(), M, B, theta.data_ptr(), float(p_dropout),
+                                                  nz, int(compute_grads), scalars.data_ptr(),
+                                                  grad.data_ptr() if grad is not None else None, out.data_ptr(), ws.data_ptr(),
+                                                  ws.numel(), self._stream()))
+        return dict(scalars=scalars, grad=grad, out=out)
+
     # -- A14 / A15 / N1 ------------------------------------------------------------------------------------
     def mixture_moments(self, mu_m: torch.Tensor, sigma_m: torch.Tensor):
         mu_m, sigma_m = _chk(mu_m, self.device, "mu_m"), _chk(sigma_m, self.device, "sigma_m")

@@ -113,7 +113,8 @@ int brl_destroy(brl_ctx* ctx);
 /* bytes of scratch needed by the calls below for B windows x S concurrently-resident samples;
  * train == 1 adds the saved activations / gradient buffers of brl_elbo_step / brl_hnn_step (with S >= 2: a second set, so
  * that brl_elbo_step runs two particles side by side on two stream lanes),
- * train == 2 the sign tensors brl_forward generates in BRL_MODE_FLIPOUT when none are injected */
+ * train == 2 the sign tensors brl_forward generates in BRL_MODE_FLIPOUT when none are injected,
+ * train == 3 the buffers of brl_hnn_step_ensemble over S = M members (all of them in one chain of launches where it can) */
 /* 1 when `engine` can run this net's forward on this build, else 0 */
 int brl_engine_available(const brl_ctx* ctx, int engine);
 int64_t brl_workspace_bytes(const brl_ctx* ctx, int64_t B, int64_t S, int train, int engine);
@@ -209,6 +210,19 @@ int brl_hnn_step(brl_ctx* ctx, const float* x, const float* y, int64_t B, const 
                  float p_dropout, const brl_noise* noise, int compute_grads, double* scalars,
                  float* grad_theta, float* out /*[B,2]*/, void* workspace, size_t workspace_bytes,
                  void* stream);
+
+/* ---- M independent heteroscedastic NNs (the members of a deep ensemble, models/deepens.py) in ONE step.
+ *      Member m is brl_hnn_step(x + m*B*540, y + m*B, B, theta + m*P, p_dropout, noise with sample0 + m, ...):
+ *      same loss (F.gaussian_nll_loss over the member's B windows), same dropout keys with MC-sample index sample0 + m,
+ *      injected drop_mask[l] laid out [M,B,out_elems(l)].  Graph-replayed under the same conditions as brl_hnn_step.
+ *      Where brl_hnn_step runs the fused Inception kernels (BRL_GEMM_TC_FUSED, B <= 4736) and the workspace holds
+ *      brl_workspace_bytes(B, M, 3), the M members share every launch (member = blockIdx.z); otherwise they run one after
+ *      another on the single-member step, with the same results.  A workspace below the single-member size returns
+ *      BRL_ERR_WORKSPACE. */
+int brl_hnn_step_ensemble(brl_ctx* ctx, const float* x /*[M,B,30,18]*/, const float* y /*[M,B]*/, int64_t M, int64_t B,
+                          const float* theta /*[M,P]*/, float p_dropout, const brl_noise* noise, int compute_grads,
+                          double* scalars /*[M,2] = {loss, mse}*/, float* grad_theta /*[M,P]*/, float* out /*[M,B,2]*/,
+                          void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- deep-ensemble mixture moments (models/deepens.py:21-24), [M,n] -> [n] ------------- */
 int brl_mixture_moments(const float* mu_m, const float* sigma_m, int64_t M, int64_t n, float* mu,
