@@ -70,6 +70,8 @@ SIGNATURES = {
     "brl_aggregate_predictions": (_i, [_vp, _i64, _i64, _vp, _vp]),
     "brl_elbo_step": (_i, [_vp, _vp, _vp, _i64, _vp, _vp, _i, _i, _i, _f, _f, _i64, _np, _i, _vp, _vp, _vp, _vp, _vp,
                            _vp, _sz, _vp]),
+    "brl_elbo_step_ensemble": (_i, [_vp, _vp, _vp, _i64, _i64, _vp, _vp, _i, _i, _i, _f, _f, _i64, _np, _i, _vp, _vp, _vp, _vp,
+                                    _vp, _vp, _sz, _vp]),
     "brl_hnn_step": (_i, [_vp, _vp, _vp, _i64, _vp, _f, _np, _i, _vp, _vp, _vp, _vp, _sz, _vp]),
     "brl_hnn_step_ensemble": (_i, [_vp, _vp, _vp, _i64, _i64, _vp, _f, _np, _i, _vp, _vp, _vp, _vp, _sz, _vp]),
     "brl_mixture_moments": (_i, [_vp, _vp, _i64, _i64, _vp, _vp, _vp]),

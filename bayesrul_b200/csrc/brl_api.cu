@@ -137,7 +137,8 @@ struct ActBufs {
   // level-fused tcgen05 training kernels (Inception conv stack, brl_tc_train.cu): images of one particle lane
   TtLane tt{};
   bool has_tt = false;
-  int tt_members = 1;         // brl_hnn_step_ensemble: members whose lanes sit back to back from `tt`, tt_stride bytes apart
+  int tt_members = 1;         // brl_hnn_step_ensemble / brl_elbo_step_ensemble: members whose lanes sit back to back from `tt`,
+                              // tt_stride bytes apart
   long long tt_stride = 0;
   // level-fused tcgen05 training kernels of the Linear net (brl_tc_train_linear.cuh): carved last, only where they fit
   TlLane tl{};
@@ -206,10 +207,11 @@ static void carve_tl(const NetSpec& n, Carve& c, long long B, ActBufs& ab) {
   (lin ? ab.has_tl : ab.has_tc3) = base != nullptr;
 }
 
-// brl_hnn_step_ensemble on the fused Inception kernels: the other M - 1 members' lanes right behind lane 0 (carve_train carves it
-// last), the members' fc-layer sums and gradients, and graph staging for M members.  A workspace without room for all of it keeps
-// the layout of the single-member step, whose body then runs once per member.
-static void carve_members(const NetSpec& n, Carve& c, long long B, long long M, ActBufs& ab) {
+// brl_hnn_step_ensemble / brl_elbo_step_ensemble (elbo) on the fused Inception kernels: the other M - 1 members' lanes right
+// behind lane 0 (carve_train carves it last), the members' fc-layer sums and gradients, and graph staging for M members; the ELBO
+// step adds its per-member weight draws, deltas, radial norms, native sign tensors and accumulators.  A workspace without room
+// for all of it keeps the layout of the single-member step, whose body then runs once per member.
+static void carve_members(const NetSpec& n, Carve& c, long long B, long long M, bool elbo, ActBufs& ab) {
   if (M < 2 || n.id != BRL_NET_INCEPTION || 2 * B * 64 > SPLITK_SCRATCH_FLOATS) return;
   Carve t = c;
   t.take<unsigned char>((M - 1) * (long long)tt_lane_bytes(B));  // tt_lane_bytes is a multiple of the carve alignment
@@ -217,17 +219,42 @@ static void carve_members(const NetSpec& n, Carve& c, long long B, long long M, 
   float* dpre = t.take<float>(M * B * 64);
   float* sx = t.take<float>(M * B * 540);
   float* sy = t.take<float>(M * B);
-  float* sout = t.take<float>(M * B * 2);
+  float* sout = t.take<float>((elbo ? GRAPH_MAX_PARTICLES : 1) * M * B * 2);
   float* sg = t.take<float>(M * n.P);
-  double* ss = t.take<double>(2 * M);
+  double* ss = t.take<double>((elbo ? 4 : 2) * M);
+  ActBufs e;  // the ELBO step's buffers, [M][...]
+  if (elbo) {
+    e.dsec.assign(1, t.take<float>(M * B * 64));
+    e.g0 = t.take<float>(M * n.P);
+    e.g1 = t.take<float>(M * n.P);
+    e.wsamp = t.take<float>(M * n.P);
+    e.delta = t.take<float>(M * n.P);
+    e.norms = t.take<float>(M * 2 * (long long)n.layers.size());
+    e.sgn_in.resize(n.layers.size());
+    e.sgn_out.resize(n.layers.size());
+    for (size_t l = 0; l < n.layers.size(); ++l) {
+      e.sgn_in[l] = t.take<float>(M * B * n.layers[l].cin);
+      e.sgn_out[l] = t.take<float>(M * B * n.layers[l].cout);
+    }
+    e.acc = t.take<double>(4 * M);
+    e.st_gsig = t.take<float>(M * n.P);
+    e.st_glog = t.take<float>(M * n.P);
+  }
   if (c.base && (!t.ok || !ab.has_tt)) return;
   c = t;
   if (!c.base) return;
   ab.tt_members = (int)M;
   ab.tt_stride = (long long)tt_lane_bytes(B);
-  ab.part[0] = part;  // hnn_body's fc split-K sums, [M][2][B][64]
+  ab.part[0] = part;  // the fc split-K sums, [M][2][B][64]
   ab.dpre[n.ops.size() - 2] = dpre;
   ab.st_x = sx; ab.st_y = sy; ab.st_out = sout; ab.st_gmu = sg; ab.st_scal = ss;
+  if (elbo) {
+    ab.dsec[n.ops.size() - 2] = e.dsec[0];
+    ab.g0 = e.g0; ab.g1 = e.g1; ab.wsamp = e.wsamp; ab.delta = e.delta; ab.norms = e.norms;
+    ab.sgn_in = e.sgn_in; ab.sgn_out = e.sgn_out;
+    ab.acc = e.acc;
+    ab.st_gsig = e.st_gsig; ab.st_glog = e.st_glog;
+  }
 }
 
 // device {seed, sample0, window0} of the step being captured (nullptr outside a capture): every Philox stream built by
@@ -790,11 +817,11 @@ int64_t brl_workspace_bytes(const brl_ctx* ctx, int64_t B, int64_t S, int train,
   const NetSpec& n = *ctx->net;
   Carve c(nullptr, 0);
   ActBufs ab;
-  if (train == 3) {  // brl_hnn_step_ensemble over S members: the layout of hnn_step
+  if (train == 3 || train == 4) {  // brl_hnn_step_ensemble / brl_elbo_step_ensemble over S members: the layout of their steps
     carve_forward(n, c, B, 1, ab);
     carve_train(n, c, B, ab);
     carve_tl(n, c, B, ab);
-    carve_members(n, c, B, S, ab);
+    carve_members(n, c, B, S, train == 4, ab);
     return (int64_t)c.used + 4096;
   }
   c.take<float>(4 * B);          // moment state
@@ -1131,11 +1158,31 @@ int brl_aggregate_predictions(const float* out, int64_t S, int64_t B, float* agg
   return BRL_OK;
 }
 
-// the launches of one ELBO step (every pointer final); captured as is by the graph path of brl_elbo_step.
+// M members of an ELBO step in ONE chain of launches: the level-fused Inception kernels with the workspace's lanes for M members
+// (at M = 1: where brl_elbo_step runs the fused Inception kernels)
+static bool elbo_batched(const brl_ctx* ctx, const ActBufs& ab, long long M, long long B, int mode) {
+  return ctx->gemm_backend == BRL_GEMM_TC_FUSED && ctx->net->id == BRL_NET_INCEPTION && ab.has_tt && ab.tt_members >= M &&
+         (mode == BRL_MODE_LRT || mode == BRL_MODE_FLIPOUT || mode == BRL_MODE_WS) &&
+         2 * B * 64 <= SPLITK_SCRATCH_FLOATS;  // fc partial sums live in the split-K scratch (B <= 4736), else per-layer
+}
+// injected Flipout signs of the member-batched kernels: member m's tensors start `particles` rows [B, C] after member m - 1's,
+// the signs generated in the workspace one row after; with several particles the kernels take one stride for all layers
+static bool signs_one_stride(const NetSpec& n, const brl_noise* nz, int particles) {
+  if (!nz || particles == 1) return true;
+  int injected = 0;
+  for (size_t l = 0; l < n.layers.size(); ++l) injected += (nz->flip_in[l] != nullptr) + (nz->flip_out[l] != nullptr);
+  return injected == 0 || injected == 2 * (int)n.layers.size();
+}
+static bool signs_injected(const brl_noise* nz) { return nz && nz->flip_in[0]; }
+
+// the launches of one ELBO step of M members (every pointer final; M > 1 only where elbo_batched holds); captured as is by the
+// graph path of elbo_step.
 // lanes[0] always exists and owns the shared accumulators; with a second buffer set (lanes[1]) two particles run side by
 // side: lane 0 on `st`, lane 1 on the context's own stream, forked / joined with events.  The gradient finalisation of the
-// particles (first one writes, the others accumulate) stays in particle order on `st`.
-static int elbo_body(brl_ctx* ctx, const ActBufs* const* lanes, int n_lanes, const float* x, const float* y, int64_t B,
+// particles (first one writes, the others accumulate) stays in particle order on `st`.  M > 1 members share every launch of one
+// lane (member m on blockIdx.z of the fused kernels, on blockIdx.y of the sampler / sign / finalisation kernels), particle after
+// particle; their accumulators are [M][4].
+static int elbo_body(brl_ctx* ctx, const ActBufs* const* lanes, int n_lanes, const float* x, const float* y, int64_t M, int64_t B,
                      const float* mu, const float* sigma, int mode, int guide, int particles, float prior_loc, float prior_scale,
                      int64_t dataset_size, const brl_noise* noise, int compute_grads, double* scalars, float* grad_mu,
                      float* grad_sigma, float* grad_log_sigma, float* out, cudaStream_t st) {
@@ -1143,9 +1190,9 @@ static int elbo_body(brl_ctx* ctx, const ActBufs* const* lanes, int n_lanes, con
   const ActBufs& ab0 = *lanes[0];
   const double cc = 1.0 / ((double)dataset_size * 30.0 * 18.0);
   const double c_nll = cc * (double)dataset_size / (double)B;
-  BRL_CUDA(cudaMemsetAsync(ab0.acc, 0, 8 * sizeof(double), st));
+  BRL_CUDA(cudaMemsetAsync(ab0.acc, 0, std::max<int64_t>(8, 4 * M) * sizeof(double), st));
   const int nsites = 2 * (int)n.layers.size();
-  if (!ctx->multi_stream) n_lanes = 1;
+  if (!ctx->multi_stream || M > 1) n_lanes = 1;
   for (int p0 = 0; p0 < particles; p0 += n_lanes) {
     const int nl = std::min(n_lanes, particles - p0);
     if (nl > 1) {
@@ -1160,9 +1207,10 @@ static int elbo_body(brl_ctx* ctx, const ActBufs* const* lanes, int n_lanes, con
       const bool need_w = mode != BRL_MODE_LRT;
       if (need_w) {
         NoiseRef eps = nref(&nz, nz.weight_eps, KIND_WEIGHT_EPS, 0);
-        if (guide == BRL_GUIDE_NORMAL) launch_sample_normal(mu, sigma, n.P, 1, eps, ab.wsamp, ab.delta, ls);
-        else launch_sample_radial(mu, sigma, n.P, 1, ctx->site_off_dev, nsites, ctx->max_site, eps,
-                                  nref(&nz, nz.radial_r, KIND_RADIAL_R, 0), ab.norms, ab.wsamp, ab.delta, ls);
+        // one draw per member: member m's posterior, MC-sample index sample0 + m particles + pt
+        if (guide == BRL_GUIDE_NORMAL) launch_sample_normal(mu, sigma, n.P, M, eps, ab.wsamp, ab.delta, ls, n.P, particles);
+        else launch_sample_radial(mu, sigma, n.P, M, ctx->site_off_dev, nsites, ctx->max_site, eps,
+                                  nref(&nz, nz.radial_r, KIND_RADIAL_R, 0), ab.norms, ab.wsamp, ab.delta, ls, n.P, particles);
       }
       std::vector<const float*> sin_(n.layers.size(), nullptr), sout_(n.layers.size(), nullptr);
       if (mode == BRL_MODE_FLIPOUT) {  // native sign tensors of all layers: one launch per particle
@@ -1180,15 +1228,13 @@ static int elbo_body(brl_ctx* ctx, const ActBufs* const* lanes, int n_lanes, con
           if (nz.flip_out[ly]) sout_[ly] = nz.flip_out[ly];
           else { add(ab.sgn_out[ly], n.layers[ly].cout, KIND_FLIP_OUT, (unsigned)ly); sout_[ly] = ab.sgn_out[ly]; }
         }
-        if (jobs.n) launch_gen_signs_multi(jobs, B, nref(&nz, nullptr, 0, 0), ls);
+        if (jobs.n) launch_gen_signs_multi(jobs, B, nref(&nz, nullptr, 0, 0), ls, (int)M, particles);
       }
       float* outp = out + (long long)pt * B * 2;
       const brl_ctx::Lane& ln = ctx->lanes[l];
       // level-fused tcgen05 kernels (BRL_GEMM_TC_FUSED): ten conv layers + the fc layer on the tensor pipe, the rest of the net
       // (fc epilogue, head, likelihood, their backward) in one tail kernel
-      const bool use_tt = ctx->gemm_backend == BRL_GEMM_TC_FUSED && n.id == BRL_NET_INCEPTION && ab.has_tt &&
-                          (mode == BRL_MODE_LRT || mode == BRL_MODE_FLIPOUT || mode == BRL_MODE_WS) &&
-                          2 * B * 64 <= SPLITK_SCRATCH_FLOATS;  // fc partial sums live in the split-K scratch (B <= 4736), else per-layer
+      const bool use_tt = elbo_batched(ctx, ab, M, B, mode);
       // the Linear net's four hidden layers on the tensor pipe, the head in the same tail kernel (width 32)
       const bool use_tl = ctx->gemm_backend == BRL_GEMM_TC_FUSED && n.id == BRL_NET_LINEAR && ab.has_tl &&
                           (mode == BRL_MODE_LRT || mode == BRL_MODE_FLIPOUT || mode == BRL_MODE_WS);
@@ -1205,8 +1251,8 @@ static int elbo_body(brl_ctx* ctx, const ActBufs* const* lanes, int n_lanes, con
           int rc = zero_grads(n, ab, B, zs);
           if (rc) return rc;
         }
-        BRL_CUDA(cudaMemsetAsync(ab.g0, 0, sizeof(float) * n.P, zs));
-        BRL_CUDA(cudaMemsetAsync(ab.g1, 0, sizeof(float) * n.P, zs));
+        BRL_CUDA(cudaMemsetAsync(ab.g0, 0, sizeof(float) * M * n.P, zs));
+        BRL_CUDA(cudaMemsetAsync(ab.g1, 0, sizeof(float) * M * n.P, zs));
         if (zs != ls) BRL_CUDA(cudaEventRecord(ln.ev_zero, zs));
       }
       FwdArgs fa{x, B, 1, mode, mu, sigma, ab.wsamp, 0.f, &nz, sin_.data(), sout_.data(), outp, compute_grads != 0};
@@ -1224,6 +1270,8 @@ static int elbo_body(brl_ctx* ctx, const ActBufs* const* lanes, int n_lanes, con
         ts.sgn_fc_in = sin_[fc_layer];
         ts.w_off_fc = n.layers[fc_layer].w_off; ts.b_off_fc = n.layers[fc_layer].b_off;
         ts.g0 = ab.g0; ts.g1 = ab.g1;
+        ts.members = (int)M; ts.P = n.P; ts.lane_stride = ab.tt_stride;
+        ts.noise_stride = particles; ts.sign_stride = signs_injected(noise) ? particles : 1;
         const TtSide tsd{ln.side[0], ln.ev_fork, ln.ev_join[0]};
         tt_forward(ab.tt, ts, ls, tsd);
         tt_fc_forward(ab.tt, ts, ab.part[0], ls);
@@ -1263,6 +1311,7 @@ static int elbo_body(brl_ctx* ctx, const ActBufs* const* lanes, int n_lanes, con
         tl.eps_head = nref(&nz, nz.lrt_eps[hd_layer], KIND_LRT_EPS, (unsigned)hd_layer);
         tl.sout_fc = sout_[fc_layer]; tl.sin_head = sin_[hd_layer]; tl.sout_head = sout_[hd_layer];
         tl.hw_off = n.layers[hd_layer].w_off; tl.hb_off = n.layers[hd_layer].b_off;
+        tl.acc_stride = 4;
         tt_tail(ts, tl, ls);
       } else if (use_tl) {
         TtTail tl{};
@@ -1315,10 +1364,11 @@ static int elbo_body(brl_ctx* ctx, const ActBufs* const* lanes, int n_lanes, con
       f.grad_mu = compute_grads ? grad_mu : nullptr; f.grad_sigma = compute_grads ? grad_sigma : nullptr;
       f.grad_log_sigma = (compute_grads && pt == particles - 1) ? grad_log_sigma : nullptr;  // the last particle completes the sum
       f.kl_acc = ab0.acc + 2;
+      f.members = (int)M; f.kl_stride = 4;
       launch_finalize(f, st);
     }
   }
-  launch_post_scalars(scalars, ab0.acc, c_nll, cc, particles, B, st);
+  launch_post_scalars(scalars, ab0.acc, c_nll, cc, particles, B, st, (int)M);
   BRL_CUDA(cudaGetLastError());
   return BRL_OK;
 }
@@ -1337,38 +1387,52 @@ int brl_set_step_graph(brl_ctx* ctx, int enable) {
   return BRL_OK;
 }
 
-int brl_elbo_step(brl_ctx* ctx, const float* x, const float* y, int64_t B, const float* mu, const float* sigma, int mode,
-                  int guide, int particles, float prior_loc, float prior_scale, int64_t dataset_size,
-                  const brl_noise* noise, int compute_grads, double* scalars, float* grad_mu, float* grad_sigma,
-                  float* grad_log_sigma, float* out, void* workspace, size_t workspace_bytes, void* stream) {
-  BRL_REQUIRE(ctx && x && y && mu && sigma && scalars && out && workspace, "brl_elbo_step: NULL argument");
-  DeviceGuard dg(ctx->device);
-  BRL_REQUIRE(B > 0 && particles > 0 && dataset_size > 0 && prior_scale > 0.f, "brl_elbo_step: bad sizes");
-  BRL_REQUIRE(guide == BRL_GUIDE_NORMAL || guide == BRL_GUIDE_RADIAL, "Guide unknown. Choose from 'normal', 'radial'.");
-  BRL_REQUIRE(mode == BRL_MODE_WS || mode == BRL_MODE_LRT || mode == BRL_MODE_FLIPOUT, "brl_elbo_step: mode must be WS, LRT or FLIPOUT");
-  BRL_REQUIRE(!compute_grads || (grad_mu && grad_sigma), "brl_elbo_step: gradient buffers are NULL");
-  if (guide == BRL_GUIDE_RADIAL) mode = BRL_MODE_WS;  // bayesian.py:81-83: radial forces nullcontext
-  cudaStream_t st = (cudaStream_t)stream;
+// brl_elbo_step (M = 1) and brl_elbo_step_ensemble: M members in one chain of launches where elbo_batched holds, else one member
+// after another on the single-member step
+static int elbo_step(brl_ctx* ctx, const float* x, const float* y, int64_t M, int64_t B, const float* mu, const float* sigma,
+                     int mode, int guide, int particles, float prior_loc, float prior_scale, int64_t dataset_size,
+                     const brl_noise* noise, int compute_grads, double* scalars, float* grad_mu, float* grad_sigma,
+                     float* grad_log_sigma, float* out, void* workspace, size_t workspace_bytes, cudaStream_t st) {
   const NetSpec& n = *ctx->net;
   Carve c(workspace, workspace_bytes);
   ActBufs ab;
   carve_forward(n, c, B, 1, ab);
   carve_train(n, c, B, ab);
-  if (!c.ok) return fail(BRL_ERR_WORKSPACE, "brl_elbo_step: workspace too small; need " +
-                                                std::to_string(brl_workspace_bytes(ctx, B, 1, 1, 0)) + " bytes");
-  // a second buffer set, if the workspace has room for it (brl_workspace_bytes(B, S >= 2, train = 1)): two particles at a time
+  if (!c.ok) return fail(BRL_ERR_WORKSPACE, std::string(M == 1 ? "brl_elbo_step" : "brl_elbo_step_ensemble") +
+                                                ": workspace too small; need " + std::to_string(brl_workspace_bytes(ctx, B, 1, 1, 0)) + " bytes");
   ActBufs ab1;
   int n_lanes = 1;
-  if (particles > 1) {
-    carve_forward(n, c, B, 1, ab1);
-    carve_train(n, c, B, ab1);
-    if (c.ok) n_lanes = 2;
-  }
-  carve_tl(n, c, B, ab);
-  if (n_lanes == 2) {
-    carve_tl(n, c, B, ab1);
-    if (!ab1.has_tl) ab.has_tl = false;  // both particle lanes run the same back-end
-    if (!ab1.has_tc3) ab.has_tc3 = false;
+  if (M > 1) {  // the members' lanes right behind lane 0 (brl_workspace_bytes(B, M, 4)), or one member after another
+    carve_tl(n, c, B, ab);
+    carve_members(n, c, B, M, true, ab);
+    if (!elbo_batched(ctx, ab, M, B, mode) || !signs_one_stride(n, noise, particles)) {
+      brl_noise base;
+      memset(&base, 0, sizeof(base));
+      if (noise) base = *noise;
+      for (int64_t m = 0; m < M; ++m) {
+        const brl_noise nm = noise_at_sample(n, &base, m * particles, B);  // MC-sample index sample0 + m particles, member m's rows
+        const int rc = elbo_step(ctx, x + m * B * 540, y + m * B, 1, B, mu + m * n.P, sigma + m * n.P, mode, guide, particles,
+                                 prior_loc, prior_scale, dataset_size, &nm, compute_grads, scalars + 4 * m,
+                                 compute_grads ? grad_mu + m * n.P : nullptr, compute_grads ? grad_sigma + m * n.P : nullptr,
+                                 (compute_grads && grad_log_sigma) ? grad_log_sigma + m * n.P : nullptr,
+                                 out + m * particles * B * 2, workspace, workspace_bytes, st);
+        if (rc != BRL_OK) return rc;
+      }
+      return BRL_OK;
+    }
+  } else {
+    // a second buffer set, if the workspace has room for it (brl_workspace_bytes(B, S >= 2, train = 1)): two particles at a time
+    if (particles > 1) {
+      carve_forward(n, c, B, 1, ab1);
+      carve_train(n, c, B, ab1);
+      if (c.ok) n_lanes = 2;
+    }
+    carve_tl(n, c, B, ab);
+    if (n_lanes == 2) {
+      carve_tl(n, c, B, ab1);
+      if (!ab1.has_tl) ab.has_tl = false;  // both particle lanes run the same back-end
+      if (!ab1.has_tc3) ab.has_tc3 = false;
+    }
   }
   const ActBufs* lanes[2] = {&ab, &ab1};
   // ---- graph replay (native Philox noise): eager on first sight of a configuration, captured on the second, replayed after
@@ -1384,6 +1448,7 @@ int brl_elbo_step(brl_ctx* ctx, const float* x, const float* y, int64_t B, const
     memset(&key, 0, sizeof(key));
     key.B = B; key.dataset_size = dataset_size; key.mode = mode; key.guide = guide; key.particles = particles;
     key.compute_grads = compute_grads; key.backend = ctx->gemm_backend; key.has_log_sigma = grad_log_sigma != nullptr;
+    key.members = (int)M;
     key.prior_loc = prior_loc; key.prior_scale = prior_scale; key.mu = mu; key.sigma = sigma; key.ws = workspace;
     key.ws_bytes = workspace_bytes;
     for (auto it = ctx->graphs.begin(); it != ctx->graphs.end(); ++it)
@@ -1406,7 +1471,7 @@ int brl_elbo_step(brl_ctx* ctx, const float* x, const float* y, int64_t B, const
         const long long l0 = launch_count();
         brl_noise zero;
         memset(&zero, 0, sizeof(zero));
-        rc = elbo_body(ctx, lanes, n_lanes, ab.st_x, ab.st_y, B, mu, sigma, mode, guide, particles, prior_loc, prior_scale, dataset_size, &zero,
+        rc = elbo_body(ctx, lanes, n_lanes, ab.st_x, ab.st_y, M, B, mu, sigma, mode, guide, particles, prior_loc, prior_scale, dataset_size, &zero,
                        compute_grads, ab.st_scal, compute_grads ? ab.st_gmu : nullptr, compute_grads ? ab.st_gsig : nullptr,
                        (compute_grads && grad_log_sigma) ? ab.st_glog : nullptr, ab.st_out, ctx->cap);
         g_dyn = nullptr;
@@ -1427,8 +1492,8 @@ int brl_elbo_step(brl_ctx* ctx, const float* x, const float* y, int64_t B, const
   if (sg && sg->exec) {
     count_launch(sg->launches);
     CopyJobs in{};  // x, y and the Philox key of this step -> staging
-    in.dst[0] = ab.st_x; in.src[0] = x; in.n[0] = B * 540;
-    in.dst[1] = ab.st_y; in.src[1] = y; in.n[1] = B;
+    in.dst[0] = ab.st_x; in.src[0] = x; in.n[0] = M * B * 540;
+    in.dst[1] = ab.st_y; in.src[1] = y; in.n[1] = M * B;
     in.njobs = 2;
     in.dyn = ab.dyn;
     in.seed = noise ? noise->seed : 0ull;
@@ -1437,21 +1502,53 @@ int brl_elbo_step(brl_ctx* ctx, const float* x, const float* y, int64_t B, const
     launch_copy_jobs(in, st);
     BRL_CUDA(cudaGraphLaunch(sg->exec, st));
     CopyJobs o{};  // staging -> the caller's result tensors (the four doubles travel as eight floats)
-    o.dst[0] = reinterpret_cast<float*>(scalars); o.src[0] = reinterpret_cast<const float*>(ab.st_scal); o.n[0] = 8;
-    o.dst[1] = out; o.src[1] = ab.st_out; o.n[1] = (long long)particles * B * 2;
+    o.dst[0] = reinterpret_cast<float*>(scalars); o.src[0] = reinterpret_cast<const float*>(ab.st_scal); o.n[0] = 8 * M;
+    o.dst[1] = out; o.src[1] = ab.st_out; o.n[1] = M * particles * B * 2;
     o.njobs = 2;
     if (compute_grads) {
-      o.dst[2] = grad_mu; o.src[2] = ab.st_gmu; o.n[2] = n.P;
-      o.dst[3] = grad_sigma; o.src[3] = ab.st_gsig; o.n[3] = n.P;
+      o.dst[2] = grad_mu; o.src[2] = ab.st_gmu; o.n[2] = M * n.P;
+      o.dst[3] = grad_sigma; o.src[3] = ab.st_gsig; o.n[3] = M * n.P;
       o.njobs = 4;
-      if (grad_log_sigma) { o.dst[4] = grad_log_sigma; o.src[4] = ab.st_glog; o.n[4] = n.P; o.njobs = 5; }
+      if (grad_log_sigma) { o.dst[4] = grad_log_sigma; o.src[4] = ab.st_glog; o.n[4] = M * n.P; o.njobs = 5; }
     }
     launch_copy_jobs(o, st);
     BRL_CUDA(cudaGetLastError());
     return BRL_OK;
   }
-  return elbo_body(ctx, lanes, n_lanes, x, y, B, mu, sigma, mode, guide, particles, prior_loc, prior_scale, dataset_size, noise, compute_grads,
-                   scalars, grad_mu, grad_sigma, grad_log_sigma, out, st);
+  return elbo_body(ctx, lanes, n_lanes, x, y, M, B, mu, sigma, mode, guide, particles, prior_loc, prior_scale, dataset_size, noise,
+                   compute_grads, scalars, grad_mu, grad_sigma, grad_log_sigma, out, st);
+}
+
+int brl_elbo_step(brl_ctx* ctx, const float* x, const float* y, int64_t B, const float* mu, const float* sigma, int mode,
+                  int guide, int particles, float prior_loc, float prior_scale, int64_t dataset_size,
+                  const brl_noise* noise, int compute_grads, double* scalars, float* grad_mu, float* grad_sigma,
+                  float* grad_log_sigma, float* out, void* workspace, size_t workspace_bytes, void* stream) {
+  BRL_REQUIRE(ctx && x && y && mu && sigma && scalars && out && workspace, "brl_elbo_step: NULL argument");
+  DeviceGuard dg(ctx->device);
+  BRL_REQUIRE(B > 0 && particles > 0 && dataset_size > 0 && prior_scale > 0.f, "brl_elbo_step: bad sizes");
+  BRL_REQUIRE(guide == BRL_GUIDE_NORMAL || guide == BRL_GUIDE_RADIAL, "Guide unknown. Choose from 'normal', 'radial'.");
+  BRL_REQUIRE(mode == BRL_MODE_WS || mode == BRL_MODE_LRT || mode == BRL_MODE_FLIPOUT, "brl_elbo_step: mode must be WS, LRT or FLIPOUT");
+  BRL_REQUIRE(!compute_grads || (grad_mu && grad_sigma), "brl_elbo_step: gradient buffers are NULL");
+  if (guide == BRL_GUIDE_RADIAL) mode = BRL_MODE_WS;  // bayesian.py:81-83: radial forces nullcontext
+  return elbo_step(ctx, x, y, 1, B, mu, sigma, mode, guide, particles, prior_loc, prior_scale, dataset_size, noise, compute_grads,
+                   scalars, grad_mu, grad_sigma, grad_log_sigma, out, workspace, workspace_bytes, (cudaStream_t)stream);
+}
+
+int brl_elbo_step_ensemble(brl_ctx* ctx, const float* x, const float* y, int64_t M, int64_t B, const float* mu, const float* sigma,
+                           int mode, int guide, int particles, float prior_loc, float prior_scale, int64_t dataset_size,
+                           const brl_noise* noise, int compute_grads, double* scalars, float* grad_mu, float* grad_sigma,
+                           float* grad_log_sigma, float* out, void* workspace, size_t workspace_bytes, void* stream) {
+  BRL_REQUIRE(ctx && x && y && mu && sigma && scalars && out && workspace, "brl_elbo_step_ensemble: NULL argument");
+  DeviceGuard dg(ctx->device);
+  BRL_REQUIRE(M > 0 && M < (1 << 16) && B > 0 && particles > 0 && dataset_size > 0 && prior_scale > 0.f,
+              "brl_elbo_step_ensemble: bad M or sizes");
+  BRL_REQUIRE(guide == BRL_GUIDE_NORMAL || guide == BRL_GUIDE_RADIAL, "Guide unknown. Choose from 'normal', 'radial'.");
+  BRL_REQUIRE(mode == BRL_MODE_WS || mode == BRL_MODE_LRT || mode == BRL_MODE_FLIPOUT,
+              "brl_elbo_step_ensemble: mode must be WS, LRT or FLIPOUT");
+  BRL_REQUIRE(!compute_grads || (grad_mu && grad_sigma), "brl_elbo_step_ensemble: gradient buffers are NULL");
+  if (guide == BRL_GUIDE_RADIAL) mode = BRL_MODE_WS;  // bayesian.py:81-83: radial forces nullcontext
+  return elbo_step(ctx, x, y, M, B, mu, sigma, mode, guide, particles, prior_loc, prior_scale, dataset_size, noise, compute_grads,
+                   scalars, grad_mu, grad_sigma, grad_log_sigma, out, workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
 // M members of an HNN step in ONE chain of launches: the level-fused Inception kernels with the workspace's lanes for M members
@@ -1584,7 +1681,7 @@ static int hnn_step(brl_ctx* ctx, const float* x, const float* y, int64_t M, int
   carve_train(n, c, B, ab);
   if (!c.ok) return fail(BRL_ERR_WORKSPACE, M == 1 ? "brl_hnn_step: workspace too small" : "brl_hnn_step_ensemble: workspace too small");
   carve_tl(n, c, B, ab);
-  carve_members(n, c, B, M, ab);
+  carve_members(n, c, B, M, false, ab);
   if (M > 1 && !hnn_batched(ctx, ab, M, B)) {
     brl_noise base;
     memset(&base, 0, sizeof(base));

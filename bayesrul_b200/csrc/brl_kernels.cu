@@ -160,18 +160,21 @@ void launch_bwd_act(const BwdAct& p, cudaStream_t st) {
 // guide samplers
 // ------------------------------------------------------------------------------------------------
 __global__ void sample_normal_kernel(const float* __restrict__ mu, const float* __restrict__ sigma, long long P,
-                                     NoiseRef eps, float* __restrict__ w, float* __restrict__ delta) {
+                                     NoiseRef eps, float* __restrict__ w, float* __restrict__ delta, long long mu_stride,
+                                     int sample_stride) {
   const long long nblk = (P + 3) >> 2;
-  const int s = blockIdx.y;
+  const int s = blockIdx.y, se = s * sample_stride;  // draw s: MC-sample index / injected row sample0 + se
+  mu += s * mu_stride;
+  sigma += s * mu_stride;
   for (long long blk = blockIdx.x * (long long)blockDim.x + threadIdx.x; blk < nblk; blk += (long long)gridDim.x * blockDim.x) {
     float z[4];
     const long long e0 = blk << 2;
     if (eps.ptr) {
 #pragma unroll
-      for (int l = 0; l < 4; ++l) z[l] = e0 + l < P ? eps.ptr[(long long)s * P + e0 + l] : 0.f;
+      for (int l = 0; l < 4; ++l) z[l] = e0 + l < P ? eps.ptr[(long long)se * P + e0 + l] : 0.f;
     } else {
       const NoiseKey k = noise_key(eps);
-      const float4 n4 = normal4(philox_block(k.seed, KIND_WEIGHT_EPS, 0, k.sample0 + s, 0, (uint32_t)blk));
+      const float4 n4 = normal4(philox_block(k.seed, KIND_WEIGHT_EPS, 0, k.sample0 + se, 0, (uint32_t)blk));
       z[0] = n4.x; z[1] = n4.y; z[2] = n4.z; z[3] = n4.w;
     }
 #pragma unroll
@@ -185,11 +188,11 @@ __global__ void sample_normal_kernel(const float* __restrict__ mu, const float* 
   }
 }
 void launch_sample_normal(const float* mu, const float* sigma, long long P, long long S, NoiseRef eps, float* w,
-                          float* delta, cudaStream_t st) {
+                          float* delta, cudaStream_t st, long long mu_stride, int sample_stride) {
   const long long nblk = (P + 3) >> 2;
   dim3 grid((unsigned)min((nblk + 255) / 256, (long long)148 * 8), (unsigned)S);
   ++g_launch_count;
-  sample_normal_kernel<<<grid, 256, 0, st>>>(mu, sigma, P, eps, w, delta);
+  sample_normal_kernel<<<grid, 256, 0, st>>>(mu, sigma, P, eps, w, delta, mu_stride, sample_stride);
 }
 
 // The radial guide needs ||eps|| over each whole site before any weight of the site exists, so the draw is two passes over
@@ -205,14 +208,14 @@ __device__ __forceinline__ void weight_eps4(const NoiseRef& eps, const NoiseKey&
   }
 }
 __global__ void radial_norm_kernel(long long P, const long long* __restrict__ site_off, int n_sites, NoiseRef eps,
-                                   float* __restrict__ norms) {
-  const int j = blockIdx.x, s = blockIdx.y;
+                                   float* __restrict__ norms, int sample_stride) {
+  const int j = blockIdx.x, s = blockIdx.y, se = s * sample_stride;
   const long long beg = site_off[j], end = site_off[j + 1];
   const NoiseKey k = noise_key(eps);
   double acc = 0.0;
   for (long long blk = (beg >> 2) + threadIdx.x; blk <= ((end - 1) >> 2); blk += blockDim.x) {
     float z[4];
-    weight_eps4(eps, k, s, P, blk, z);
+    weight_eps4(eps, k, se, P, blk, z);
 #pragma unroll
     for (int l = 0; l < 4; ++l) {
       const long long e = (blk << 2) + l;
@@ -224,13 +227,16 @@ __global__ void radial_norm_kernel(long long P, const long long* __restrict__ si
 }
 __global__ void radial_apply_kernel(const float* __restrict__ mu, const float* __restrict__ sigma, long long P,
                                     const long long* __restrict__ site_off, int n_sites, NoiseRef eps, NoiseRef r,
-                                    const float* __restrict__ norms, float* __restrict__ w, float* __restrict__ delta) {
-  const int s = blockIdx.y;
+                                    const float* __restrict__ norms, float* __restrict__ w, float* __restrict__ delta,
+                                    long long mu_stride, int sample_stride) {
+  const int s = blockIdx.y, se = s * sample_stride;
+  mu += s * mu_stride;
+  sigma += s * mu_stride;
   const long long nblk = (P + 3) >> 2;
   const NoiseKey k = noise_key(eps), rk = noise_key(r);
   for (long long blk = blockIdx.x * (long long)blockDim.x + threadIdx.x; blk < nblk; blk += (long long)gridDim.x * blockDim.x) {
     float z[4];
-    weight_eps4(eps, k, s, P, blk, z);
+    weight_eps4(eps, k, se, P, blk, z);
     const long long e0 = blk << 2;
     int lo = 0, hi = n_sites - 1;  // site of e0: last j with site_off[j] <= e0
     while (lo < hi) {
@@ -246,8 +252,8 @@ __global__ void radial_apply_kernel(const float* __restrict__ mu, const float* _
       if (e >= P) break;
       while (e >= site_off[j + 1]) { ++j; have = false; }
       if (!have) {
-        const float rr = r.ptr ? r.ptr[(long long)s * n_sites + j]
-                               : philox_normal(rk.seed, KIND_RADIAL_R, 0, rk.sample0 + s, 0, (uint32_t)j);
+        const float rr = r.ptr ? r.ptr[(long long)se * n_sites + j]
+                               : philox_normal(rk.seed, KIND_RADIAL_R, 0, rk.sample0 + se, 0, (uint32_t)j);
         scale = rr / norms[(long long)s * n_sites + j];
         have = true;
       }
@@ -259,13 +265,13 @@ __global__ void radial_apply_kernel(const float* __restrict__ mu, const float* _
 }
 void launch_sample_radial(const float* mu, const float* sigma, long long P, long long S, const long long* site_off,
                           int n_sites, int max_site, NoiseRef eps, NoiseRef r, float* norms, float* w, float* delta,
-                          cudaStream_t st) {
+                          cudaStream_t st, long long mu_stride, int sample_stride) {
   ++g_launch_count;
-  radial_norm_kernel<<<dim3(n_sites, (unsigned)S), 256, 0, st>>>(P, site_off, n_sites, eps, norms);
+  radial_norm_kernel<<<dim3(n_sites, (unsigned)S), 256, 0, st>>>(P, site_off, n_sites, eps, norms, sample_stride);
   ++g_launch_count;
   const long long nblk = (P + 3) >> 2;
   radial_apply_kernel<<<dim3((unsigned)min((nblk + 255) / 256, (long long)148 * 8), (unsigned)S), 256, 0, st>>>(
-      mu, sigma, P, site_off, n_sites, eps, r, norms, w, delta);
+      mu, sigma, P, site_off, n_sites, eps, r, norms, w, delta, mu_stride, sample_stride);
 }
 
 __global__ void gen_signs_kernel(float* dst, long long S, long long B, int C, NoiseRef nz) {
@@ -278,9 +284,11 @@ __global__ void gen_signs_kernel(float* dst, long long S, long long B, int C, No
     dst[i] = philox_sign(k.seed, nz.kind, nz.site, k.sample0 + s, k.window0 + b, c);
   }
 }
-__global__ void gen_signs_multi_kernel(const SignJobs jobs, long long B, NoiseRef base) {
+__global__ void gen_signs_multi_kernel(const SignJobs jobs, long long B, NoiseRef base, int sample_stride) {
   const long long total = jobs.start[jobs.n];
-  const NoiseKey k = noise_key(base);
+  const int m = blockIdx.y;  // member: its tensors [B, C] follow the previous member's, MC-sample index + m sample_stride
+  NoiseKey k = noise_key(base);
+  k.sample0 += (unsigned)(m * sample_stride);
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
     int j = 0;
     while (j + 1 < jobs.n && i >= jobs.start[j + 1]) ++j;
@@ -289,18 +297,19 @@ __global__ void gen_signs_multi_kernel(const SignJobs jobs, long long B, NoiseRe
     const long long e = i - jobs.start[j];
     const int C = jobs.C[j], Q = (C + 3) >> 2, q = (int)(e % Q), b = (int)(e / Q);
     const uint4 r = philox_block(k.seed, jobs.kind[j], jobs.site[j], k.sample0, k.window0 + b, (uint32_t)q);
-    float* d = jobs.dst[j] + (long long)b * C + 4 * q;
+    float* d = jobs.dst[j] + ((long long)m * B + b) * C + 4 * q;
     const uint32_t w[4] = {r.x, r.y, r.z, r.w};
 #pragma unroll
     for (int l = 0; l < 4; ++l)
       if (4 * q + l < C) d[l] = (w[l] >> 31) ? -1.0f : 1.0f;
   }
 }
-void launch_gen_signs_multi(const SignJobs& jobs, long long B, NoiseRef base, cudaStream_t st) {
+void launch_gen_signs_multi(const SignJobs& jobs, long long B, NoiseRef base, cudaStream_t st, int members, int sample_stride) {
   const long long total = jobs.start[jobs.n];
   if (total <= 0) return;
   ++g_launch_count;
-  gen_signs_multi_kernel<<<(unsigned)min((total + 255) / 256, (long long)148 * 8), 256, 0, st>>>(jobs, B, base);
+  gen_signs_multi_kernel<<<dim3((unsigned)min((total + 255) / 256, (long long)148 * 8), (unsigned)members), 256, 0, st>>>(
+      jobs, B, base, sample_stride);
 }
 void launch_gen_signs(float* dst, long long S, long long B, int C, NoiseRef nz, cudaStream_t st) {
   const long long total = S * B * C;
@@ -369,7 +378,17 @@ void launch_nll_hnn(const float* out, const float* y, long long B, double* acc, 
 // ------------------------------------------------------------------------------------------------
 // KL + gradient finalisation
 // ------------------------------------------------------------------------------------------------
-__global__ void finalize_kernel(const Finalize p) {
+// member blockIdx.y: its parameters, draws and gradients P floats after the previous member's, its KL at kl_acc + m kl_stride
+__device__ __forceinline__ Finalize member_finalize(Finalize p) {
+  const long long o = p.P * blockIdx.y;
+  auto sh = [o](auto* q) { return q ? q + o : q; };
+  p.mu = sh(p.mu); p.sigma = sh(p.sigma); p.w = sh(p.w); p.delta = sh(p.delta); p.g0 = sh(p.g0); p.g1 = sh(p.g1);
+  p.grad_mu = sh(p.grad_mu); p.grad_sigma = sh(p.grad_sigma); p.grad_log_sigma = sh(p.grad_log_sigma);
+  p.kl_acc += (long long)p.kl_stride * blockIdx.y;
+  return p;
+}
+__global__ void finalize_kernel(const Finalize p_) {
+  const Finalize p = member_finalize(p_);
   double kl = 0.0;
   const float isp2 = 1.0f / (p.prior_scale * p.prior_scale);
   const float lsp = logf(p.prior_scale);
@@ -409,21 +428,23 @@ __global__ void finalize_kernel(const Finalize p) {
 }
 void launch_finalize(const Finalize& p, cudaStream_t st) {
   ++g_launch_count;
-  finalize_kernel<<<(unsigned)min((p.P + 255) / 256, (long long)148 * 4), 256, 0, st>>>(p);
+  finalize_kernel<<<dim3((unsigned)min((p.P + 255) / 256, (long long)148 * 4), (unsigned)max(1, p.members)), 256, 0, st>>>(p);
 }
 
 __global__ void post_scalars_kernel(double* scalars, const double* acc, double c_nll, double c, int particles,
                                     long long B) {
-  // acc = {nll_sum over particles, squared error sum over particles, kl sum over particles}
+  // acc = {nll_sum over particles, squared error sum over particles, kl sum over particles}; member m (thread m): [m][4]
+  scalars += 4 * threadIdx.x;
+  acc += 4 * threadIdx.x;
   scalars[0] = (c_nll * acc[0] + c * acc[2]) / particles;
   scalars[1] = acc[0] / particles;
   scalars[2] = acc[2] / particles;
   scalars[3] = acc[1] / ((double)particles * (double)B);
 }
 void launch_post_scalars(double* scalars, const double* acc, double c_nll, double c, int particles, long long B,
-                         cudaStream_t st) {
+                         cudaStream_t st, int members) {
   ++g_launch_count;
-  post_scalars_kernel<<<1, 1, 0, st>>>(scalars, acc, c_nll, c, particles, B);
+  post_scalars_kernel<<<1, members, 0, st>>>(scalars, acc, c_nll, c, particles, B);
 }
 
 __global__ void log_sigma_grad_kernel(const float* gs, const float* sigma, float* gls, long long P) {

@@ -143,14 +143,17 @@ struct BwdAct {
 };
 void launch_bwd_act(const BwdAct& p, cudaStream_t st);
 
+// S draws [S,P]: draw s reads mu / sigma + s mu_stride (0: S draws of one posterior; P: one draw from each of S posteriors, the
+// members of an ensemble step) and MC-sample index / injected noise row sample0 + s sample_stride
 void launch_sample_normal(const float* mu, const float* sigma, long long P, long long S, NoiseRef eps, float* w,
-                          float* delta, cudaStream_t st);
+                          float* delta, cudaStream_t st, long long mu_stride = 0, int sample_stride = 1);
 void launch_sample_radial(const float* mu, const float* sigma, long long P, long long S, const long long* site_off,
                           int n_sites, int max_site, NoiseRef eps, NoiseRef r, float* norms /*[S,n_sites]*/, float* w,
-                          float* delta, cudaStream_t st);
+                          float* delta, cudaStream_t st, long long mu_stride = 0, int sample_stride = 1);
 void launch_gen_signs(float* dst, long long S, long long B, int C, NoiseRef nz, cudaStream_t st);
 // all sign tensors of one particle in ONE launch (a Flipout step needs 2 per layer): job j fills dst[j][B][C[j]] with stream
-// (kind[j], site[j]) of the key in `base`
+// (kind[j], site[j]) of the key in `base`; with `members` > 1, member m fills dst[j][m][B][C[j]] with MC-sample index
+// sample0 + m sample_stride
 struct SignJobs {
   float* dst[32];
   int C[32];
@@ -158,7 +161,8 @@ struct SignJobs {
   long long start[33];  // offsets of the jobs in the launch's index space (work item = four consecutive channels of a window)
   int n;
 };
-void launch_gen_signs_multi(const SignJobs& jobs, long long B, NoiseRef base, cudaStream_t st);
+void launch_gen_signs_multi(const SignJobs& jobs, long long B, NoiseRef base, cudaStream_t st, int members = 1,
+                            int sample_stride = 1);
 
 void launch_nll_elbo(const float* out, const float* y, long long B, float gscale, double* acc /*[nll, mse]*/,
                      float* gout, cudaStream_t st);
@@ -173,10 +177,14 @@ struct Finalize {
   float *grad_mu, *grad_sigma;
   float* grad_log_sigma;  // last particle only (nullable): d/d(log sigma) = d/d(sigma) * sigma of the summed gradient
   double* kl_acc;  // += KL (unscaled) of this particle
+  // members > 1 (ensemble step): member m's mu / sigma / w / delta / g0 / g1 / grad_* sit m P floats further, its KL at
+  // kl_acc + m kl_stride
+  int members, kl_stride;
 };
 void launch_finalize(const Finalize& p, cudaStream_t st);
+// scalars [members][4] from acc [members][4]
 void launch_post_scalars(double* scalars, const double* acc, double c_nll, double c, int particles, long long B,
-                         cudaStream_t st);
+                         cudaStream_t st, int members = 1);
 void launch_log_sigma_grad(const float* gs, const float* sigma, float* gls, long long P, cudaStream_t st);
 
 void launch_moments_update(const float* out, long long S, long long B, float* state /*[4,B]*/, int first,

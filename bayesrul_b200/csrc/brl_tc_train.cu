@@ -197,10 +197,11 @@ __device__ __forceinline__ TtLane member_lane(TtLane ln, long long stride) {
   ln.fcblob = sh(ln.fcblob);
   return ln;
 }
-// the member's dropout stream: injected masks [members, B, per_window], Philox keys with MC-sample index sample0 + member
-__device__ __forceinline__ NoiseRef member_noise(NoiseRef nz, long long per_window, int B) {
-  if (nz.ptr) nz.ptr += (long long)blockIdx.z * B * per_window;
-  else nz.sample0 += blockIdx.z;
+// the member's noise stream: `stride` MC samples per member (1 for the HNN step, `particles` for the ELBO step), i.e. injected
+// tensors [members * stride, B, per_window] and Philox keys with MC-sample index sample0 + member * stride
+__device__ __forceinline__ NoiseRef member_noise(NoiseRef nz, long long per_window, int B, int stride) {
+  if (nz.ptr) nz.ptr += (long long)blockIdx.z * stride * B * per_window;
+  else nz.sample0 += blockIdx.z * (unsigned)stride;
   return nz;
 }
 template <typename T>
@@ -309,7 +310,8 @@ struct TtFwdArgs {
   const float* sgn_fc_in;  // Flipout: s_in of the fc layer [B, 2400] (the feature producers build its perturbation operand)
   NoiseRef drop[4];        // PLAIN mode: dropout site behind the layer (injected masks [B, N, 30] or Philox)
   float keep[4];           // its keep probability (1 = no dropout site / dropout off)
-  long long lane_stride;   // ensemble members (blockIdx.z, PLAIN mode): bytes between their lanes
+  long long lane_stride;   // ensemble members (blockIdx.z): bytes between their lanes
+  int noise_stride, sign_stride;  // ensemble members: MC samples / sign-tensor rows [B, C] between their noise (TtStep)
   int* status;
   long long* trace;  // debug: clock64 stamps of CTA (0, y), [4 layers][16] (nullptr = off)
 };
@@ -370,7 +372,7 @@ __global__ void __launch_bounds__(NT, 1) tt_fwd_kernel(const TtFwdArgs a) {
   const TtLayer& L = a.lay[blockIdx.y];
   const int tile = blockIdx.x, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   long long* tr = (a.trace && blockIdx.x == 0 && blockIdx.z == 0 && tid == 0) ? a.trace + blockIdx.y * 16 : nullptr;
-  const TtLane ln = MODE == TT_PLAIN ? member_lane(a.ln, a.lane_stride) : a.ln;
+  const TtLane ln = member_lane(a.ln, a.lane_stride);
   if (tr) tr[0] = clock64();
   const uint32_t sbase = smem_u32(smem);
   const uint32_t bar_ld = sbase + F_BAR, bar_mma = bar_ld + 8;
@@ -405,7 +407,9 @@ __global__ void __launch_bounds__(NT, 1) tt_fwd_kernel(const TtFwdArgs a) {
     __syncthreads();
   }
   constexpr bool P1H = MODE == BRL_MODE_FLIPOUT;  // perturbation path: fp16 operands (W - mu is far above fp16's subnormals for q_scale >= 1e-4)
-  if (MODE != TT_PLAIN) second_operand<MODE, P1H>(smem + F_A, smem + F_A2, nullptr, L, a.sgn_in[blockIdx.y], tile, a.B, tid);
+  if (MODE != TT_PLAIN)
+    second_operand<MODE, P1H>(smem + F_A, smem + F_A2, nullptr, L,
+                              member_ptr(a.sgn_in[blockIdx.y], (long long)a.sign_stride * a.B * L.cin), tile, a.B, tid);
   fence_async_smem();
   tc_fence_before();
   __syncthreads();
@@ -435,10 +439,10 @@ __global__ void __launch_bounds__(NT, 1) tt_fwd_kernel(const TtFwdArgs a) {
   const RowInfo ri = row_info(ROW0 + row, tile, a.B);
   const uint32_t la = tmem + ((uint32_t)((warp & 3) * 32) << 16);
   const float* bias = reinterpret_cast<const float*>(smem + F_BIAS);
-  const NoiseRef& nz = a.eps[blockIdx.y];
+  const NoiseRef nz = MODE == BRL_MODE_LRT ? member_noise(a.eps[blockIdx.y], (long long)L.N * 30, a.B, a.noise_stride) : a.eps[blockIdx.y];
   const NoiseKey nk = noise_key(nz);
-  const float* sout = a.sgn_out[blockIdx.y];
-  const NoiseRef dz = MODE == TT_PLAIN ? member_noise(a.drop[blockIdx.y], (long long)L.N * 30, a.B) : a.drop[blockIdx.y];
+  const float* sout = member_ptr(a.sgn_out[blockIdx.y], (long long)a.sign_stride * a.B * L.N);
+  const NoiseRef dz = MODE == TT_PLAIN ? member_noise(a.drop[blockIdx.y], (long long)L.N * 30, a.B, a.noise_stride) : a.drop[blockIdx.y];
   float* rb = ln.rbuf ? ln.rbuf + (long long)tile * RBUF_PER_TILE + L.roff_per_tile : nullptr;
   unsigned char* oimg = L.out == OUT_M1 ? ln.m1 + (long long)tile * 16 * CS
                         : L.out == OUT_T2 ? ln.t2 + (long long)tile * 8 * CS
@@ -504,7 +508,7 @@ __global__ void __launch_bounds__(NT, 1) tt_fwd_kernel(const TtFwdArgs a) {
 #pragma unroll
       for (int j = 0; j < 8; ++j)
         f2[j] = MODE == BRL_MODE_LRT ? fr[j] * fr[j]
-                : MODE == BRL_MODE_FLIPOUT ? fr[j] * __ldg(a.sgn_fc_in + (long long)ri.gw * 2400 + (c0 + j) * 30 + ri.t) : 0.f;
+                : MODE == BRL_MODE_FLIPOUT ? fr[j] * __ldg(a.sgn_fc_in + ((long long)blockIdx.z * a.sign_stride * a.B + ri.gw) * 2400 + (c0 + j) * 30 + ri.t) : 0.f;
       *reinterpret_cast<uint4*>(ln.fimg + fa) = fh;
       *reinterpret_cast<uint4*>(ln.fbimg + fa) = pack_b8(fr);
       if (MODE == BRL_MODE_LRT) {
@@ -541,7 +545,8 @@ struct TtBwdArgs {
   const float* sgn_out[4];
   float *g0, *g1;
   float keep[4];  // PLAIN mode: keep probability of the dropout site behind each layer (1 = none)
-  long long lane_stride;  // ensemble members (blockIdx.z, PLAIN mode): bytes between their lanes
+  long long lane_stride;  // ensemble members (blockIdx.z): bytes between their lanes
+  int sign_stride;        // ensemble members: sign-tensor rows [B, C] between theirs (TtStep)
   int part_floats;
   int* status;
   long long* trace;
@@ -618,7 +623,7 @@ __global__ void __launch_bounds__(NT, 1) tt_bwd_kernel(const TtBwdArgs a) {
   const TtLayer& L = a.lay[blockIdx.y];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   long long* tr = (a.trace && blockIdx.x == 0 && blockIdx.z == 0 && tid == 0) ? a.trace + blockIdx.y * 16 : nullptr;
-  const TtLane ln = MODE == TT_PLAIN ? member_lane(a.ln, a.lane_stride) : a.ln;
+  const TtLane ln = member_lane(a.ln, a.lane_stride);
   if (tr) tr[0] = clock64();
   const uint32_t sbase = smem_u32(smem);
   const uint32_t bar_ld = sbase + B_BAR, bar_mma = bar_ld + 8;
@@ -668,7 +673,7 @@ __global__ void __launch_bounds__(NT, 1) tt_bwd_kernel(const TtBwdArgs a) {
     const int row = (warp & 3) * 32 + lane, cq = warp >> 2;
     const RowInfo ri = row_info(ROW0 + row, tile, a.B);
     const float* rb = ln.rbuf + (long long)tile * RBUF_PER_TILE + L.roff_per_tile;
-    const float* sout = a.sgn_out[blockIdx.y];
+    const float* sout = member_ptr(a.sgn_out[blockIdx.y], (long long)a.sign_stride * a.B * L.N);
     for (int c = cq; c < L.NP / 8; c += 4) {
       float d[8], d1[8];
       output_grad<MODE>(ln, L, tile, row, ri, c * 8, d);
@@ -700,7 +705,8 @@ __global__ void __launch_bounds__(NT, 1) tt_bwd_kernel(const TtBwdArgs a) {
       pool_image(smem + B_AB, smem + B_AH, L.KC, tile, a.B, tid);
       __syncthreads();
     }
-    second_operand<MODE, false>(smem + B_AH, smem + B_A2, smem + B_AB, L, a.sgn_in[blockIdx.y], tile, a.B, tid);
+    second_operand<MODE, false>(smem + B_AH, smem + B_A2, smem + B_AB, L,
+                                member_ptr(a.sgn_in[blockIdx.y], (long long)a.sign_stride * a.B * L.cin), tile, a.B, tid);
     fence_async_smem();
     tc_fence_before();
     __syncthreads();
@@ -738,7 +744,7 @@ __global__ void __launch_bounds__(NT, 1) tt_bwd_kernel(const TtBwdArgs a) {
     if (has_dx) {  // ---- input gradient of this tile -> bf16 image (thread = row x column quarter)
       unsigned char* gi = member_ptr(a.ln.g[L.gdst], a.lane_stride) + (long long)tile * L.KC * CS;  // (ln.g[L.gdst]: a local-memory copy)
       const uint32_t la = tmem + ((uint32_t)((warp & 3) * 32) << 16);
-      const float* sin_ = a.sgn_in[blockIdx.y];
+      const float* sin_ = member_ptr(a.sgn_in[blockIdx.y], (long long)a.sign_stride * a.B * L.cin);
       for (int g = cq; g < dxw / 8; g += 4) {
         float v0[8], v1[8], o[8], av[8];
         tmem_ld8(la + g * 8, v0);
@@ -947,7 +953,7 @@ __device__ __forceinline__ TtFcBwdArgs member_fc(TtFcBwdArgs a) {
 template <int MODE>
 __global__ void __launch_bounds__(256, 1) tt_fc_dx_kernel(const TtFcBwdArgs a_) {
   extern __shared__ __align__(128) unsigned char smem[];
-  const TtFcBwdArgs a = MODE == TT_PLAIN ? member_fc(a_) : a_;
+  const TtFcBwdArgs a = member_fc(a_);
   const int mt = blockIdx.x, ns = blockIdx.y, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const uint32_t sbase = smem_u32(smem), bar_ld = sbase + FX_BAR, bar_mma = bar_ld + 8;
   uint32_t* tslot = reinterpret_cast<uint32_t*>(smem + FX_BAR + 16);
@@ -1020,7 +1026,7 @@ constexpr int FW_SMEM = FW_BAR + 64;
 template <int MODE>
 __global__ void __launch_bounds__(256, 1) tt_fc_dw_kernel(const TtFcBwdArgs a_) {
   extern __shared__ __align__(128) unsigned char smem[];
-  const TtFcBwdArgs a = MODE == TT_PLAIN ? member_fc(a_) : a_;
+  const TtFcBwdArgs a = member_fc(a_);
   const int kt = blockIdx.x, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const uint32_t sbase = smem_u32(smem), bar_ld = sbase + FW_BAR, bar_mma = bar_ld + 8;
   uint32_t* tslot = reinterpret_cast<uint32_t*>(smem + FW_BAR + 16);
@@ -1151,8 +1157,10 @@ struct TtTailArgs {
   float keep_fc;               // keep probability of the dropout site behind the fc layer (1 = none)
   NoiseRef drop_fc;            // its masks: injected [B, HW] or Philox
   long long P, part_stride;    // ensemble members (blockIdx.z): floats between their parameters / gradients and their `part`
+  int noise_stride, sign_stride, acc_stride;  // ... MC samples / sign rows [B, C] / accumulator doubles between theirs
 };
-// the arguments as ensemble member blockIdx.z sees them (y, out, dpre, dsec: [members][B][...]; acc: [members][2])
+// the arguments as ensemble member blockIdx.z sees them (y, dpre, dsec: [members][B][...]; out: [members][noise_stride][B][2];
+// acc: [members][acc_stride])
 template <int HW>
 __device__ __forceinline__ TtTailArgs member_tail(TtTailArgs a) {
   a.part = member_ptr(a.part, a.part_stride);
@@ -1160,16 +1168,20 @@ __device__ __forceinline__ TtTailArgs member_tail(TtTailArgs a) {
   a.hw0 = member_ptr(a.hw0, a.P); a.hw1 = member_ptr(a.hw1, a.P);
   a.hb0 = member_ptr(a.hb0, a.P); a.hb1 = member_ptr(a.hb1, a.P);
   a.y = member_ptr(a.y, (long long)a.B);
-  a.acc = member_ptr(a.acc, 2ll);
-  a.out = member_ptr(a.out, 2ll * a.B);
+  a.acc = member_ptr(a.acc, (long long)a.acc_stride);
+  a.out = member_ptr(a.out, 2ll * a.noise_stride * a.B);
   a.dpre = member_ptr(a.dpre, (long long)HW * a.B); a.dsec = member_ptr(a.dsec, (long long)HW * a.B);
   a.g0 = member_ptr(a.g0, a.P); a.g1 = member_ptr(a.g1, a.P);
-  a.drop_fc = member_noise(a.drop_fc, HW, a.B);
+  a.drop_fc = member_noise(a.drop_fc, HW, a.B, a.noise_stride);
+  a.eps_fc = member_noise(a.eps_fc, HW, a.B, a.noise_stride);
+  a.eps_head = member_noise(a.eps_head, 2, a.B, a.noise_stride);
+  const long long sr = (long long)a.sign_stride * a.B;
+  a.sout_fc = member_ptr(a.sout_fc, sr * HW); a.sin_head = member_ptr(a.sin_head, sr * HW); a.sout_head = member_ptr(a.sout_head, sr * 2);
   return a;
 }
 template <int MODE, int HW>
 __global__ void __launch_bounds__(256) tt_tail_kernel(const TtTailArgs a_) {
-  const TtTailArgs a = MODE == TT_PLAIN ? member_tail<HW>(a_) : a_;
+  const TtTailArgs a = member_tail<HW>(a_);
   __shared__ float sg[2][2][HW + 1];  // [path][output][hidden unit | bias] head weight-gradient partials of the CTA
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   for (int i = tid; i < 2 * 2 * (HW + 1); i += 256) (&sg[0][0][0])[i] = 0.f;
@@ -1524,6 +1536,7 @@ void tt_forward(const TtLane& ln, const TtStep& s, cudaStream_t st, const TtSide
     fa.ln = ln;
     if (s.mode != BRL_MODE_LRT) fa.ln.rbuf = nullptr;
     fa.B = (int)s.B; fa.ntile = nt; fa.sgn_fc_in = s.sgn_fc_in; fa.lane_stride = s.lane_stride; fa.status = tt_status_word();
+    fa.noise_stride = s.noise_stride; fa.sign_stride = s.sign_stride;
     fa.trace = g_tt_trace ? g_tt_trace + lv * 64 : nullptr;
     int nl = 0;
     for (int k = 0; k < 4; ++k) {
@@ -1539,8 +1552,8 @@ void tt_forward(const TtLane& ln, const TtStep& s, cudaStream_t st, const TtSide
     }
     fa.nl = nl;
     ++g_launch_count;
-    if (s.mode == BRL_MODE_LRT) tt_fwd_kernel<BRL_MODE_LRT><<<dim3(nt, nl), NT, F_SMEM, st>>>(fa);
-    else if (s.mode == BRL_MODE_FLIPOUT) tt_fwd_kernel<BRL_MODE_FLIPOUT><<<dim3(nt, nl), NT, F_SMEM, st>>>(fa);
+    if (s.mode == BRL_MODE_LRT) tt_fwd_kernel<BRL_MODE_LRT><<<dim3(nt, nl, M), NT, F_SMEM, st>>>(fa);
+    else if (s.mode == BRL_MODE_FLIPOUT) tt_fwd_kernel<BRL_MODE_FLIPOUT><<<dim3(nt, nl, M), NT, F_SMEM, st>>>(fa);
     else tt_fwd_kernel<TT_PLAIN><<<dim3(nt, nl, M), NT, F_SMEM, st>>>(fa);
   }
 }
@@ -1570,6 +1583,7 @@ void tt_tail(const TtStep& s, const TtTail& t, cudaStream_t st) {
   a.y = t.y; a.gscale = t.gscale; a.acc = t.acc; a.out = t.out; a.dpre = t.dpre; a.dsec = t.dsec;
   a.g0 = s.g0; a.g1 = s.g1; a.hw_off = t.hw_off; a.hb_off = t.hb_off;
   a.P = s.P; a.part_stride = 2 * s.B * t.width;
+  a.noise_stride = s.noise_stride; a.sign_stride = s.sign_stride; a.acc_stride = t.acc_stride;
   const dim3 grid((unsigned)std::min<long long>((s.B + 7) / 8, 148), 1, (unsigned)s.members);
   ++g_launch_count;
   if (t.width == 320) {
@@ -1599,14 +1613,14 @@ void tt_fc_backward(const TtLane& ln, const TtStep& s, const float* dpre, const 
   cudaEventRecord(sd.fork, st);
   cudaStreamWaitEvent(sd.side, sd.fork, 0);
   if (s.mode == BRL_MODE_LRT) {
-    tt_fc_dx_kernel<BRL_MODE_LRT><<<dim3(ba.nmt, FC_NS), 256, FX_SMEM, st>>>(ba);
-    tt_fc_dw_kernel<BRL_MODE_LRT><<<(FC_KC + 15) / 16, 256, FW_SMEM, sd.side>>>(ba);
+    tt_fc_dx_kernel<BRL_MODE_LRT><<<dim3(ba.nmt, FC_NS, s.members), 256, FX_SMEM, st>>>(ba);
+    tt_fc_dw_kernel<BRL_MODE_LRT><<<dim3((FC_KC + 15) / 16, 1, s.members), 256, FW_SMEM, sd.side>>>(ba);
   } else if (s.mode != BRL_MODE_FLIPOUT) {
     tt_fc_dx_kernel<TT_PLAIN><<<dim3(ba.nmt, FC_NS, s.members), 256, FX_SMEM, st>>>(ba);
     tt_fc_dw_kernel<TT_PLAIN><<<dim3((FC_KC + 15) / 16, 1, s.members), 256, FW_SMEM, sd.side>>>(ba);
   } else {
-    tt_fc_dx_kernel<BRL_MODE_FLIPOUT><<<dim3(ba.nmt, FC_NS), 256, FX_SMEM, st>>>(ba);
-    tt_fc_dw_kernel<BRL_MODE_FLIPOUT><<<(FC_KC + 15) / 16, 256, FW_SMEM, sd.side>>>(ba);
+    tt_fc_dx_kernel<BRL_MODE_FLIPOUT><<<dim3(ba.nmt, FC_NS, s.members), 256, FX_SMEM, st>>>(ba);
+    tt_fc_dw_kernel<BRL_MODE_FLIPOUT><<<dim3((FC_KC + 15) / 16, 1, s.members), 256, FW_SMEM, sd.side>>>(ba);
   }
   cudaEventRecord(sd.join, sd.side);
 }
@@ -1624,6 +1638,7 @@ void tt_backward(const TtLane& ln, const TtStep& s, cudaStream_t st, const TtSid
     ba.ln = ln;
     ba.part_floats = tb.part_floats;
     ba.B = (int)s.B; ba.ntile = nt; ba.g0 = s.g0; ba.g1 = s.g1; ba.lane_stride = s.lane_stride; ba.status = tt_status_word();
+    ba.sign_stride = s.sign_stride;
     ba.trace = g_tt_trace ? g_tt_trace + (3 + lv) * 64 : nullptr;
     int nl = 0;
     for (int k = 0; k < 4; ++k) {
@@ -1641,9 +1656,10 @@ void tt_backward(const TtLane& ln, const TtStep& s, cudaStream_t st, const TtSid
     for (int k = 0; k < 4; ++k)
       if (levels[lv][k] >= 0) ra.ngroups[levels[lv][k]] = ngroups;
     ++g_launch_count;
-    if (s.mode == BRL_MODE_LRT) tt_bwd_kernel<BRL_MODE_LRT><<<dim3(ngroups, nl), NT, B_SMEM, st>>>(ba);
-    else if (s.mode == BRL_MODE_FLIPOUT) tt_bwd_kernel<BRL_MODE_FLIPOUT><<<dim3(ngroups, nl), NT, B_SMEM, st>>>(ba);
-    else tt_bwd_kernel<TT_PLAIN><<<dim3(ngroups, nl, s.members), NT, B_SMEM, st>>>(ba);
+    const dim3 grid(ngroups, nl, s.members);
+    if (s.mode == BRL_MODE_LRT) tt_bwd_kernel<BRL_MODE_LRT><<<grid, NT, B_SMEM, st>>>(ba);
+    else if (s.mode == BRL_MODE_FLIPOUT) tt_bwd_kernel<BRL_MODE_FLIPOUT><<<grid, NT, B_SMEM, st>>>(ba);
+    else tt_bwd_kernel<TT_PLAIN><<<grid, NT, B_SMEM, st>>>(ba);
   }
   int tot = 0;
   for (int i = 0; i < TT_LAYERS; ++i) {

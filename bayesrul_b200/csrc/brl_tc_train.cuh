@@ -50,12 +50,16 @@ struct TtStep {
   float* g0;             // flat gradient accumulators [P] (brl_kernels.cuh: Finalize): mean path / variance or perturbation path
   float* g1;
   long long w_off[TT_LAYERS], b_off[TT_LAYERS];
-  // Inception, BRL_MODE_DET: `members` independent nets (a deep ensemble) in the same launches, member m on blockIdx.z.  Member m
-  // reads x + m B 540, mu + m P, its lane images at lane + m lane_stride bytes, and writes g0 + m P; its dropout streams are the
-  // injected masks + m B out_elems or Philox with MC-sample index sample0 + m.  The tail's y / out / acc / part / dpre follow.
+  // Inception: `members` independent nets (the members of a deep ensemble, the seeds of a BNN experiment) in the same launches,
+  // member m on blockIdx.z.  Member m reads x + m B 540, mu / sigma / wsamp + m P, its lane images at lane + m lane_stride bytes,
+  // and writes g0 / g1 + m P; its noise streams (LRT eps, dropout masks) are the injected tensors + m noise_stride B per_window or
+  // Philox with MC-sample index sample0 + m noise_stride, its sign tensors sgn_in / sgn_out / sgn_fc_in + m sign_stride B C.  The
+  // tail's y / out / acc / part / dpre / dsec follow (TtTail).
   int members = 1;
   long long P = 0;            // floats between members' parameters / gradients
   long long lane_stride = 0;  // bytes between members' TtLane images (tt_carve of M lanes back to back)
+  int noise_stride = 1;       // MC samples between members: 1 (HNN step), `particles` (ELBO step: member-major, particle-minor)
+  int sign_stride = 1;        // sign-tensor rows [B, C] between members: 1 (generated per member), `particles` (injected)
 };
 // forward of the ten conv layers: x -> feature images (+ the activation / eps images the backward pass re-reads); 6 launches
 // side stream + two events of the calling lane: independent kernels of a step (weight packing next to the window packing, the fc
@@ -86,6 +90,8 @@ struct TtTail {
   NoiseRef drop_fc{};
   int width = 64;            // hidden units in front of the head: 64 (Inception fc layer), 32 (Linear layer 3), 320 (Conv-D3: the
                              // pooled conv3 features, given in `part` as [B, 320]; their gradient goes to `dpre`)
+  int acc_stride = 2;        // TtStep::members: doubles between members' accumulators (HNN [M][2] = {loss, mse}; ELBO [M][4] =
+                             // {nll, squared error, kl, -}); out is [members][noise_stride][B][2], part / dpre / dsec per member
 };
 void tt_tail(const TtStep& s, const TtTail& t, cudaStream_t st);
 // backward: feature-gradient image -> g0 / g1 of the ten conv layers (accumulated: the buffers must be zeroed); 4 launches

@@ -332,6 +332,41 @@ class Engine:
                                           ws.numel(), self._stream()))
         return dict(scalars=scalars, grad_mu=g[0], grad_sigma=g[1], grad_log_sigma=g[2], out=out, flat=flat)
 
+    def elbo_step_ensemble(self, x, y, mu, sigma, *, mode: str = "lrt", guide: str = "normal", particles: int = 1,
+                           prior_loc: float = 0.0, prior_scale: float = 1.0, dataset_size: int, noise: Optional[Noise] = None,
+                           compute_grads: bool = True):
+        """elbo_step of M independent variational posteriors (the seeds of an experiment) in one call: x [M,B,30,18], y [M,B],
+        mu / sigma [M,P].  Member m is elbo_step(x[m], y[m], mu[m], sigma[m], noise with sample0 + m * particles); injected
+        noise is member-major, particle-minor ([M * particles, ...]).  Returns dict(scalars [M,4] (device, float64: loss,
+        nll_sum, kl, mse), grad_mu, grad_sigma, grad_log_sigma [M,P], out [M,particles,B,2]).  clipped_adam_vi over the
+        [M,P] stacks is elementwise: M independent optimisers."""
+        x = _chk(x, self.device, "x")
+        if x.dim() != 4 or x.shape[2] != WIN_LENGTH or x.shape[3] != N_FEATURES:
+            raise RuntimeError(f"bayesrul_b200: x must be [M,B,{WIN_LENGTH},{N_FEATURES}], got {tuple(x.shape)}")
+        M, B = x.shape[0], x.shape[1]
+        if M == 0 or B == 0:
+            raise RuntimeError("bayesrul_b200: empty ensemble or batch")
+        y = _chk(y, self.device, "y")
+        if tuple(y.shape) != (M, B):
+            raise RuntimeError(f"bayesrul_b200: y must have shape {(M, B)}, got {tuple(y.shape)}")
+        mu, sigma = self._theta(mu, "mu", (M,)), self._theta(sigma, "sigma", (M,))
+        if guide not in GUIDE_IDS:
+            raise RuntimeError("Guide unknown. Choose from 'normal', 'radial'.")
+        if mode is None:
+            mode = "ws"
+        scalars = torch.empty(M, 4, dtype=torch.float64, device=self.device)
+        out = torch.empty(M, particles, B, 2, device=self.device)
+        g = [torch.empty(M, self.P, device=self.device) for _ in range(3)] if compute_grads else [None] * 3
+        ws = self._ws_for(B, M, 4, "simt")
+        nz, keep = self._noise(noise)
+        p = lambda t: t.data_ptr() if t is not None else None
+        _lib.check(self.lib.brl_elbo_step_ensemble(self.ctx, x.data_ptr(), y.data_ptr(), M, B, mu.data_ptr(), sigma.data_ptr(),
+                                                   MODE_IDS[mode], GUIDE_IDS[guide], particles, float(prior_loc),
+                                                   float(prior_scale), int(dataset_size), nz, int(compute_grads),
+                                                   scalars.data_ptr(), p(g[0]), p(g[1]), p(g[2]), out.data_ptr(), ws.data_ptr(),
+                                                   ws.numel(), self._stream()))
+        return dict(scalars=scalars, grad_mu=g[0], grad_sigma=g[1], grad_log_sigma=g[2], out=out)
+
     # -- A13: HNN step -----------------------------------------------------------------------------------
     def hnn_step(self, x, y, theta, p_dropout: float = 0.0, noise: Optional[Noise] = None, compute_grads: bool = True,
                  out_grad: Optional[torch.Tensor] = None):

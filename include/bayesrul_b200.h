@@ -114,7 +114,8 @@ int brl_destroy(brl_ctx* ctx);
  * train == 1 adds the saved activations / gradient buffers of brl_elbo_step / brl_hnn_step (with S >= 2: a second set, so
  * that brl_elbo_step runs two particles side by side on two stream lanes),
  * train == 2 the sign tensors brl_forward generates in BRL_MODE_FLIPOUT when none are injected,
- * train == 3 the buffers of brl_hnn_step_ensemble over S = M members (all of them in one chain of launches where it can) */
+ * train == 3 the buffers of brl_hnn_step_ensemble over S = M members (all of them in one chain of launches where it can),
+ * train == 4 the buffers of brl_elbo_step_ensemble over S = M members (the same, one particle lane of M members) */
 /* 1 when `engine` can run this net's forward on this build, else 0 */
 int brl_engine_available(const brl_ctx* ctx, int engine);
 int64_t brl_workspace_bytes(const brl_ctx* ctx, int64_t B, int64_t S, int train, int engine);
@@ -194,6 +195,28 @@ int brl_elbo_step(brl_ctx* ctx, const float* x, const float* y, int64_t B, const
                   float prior_scale, int64_t dataset_size, const brl_noise* noise, int compute_grads,
                   double* scalars, float* grad_mu, float* grad_sigma, float* grad_log_sigma, float* out,
                   void* workspace, size_t workspace_bytes, void* stream);
+
+/* ---- M independent variational posteriors (the seeds of a BNN experiment) in ONE ELBO step.
+ *      Member m is brl_elbo_step(x + m*B*540, y + m*B, B, mu + m*P, sigma + m*P, mode, guide, particles, prior_loc,
+ *      prior_scale, dataset_size, noise with sample0 + m*particles, ...): mode, guide, particles, prior, dataset size and seed
+ *      are shared; particle pt of member m draws with MC-sample index sample0 + m*particles + pt.  Injected noise is
+ *      member-major, particle-minor (member m's tensors are rows [m*particles, (m+1)*particles)): weight_eps [M*particles,P],
+ *      radial_r [M*particles,n_sites], lrt_eps[l] [M*particles,B,out_elems(l)], flip_in[l] / flip_out[l] [M*particles,B,C].
+ *      Graph-replayed under the same conditions as brl_elbo_step.  brl_clipped_adam_vi over n = M*P is elementwise: M
+ *      independent optimisers.
+ *      Where brl_elbo_step runs the fused Inception kernels (BRL_GEMM_TC_FUSED; LRT, Flipout or weight sampling; B <= 4736)
+ *      and the workspace holds brl_workspace_bytes(B, M, 4), the M members share every launch: one weight-sampler and one
+ *      sign-generator launch per particle for all members, the fused forward / fc / tail / backward / reduction kernels with
+ *      member = blockIdx.z, the finalisation over M*P with per-member KL, and one scalars launch; the particles run one after
+ *      another.  Otherwise (simt / tc back-ends, Linear and Conv-D3 nets, B > 4736, a workspace that holds one member only,
+ *      Flipout with several particles and only some of the sign tensors injected) the members run one after another on
+ *      brl_elbo_step, with the same results.  A workspace below the single-member size returns BRL_ERR_WORKSPACE. */
+int brl_elbo_step_ensemble(brl_ctx* ctx, const float* x /*[M,B,30,18]*/, const float* y /*[M,B]*/, int64_t M, int64_t B,
+                           const float* mu /*[M,P]*/, const float* sigma /*[M,P]*/, int mode, int guide, int particles,
+                           float prior_loc, float prior_scale, int64_t dataset_size, const brl_noise* noise, int compute_grads,
+                           double* scalars /*[M,4] = {loss, nll_sum, kl, mse}*/, float* grad_mu /*[M,P]*/,
+                           float* grad_sigma /*[M,P]*/, float* grad_log_sigma /*[M,P] or NULL*/,
+                           float* out /*[M,particles,B,2]*/, void* workspace, size_t workspace_bytes, void* stream);
 
 /* brl_elbo_step replays a CUDA graph of the step when the noise is native Philox (no injected tensor): the first call with
  * a given configuration (sizes, mode, parameter / workspace pointers) runs eagerly, the second captures it, later calls
