@@ -64,6 +64,7 @@ SIGNATURES = {
     "brl_sample_weights": (_i, [_vp, _vp, _vp, _i, _i64, _np, _vp, _vp, _vp, _sz, _vp]),
     "brl_forward": (_i, [_vp, _vp, _i64, _i64, _i, _vp, _vp, _vp, _f, _np, _vp, _i, _vp, _sz, _vp]),
     "brl_predict_moments": (_i, [_vp, _vp, _i64, _i64, _i, _vp, _vp, _f, _np, _vp, _vp, _vp, _vp, _i, _vp, _sz, _vp]),
+    "brl_predict_moments_ensemble": (_i, [_vp, _vp, _i64, _i64, _i64, _i, _vp, _vp, _f, _np, _vp, _i, _vp, _sz, _vp]),
     "brl_workspace_bytes_host": (_i64, [_vp, _i64, _i64, _i]),
     "brl_predict_moments_host": (_i, [_vp, _vp, _i64, _i64, _i, _vp, _vp, _f, _np, _vp, _i, _vp, _sz, _vp]),
     "brl_moments": (_i, [_vp, _i64, _i64, _vp, _vp, _vp, _vp, _vp]),
@@ -76,6 +77,7 @@ SIGNATURES = {
     "brl_hnn_step_ensemble": (_i, [_vp, _vp, _vp, _i64, _i64, _vp, _f, _np, _i, _vp, _vp, _vp, _vp, _sz, _vp]),
     "brl_mixture_moments": (_i, [_vp, _vp, _i64, _i64, _vp, _vp, _vp]),
     "brl_step_metrics": (_i, [_vp, _vp, _vp, _i64, _vp, _vp, _sz, _vp]),
+    "brl_step_metrics_ensemble": (_i, [_vp, _vp, _vp, _i64, _i64, _vp, _vp, _sz, _vp]),
     "brl_clipped_adam_vi_scaled": (_i, [_vp] * 9 + [_i64, _i64] + [_f] * 8 + [_vp]),
     "brl_test_metrics": (_i, [_vp, _vp, _vp, _i64, _vp, _vp, _sz, _vp]),
     "brl_clipped_adam": (_i, [_vp, _vp, _vp, _vp, _i64, _i64, _f, _f, _f, _f, _f, _f, _f, _vp]),

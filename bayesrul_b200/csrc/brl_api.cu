@@ -930,6 +930,19 @@ int brl_forward(brl_ctx* ctx, const float* x, int64_t B, int64_t S, int mode, co
   return BRL_OK;
 }
 
+// largest chunk of S samples whose brl_predict_moments buffers fit `bytes` of workspace (at most 128 on the fused engine, whose
+// per-sample footprint is 4.8 KB per window -- B = 10 000 x S = 100 is ONE pass over a 4.9 GB feature tensor: measured 4.60 /
+// 4.50 / 4.46 ms per step for 25 / 50 / 100 samples per launch; 16 on the per-layer engines), then equal chunks; 0 when not
+// even one sample fits
+static long long sample_chunk(brl_ctx* ctx, long long B, long long S, int engine, size_t bytes) {
+  static const int env_sc = getenv("BRL_TC_SC") ? atoi(getenv("BRL_TC_SC")) : 0;  // experiment knob
+  long long Sc = std::min<long long>(S, engine == BRL_ENGINE_TC_FP16 ? (env_sc > 0 ? env_sc : 128) : 16);
+  for (; Sc >= 1; --Sc)
+    if ((size_t)brl_workspace_bytes(ctx, B, Sc, 0, engine) <= bytes) break;
+  if (Sc >= 1) Sc = (S + (S + Sc - 1) / Sc - 1) / ((S + Sc - 1) / Sc);
+  return std::max(Sc, 0ll);
+}
+
 int brl_predict_moments(brl_ctx* ctx, const float* x, int64_t B, int64_t S, int guide, const float* mu,
                         const float* sigma, float p_dropout, const brl_noise* noise, float* pred, float* std,
                         float* ep_var, float* al_var, int engine, void* workspace, size_t workspace_bytes, void* stream) {
@@ -941,14 +954,7 @@ int brl_predict_moments(brl_ctx* ctx, const float* x, int64_t B, int64_t S, int 
   cudaStream_t st = (cudaStream_t)stream;
   const NetSpec& n = *ctx->net;
   const int nsites = 2 * (int)n.layers.size();
-  // largest chunk of samples that fits the workspace (at most 128 on the fused engine, whose per-sample footprint is 4.8 KB
-  // per window -- B = 10 000 x S = 100 is ONE pass over a 4.9 GB feature tensor: measured 4.60 / 4.50 / 4.46 ms per step
-  // for 25 / 50 / 100 samples per launch; 16 on the per-layer engines), then equal chunks
-  static const int env_sc = getenv("BRL_TC_SC") ? atoi(getenv("BRL_TC_SC")) : 0;  // experiment knob
-  long long Sc = std::min<long long>(S, engine == BRL_ENGINE_TC_FP16 ? (env_sc > 0 ? env_sc : 128) : 16);
-  for (; Sc >= 1; --Sc)
-    if ((size_t)brl_workspace_bytes(ctx, B, Sc, 0, engine) <= workspace_bytes) break;
-  if (Sc >= 1) Sc = (S + (S + Sc - 1) / Sc - 1) / ((S + Sc - 1) / Sc);
+  const long long Sc = sample_chunk(ctx, B, S, engine, workspace_bytes);
   if (Sc < 1) return fail(BRL_ERR_WORKSPACE, "brl_predict_moments: workspace too small for one MC sample; need " +
                                                  std::to_string(brl_workspace_bytes(ctx, B, 1, 0, engine)) + " bytes");
   Carve c(workspace, workspace_bytes);
@@ -989,6 +995,77 @@ int brl_predict_moments(brl_ctx* ctx, const float* x, int64_t B, int64_t S, int 
     launch_moments_update(outc, sc, B, state, s0 == 0, st);
   }
   launch_moments_final(state, B, pred, std, ep_var, al_var, st);
+  BRL_CUDA(cudaGetLastError());
+  return BRL_OK;
+}
+
+// M members' moments over one batch.  The M S draws form ONE member-major sample axis j = m S + s (MC-sample index sample0 + j,
+// injected noise row j), cut into chunks as brl_predict_moments cuts S.  On the tensor-core engine each chunk is one sampler
+// launch (draw j from member j / S), one pack launch (one image per draw, or per member for MC-dropout / deterministic
+// members), the engine's kernels and one member-routed Welford update; every member's samples go through the same arithmetic
+// as in its own call, whatever chunk they fall in.  Elsewhere the members run one after another on brl_predict_moments.
+int brl_predict_moments_ensemble(brl_ctx* ctx, const float* x, int64_t M, int64_t B, int64_t S, int guide, const float* mu,
+                                 const float* sigma, float p_dropout, const brl_noise* noise, float* out, int engine, void* workspace,
+                                 size_t workspace_bytes, void* stream) {
+  BRL_REQUIRE(ctx && x && mu && out && workspace, "brl_predict_moments_ensemble: NULL argument");
+  DeviceGuard dg(ctx->device);
+  BRL_REQUIRE(M > 0 && M < (1 << 16) && B > 0 && S > 0 && B * 30 < (1ll << 31) / 512 && S < (1ll << 31) / M,
+              "brl_predict_moments_ensemble: bad M, B or S");
+  BRL_REQUIRE(p_dropout >= 0.f && p_dropout < 1.f, "brl_predict_moments_ensemble: p_dropout must be in [0,1)");
+  BRL_REQUIRE(guide < 0 || sigma, "brl_predict_moments_ensemble: sigma is NULL");
+  BRL_REQUIRE(guide <= BRL_GUIDE_RADIAL, "Guide unknown. Choose from 'normal', 'radial'.");
+  cudaStream_t st = (cudaStream_t)stream;
+  const NetSpec& n = *ctx->net;
+  const size_t state_bytes = ((size_t)(M * 4 * B) * sizeof(float) + 255) & ~(size_t)255;  // Welford state [M,4,B]
+  const size_t need = (size_t)brl_workspace_bytes(ctx, B, 1, 0, engine) + state_bytes;
+  if (workspace_bytes < need)
+    return fail(BRL_ERR_WORKSPACE, "brl_predict_moments_ensemble: workspace too small; need " + std::to_string(need) + " bytes");
+  brl_noise base;
+  memset(&base, 0, sizeof(base));
+  if (noise) base = *noise;
+  // the Linear and Conv-D3 tensor-core engines have no dropout path: their members run (and fail) as single calls
+  const bool batched = engine == BRL_ENGINE_TC_FP16 && tc_available(ctx->tc) && (p_dropout == 0.f || n.id == BRL_NET_INCEPTION);
+  if (!batched) {
+    for (int64_t m = 0; m < M; ++m) {
+      const brl_noise nm = noise_at_sample(n, &base, m * S, B);  // MC-sample index sample0 + m S, injected rows of member m
+      const int rc = brl_predict_moments(ctx, x, B, S, guide, mu + m * n.P, guide >= 0 ? sigma + m * n.P : nullptr, p_dropout, &nm,
+                                         out + m * B, out + (M + m) * B, out + (2 * M + m) * B, out + (3 * M + m) * B, engine,
+                                         workspace, workspace_bytes, stream);
+      if (rc != BRL_OK) return rc;
+    }
+    return BRL_OK;
+  }
+  const long long T = M * S;
+  const long long Sc = sample_chunk(ctx, B, T, engine, workspace_bytes - state_bytes);
+  const int nsites = 2 * (int)n.layers.size();
+  Carve c(workspace, workspace_bytes);
+  float* state = c.take<float>(M * 4 * B);
+  float* wsamp = c.take<float>(Sc * n.P);
+  float* norms = c.take<float>(Sc * nsites);
+  float* outc = c.take<float>(Sc * B * 2);
+  const size_t tc_bytes = tc_workspace_bytes(ctx->tc, B, Sc);
+  void* tc_ws = c.take<char>((long long)tc_bytes);
+  if (Sc < 1 || !c.ok) return fail(BRL_ERR_WORKSPACE, "brl_predict_moments_ensemble: workspace carve failed");
+  for (long long j0 = 0; j0 < T; j0 += Sc) {
+    const long long sc = std::min(Sc, T - j0), m0 = j0 / S, phase = j0 - m0 * S;  // the chunk starts `phase` samples into member m0
+    brl_noise nz = noise_at_sample(n, &base, j0, B);
+    const char* err;
+    if (guide >= 0) {
+      NoiseRef eps = nref(&nz, nz.weight_eps, KIND_WEIGHT_EPS, 0);
+      if (guide == BRL_GUIDE_NORMAL)
+        launch_sample_normal(mu + m0 * n.P, sigma + m0 * n.P, n.P, sc, eps, wsamp, nullptr, st, n.P, 1, (int)S, (int)phase);
+      else
+        launch_sample_radial(mu + m0 * n.P, sigma + m0 * n.P, n.P, sc, ctx->site_off_dev, nsites, ctx->max_site, eps,
+                             nref(&nz, nz.radial_r, KIND_RADIAL_R, 0), norms, wsamp, nullptr, st, n.P, 1, (int)S, (int)phase);
+      err = tc_forward(ctx->tc, x, B, sc, wsamp, n.P, p_dropout, &nz, outc, tc_ws, tc_bytes, j0 == 0, st);
+    } else {  // one image per member: draw j reads image j / S of the members from m0 on
+      err = tc_forward(ctx->tc, x, B, sc, mu + m0 * n.P, n.P, p_dropout, &nz, outc, tc_ws, tc_bytes, j0 == 0, st, nullptr, (int)S,
+                       (int)phase);
+    }
+    if (err) return fail(BRL_ERR_UNSUPPORTED, err);
+    launch_moments_update_members(outc, j0, sc, S, B, state, st);
+  }
+  launch_moments_final_members(state, M, B, out, st);
   BRL_CUDA(cudaGetLastError());
   return BRL_OK;
 }
@@ -1811,6 +1888,16 @@ int brl_step_metrics(const float* pred, const float* std, const float* y, int64_
   BRL_REQUIRE(pred && std && y && scalars && workspace && nn > 0, "brl_step_metrics: bad argument");
   if (workspace_bytes < 1024) return fail(BRL_ERR_WORKSPACE, "brl_step_metrics: workspace must be >= 1024 bytes");
   launch_test_metrics(pred, std, y, nn, scalars, (unsigned int*)workspace, (cudaStream_t)stream, 5);
+  BRL_CUDA(cudaGetLastError());
+  return BRL_OK;
+}
+
+int brl_step_metrics_ensemble(const float* pred, const float* std, const float* y, int64_t M, int64_t nn, double* scalars,
+                              void* workspace, size_t workspace_bytes, void* stream) {
+  BRL_REQUIRE(pred && std && y && scalars && workspace && M > 0 && M < (1 << 16) && nn > 0, "brl_step_metrics_ensemble: bad argument");
+  if (workspace_bytes < (size_t)M * 1024)
+    return fail(BRL_ERR_WORKSPACE, "brl_step_metrics_ensemble: workspace must be >= M x 1024 bytes");
+  launch_test_metrics(pred, std, y, nn, scalars, (unsigned int*)workspace, (cudaStream_t)stream, 5, (int)M);
   BRL_CUDA(cudaGetLastError());
   return BRL_OK;
 }

@@ -161,11 +161,11 @@ void launch_bwd_act(const BwdAct& p, cudaStream_t st) {
 // ------------------------------------------------------------------------------------------------
 __global__ void sample_normal_kernel(const float* __restrict__ mu, const float* __restrict__ sigma, long long P,
                                      NoiseRef eps, float* __restrict__ w, float* __restrict__ delta, long long mu_stride,
-                                     int sample_stride) {
+                                     int sample_stride, int per, int phase) {
   const long long nblk = (P + 3) >> 2;
   const int s = blockIdx.y, se = s * sample_stride;  // draw s: MC-sample index / injected row sample0 + se
-  mu += s * mu_stride;
-  sigma += s * mu_stride;
+  mu += (long long)((s + phase) / per) * mu_stride;
+  sigma += (long long)((s + phase) / per) * mu_stride;
   for (long long blk = blockIdx.x * (long long)blockDim.x + threadIdx.x; blk < nblk; blk += (long long)gridDim.x * blockDim.x) {
     float z[4];
     const long long e0 = blk << 2;
@@ -188,11 +188,11 @@ __global__ void sample_normal_kernel(const float* __restrict__ mu, const float* 
   }
 }
 void launch_sample_normal(const float* mu, const float* sigma, long long P, long long S, NoiseRef eps, float* w,
-                          float* delta, cudaStream_t st, long long mu_stride, int sample_stride) {
+                          float* delta, cudaStream_t st, long long mu_stride, int sample_stride, int per, int phase) {
   const long long nblk = (P + 3) >> 2;
   dim3 grid((unsigned)min((nblk + 255) / 256, (long long)148 * 8), (unsigned)S);
   ++g_launch_count;
-  sample_normal_kernel<<<grid, 256, 0, st>>>(mu, sigma, P, eps, w, delta, mu_stride, sample_stride);
+  sample_normal_kernel<<<grid, 256, 0, st>>>(mu, sigma, P, eps, w, delta, mu_stride, sample_stride, per, phase);
 }
 
 // The radial guide needs ||eps|| over each whole site before any weight of the site exists, so the draw is two passes over
@@ -228,10 +228,10 @@ __global__ void radial_norm_kernel(long long P, const long long* __restrict__ si
 __global__ void radial_apply_kernel(const float* __restrict__ mu, const float* __restrict__ sigma, long long P,
                                     const long long* __restrict__ site_off, int n_sites, NoiseRef eps, NoiseRef r,
                                     const float* __restrict__ norms, float* __restrict__ w, float* __restrict__ delta,
-                                    long long mu_stride, int sample_stride) {
+                                    long long mu_stride, int sample_stride, int per, int phase) {
   const int s = blockIdx.y, se = s * sample_stride;
-  mu += s * mu_stride;
-  sigma += s * mu_stride;
+  mu += (long long)((s + phase) / per) * mu_stride;
+  sigma += (long long)((s + phase) / per) * mu_stride;
   const long long nblk = (P + 3) >> 2;
   const NoiseKey k = noise_key(eps), rk = noise_key(r);
   for (long long blk = blockIdx.x * (long long)blockDim.x + threadIdx.x; blk < nblk; blk += (long long)gridDim.x * blockDim.x) {
@@ -265,13 +265,13 @@ __global__ void radial_apply_kernel(const float* __restrict__ mu, const float* _
 }
 void launch_sample_radial(const float* mu, const float* sigma, long long P, long long S, const long long* site_off,
                           int n_sites, int max_site, NoiseRef eps, NoiseRef r, float* norms, float* w, float* delta,
-                          cudaStream_t st, long long mu_stride, int sample_stride) {
+                          cudaStream_t st, long long mu_stride, int sample_stride, int per, int phase) {
   ++g_launch_count;
   radial_norm_kernel<<<dim3(n_sites, (unsigned)S), 256, 0, st>>>(P, site_off, n_sites, eps, norms, sample_stride);
   ++g_launch_count;
   const long long nblk = (P + 3) >> 2;
   radial_apply_kernel<<<dim3((unsigned)min((nblk + 255) / 256, (long long)148 * 8), (unsigned)S), 256, 0, st>>>(
-      mu, sigma, P, site_off, n_sites, eps, r, norms, w, delta, mu_stride, sample_stride);
+      mu, sigma, P, site_off, n_sites, eps, r, norms, w, delta, mu_stride, sample_stride, per, phase);
 }
 
 __global__ void gen_signs_kernel(float* dst, long long S, long long B, int C, NoiseRef nz) {
@@ -512,6 +512,71 @@ void launch_moments_final(const float* state, long long B, float* pred, float* s
   moments_final_kernel<<<(unsigned)min((B + 255) / 256, (long long)148 * 8), 256, 0, st>>>(state, B, pred, std, ep, al);
 }
 
+// Samples [j0, j0 + sc) of the member-major sample axis j = m S + s of brl_predict_moments_ensemble (out [sc,B,2]): member
+// m = j0 / S + blockIdx.y takes its segment of the chunk, a sequential Welford into its own state [4,B] in the arithmetic
+// order of moments_update_kernel (a member whose first sample is in the chunk starts from zero)
+__global__ void moments_update_members_kernel(const float* __restrict__ out, long long j0, long long sc, long long S, long long B,
+                                              float* state /*[M,4,B]*/) {
+  const long long m = j0 / S + blockIdx.y;
+  const long long lo = max(j0, m * S), hi = min(j0 + sc, (m + 1) * S), ns = hi - lo;
+  const bool first = lo == m * S;
+  out += (lo - j0) * B * 2;
+  state += m * 4 * B;
+  for (long long b = blockIdx.x * (long long)blockDim.x + threadIdx.x; b < B; b += (long long)gridDim.x * blockDim.x) {
+    float n = 0.f, mean = 0.f, m2 = 0.f, s2 = 0.f;
+    if (!first) { n = state[b]; mean = state[B + b]; m2 = state[2 * B + b]; s2 = state[3 * B + b]; }
+    long long s = 0;
+    for (; s + 16 <= ns; s += 16) {
+      float2 o[16];
+#pragma unroll
+      for (int u = 0; u < 16; ++u) o[u] = __ldcs(reinterpret_cast<const float2*>(out + ((s + u) * B + b) * 2));
+#pragma unroll
+      for (int u = 0; u < 16; ++u) {
+        n += 1.f;
+        const float d = o[u].x - mean;
+        mean += d / n;
+        m2 = fmaf(d, o[u].x - mean, m2);
+        s2 = fmaf(o[u].y, o[u].y, s2);
+      }
+    }
+    for (; s < ns; ++s) {
+      const float2 o = *reinterpret_cast<const float2*>(out + (s * B + b) * 2);
+      n += 1.f;
+      const float d = o.x - mean;
+      mean += d / n;
+      m2 = fmaf(d, o.x - mean, m2);
+      s2 = fmaf(o.y, o.y, s2);
+    }
+    state[b] = n; state[B + b] = mean; state[2 * B + b] = m2; state[3 * B + b] = s2;
+  }
+}
+void launch_moments_update_members(const float* out, long long j0, long long sc, long long S, long long B, float* state,
+                                   cudaStream_t st) {
+  const long long members = (j0 + sc - 1) / S - j0 / S + 1;
+  ++g_launch_count;
+  moments_update_members_kernel<<<dim3((unsigned)min((B + 127) / 128, (long long)148 * 8), (unsigned)members), 128, 0, st>>>(
+      out, j0, sc, S, B, state);
+}
+// state [M,4,B] -> out [4,M,B] = (pred, std, ep_var, al_var), the arithmetic of moments_final_kernel
+__global__ void moments_final_members_kernel(const float* __restrict__ state, long long M, long long B, float* out) {
+  const long long MB = M * B;
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < MB; i += (long long)gridDim.x * blockDim.x) {
+    const long long m = i / B, b = i % B;
+    const float* st = state + m * 4 * B;
+    const float n = st[b];
+    const float e = st[2 * B + b] / (n - 1.f);
+    const float a = st[3 * B + b] / n;
+    out[i] = st[B + b];
+    out[2 * MB + i] = e;
+    out[3 * MB + i] = a;
+    out[MB + i] = sqrtf(a + e);
+  }
+}
+void launch_moments_final_members(const float* state, long long M, long long B, float* out, cudaStream_t st) {
+  ++g_launch_count;
+  moments_final_members_kernel<<<(unsigned)min((M * B + 255) / 256, (long long)148 * 8), 256, 0, st>>>(state, M, B, out);
+}
+
 __global__ void moments_direct_kernel(const float* __restrict__ out, long long S, long long B, float* pred, float* std,
                                       float* ep, float* al) {
   for (long long b = blockIdx.x * (long long)blockDim.x + threadIdx.x; b < B; b += (long long)gridDim.x * blockDim.x) {
@@ -581,8 +646,15 @@ void launch_mixture(const float* mu_m, const float* sd_m, long long M, long long
 // ------------------------------------------------------------------------------------------------
 // test-time scalar metrics (bayesian.py:217-224; results/metrics.py:210-274)
 // ------------------------------------------------------------------------------------------------
+// member m = blockIdx.y (grid.y = M) of [M,n] inputs: its scratch is the m-th 1024 bytes (hist[100] u32, acc[3] doubles at +512 B)
 __global__ void test_metrics_acc_kernel(const float* __restrict__ pred, const float* __restrict__ std,
-                                        const float* __restrict__ y, long long n, double* acc, unsigned int* hist) {
+                                        const float* __restrict__ y, long long n, unsigned int* hist) {
+  const long long m = blockIdx.y;
+  pred += m * n;
+  std += m * n;
+  y += m * n;
+  hist += m * 256;
+  double* acc = reinterpret_cast<double*>(hist + 128);
   __shared__ unsigned int sh[100];
   for (int i = threadIdx.x; i < 100; i += blockDim.x) sh[i] = 0;
   __syncthreads();
@@ -607,8 +679,11 @@ __global__ void test_metrics_acc_kernel(const float* __restrict__ pred, const fl
   for (int i = threadIdx.x; i < 100; i += blockDim.x)
     if (sh[i]) atomicAdd(hist + i, sh[i]);
 }
-__global__ void test_metrics_final_kernel(const double* acc, const unsigned int* hist, long long n, double* scalars, int nscal) {
+__global__ void test_metrics_final_kernel(const unsigned int* hist, long long n, double* scalars, int nscal) {  // member = blockIdx.x
   if (threadIdx.x != 0) return;
+  hist += blockIdx.x * 256ll;
+  scalars += blockIdx.x * (long long)nscal;
+  const double* acc = reinterpret_cast<const double*>(hist + 128);
   scalars[0] = acc[0] / (double)n;
   scalars[1] = acc[1] / (double)n;
   scalars[2] = sqrt(acc[2] / (double)n);
@@ -623,14 +698,14 @@ __global__ void test_metrics_final_kernel(const double* acc, const unsigned int*
   if (nscal > 4) scalars[4] = ab / 100.0;  // mean absolute calibration error (results/metrics.py:277-297)
 }
 void launch_test_metrics(const float* pred, const float* std, const float* y, long long n, double* scalars,
-                         unsigned int* hist, cudaStream_t st, int nscal) {
-  // workspace layout: hist[100] u32 followed (at +512 B) by acc[3] doubles
-  double* acc = reinterpret_cast<double*>(reinterpret_cast<char*>(hist) + 512);
-  cudaMemsetAsync(hist, 0, 512 + 3 * sizeof(double), st);
+                         unsigned int* hist, cudaStream_t st, int nscal, int members) {
+  // workspace layout, 1024 bytes per member: hist[100] u32 followed (at +512 B) by acc[3] doubles
+  cudaMemsetAsync(hist, 0, (size_t)(members - 1) * 1024 + 512 + 3 * sizeof(double), st);
   ++g_launch_count;
-  test_metrics_acc_kernel<<<(unsigned)min((n + 255) / 256, (long long)148 * 4), 256, 0, st>>>(pred, std, y, n, acc, hist);
+  test_metrics_acc_kernel<<<dim3((unsigned)min((n + 255) / 256, (long long)148 * 4), (unsigned)members), 256, 0, st>>>(pred, std, y, n,
+                                                                                                                   hist);
   ++g_launch_count;
-  test_metrics_final_kernel<<<1, 32, 0, st>>>(acc, hist, n, scalars, nscal);
+  test_metrics_final_kernel<<<members, 32, 0, st>>>(hist, n, scalars, nscal);
 }
 
 // ------------------------------------------------------------------------------------------------

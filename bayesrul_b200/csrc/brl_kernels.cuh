@@ -143,13 +143,17 @@ struct BwdAct {
 };
 void launch_bwd_act(const BwdAct& p, cudaStream_t st);
 
-// S draws [S,P]: draw s reads mu / sigma + s mu_stride (0: S draws of one posterior; P: one draw from each of S posteriors, the
-// members of an ensemble step) and MC-sample index / injected noise row sample0 + s sample_stride
+// S draws [S,P]: draw s reads mu / sigma + ((s + phase) / per) mu_stride (mu_stride 0: S draws of one posterior; P with per 1:
+// one draw from each of S posteriors, the members of an ensemble step; P with per > 1: `per` draws per posterior, the first
+// posterior already `phase` draws in, a chunk of the member-major sample axis of brl_predict_moments_ensemble) and MC-sample
+// index / injected noise row sample0 + s sample_stride
 void launch_sample_normal(const float* mu, const float* sigma, long long P, long long S, NoiseRef eps, float* w,
-                          float* delta, cudaStream_t st, long long mu_stride = 0, int sample_stride = 1);
+                          float* delta, cudaStream_t st, long long mu_stride = 0, int sample_stride = 1, int per = 1,
+                          int phase = 0);
 void launch_sample_radial(const float* mu, const float* sigma, long long P, long long S, const long long* site_off,
                           int n_sites, int max_site, NoiseRef eps, NoiseRef r, float* norms /*[S,n_sites]*/, float* w,
-                          float* delta, cudaStream_t st, long long mu_stride = 0, int sample_stride = 1);
+                          float* delta, cudaStream_t st, long long mu_stride = 0, int sample_stride = 1, int per = 1,
+                          int phase = 0);
 void launch_gen_signs(float* dst, long long S, long long B, int C, NoiseRef nz, cudaStream_t st);
 // all sign tensors of one particle in ONE launch (a Flipout step needs 2 per layer): job j fills dst[j][B][C[j]] with stream
 // (kind[j], site[j]) of the key in `base`; with `members` > 1, member m fills dst[j][m][B][C[j]] with MC-sample index
@@ -191,13 +195,19 @@ void launch_moments_update(const float* out, long long S, long long B, float* st
                            cudaStream_t st);
 void launch_moments_final(const float* state, long long B, float* pred, float* std, float* ep, float* al,
                           cudaStream_t st);
+// brl_predict_moments_ensemble: the Welford update of samples [j0, j0 + sc) of the member-major sample axis j = m S + s (out
+// [sc,B,2]) into state [M,4,B], and the final moments of all members, out [4,M,B] = (pred, std, ep_var, al_var)
+void launch_moments_update_members(const float* out, long long j0, long long sc, long long S, long long B, float* state,
+                                   cudaStream_t st);
+void launch_moments_final_members(const float* state, long long M, long long B, float* out, cudaStream_t st);
 void launch_moments_direct(const float* out, long long S, long long B, float* pred, float* std, float* ep, float* al,
                            cudaStream_t st);
 void launch_aggregate(const float* out, long long S, long long B, float* agg, cudaStream_t st);
 void launch_mixture(const float* mu_m, const float* sd_m, long long M, long long n, float* mu, float* sd,
                     cudaStream_t st);
+// members > 1: row m of pred / std / y [members,n] -> scalars + m nscal, with the m-th 1024 bytes of the scratch at `hist`
 void launch_test_metrics(const float* pred, const float* std, const float* y, long long n, double* scalars,
-                         unsigned int* hist, cudaStream_t st, int nscal = 4);
+                         unsigned int* hist, cudaStream_t st, int nscal = 4, int members = 1);
 void launch_clipped_adam(float* p, const float* g, float* m, float* v, long long n, float step_size, float b1,
                          float b2, float eps, float clip, float wd, cudaStream_t st);
 void launch_clipped_adam_vi(float* loc, float* ls, float* scale, const float* g_loc, const float* g_ls, float* m_loc, float* v_loc,

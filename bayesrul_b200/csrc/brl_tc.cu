@@ -209,6 +209,7 @@ constexpr int PACK_THREADS_TOTAL = 12 * 1024 + 144 * 128 + 32 * 128 + 3 * 1024 +
 struct FcArgs {
   const unsigned char* blob;
   long long blob_stride;
+  int img_per, img_phase;  // MC sample s reads image (s + img_phase) / img_per (ConvArgs)
   float* out;  // [S,B,2]
   int B, S, ntile128;  // feature rows per sample = ntile128 * 128
   float keep;  // dropout keep of the fc site
@@ -257,7 +258,7 @@ __global__ void __launch_bounds__(192, 1) tc_fc_kernel(const FcArgs a, const __g
       for (long long it = blockIdx.x; it < total && ok; it += gridDim.x) {
         const int s = (int)(it / a.ntile128);
         const int row0 = (int)(it * 128);  // == (s * ntile128 + tile) * 128: rows of the [S * Bpad, 2400] feature matrix
-        const unsigned char* gb = a.blob + (long long)s * a.blob_stride + BLOB_FC;
+        const unsigned char* gb = a.blob + (long long)((s + a.img_phase) / a.img_per) * a.blob_stride + BLOB_FC;
         for (int kb = 0; kb < NKB && ok; ++kb) {
           ok = mbar_wait(bars + 48 + 8 * stage, ph, a.status, 10);
           const uint32_t dst = sbase + stage * FC_STAGE_BYTES;
@@ -296,7 +297,7 @@ __global__ void __launch_bounds__(192, 1) tc_fc_kernel(const FcArgs a, const __g
     bool ok = true;
     for (long long it = blockIdx.x; it < total && ok; it += gridDim.x) {
       const int s = (int)(it / a.ntile128), tile = (int)(it % a.ntile128);
-      const float* tail = reinterpret_cast<const float*>(a.blob + (long long)s * a.blob_stride + BLOB_TAIL);
+      const float* tail = reinterpret_cast<const float*>(a.blob + (long long)((s + a.img_phase) / a.img_per) * a.blob_stride + BLOB_TAIL);
       ok = mbar_wait(bars + 96 + 8 * acc_i, aph, a.status, 13);
       tc_fence_after();
       float acc[4][16];
@@ -454,7 +455,7 @@ static TmaEncodeFn tma_encode_fn() {
 
 // Linear net: windows -> fp16 matrix, weights -> fp16 images, one persistent launch (brl_tc_linear.cuh)
 static const char* tcl_forward(TcState* st, const float* x, long long B, long long S, const float* weights, long long w_sample_stride,
-                               float p_dropout, float* out, void* ws, bool pack_x, cudaStream_t stream) {
+                               float p_dropout, float* out, void* ws, bool pack_x, cudaStream_t stream, int img_per, int img_phase) {
   if (p_dropout > 0.f) return "bayesrul_b200: the Linear net's tensor-core engine has no dropout path (use engine 'simt')";
   const long long nt128 = (B + 127) / 128, Bpad = nt128 * 128;
   unsigned char* x16 = reinterpret_cast<unsigned char*>(ws);
@@ -466,7 +467,7 @@ static const char* tcl_forward(TcState* st, const float* x, long long B, long lo
   LinPackArgs pa;
   pa.w = weights; pa.w_stride = w_sample_stride; pa.img = img;
   for (int l = 0; l < 5; ++l) { pa.w_off[l] = st->loff[l][0]; pa.b_off[l] = st->loff[l][1]; }
-  const long long nimg = w_sample_stride ? S : 1;
+  const long long nimg = w_sample_stride ? (img_phase + S - 1) / img_per + 1 : 1;
   tcl_pack_kernel<<<dim3((lin::IMG_HALVES + lin::TAIL_FLOATS + 255) / 256, (unsigned)nimg), 256, 0, stream>>>(pa);
   CUtensorMap xmap;
   {
@@ -481,7 +482,7 @@ static const char* tcl_forward(TcState* st, const float* x, long long B, long lo
       return "bayesrul_b200: cuTensorMapEncodeTiled failed for the window matrix";
   }
   LinArgs la;
-  la.img = img; la.img_stride = w_sample_stride ? lin::IMG_BYTES : 0; la.out = out;
+  la.img = img; la.img_stride = w_sample_stride ? lin::IMG_BYTES : 0; la.img_per = img_per; la.img_phase = img_phase; la.out = out;
   la.B = (int)B; la.S = (int)S; la.ntile128 = (int)nt128; la.status = st->status;
   const int grid = (int)std::min<long long>(st->sm_count, S * nt128);
   tcl_kernel<<<grid, 128, lin::SMEM, stream>>>(la, xmap);
@@ -491,7 +492,7 @@ static const char* tcl_forward(TcState* st, const float* x, long long B, long lo
 
 // Conv-D3 net: windows -> per-tile fp16 images, weights -> fp16 images, one persistent launch (brl_tc_convd3.cuh)
 static const char* tcc_forward(TcState* st, const float* x, long long B, long long S, const float* weights, long long w_sample_stride,
-                               float p_dropout, float* out, void* ws, bool pack_x, cudaStream_t stream) {
+                               float p_dropout, float* out, void* ws, bool pack_x, cudaStream_t stream, int img_per, int img_phase) {
   if (p_dropout > 0.f) return "bayesrul_b200: the Conv-D3 net's tensor-core engine has no dropout path (use engine 'simt')";
   const long long ntile = (B + 3) / 4;
   unsigned char* ximg = reinterpret_cast<unsigned char*>(ws);
@@ -503,10 +504,11 @@ static const char* tcc_forward(TcState* st, const float* x, long long B, long lo
   Cd3PackArgs pa;
   pa.w = weights; pa.w_stride = w_sample_stride; pa.img = img;
   for (int l = 0; l < 4; ++l) { pa.w_off[l] = st->loff[l][0]; pa.b_off[l] = st->loff[l][1]; }
-  const long long nimg = w_sample_stride ? S : 1;
+  const long long nimg = w_sample_stride ? (img_phase + S - 1) / img_per + 1 : 1;
   tcc_pack_kernel<<<dim3((cd3::IMG_HALVES + cd3::TAIL_FLOATS + 255) / 256, (unsigned)nimg), 256, 0, stream>>>(pa);
   Cd3Args ca;
-  ca.ximg = ximg; ca.img = img; ca.img_stride = w_sample_stride ? cd3::IMG_BYTES : 0; ca.out = out;
+  ca.ximg = ximg; ca.img = img; ca.img_stride = w_sample_stride ? cd3::IMG_BYTES : 0; ca.img_per = img_per; ca.img_phase = img_phase;
+  ca.out = out;
   ca.B = (int)B; ca.S = (int)S; ca.ntile = (int)ntile; ca.status = st->status;
   const int grid = (int)std::min<long long>(2ll * st->sm_count, S * ntile);
   tcc_kernel<<<grid, 128, cd3::SMEM, stream>>>(ca);
@@ -516,23 +518,23 @@ static const char* tcc_forward(TcState* st, const float* x, long long B, long lo
 
 const char* tc_forward(TcState* st, const float* x, long long B, long long S, const float* weights, long long w_sample_stride,
                        float p_dropout, const brl_noise* noise, float* out, void* ws, size_t ws_bytes, bool pack_x,
-                       cudaStream_t stream, const unsigned char* prepacked) {
+                       cudaStream_t stream, const unsigned char* prepacked, int img_per, int img_phase) {
   if (!tc_available(st)) return "bayesrul_b200: tensor-core engine unavailable (no sm_100 context)";
   if (ws_bytes < tc_workspace_bytes(st, B, S)) return "bayesrul_b200: workspace too small for the tensor-core engine";
   if (st->net == BRL_NET_LINEAR) {
     if (prepacked) return "bayesrul_b200: prepacked weight images are implemented for the Inception net only";
-    return tcl_forward(st, x, B, S, weights, w_sample_stride, p_dropout, out, ws, pack_x, stream);
+    return tcl_forward(st, x, B, S, weights, w_sample_stride, p_dropout, out, ws, pack_x, stream, img_per, img_phase);
   }
   if (st->net == BRL_NET_CONV) {
     if (prepacked) return "bayesrul_b200: prepacked weight images are implemented for the Inception net only";
-    return tcc_forward(st, x, B, S, weights, w_sample_stride, p_dropout, out, ws, pack_x, stream);
+    return tcc_forward(st, x, B, S, weights, w_sample_stride, p_dropout, out, ws, pack_x, stream, img_per, img_phase);
   }
   const long long nt128 = (B + 127) / 128, nt4 = (B + 3) / 4;
   // workspace: window images (independent of S, so later sample chunks of a batch find them again) | blobs | features
   const int ntx = (int)((nt4 + 1) / 2 * 2);
   unsigned char* ximg = reinterpret_cast<unsigned char*>(ws);
   unsigned char* blob = ximg + (((long long)ntx * XIMG_TILE_BYTES + 255) / 256) * 256;
-  const long long nblob = w_sample_stride ? S : 1;
+  const long long nblob = w_sample_stride ? (img_phase + S - 1) / img_per + 1 : 1;
   unsigned char* feat = blob + ((S * (long long)BLOB_BYTES + 255) / 256) * 256;
   if (pack_x) {  // the windows are shared by all MC samples: their fp16 chunk images are built once per batch
     tc_packx_kernel<<<(unsigned)(((long long)ntx * 384 + 255) / 256), 256, 0, stream>>>(x, ximg, (int)B, ntx);
@@ -560,6 +562,7 @@ const char* tc_forward(TcState* st, const float* x, long long B, long long S, co
   };
   ConvArgs ca;
   ca.ximg = ximg; ca.blob = blob; ca.blob_stride = w_sample_stride ? BLOB_BYTES : 0; ca.feat = feat;
+  ca.img_per = img_per; ca.img_phase = img_phase;
   ca.B = (int)B; ca.S = (int)S; ca.ntile4 = (int)nt4; ca.ntile128 = (int)nt128;
   ca.keep4 = drop ? 1.0f - p_dropout * 0.25f : 1.0f;
   for (int l = 0; l < 12; ++l) ca.drop[l] = nr(l);
@@ -585,7 +588,7 @@ const char* tc_forward(TcState* st, const float* x, long long B, long long S, co
   else tc_conv_kernel<false><<<grid, CONV_THREADS, CONV_SMEM, stream>>>(ca);
   tc_time_end(st, 0, stream);
   FcArgs fa;
-  fa.blob = blob; fa.blob_stride = ca.blob_stride; fa.out = out;
+  fa.blob = blob; fa.blob_stride = ca.blob_stride; fa.img_per = img_per; fa.img_phase = img_phase; fa.out = out;
   fa.B = (int)B; fa.S = (int)S; fa.ntile128 = (int)nt128;
   fa.keep = drop ? 1.0f - p_dropout : 1.0f;
   fa.drop = nr(10);

@@ -20,9 +20,12 @@ size_t tc_workspace_bytes(const TcState*, long long B, long long S);
 // call built in the same workspace for the same x (later chunks of MC samples of one batch).
 // prepacked != nullptr: the fp16 weight images of the S samples (tc_pack_weights) are taken from there instead of being
 // packed from `weights` into the workspace (window chunks of one batch share the images of all MC samples).
+// With w_sample_stride != 0, MC sample s uses weight row / image (s + img_phase) / img_per: img_per = 1 is one image per sample;
+// img_per = S serves the samples of several ensemble members (S each, the first member img_phase samples in) from one image per
+// member.  w_sample_stride == 0: one image shared by all samples.
 const char* tc_forward(TcState*, const float* x, long long B, long long S, const float* weights, long long w_sample_stride,
                        float p_dropout, const brl_noise* noise, float* out, void* ws, size_t ws_bytes, bool pack_x,
-                       cudaStream_t st, const unsigned char* prepacked = nullptr);
+                       cudaStream_t st, const unsigned char* prepacked = nullptr, int img_per = 1, int img_phase = 0);
 size_t tc_weight_image_bytes();  // bytes of one sample's fp16 weight image
 // fp32 weights [n, P] (or one shared [P] vector: n = 1) -> n fp16 weight images at `images` (tc_weight_image_bytes() apart).
 // The images depend on p_dropout (inverted dropout's 1 / keep is folded into the weights behind a dropout site): pass the value

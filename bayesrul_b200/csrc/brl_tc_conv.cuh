@@ -28,8 +28,9 @@
 
 struct ConvArgs {
   const unsigned char* ximg;  // [2 * npair][X0 X1 X2 XP0 XP1 XP2][132 rows][16 B]  (tc_packx_kernel)
-  const unsigned char* blob;  // [S or 1][BLOB_BYTES]
+  const unsigned char* blob;  // [images][BLOB_BYTES]: MC sample s reads image (s + img_phase) / img_per
   long long blob_stride;      // BLOB_BYTES or 0
+  int img_per, img_phase;     // 1, 0: one image per sample; S, phase: one image per ensemble member of S samples
   unsigned char* feat;        // row-major [S][ntile128 * 128 windows][10 chunks][30 steps][8 fp16] (= [.., 2400] for the fc GEMM)
   int B, S, ntile4, ntile128;
   float keep4;                // dropout keep of the branch sites (1 = off)
@@ -263,7 +264,7 @@ __global__ void __launch_bounds__(CONV_THREADS, 1) tc_conv_kernel(const ConvArgs
         const uint64_t pol = l2_policy_evict_last();
         auto load_w = [&](int s) {
           if (elect_one()) {
-            const unsigned char* src = a.blob + (long long)s * a.blob_stride;
+            const unsigned char* src = a.blob + (long long)((s + a.img_phase) / a.img_per) * a.blob_stride;
             mbar_expect_tx(bars + BAR_W, CONV_IMG);
             for (int o = 0; o < CONV_IMG; o += 16384) bulk_g2s_hint(sbase + OFF_W + o, src + o, min(16384, CONV_IMG - o), bars + BAR_W, pol);
           }

@@ -100,6 +100,7 @@ struct Cd3Args {
   const unsigned char* ximg;  // [ntile][XQ_BYTES]
   const unsigned char* img;
   long long img_stride;
+  int img_per, img_phase;  // MC sample s reads image (s + img_phase) / img_per
   float* out;  // [S,B,2]
   int B, S, ntile;
   int* status;
@@ -155,7 +156,7 @@ __global__ void __launch_bounds__(128, 2) tcc_kernel(const Cd3Args a) {
         const bool neww = s != s_loaded;
         mbar_expect_tx(bar_full, XQ_BYTES + (neww ? IMG_BYTES : 0));
         cd3_bulk(xs, a.ximg + (long long)tile * XQ_BYTES, XQ_BYTES, bar_full);
-        if (neww) cd3_bulk(ws, a.img + (long long)s * a.img_stride, IMG_BYTES, bar_full);
+        if (neww) cd3_bulk(ws, a.img + (long long)((s + a.img_phase) / a.img_per) * a.img_stride, IMG_BYTES, bar_full);
       }
       ok = mbar_wait(bar_full, fph, a.status, 30) && ok;
       tc_fence_after();

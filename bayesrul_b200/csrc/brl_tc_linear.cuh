@@ -87,6 +87,7 @@ __global__ void tcl_packx_kernel(const float* __restrict__ x, unsigned char* __r
 struct LinArgs {
   const unsigned char* img;
   long long img_stride;  // IMG_BYTES or 0
+  int img_per, img_phase;  // MC sample s reads image (s + img_phase) / img_per
   float* out;            // [S,B,2]
   int B, S, ntile128;
   int* status;
@@ -121,7 +122,7 @@ __global__ void __launch_bounds__(128, 1) tcl_kernel(const LinArgs a, const __gr
 
   for (long long it = beg; it < end && ok; ++it) {
     const int s = (int)(it / a.ntile128), tile = (int)(it % a.ntile128);
-    const unsigned char* img = a.img + (long long)s * a.img_stride;
+    const unsigned char* img = a.img + (long long)((s + a.img_phase) / a.img_per) * a.img_stride;
     const float* tail = reinterpret_cast<const float*>(img + L_TAIL);
     const int row0 = tile * 128;
 
@@ -196,7 +197,7 @@ __global__ void __launch_bounds__(128, 1) tcl_kernel(const LinArgs a, const __gr
     layer_done();
     if (tid == 0 && it + 1 < end) {  // the ring is idle from here on: the next item's first two fc1 k-blocks travel underneath the head
       const int s2 = (int)((it + 1) / a.ntile128), tile2 = (int)((it + 1) % a.ntile128);
-      const unsigned char* img2 = a.img + (long long)s2 * a.img_stride;
+      const unsigned char* img2 = a.img + (long long)((s2 + a.img_phase) / a.img_per) * a.img_stride;
       load(true, 0, img2 + L_W1, KB1_BYTES, tile2 * 128);
       load(true, 1, img2 + L_W1, KB1_BYTES, tile2 * 128);
     }

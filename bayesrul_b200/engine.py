@@ -243,6 +243,38 @@ class Engine:
                                                 ws.data_ptr(), nbytes, self._stream()))
         return tuple(outs)
 
+    def predict_moments_ensemble(self, x, mu, sigma=None, S: int = 20, guide: Optional[str] = "normal", p_dropout: float = 0.0,
+                                 noise: Optional[Noise] = None, engine: str = "simt", chunk: Optional[int] = None):
+        """predict_moments of M models over one batch x [B,30,18] in one call: mu (and sigma with a guide) [M,P].  Member m is
+        predict_moments(x, mu[m], sigma[m], S, guide, p_dropout, noise with sample0 + m * S); injected noise is member-major
+        ([M * S, ...]).  Returns (pred, std, ep_var, al_var), each an [M,B] view of one [4,M,B] tensor (pred / std are the
+        inputs of mixture_moments).  `chunk` caps the draws per pass of the flattened M * S sample axis."""
+        x = self._x(x)
+        B = x.shape[0]
+        mu = _chk(mu, self.device, "mu")
+        if mu.dim() != 2 or mu.shape[0] == 0 or mu.shape[1] != self.P:
+            raise RuntimeError(f"bayesrul_b200: mu must have shape (M, {self.P}), got {tuple(mu.shape)}")
+        M = mu.shape[0]
+        if guide is not None:
+            if guide not in GUIDE_IDS:
+                raise RuntimeError("Guide unknown. Choose from 'normal', 'radial'.")
+            if sigma is None:
+                raise RuntimeError("bayesrul_b200: sigma is required with a guide")
+            sigma = self._theta(sigma, "sigma", (M,))
+        eid = ENGINE_IDS[engine]
+        sc = min(M * S, chunk or (128 if engine == "tc" else 16))
+        while sc > 1 and self.lib.brl_workspace_bytes(self.ctx, B, sc, 0, eid) > self.max_workspace_bytes:
+            sc -= 1
+        nbytes = self.lib.brl_workspace_bytes(self.ctx, B, sc, 0, eid) + (M * 4 * B * 4 + 255) // 256 * 256  # + Welford state
+        ws = self.workspace(nbytes)
+        out = torch.empty(4, M, B, device=self.device)
+        nz, keep = self._noise(noise)
+        _lib.check(self.lib.brl_predict_moments_ensemble(self.ctx, x.data_ptr(), M, B, S, GUIDE_IDS[guide] if guide else -1,
+                                                         mu.data_ptr(), sigma.data_ptr() if guide is not None else None,
+                                                         float(p_dropout), nz, out.data_ptr(), eid, ws.data_ptr(), nbytes,
+                                                         self._stream()))
+        return tuple(out.unbind(0))
+
     def predict_moments_host(self, x_host: torch.Tensor, mu, sigma=None, S: int = 20, guide: Optional[str] = "normal",
                              p_dropout: float = 0.0, noise: Optional[Noise] = None, engine: str = "simt") -> torch.Tensor:
         """predict_moments for a HOST batch [B,30,18] (pinned memory makes the copies asynchronous).  Returns a pinned
@@ -458,6 +490,21 @@ class Engine:
         with self._on_device():
             _lib.check(self.lib.brl_step_metrics(pred.data_ptr(), std.data_ptr(), y.data_ptr(), pred.numel(), scalars.data_ptr(),
                                                  self._metrics_ws.data_ptr(), self._metrics_ws.numel(), self._stream()))
+        return scalars
+
+    def step_metrics_ensemble(self, pred, std, y) -> torch.Tensor:
+        """step_metrics of M rows in one pass: pred / std / y [M,n] -> device float64 [M,5], row m = step_metrics(pred[m],
+        std[m], y[m])."""
+        pred, std, y = (_chk(t, self.device, n) for t, n in ((pred, "pred"), (std, "std"), (y, "y")))
+        if pred.dim() != 2 or not (pred.shape == std.shape == y.shape) or pred.numel() == 0:
+            raise RuntimeError("bayesrul_b200: pred / std / y must all be [M,n] with M, n > 0")
+        M, n = pred.shape
+        scalars = torch.empty(M, 5, dtype=torch.float64, device=self.device)
+        if getattr(self, "_metrics_ws", None) is None or self._metrics_ws.numel() < M * 1024:
+            self._metrics_ws = torch.empty(max(4096, M * 1024), dtype=torch.uint8, device=self.device)
+        with self._on_device():
+            _lib.check(self.lib.brl_step_metrics_ensemble(pred.data_ptr(), std.data_ptr(), y.data_ptr(), M, n, scalars.data_ptr(),
+                                                          self._metrics_ws.data_ptr(), self._metrics_ws.numel(), self._stream()))
         return scalars
 
     def clipped_adam(self, param, grad, exp_avg, exp_avg_sq, step: int, lr: float, betas=(0.95, 0.999), eps=1e-8,

@@ -166,6 +166,25 @@ int brl_predict_moments(brl_ctx* ctx, const float* x, int64_t B, int64_t S, int 
                         float* std, float* ep_var, float* al_var, int engine, void* workspace,
                         size_t workspace_bytes, void* stream);
 
+/* ---- M models' S-sample predictive moments over ONE batch of windows in one call (the seeds of a BNN experiment or the members
+ *      of a deep ensemble at test / predict / validation time).
+ *      Member m is brl_predict_moments(x, B, S, guide, mu + m*P, sigma + m*P, p_dropout, noise with sample0 + m*S, ...):
+ *      guide >= 0: M variational posteriors (the seeds of a BNN experiment), weight sampling;
+ *      guide < 0 : M weight vectors (deep-ensemble members), MC-dropout when p_dropout > 0.
+ *      Injected noise is member-major, sample-minor: weight_eps [M*S,P], radial_r [M*S,n_sites], drop_mask[l] [M*S,B,out_elems(l)].
+ *      out [4][M][B] = (pred, std, ep_var, al_var), so out + 0 and out + M*B are the [M,B] inputs of brl_mixture_moments.
+ *      Each member's results are bit-identical to its single call on the same engine.  On BRL_ENGINE_TC_FP16 the M*S draws form
+ *      one sample axis j = m*S + s, cut into chunks that fit the workspace; per chunk the members share one sampler, one pack,
+ *      the engine's and one moment-update launch, so a call whose M*S draws fit one chunk issues as many launches as one
+ *      member's call.  Elsewhere (SIMT engine; MC-dropout on the Linear and Conv-D3 nets, which the tensor-core engine refuses)
+ *      the members run one after another on brl_predict_moments.  Workspace: at least brl_workspace_bytes(B, 1, 0, engine) plus
+ *      the [M,4,B] float Welford state (rounded up to 256 bytes); more workspace gives larger chunks.  Less returns
+ *      BRL_ERR_WORKSPACE. */
+int brl_predict_moments_ensemble(brl_ctx* ctx, const float* x /*[B,30,18]*/, int64_t M, int64_t B, int64_t S, int guide,
+                                 const float* mu /*[M,P]*/, const float* sigma /*[M,P] or NULL*/, float p_dropout,
+                                 const brl_noise* noise, float* out /*[4,M,B]*/, int engine, void* workspace,
+                                 size_t workspace_bytes, void* stream);
+
 /* ---- the same with HOST buffers (replaces predict_step as a whole, bayesian.py:231-250: `x.to(device)`, bnn.predict,
  *      the moments and the five `.cpu()` reads).  x_host [B,30,18] and out_host [4,B] = (pred, std, ep_var, al_var) are HOST
  *      pointers (pinned memory makes the copies asynchronous).  On the fused engine the batch travels in window chunks on a
@@ -262,6 +281,11 @@ int brl_test_metrics(const float* pred, const float* std, const float* y, int64_
  *      100-bin coverage histogram, instead of ~30 small torch launches per step */
 int brl_step_metrics(const float* pred, const float* std, const float* y, int64_t n, double* scalars,
                      void* workspace, size_t workspace_bytes, void* stream);
+
+/* brl_step_metrics of M rows in one pass: row m of scalars [M,5] is brl_step_metrics(pred + m*n, std + m*n, y + m*n, n).
+ * Workspace: M x 1024 bytes (less returns BRL_ERR_WORKSPACE). */
+int brl_step_metrics_ensemble(const float* pred /*[M,n]*/, const float* std /*[M,n]*/, const float* y /*[M,n]*/, int64_t M,
+                              int64_t n, double* scalars /*[M,5]*/, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- fused ClippedAdam over a flat buffer (pyro.optim.ClippedAdam, conf/model/bnn.yaml:6-10) */
 int brl_clipped_adam(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, int64_t n,
