@@ -134,18 +134,15 @@ struct ActBufs {
   float *st_x = nullptr, *st_y = nullptr, *st_out = nullptr, *st_gmu = nullptr, *st_gsig = nullptr, *st_glog = nullptr;
   double* st_scal = nullptr;
   unsigned long long* dyn = nullptr;
-  // level-fused tcgen05 training kernels (Inception conv stack, brl_tc_train.cu): images of one particle lane
+  // images of one particle lane of the level-fused tcgen05 training kernels (brl_tc_train*.cu), one set per net: `tt` for the
+  // Inception conv stack, `tl` for the Linear net, `tc3` for the Conv-D3 net (the latter two carved last, only where they fit)
   TtLane tt{};
-  bool has_tt = false;
-  int tt_members = 1;         // brl_hnn_step_ensemble / brl_elbo_step_ensemble: members whose lanes sit back to back from `tt`,
-                              // tt_stride bytes apart
-  long long tt_stride = 0;
-  // level-fused tcgen05 training kernels of the Linear net (brl_tc_train_linear.cuh): carved last, only where they fit
   TlLane tl{};
-  bool has_tl = false;
-  // level-fused tcgen05 training kernels of the Conv-D3 net (brl_tc_train_convd3.cuh): carved last, only where they fit
   Tc3Lane tc3{};
-  bool has_tc3 = false;
+  bool fused = false;         // this net's images were carved
+  int fused_members = 1;      // brl_hnn_step_ensemble / brl_elbo_step_ensemble: members whose lanes sit back to back from `tt`,
+                              // fused_stride bytes apart
+  long long fused_stride = 0;
 };
 constexpr int GRAPH_MAX_PARTICLES = 8;
 
@@ -190,7 +187,7 @@ static void carve_train(const NetSpec& n, Carve& c, long long B, ActBufs& ab) {
   if (n.id == BRL_NET_INCEPTION) {
     unsigned char* base = c.take<unsigned char>((long long)tt_lane_bytes(B));
     if (base) tt_carve(base, B, ab.tt);
-    ab.has_tt = base != nullptr;
+    ab.fused = base != nullptr;
   }
 }
 
@@ -204,7 +201,7 @@ static void carve_tl(const NetSpec& n, Carve& c, long long B, ActBufs& ab) {
   unsigned char* base = c.take<unsigned char>((long long)bytes);
   if (base && lin) tl_carve(base, B, ab.tl);
   if (base && !lin) tc3_carve(base, B, ab.tc3);
-  (lin ? ab.has_tl : ab.has_tc3) = base != nullptr;
+  ab.fused = base != nullptr;
 }
 
 // brl_hnn_step_ensemble / brl_elbo_step_ensemble (elbo) on the fused Inception kernels: the other M - 1 members' lanes right
@@ -240,11 +237,11 @@ static void carve_members(const NetSpec& n, Carve& c, long long B, long long M, 
     e.st_gsig = t.take<float>(M * n.P);
     e.st_glog = t.take<float>(M * n.P);
   }
-  if (c.base && (!t.ok || !ab.has_tt)) return;
+  if (c.base && (!t.ok || !ab.fused)) return;
   c = t;
   if (!c.base) return;
-  ab.tt_members = (int)M;
-  ab.tt_stride = (long long)tt_lane_bytes(B);
+  ab.fused_members = (int)M;
+  ab.fused_stride = (long long)tt_lane_bytes(B);
   ab.part[0] = part;  // the fc split-K sums, [M][2][B][64]
   ab.dpre[n.ops.size() - 2] = dpre;
   ab.st_x = sx; ab.st_y = sy; ab.st_out = sout; ab.st_gmu = sg; ab.st_scal = ss;
@@ -602,6 +599,74 @@ static void run_backward(const brl_ctx* ctx, const ActBufs& ab, const BwdArgs& a
 static int zero_grads(const NetSpec& n, const ActBufs& ab, long long B, cudaStream_t st) {
   for (size_t i = 0; i < n.bufs.size(); ++i)
     if (ab.grad[i]) BRL_CUDA(cudaMemsetAsync(ab.grad[i], 0, sizeof(float) * B * n.bufs[i].elems(), st));
+  return BRL_OK;
+}
+
+// Graph replay of a training step whose configuration is `key`, where `graphable` (native Philox noise): eager on first sight of
+// the key, captured on the second, replayed after.  body(x, y, noise, staged, stream) issues the step's launches; `staged` selects
+// the outputs among ab's staging buffers instead of the caller's.  The capture runs it over the staging inputs with the Philox key
+// read from ab.dyn; a replay copies x, y (MB windows) and the key in, launches the graph and copies `out` back.
+template <class Body>
+static int run_step(brl_ctx* ctx, const brl_ctx::StepKey& key, bool graphable, const ActBufs& ab, const float* x, const float* y,
+                    long long MB, const brl_noise* noise, CopyJobs out, Body body, cudaStream_t st) {
+  brl_ctx::StepGraph* sg = nullptr;
+  bool caller_captures = false;  // the caller is capturing `st` itself (e.g. torch.cuda.graph): stay on the eager, capturable path
+  {
+    cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+    if (cudaStreamIsCapturing(st, &cs) != cudaSuccess) { cudaGetLastError(); caller_captures = true; }
+    else caller_captures = cs != cudaStreamCaptureStatusNone;
+  }
+  if (ctx->graph_enabled && !caller_captures && graphable) {
+    for (auto it = ctx->graphs.begin(); it != ctx->graphs.end(); ++it)
+      if (it->key == key) { ctx->graphs.splice(ctx->graphs.begin(), ctx->graphs, it); sg = &ctx->graphs.front(); break; }
+    if (!sg) {
+      if (ctx->graphs.size() >= 16) {
+        if (ctx->graphs.back().exec) cudaGraphExecDestroy(ctx->graphs.back().exec);
+        ctx->graphs.pop_back();
+      }
+      ctx->graphs.emplace_front();
+      ctx->graphs.front().key = key;
+      sg = &ctx->graphs.front();
+    }
+    ++sg->seen;
+    if (sg->seen >= 2 && !sg->exec && !sg->bad) {
+      cudaGraph_t graph = nullptr;
+      // on `cap`, since the caller's stream may be the legacy default stream
+      if (cudaStreamBeginCapture(ctx->cap, cudaStreamCaptureModeThreadLocal) == cudaSuccess) {
+        g_dyn = ab.dyn;
+        const long long l0 = launch_count();
+        brl_noise zero;
+        memset(&zero, 0, sizeof(zero));
+        const int rc = body(ab.st_x, ab.st_y, &zero, true, ctx->cap);
+        g_dyn = nullptr;
+        sg->launches = (int)(launch_count() - l0);
+        count_launch(-sg->launches);  // captured, not executed
+        const cudaError_t e = cudaStreamEndCapture(ctx->cap, &graph);
+        if (rc != BRL_OK || e != cudaSuccess || !graph || cudaGraphInstantiate(&sg->exec, graph, 0) != cudaSuccess) {
+          sg->exec = nullptr;
+          sg->bad = true;
+        }
+        if (graph) cudaGraphDestroy(graph);
+      } else {
+        sg->bad = true;
+      }
+      cudaGetLastError();  // a failed capture must not poison the eager path below
+    }
+  }
+  if (!sg || !sg->exec) return body(x, y, noise, false, st);
+  count_launch(sg->launches);
+  CopyJobs in{};  // x, y and the Philox key of this step -> staging
+  in.dst[0] = ab.st_x; in.src[0] = x; in.n[0] = MB * 540;
+  in.dst[1] = ab.st_y; in.src[1] = y; in.n[1] = MB;
+  in.njobs = 2;
+  in.dyn = ab.dyn;
+  in.seed = noise ? noise->seed : 0ull;
+  in.sample0 = noise ? (unsigned long long)noise->sample0 : 0ull;
+  in.window0 = noise ? (unsigned long long)noise->window0 : 0ull;
+  launch_copy_jobs(in, st);
+  BRL_CUDA(cudaGraphLaunch(sg->exec, st));
+  launch_copy_jobs(out, st);
+  BRL_CUDA(cudaGetLastError());
   return BRL_OK;
 }
 
@@ -1235,13 +1300,104 @@ int brl_aggregate_predictions(const float* out, int64_t S, int64_t B, float* agg
   return BRL_OK;
 }
 
-// M members of an ELBO step in ONE chain of launches: the level-fused Inception kernels with the workspace's lanes for M members
-// (at M = 1: where brl_elbo_step runs the fused Inception kernels)
-static bool elbo_batched(const brl_ctx* ctx, const ActBufs& ab, long long M, long long B, int mode) {
-  return ctx->gemm_backend == BRL_GEMM_TC_FUSED && ctx->net->id == BRL_NET_INCEPTION && ab.has_tt && ab.tt_members >= M &&
-         (mode == BRL_MODE_LRT || mode == BRL_MODE_FLIPOUT || mode == BRL_MODE_WS) &&
-         2 * B * 64 <= SPLITK_SCRATCH_FLOATS;  // fc partial sums live in the split-K scratch (B <= 4736), else per-layer
+// ---- level-fused tcgen05 training kernels (BRL_GEMM_TC_FUSED) of the three nets, shared by the ELBO and HNN steps: layers 0..L-1
+// on the tensor pipe, the rest of the net (the epilogue of fc layer `fc` if there is one, the head, the likelihood and their
+// backward) in one tt_tail launch over the `width` hidden units in front of the head (always the last layer)
+struct FusedNet { int L, fc, width; };
+static FusedNet fused_net(const NetSpec& n) {
+  if (n.id == BRL_NET_INCEPTION) return {TT_LAYERS, TT_LAYERS, 64};  // ten convs, fc layer 10
+  if (n.id == BRL_NET_LINEAR) return {4, 3, 32};                      // four hidden layers, the tail runs layer 3's epilogue
+  return {3, -1, 320};                                                 // Conv-D3: three convs, the head reads the pooled features
 }
+
+// M members of a step in ONE chain of launches on the fused kernels: this net's images carved for M members (more than one: the
+// Inception net only) and, for the Inception net, the fc layer's partial sums within the split-K scratch (B <= 4736).  Every mode
+// the ELBO step (LRT / Flipout / WS) and the HNN step (DET) accept runs on them.
+static bool fused_ok(const brl_ctx* ctx, const ActBufs& ab, long long M, long long B) {
+  return ctx->gemm_backend == BRL_GEMM_TC_FUSED && ab.fused && M <= ab.fused_members &&
+         (ctx->net->id != BRL_NET_INCEPTION || 2 * B * 64 <= SPLITK_SCRATCH_FLOATS);
+}
+
+static float keep_prob(const LayerSpec& L, float p_dropout) {
+  return (p_dropout > 0.f && L.drop_factor > 0.f) ? 1.0f - p_dropout * L.drop_factor : 1.0f;
+}
+
+// the fused kernels' view of one particle lane of the step `a` describes: LRT eps (ELBO) or dropout sites (mode DET: the HNN step)
+// and the sign tensors of layers 0..L-1, the members' strides (read against blockIdx.z only, so inert at M = 1)
+static TtStep fused_step(const brl_ctx* ctx, const ActBufs& ab, const FwdArgs& a, long long M, float* g0, float* g1, int particles) {
+  const NetSpec& n = *ctx->net;
+  const FusedNet f = fused_net(n);
+  const brl_noise& nz = *a.noise;
+  auto sin_ = [&](int ly) { return a.sgn_in ? a.sgn_in[ly] : nullptr; };
+  TtStep ts{};
+  // weight-sampling ELBO (radial guide / no fit context): ONE contraction with the particle's weight draw
+  ts.x = a.x; ts.B = a.B; ts.mode = a.mode; ts.mu = a.mode == BRL_MODE_WS ? a.wsamp : a.theta; ts.sigma = a.sigma; ts.wsamp = a.wsamp;
+  for (int ly = 0; ly < f.L; ++ly) {
+    if (a.mode == BRL_MODE_DET) ts.drop[ly] = nref(&nz, nz.drop_mask[ly], KIND_DROPOUT, (unsigned)ly);
+    else ts.eps[ly] = nref(&nz, nz.lrt_eps[ly], KIND_LRT_EPS, (unsigned)ly);
+    ts.keep[ly] = keep_prob(n.layers[ly], a.p_dropout);
+    ts.sgn_in[ly] = sin_(ly); ts.sgn_out[ly] = a.sgn_out ? a.sgn_out[ly] : nullptr;
+    ts.w_off[ly] = n.layers[ly].w_off; ts.b_off[ly] = n.layers[ly].b_off;
+  }
+  (f.L < TT_LAYERS ? ts.sgn_in[f.L] : ts.sgn_fc_in) = sin_(f.L);  // s_in of the first layer behind the tensor pipe
+  if (f.fc >= 0) { ts.w_off_fc = n.layers[f.fc].w_off; ts.b_off_fc = n.layers[f.fc].b_off; }
+  ts.g0 = g0; ts.g1 = g1;
+  ts.members = (int)M; ts.P = n.P; ts.lane_stride = ab.fused_stride;
+  ts.noise_stride = particles; ts.sign_stride = nz.flip_in[0] ? particles : 1;
+  return ts;
+}
+
+static void fused_forward(const brl_ctx* ctx, const ActBufs& ab, const TtStep& ts, cudaStream_t st, const TtSide& sd) {
+  if (ctx->net->id == BRL_NET_INCEPTION) {
+    tt_forward(ab.tt, ts, st, sd);
+    tt_fc_forward(ab.tt, ts, ab.part[0], st);
+  } else if (ctx->net->id == BRL_NET_LINEAR) {
+    tl_forward(ab.tl, ts, st, sd);
+  } else {
+    tc3_forward(ab.tc3, ts, st, sd);
+  }
+}
+
+// the tail: the ELBO likelihood (gscale = c_nll / particles, acc [M][4]) or in mode DET the HNN loss (acc [M][2]) of `a`'s lane
+static void fused_tail(const brl_ctx* ctx, const ActBufs& ab, const TtStep& ts, const FwdArgs& a, const float* y, float gscale,
+                       int compute_grads, double* acc, cudaStream_t st) {
+  const NetSpec& n = *ctx->net;
+  const FusedNet f = fused_net(n);
+  const brl_noise& nz = *a.noise;
+  const int hd = (int)n.layers.size() - 1, fc_op = (int)n.ops.size() - 2;
+  TtTail tl{};
+  tl.part = n.id == BRL_NET_INCEPTION ? ab.part[0] : n.id == BRL_NET_LINEAR ? ab.tl.part : ab.tc3.feat;
+  tl.width = f.width; tl.y = y; tl.gscale = gscale; tl.compute_grads = compute_grads; tl.acc = acc; tl.out = a.out;
+  tl.dpre = f.fc >= 0 ? ab.dpre[fc_op] : ab.tc3.dfeat;
+  tl.dsec = f.fc >= 0 ? ab.dsec[fc_op] : nullptr;
+  tl.hw_off = n.layers[hd].w_off; tl.hb_off = n.layers[hd].b_off;
+  if (a.mode == BRL_MODE_DET) {
+    tl.loss_kind = 1;
+    if (f.fc >= 0) {
+      tl.keep_fc = keep_prob(n.layers[f.fc], a.p_dropout);
+      tl.drop_fc = nref(&nz, nz.drop_mask[f.fc], KIND_DROPOUT, (unsigned)f.fc);
+    }
+  } else {
+    if (f.fc >= 0) { tl.eps_fc = nref(&nz, nz.lrt_eps[f.fc], KIND_LRT_EPS, (unsigned)f.fc); tl.sout_fc = a.sgn_out[f.fc]; }
+    tl.eps_head = nref(&nz, nz.lrt_eps[hd], KIND_LRT_EPS, (unsigned)hd);
+    tl.sin_head = a.sgn_in[hd]; tl.sout_head = a.sgn_out[hd];
+    tl.acc_stride = 4;
+  }
+  tt_tail(ts, tl, st);
+}
+
+static void fused_backward(const brl_ctx* ctx, const ActBufs& ab, const TtStep& ts, cudaStream_t st, const TtSide& sd) {
+  const int fc_op = (int)ctx->net->ops.size() - 2;
+  if (ctx->net->id == BRL_NET_INCEPTION) {
+    tt_fc_backward(ab.tt, ts, ab.dpre[fc_op], ab.dsec[fc_op], st, sd);
+    tt_backward(ab.tt, ts, st, sd);
+  } else if (ctx->net->id == BRL_NET_LINEAR) {
+    tl_backward(ab.tl, ts, ab.dpre.data(), ab.dsec.data(), st, sd);
+  } else {
+    tc3_backward(ab.tc3, ts, st, sd);
+  }
+}
+
 // injected Flipout signs of the member-batched kernels: member m's tensors start `particles` rows [B, C] after member m - 1's,
 // the signs generated in the workspace one row after; with several particles the kernels take one stride for all layers
 static bool signs_one_stride(const NetSpec& n, const brl_noise* nz, int particles) {
@@ -1250,9 +1406,8 @@ static bool signs_one_stride(const NetSpec& n, const brl_noise* nz, int particle
   for (size_t l = 0; l < n.layers.size(); ++l) injected += (nz->flip_in[l] != nullptr) + (nz->flip_out[l] != nullptr);
   return injected == 0 || injected == 2 * (int)n.layers.size();
 }
-static bool signs_injected(const brl_noise* nz) { return nz && nz->flip_in[0]; }
 
-// the launches of one ELBO step of M members (every pointer final; M > 1 only where elbo_batched holds); captured as is by the
+// the launches of one ELBO step of M members (every pointer final; M > 1 only where fused_ok holds); captured as is by the
 // graph path of elbo_step.
 // lanes[0] always exists and owns the shared accumulators; with a second buffer set (lanes[1]) two particles run side by
 // side: lane 0 on `st`, lane 1 on the context's own stream, forked / joined with events.  The gradient finalisation of the
@@ -1309,22 +1464,15 @@ static int elbo_body(brl_ctx* ctx, const ActBufs* const* lanes, int n_lanes, con
       }
       float* outp = out + (long long)pt * B * 2;
       const brl_ctx::Lane& ln = ctx->lanes[l];
-      // level-fused tcgen05 kernels (BRL_GEMM_TC_FUSED): ten conv layers + the fc layer on the tensor pipe, the rest of the net
-      // (fc epilogue, head, likelihood, their backward) in one tail kernel
-      const bool use_tt = elbo_batched(ctx, ab, M, B, mode);
-      // the Linear net's four hidden layers on the tensor pipe, the head in the same tail kernel (width 32)
-      const bool use_tl = ctx->gemm_backend == BRL_GEMM_TC_FUSED && n.id == BRL_NET_LINEAR && ab.has_tl &&
-                          (mode == BRL_MODE_LRT || mode == BRL_MODE_FLIPOUT || mode == BRL_MODE_WS);
-      // the Conv-D3 net's three convs on the tensor pipe, the head in the same tail kernel (width 320)
-      const bool use_tc3 = ctx->gemm_backend == BRL_GEMM_TC_FUSED && n.id == BRL_NET_CONV && ab.has_tc3 &&
-                           (mode == BRL_MODE_LRT || mode == BRL_MODE_FLIPOUT || mode == BRL_MODE_WS);
+      const TtSide sd{ln.side[0], ln.ev_fork, ln.ev_join[0]};
+      const bool fused = fused_ok(ctx, ab, M, B);
       if (compute_grads) {  // a dozen memsets: on a side stream underneath the forward pass, joined before the NLL
         cudaStream_t zs = ctx->multi_stream ? ln.zero : ls;
         if (zs != ls) {
           BRL_CUDA(cudaEventRecord(ln.ev_zero, ls));
           BRL_CUDA(cudaStreamWaitEvent(zs, ln.ev_zero, 0));
         }
-        if (!use_tt && !use_tl && !use_tc3) {  // the fused back-end keeps its gradients in bf16 images that are written, not accumulated
+        if (!fused) {  // the fused back-end keeps its gradients in bf16 images that are written, not accumulated
           int rc = zero_grads(n, ab, B, zs);
           if (rc) return rc;
         }
@@ -1333,97 +1481,16 @@ static int elbo_body(brl_ctx* ctx, const ActBufs* const* lanes, int n_lanes, con
         if (zs != ls) BRL_CUDA(cudaEventRecord(ln.ev_zero, zs));
       }
       FwdArgs fa{x, B, 1, mode, mu, sigma, ab.wsamp, 0.f, &nz, sin_.data(), sout_.data(), outp, compute_grads != 0};
-      TtStep ts{};
-      if (use_tt) {
-        // weight-sampling ELBO (radial guide / no fit context): ONE contraction with the particle's weight draw
-        ts.x = x; ts.B = B; ts.mode = mode; ts.mu = mode == BRL_MODE_WS ? ab.wsamp : mu; ts.sigma = sigma; ts.wsamp = ab.wsamp;
-        for (int ly = 0; ly < TT_LAYERS; ++ly) {
-          ts.eps[ly] = nref(&nz, nz.lrt_eps[ly], KIND_LRT_EPS, (unsigned)ly);
-          ts.keep[ly] = 1.0f;
-          ts.sgn_in[ly] = sin_[ly]; ts.sgn_out[ly] = sout_[ly];
-          ts.w_off[ly] = n.layers[ly].w_off; ts.b_off[ly] = n.layers[ly].b_off;
-        }
-        const int fc_op = (int)n.ops.size() - 2, fc_layer = n.ops[fc_op].layer;
-        ts.sgn_fc_in = sin_[fc_layer];
-        ts.w_off_fc = n.layers[fc_layer].w_off; ts.b_off_fc = n.layers[fc_layer].b_off;
-        ts.g0 = ab.g0; ts.g1 = ab.g1;
-        ts.members = (int)M; ts.P = n.P; ts.lane_stride = ab.tt_stride;
-        ts.noise_stride = particles; ts.sign_stride = signs_injected(noise) ? particles : 1;
-        const TtSide tsd{ln.side[0], ln.ev_fork, ln.ev_join[0]};
-        tt_forward(ab.tt, ts, ls, tsd);
-        tt_fc_forward(ab.tt, ts, ab.part[0], ls);
-      } else if (use_tl) {
-        ts.x = x; ts.B = B; ts.mode = mode; ts.mu = mode == BRL_MODE_WS ? ab.wsamp : mu; ts.sigma = sigma; ts.wsamp = ab.wsamp;
-        for (int ly = 0; ly < 4; ++ly) {
-          ts.eps[ly] = nref(&nz, nz.lrt_eps[ly], KIND_LRT_EPS, (unsigned)ly);
-          ts.keep[ly] = 1.0f;
-          ts.sgn_out[ly] = sout_[ly];
-          ts.w_off[ly] = n.layers[ly].w_off; ts.b_off[ly] = n.layers[ly].b_off;
-        }
-        for (int ly = 0; ly < 5; ++ly) ts.sgn_in[ly] = sin_[ly];
-        ts.w_off_fc = n.layers[3].w_off; ts.b_off_fc = n.layers[3].b_off;
-        ts.g0 = ab.g0; ts.g1 = ab.g1;
-        tl_forward(ab.tl, ts, ls, TtSide{ln.side[0], ln.ev_fork, ln.ev_join[0]});
-      } else if (use_tc3) {
-        ts.x = x; ts.B = B; ts.mode = mode; ts.mu = mode == BRL_MODE_WS ? ab.wsamp : mu; ts.sigma = sigma; ts.wsamp = ab.wsamp;
-        for (int ly = 0; ly < 3; ++ly) {
-          ts.eps[ly] = nref(&nz, nz.lrt_eps[ly], KIND_LRT_EPS, (unsigned)ly);
-          ts.keep[ly] = 1.0f;
-          ts.sgn_out[ly] = sout_[ly];
-          ts.w_off[ly] = n.layers[ly].w_off; ts.b_off[ly] = n.layers[ly].b_off;
-        }
-        for (int ly = 0; ly < 4; ++ly) ts.sgn_in[ly] = sin_[ly];
-        ts.g0 = ab.g0; ts.g1 = ab.g1;
-        tc3_forward(ab.tc3, ts, ls, TtSide{ln.side[0], ln.ev_fork, ln.ev_join[0]});
-      } else {
-        run_forward(ctx, ab, fa, ls, l);
-      }
+      const TtStep ts = fused ? fused_step(ctx, ab, fa, M, ab.g0, ab.g1, particles) : TtStep{};
+      if (fused) fused_forward(ctx, ab, ts, ls, sd);
+      else run_forward(ctx, ab, fa, ls, l);
       if (compute_grads && ctx->multi_stream) BRL_CUDA(cudaStreamWaitEvent(ls, ln.ev_zero, 0));
-      if (use_tt) {
-        const int fc_op = (int)n.ops.size() - 2, fc_layer = n.ops[fc_op].layer, hd_layer = n.ops[fc_op + 1].layer;
-        TtTail tl{};
-        tl.part = ab.part[0]; tl.y = y; tl.gscale = (float)(c_nll / particles); tl.compute_grads = compute_grads;
-        tl.acc = ab0.acc; tl.out = outp; tl.dpre = ab.dpre[fc_op]; tl.dsec = ab.dsec[fc_op];
-        tl.eps_fc = nref(&nz, nz.lrt_eps[fc_layer], KIND_LRT_EPS, (unsigned)fc_layer);
-        tl.eps_head = nref(&nz, nz.lrt_eps[hd_layer], KIND_LRT_EPS, (unsigned)hd_layer);
-        tl.sout_fc = sout_[fc_layer]; tl.sin_head = sin_[hd_layer]; tl.sout_head = sout_[hd_layer];
-        tl.hw_off = n.layers[hd_layer].w_off; tl.hb_off = n.layers[hd_layer].b_off;
-        tl.acc_stride = 4;
-        tt_tail(ts, tl, ls);
-      } else if (use_tl) {
-        TtTail tl{};
-        tl.part = ab.tl.part; tl.width = 32; tl.y = y; tl.gscale = (float)(c_nll / particles); tl.compute_grads = compute_grads;
-        tl.acc = ab0.acc; tl.out = outp; tl.dpre = ab.dpre[3]; tl.dsec = ab.dsec[3];
-        tl.eps_fc = nref(&nz, nz.lrt_eps[3], KIND_LRT_EPS, 3u);
-        tl.eps_head = nref(&nz, nz.lrt_eps[4], KIND_LRT_EPS, 4u);
-        tl.sout_fc = sout_[3]; tl.sin_head = sin_[4]; tl.sout_head = sout_[4];
-        tl.hw_off = n.layers[4].w_off; tl.hb_off = n.layers[4].b_off;
-        tt_tail(ts, tl, ls);
-      } else if (use_tc3) {
-        TtTail tl{};
-        tl.part = ab.tc3.feat; tl.width = 320; tl.y = y; tl.gscale = (float)(c_nll / particles); tl.compute_grads = compute_grads;
-        tl.acc = ab0.acc; tl.out = outp; tl.dpre = ab.tc3.dfeat;
-        tl.eps_head = nref(&nz, nz.lrt_eps[3], KIND_LRT_EPS, 3u);
-        tl.sin_head = sin_[3]; tl.sout_head = sout_[3];
-        tl.hw_off = n.layers[3].w_off; tl.hb_off = n.layers[3].b_off;
-        tt_tail(ts, tl, ls);
-      } else {
-        launch_nll_elbo(outp, y, B, (float)(c_nll / particles), ab0.acc, compute_grads ? ab.grad[n.out_buf] : nullptr, ls);
-      }
+      if (fused) fused_tail(ctx, ab, ts, fa, y, (float)(c_nll / particles), compute_grads, ab0.acc, ls);
+      else launch_nll_elbo(outp, y, B, (float)(c_nll / particles), ab0.acc, compute_grads ? ab.grad[n.out_buf] : nullptr, ls);
       if (compute_grads) {
         BwdArgs ba{x, B, mode, mode == BRL_MODE_WS ? ab.wsamp : mu, sigma, ab.wsamp, 0.f, &nz, sin_.data(), sout_.data(), outp, ab.g0, ab.g1};
-        if (use_tt) {
-          const int fc_op = (int)n.ops.size() - 2;
-          const TtSide tsd{ln.side[0], ln.ev_fork, ln.ev_join[0]};
-          tt_fc_backward(ab.tt, ts, ab.dpre[fc_op], ab.dsec[fc_op], ls, tsd);
-          tt_backward(ab.tt, ts, ls, tsd);
-        } else if (use_tl) {
-          tl_backward(ab.tl, ts, ab.dpre.data(), ab.dsec.data(), ls, TtSide{ln.side[0], ln.ev_fork, ln.ev_join[0]});
-        } else if (use_tc3) {
-          tc3_backward(ab.tc3, ts, ls, TtSide{ln.side[0], ln.ev_fork, ln.ev_join[0]});
-        } else {
-          run_backward(ctx, ab, ba, ls, l);
-        }
+        if (fused) fused_backward(ctx, ab, ts, ls, sd);
+        else run_backward(ctx, ab, ba, ls, l);
       }
     }
     if (nl > 1) {
@@ -1464,7 +1531,7 @@ int brl_set_step_graph(brl_ctx* ctx, int enable) {
   return BRL_OK;
 }
 
-// brl_elbo_step (M = 1) and brl_elbo_step_ensemble: M members in one chain of launches where elbo_batched holds, else one member
+// brl_elbo_step (M = 1) and brl_elbo_step_ensemble: M members in one chain of launches where fused_ok holds, else one member
 // after another on the single-member step
 static int elbo_step(brl_ctx* ctx, const float* x, const float* y, int64_t M, int64_t B, const float* mu, const float* sigma,
                      int mode, int guide, int particles, float prior_loc, float prior_scale, int64_t dataset_size,
@@ -1482,7 +1549,7 @@ static int elbo_step(brl_ctx* ctx, const float* x, const float* y, int64_t M, in
   if (M > 1) {  // the members' lanes right behind lane 0 (brl_workspace_bytes(B, M, 4)), or one member after another
     carve_tl(n, c, B, ab);
     carve_members(n, c, B, M, true, ab);
-    if (!elbo_batched(ctx, ab, M, B, mode) || !signs_one_stride(n, noise, particles)) {
+    if (!fused_ok(ctx, ab, M, B) || !signs_one_stride(n, noise, particles)) {
       brl_noise base;
       memset(&base, 0, sizeof(base));
       if (noise) base = *noise;
@@ -1507,93 +1574,36 @@ static int elbo_step(brl_ctx* ctx, const float* x, const float* y, int64_t M, in
     carve_tl(n, c, B, ab);
     if (n_lanes == 2) {
       carve_tl(n, c, B, ab1);
-      if (!ab1.has_tl) ab.has_tl = false;  // both particle lanes run the same back-end
-      if (!ab1.has_tc3) ab.has_tc3 = false;
+      if (!ab1.fused) ab.fused = false;  // both particle lanes run the same back-end
     }
   }
   const ActBufs* lanes[2] = {&ab, &ab1};
-  // ---- graph replay (native Philox noise): eager on first sight of a configuration, captured on the second, replayed after
-  brl_ctx::StepGraph* sg = nullptr;
-  bool caller_captures = false;  // the caller is capturing `st` itself (e.g. torch.cuda.graph): stay on the eager, capturable path
-  {
-    cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
-    if (cudaStreamIsCapturing(st, &cs) != cudaSuccess) { cudaGetLastError(); caller_captures = true; }
-    else caller_captures = cs != cudaStreamCaptureStatusNone;
+  brl_ctx::StepKey key;
+  memset(&key, 0, sizeof(key));
+  key.B = B; key.dataset_size = dataset_size; key.mode = mode; key.guide = guide; key.particles = particles;
+  key.compute_grads = compute_grads; key.backend = ctx->gemm_backend; key.has_log_sigma = grad_log_sigma != nullptr;
+  key.members = (int)M;
+  key.prior_loc = prior_loc; key.prior_scale = prior_scale; key.mu = mu; key.sigma = sigma; key.ws = workspace;
+  key.ws_bytes = workspace_bytes;
+  CopyJobs o{};  // staging -> the caller's result tensors (the four doubles travel as eight floats)
+  o.dst[0] = reinterpret_cast<float*>(scalars); o.src[0] = reinterpret_cast<const float*>(ab.st_scal); o.n[0] = 8 * M;
+  o.dst[1] = out; o.src[1] = ab.st_out; o.n[1] = M * particles * B * 2;
+  o.njobs = 2;
+  if (compute_grads) {
+    o.dst[2] = grad_mu; o.src[2] = ab.st_gmu; o.n[2] = M * n.P;
+    o.dst[3] = grad_sigma; o.src[3] = ab.st_gsig; o.n[3] = M * n.P;
+    o.njobs = 4;
+    if (grad_log_sigma) { o.dst[4] = grad_log_sigma; o.src[4] = ab.st_glog; o.n[4] = M * n.P; o.njobs = 5; }
   }
-  if (ctx->graph_enabled && !caller_captures && noise_is_native(noise) && particles <= GRAPH_MAX_PARTICLES) {
-    brl_ctx::StepKey key;
-    memset(&key, 0, sizeof(key));
-    key.B = B; key.dataset_size = dataset_size; key.mode = mode; key.guide = guide; key.particles = particles;
-    key.compute_grads = compute_grads; key.backend = ctx->gemm_backend; key.has_log_sigma = grad_log_sigma != nullptr;
-    key.members = (int)M;
-    key.prior_loc = prior_loc; key.prior_scale = prior_scale; key.mu = mu; key.sigma = sigma; key.ws = workspace;
-    key.ws_bytes = workspace_bytes;
-    for (auto it = ctx->graphs.begin(); it != ctx->graphs.end(); ++it)
-      if (it->key == key) { ctx->graphs.splice(ctx->graphs.begin(), ctx->graphs, it); sg = &ctx->graphs.front(); break; }
-    if (!sg) {
-      if (ctx->graphs.size() >= 16) {
-        if (ctx->graphs.back().exec) cudaGraphExecDestroy(ctx->graphs.back().exec);
-        ctx->graphs.pop_back();
-      }
-      ctx->graphs.emplace_front();
-      ctx->graphs.front().key = key;
-      sg = &ctx->graphs.front();
-    }
-    ++sg->seen;
-    if (sg->seen >= 2 && !sg->exec && !sg->bad) {
-      cudaGraph_t graph = nullptr;
-      int rc = BRL_OK;
-      if (cudaStreamBeginCapture(ctx->cap, cudaStreamCaptureModeThreadLocal) == cudaSuccess) {
-        g_dyn = ab.dyn;
-        const long long l0 = launch_count();
-        brl_noise zero;
-        memset(&zero, 0, sizeof(zero));
-        rc = elbo_body(ctx, lanes, n_lanes, ab.st_x, ab.st_y, M, B, mu, sigma, mode, guide, particles, prior_loc, prior_scale, dataset_size, &zero,
-                       compute_grads, ab.st_scal, compute_grads ? ab.st_gmu : nullptr, compute_grads ? ab.st_gsig : nullptr,
-                       (compute_grads && grad_log_sigma) ? ab.st_glog : nullptr, ab.st_out, ctx->cap);
-        g_dyn = nullptr;
-        sg->launches = (int)(launch_count() - l0);
-        count_launch(-sg->launches);  // captured, not executed
-        const cudaError_t e = cudaStreamEndCapture(ctx->cap, &graph);
-        if (rc != BRL_OK || e != cudaSuccess || !graph || cudaGraphInstantiate(&sg->exec, graph, 0) != cudaSuccess) {
-          sg->exec = nullptr;
-          sg->bad = true;
-        }
-        if (graph) cudaGraphDestroy(graph);
-      } else {
-        sg->bad = true;
-      }
-      cudaGetLastError();  // a failed capture must not poison the eager path below
-    }
-  }
-  if (sg && sg->exec) {
-    count_launch(sg->launches);
-    CopyJobs in{};  // x, y and the Philox key of this step -> staging
-    in.dst[0] = ab.st_x; in.src[0] = x; in.n[0] = M * B * 540;
-    in.dst[1] = ab.st_y; in.src[1] = y; in.n[1] = M * B;
-    in.njobs = 2;
-    in.dyn = ab.dyn;
-    in.seed = noise ? noise->seed : 0ull;
-    in.sample0 = noise ? (unsigned long long)noise->sample0 : 0ull;
-    in.window0 = noise ? (unsigned long long)noise->window0 : 0ull;
-    launch_copy_jobs(in, st);
-    BRL_CUDA(cudaGraphLaunch(sg->exec, st));
-    CopyJobs o{};  // staging -> the caller's result tensors (the four doubles travel as eight floats)
-    o.dst[0] = reinterpret_cast<float*>(scalars); o.src[0] = reinterpret_cast<const float*>(ab.st_scal); o.n[0] = 8 * M;
-    o.dst[1] = out; o.src[1] = ab.st_out; o.n[1] = M * particles * B * 2;
-    o.njobs = 2;
-    if (compute_grads) {
-      o.dst[2] = grad_mu; o.src[2] = ab.st_gmu; o.n[2] = M * n.P;
-      o.dst[3] = grad_sigma; o.src[3] = ab.st_gsig; o.n[3] = M * n.P;
-      o.njobs = 4;
-      if (grad_log_sigma) { o.dst[4] = grad_log_sigma; o.src[4] = ab.st_glog; o.n[4] = M * n.P; o.njobs = 5; }
-    }
-    launch_copy_jobs(o, st);
-    BRL_CUDA(cudaGetLastError());
-    return BRL_OK;
-  }
-  return elbo_body(ctx, lanes, n_lanes, x, y, M, B, mu, sigma, mode, guide, particles, prior_loc, prior_scale, dataset_size, noise,
-                   compute_grads, scalars, grad_mu, grad_sigma, grad_log_sigma, out, st);
+  auto body = [&](const float* bx, const float* by, const brl_noise* bnoise, bool staged, cudaStream_t bst) {
+    return elbo_body(ctx, lanes, n_lanes, bx, by, M, B, mu, sigma, mode, guide, particles, prior_loc, prior_scale, dataset_size,
+                     bnoise, compute_grads, staged ? ab.st_scal : scalars,
+                     staged ? (compute_grads ? ab.st_gmu : nullptr) : grad_mu,
+                     staged ? (compute_grads ? ab.st_gsig : nullptr) : grad_sigma,
+                     staged ? ((compute_grads && grad_log_sigma) ? ab.st_glog : nullptr) : grad_log_sigma,
+                     staged ? ab.st_out : out, bst);
+  };
+  return run_step(ctx, key, noise_is_native(noise) && particles <= GRAPH_MAX_PARTICLES, ab, x, y, M * B, noise, o, body, st);
 }
 
 int brl_elbo_step(brl_ctx* ctx, const float* x, const float* y, int64_t B, const float* mu, const float* sigma, int mode,
@@ -1628,108 +1638,28 @@ int brl_elbo_step_ensemble(brl_ctx* ctx, const float* x, const float* y, int64_t
                    scalars, grad_mu, grad_sigma, grad_log_sigma, out, workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
-// M members of an HNN step in ONE chain of launches: the level-fused Inception kernels with the workspace's lanes for M members
-static bool hnn_batched(const brl_ctx* ctx, const ActBufs& ab, long long M, long long B) {
-  return ctx->gemm_backend == BRL_GEMM_TC_FUSED && ctx->net->id == BRL_NET_INCEPTION && ab.has_tt && ab.tt_members >= M &&
-         2 * B * 64 <= SPLITK_SCRATCH_FLOATS;
-}
-
-// the launches of one heteroscedastic-NN step of M members (every pointer final; M > 1 only where hnn_batched holds); captured
+// the launches of one heteroscedastic-NN step of M members (every pointer final; M > 1 only where fused_ok holds); captured
 // as is by the graph path of hnn_step
 static int hnn_body(brl_ctx* ctx, const ActBufs& ab, const float* x, const float* y, int64_t M, int64_t B, const float* theta,
                     float p_dropout, const brl_noise* noise, int compute_grads, double* scalars, float* grad_theta, float* out,
                     cudaStream_t st) {
   const NetSpec& n = *ctx->net;
   brl_noise nz = noise_at_sample(n, noise, 0, B);
-  if (hnn_batched(ctx, ab, M, B)) {
+  FwdArgs fa{x, B, 1, BRL_MODE_DET, theta, nullptr, nullptr, p_dropout, &nz, nullptr, nullptr, out, false};
+  if (fused_ok(ctx, ab, M, B)) {
     // level-fused tcgen05 kernels, one contraction with the deterministic weights; dropout masks in the epilogues; member m on
     // blockIdx.z with its own lane, parameters, gradients and MC-sample index sample0 + m
     const brl_ctx::Lane& ln = ctx->lanes[0];
-    const int fc_op = (int)n.ops.size() - 2, fc_layer = n.ops[fc_op].layer, hd_layer = n.ops[fc_op + 1].layer;
-    auto keep_of = [&](int ly) { return (p_dropout > 0.f && n.layers[ly].drop_factor > 0.f) ? 1.0f - p_dropout * n.layers[ly].drop_factor : 1.0f; };
-    TtStep ts{};
-    ts.x = x; ts.B = B; ts.mode = BRL_MODE_DET; ts.mu = theta;
-    for (int ly = 0; ly < TT_LAYERS; ++ly) {
-      ts.drop[ly] = nref(&nz, nz.drop_mask[ly], KIND_DROPOUT, (unsigned)ly);
-      ts.keep[ly] = keep_of(ly);
-      ts.w_off[ly] = n.layers[ly].w_off; ts.b_off[ly] = n.layers[ly].b_off;
-    }
-    ts.w_off_fc = n.layers[fc_layer].w_off; ts.b_off_fc = n.layers[fc_layer].b_off;
-    ts.g0 = grad_theta; ts.g1 = nullptr;
-    ts.members = (int)M; ts.P = n.P; ts.lane_stride = ab.tt_stride;
-    const TtSide tsd{ln.side[0], ln.ev_fork, ln.ev_join[0]};
+    const TtSide sd{ln.side[0], ln.ev_fork, ln.ev_join[0]};
+    const TtStep ts = fused_step(ctx, ab, fa, M, grad_theta, nullptr, 1);
     BRL_CUDA(cudaMemsetAsync(scalars, 0, 2 * M * sizeof(double), st));
     if (compute_grads) BRL_CUDA(cudaMemsetAsync(grad_theta, 0, sizeof(float) * M * n.P, st));
-    tt_forward(ab.tt, ts, st, tsd);
-    tt_fc_forward(ab.tt, ts, ab.part[0], st);
-    TtTail tl{};
-    tl.part = ab.part[0]; tl.y = y; tl.gscale = 0.f; tl.compute_grads = compute_grads; tl.acc = scalars; tl.out = out;
-    tl.dpre = ab.dpre[fc_op]; tl.dsec = ab.dsec[fc_op];
-    tl.hw_off = n.layers[hd_layer].w_off; tl.hb_off = n.layers[hd_layer].b_off;
-    tl.loss_kind = 1; tl.keep_fc = keep_of(fc_layer); tl.drop_fc = nref(&nz, nz.drop_mask[fc_layer], KIND_DROPOUT, (unsigned)fc_layer);
-    tt_tail(ts, tl, st);
-    if (compute_grads) {
-      tt_fc_backward(ab.tt, ts, ab.dpre[fc_op], ab.dsec[fc_op], st, tsd);
-      tt_backward(ab.tt, ts, st, tsd);
-    }
+    fused_forward(ctx, ab, ts, st, sd);
+    fused_tail(ctx, ab, ts, fa, y, 0.f, compute_grads, scalars, st);
+    if (compute_grads) fused_backward(ctx, ab, ts, st, sd);
     BRL_CUDA(cudaGetLastError());
     return BRL_OK;
   }
-  if (M != 1) return fail(BRL_ERR_INVALID, "bayesrul_b200: hnn_body: members need the batched path");
-  if (ctx->gemm_backend == BRL_GEMM_TC_FUSED && n.id == BRL_NET_LINEAR && ab.has_tl) {
-    // the Linear net's fused kernels, one contraction with the deterministic weights; keep decisions in the epilogues
-    const brl_ctx::Lane& ln = ctx->lanes[0];
-    auto keep_of = [&](int ly) { return (p_dropout > 0.f && n.layers[ly].drop_factor > 0.f) ? 1.0f - p_dropout * n.layers[ly].drop_factor : 1.0f; };
-    TtStep ts{};
-    ts.x = x; ts.B = B; ts.mode = BRL_MODE_DET; ts.mu = theta;
-    for (int ly = 0; ly < 4; ++ly) {
-      ts.drop[ly] = nref(&nz, nz.drop_mask[ly], KIND_DROPOUT, (unsigned)ly);
-      ts.keep[ly] = keep_of(ly);
-      ts.w_off[ly] = n.layers[ly].w_off; ts.b_off[ly] = n.layers[ly].b_off;
-    }
-    ts.w_off_fc = n.layers[3].w_off; ts.b_off_fc = n.layers[3].b_off;
-    ts.g0 = grad_theta; ts.g1 = nullptr;
-    const TtSide tsd{ln.side[0], ln.ev_fork, ln.ev_join[0]};
-    BRL_CUDA(cudaMemsetAsync(scalars, 0, 2 * sizeof(double), st));
-    if (compute_grads) BRL_CUDA(cudaMemsetAsync(grad_theta, 0, sizeof(float) * n.P, st));
-    tl_forward(ab.tl, ts, st, tsd);
-    TtTail tl{};
-    tl.part = ab.tl.part; tl.width = 32; tl.y = y; tl.gscale = 0.f; tl.compute_grads = compute_grads; tl.acc = scalars; tl.out = out;
-    tl.dpre = ab.dpre[3]; tl.dsec = ab.dsec[3];
-    tl.hw_off = n.layers[4].w_off; tl.hb_off = n.layers[4].b_off;
-    tl.loss_kind = 1; tl.keep_fc = keep_of(3); tl.drop_fc = nref(&nz, nz.drop_mask[3], KIND_DROPOUT, 3u);
-    tt_tail(ts, tl, st);
-    if (compute_grads) tl_backward(ab.tl, ts, ab.dpre.data(), ab.dsec.data(), st, tsd);
-    BRL_CUDA(cudaGetLastError());
-    return BRL_OK;
-  }
-  if (ctx->gemm_backend == BRL_GEMM_TC_FUSED && n.id == BRL_NET_CONV && ab.has_tc3) {
-    // the Conv-D3 net's fused kernels, one contraction with the deterministic weights; keep decisions in the conv epilogues
-    const brl_ctx::Lane& ln = ctx->lanes[0];
-    auto keep_of = [&](int ly) { return (p_dropout > 0.f && n.layers[ly].drop_factor > 0.f) ? 1.0f - p_dropout * n.layers[ly].drop_factor : 1.0f; };
-    TtStep ts{};
-    ts.x = x; ts.B = B; ts.mode = BRL_MODE_DET; ts.mu = theta;
-    for (int ly = 0; ly < 3; ++ly) {
-      ts.drop[ly] = nref(&nz, nz.drop_mask[ly], KIND_DROPOUT, (unsigned)ly);
-      ts.keep[ly] = keep_of(ly);
-      ts.w_off[ly] = n.layers[ly].w_off; ts.b_off[ly] = n.layers[ly].b_off;
-    }
-    ts.g0 = grad_theta; ts.g1 = nullptr;
-    const TtSide tsd{ln.side[0], ln.ev_fork, ln.ev_join[0]};
-    BRL_CUDA(cudaMemsetAsync(scalars, 0, 2 * sizeof(double), st));
-    if (compute_grads) BRL_CUDA(cudaMemsetAsync(grad_theta, 0, sizeof(float) * n.P, st));
-    tc3_forward(ab.tc3, ts, st, tsd);
-    TtTail tl{};
-    tl.part = ab.tc3.feat; tl.width = 320; tl.y = y; tl.gscale = 0.f; tl.compute_grads = compute_grads; tl.acc = scalars; tl.out = out;
-    tl.dpre = ab.tc3.dfeat;
-    tl.hw_off = n.layers[3].w_off; tl.hb_off = n.layers[3].b_off;
-    tl.loss_kind = 1;
-    tt_tail(ts, tl, st);
-    if (compute_grads) tc3_backward(ab.tc3, ts, st, tsd);
-    BRL_CUDA(cudaGetLastError());
-    return BRL_OK;
-  }
-  FwdArgs fa{x, B, 1, BRL_MODE_DET, theta, nullptr, nullptr, p_dropout, &nz, nullptr, nullptr, out, false};
   run_forward(ctx, ab, fa, st);
   BRL_CUDA(cudaMemsetAsync(scalars, 0, 2 * sizeof(double), st));
   if (compute_grads) {
@@ -1746,7 +1676,7 @@ static int hnn_body(brl_ctx* ctx, const ActBufs& ab, const float* x, const float
   return BRL_OK;
 }
 
-// brl_hnn_step (M = 1) and brl_hnn_step_ensemble: M members in one chain of launches where hnn_batched holds, else one member
+// brl_hnn_step (M = 1) and brl_hnn_step_ensemble: M members in one chain of launches where fused_ok holds, else one member
 // after another on the single-member step
 static int hnn_step(brl_ctx* ctx, const float* x, const float* y, int64_t M, int64_t B, const float* theta, float p_dropout,
                     const brl_noise* noise, int compute_grads, double* scalars, float* grad_theta, float* out,
@@ -1759,7 +1689,7 @@ static int hnn_step(brl_ctx* ctx, const float* x, const float* y, int64_t M, int
   if (!c.ok) return fail(BRL_ERR_WORKSPACE, M == 1 ? "brl_hnn_step: workspace too small" : "brl_hnn_step_ensemble: workspace too small");
   carve_tl(n, c, B, ab);
   carve_members(n, c, B, M, false, ab);
-  if (M > 1 && !hnn_batched(ctx, ab, M, B)) {
+  if (M > 1 && !fused_ok(ctx, ab, M, B)) {
     brl_noise base;
     memset(&base, 0, sizeof(base));
     if (noise) base = *noise;
@@ -1771,78 +1701,22 @@ static int hnn_step(brl_ctx* ctx, const float* x, const float* y, int64_t M, int
     }
     return BRL_OK;
   }
-  // ---- graph replay, same scheme as brl_elbo_step (native dropout masks or no dropout): eager, capture, replay
-  brl_ctx::StepGraph* sg = nullptr;
-  bool caller_captures = false;
-  {
-    cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
-    if (cudaStreamIsCapturing(st, &cs) != cudaSuccess) { cudaGetLastError(); caller_captures = true; }
-    else caller_captures = cs != cudaStreamCaptureStatusNone;
-  }
-  if (ctx->graph_enabled && !caller_captures && noise_is_native(noise)) {
-    brl_ctx::StepKey key;
-    memset(&key, 0, sizeof(key));
-    key.B = B; key.mode = -1 /* HNN */; key.particles = 1; key.compute_grads = compute_grads; key.backend = ctx->gemm_backend;
-    key.members = (int)M;
-    key.prior_loc = p_dropout; key.mu = theta; key.ws = workspace; key.ws_bytes = workspace_bytes;
-    for (auto it = ctx->graphs.begin(); it != ctx->graphs.end(); ++it)
-      if (it->key == key) { ctx->graphs.splice(ctx->graphs.begin(), ctx->graphs, it); sg = &ctx->graphs.front(); break; }
-    if (!sg) {
-      if (ctx->graphs.size() >= 16) {
-        if (ctx->graphs.back().exec) cudaGraphExecDestroy(ctx->graphs.back().exec);
-        ctx->graphs.pop_back();
-      }
-      ctx->graphs.emplace_front();
-      ctx->graphs.front().key = key;
-      sg = &ctx->graphs.front();
-    }
-    ++sg->seen;
-    if (sg->seen >= 2 && !sg->exec && !sg->bad) {
-      cudaGraph_t graph = nullptr;
-      if (cudaStreamBeginCapture(ctx->cap, cudaStreamCaptureModeThreadLocal) == cudaSuccess) {
-        g_dyn = ab.dyn;
-        const long long l0 = launch_count();
-        brl_noise zero;
-        memset(&zero, 0, sizeof(zero));
-        const int rc = hnn_body(ctx, ab, ab.st_x, ab.st_y, M, B, theta, p_dropout, &zero, compute_grads, ab.st_scal,
-                                compute_grads ? ab.st_gmu : nullptr, ab.st_out, ctx->cap);
-        g_dyn = nullptr;
-        sg->launches = (int)(launch_count() - l0);
-        count_launch(-sg->launches);  // captured, not executed
-        const cudaError_t e = cudaStreamEndCapture(ctx->cap, &graph);
-        if (rc != BRL_OK || e != cudaSuccess || !graph || cudaGraphInstantiate(&sg->exec, graph, 0) != cudaSuccess) {
-          sg->exec = nullptr;
-          sg->bad = true;
-        }
-        if (graph) cudaGraphDestroy(graph);
-      } else {
-        sg->bad = true;
-      }
-      cudaGetLastError();
-    }
-  }
-  if (sg && sg->exec) {
-    count_launch(sg->launches);
-    CopyJobs in{};
-    in.dst[0] = ab.st_x; in.src[0] = x; in.n[0] = M * B * 540;
-    in.dst[1] = ab.st_y; in.src[1] = y; in.n[1] = M * B;
-    in.njobs = 2;
-    in.dyn = ab.dyn;
-    in.seed = noise ? noise->seed : 0ull;
-    in.sample0 = noise ? (unsigned long long)noise->sample0 : 0ull;
-    in.window0 = noise ? (unsigned long long)noise->window0 : 0ull;
-    launch_copy_jobs(in, st);
-    BRL_CUDA(cudaGraphLaunch(sg->exec, st));
-    CopyJobs o{};
-    o.dst[0] = reinterpret_cast<float*>(scalars); o.src[0] = reinterpret_cast<const float*>(ab.st_scal); o.n[0] = 4 * M;
-    o.dst[1] = out; o.src[1] = ab.st_out; o.n[1] = M * B * 2;
-    o.njobs = 2;
-    if (compute_grads) { o.dst[2] = grad_theta; o.src[2] = ab.st_gmu; o.n[2] = M * n.P; o.njobs = 3; }
-    launch_copy_jobs(o, st);
-    BRL_CUDA(cudaGetLastError());
-    return BRL_OK;
-  }
-  return hnn_body(ctx, ab, x, y, M, B, theta, p_dropout, noise, compute_grads, scalars, grad_theta, out, st);
+  // graph replay of native dropout masks or no dropout
+  brl_ctx::StepKey key;
+  memset(&key, 0, sizeof(key));
+  key.B = B; key.mode = -1 /* HNN */; key.particles = 1; key.compute_grads = compute_grads; key.backend = ctx->gemm_backend;
+  key.members = (int)M;
+  key.prior_loc = p_dropout; key.mu = theta; key.ws = workspace; key.ws_bytes = workspace_bytes;
+  CopyJobs o{};
+  o.dst[0] = reinterpret_cast<float*>(scalars); o.src[0] = reinterpret_cast<const float*>(ab.st_scal); o.n[0] = 4 * M;
+  o.dst[1] = out; o.src[1] = ab.st_out; o.n[1] = M * B * 2;
+  o.njobs = 2;
+  if (compute_grads) { o.dst[2] = grad_theta; o.src[2] = ab.st_gmu; o.n[2] = M * n.P; o.njobs = 3; }
+  auto body = [&](const float* bx, const float* by, const brl_noise* bnoise, bool staged, cudaStream_t bst) {
+    return hnn_body(ctx, ab, bx, by, M, B, theta, p_dropout, bnoise, compute_grads, staged ? ab.st_scal : scalars,
+                    staged ? (compute_grads ? ab.st_gmu : nullptr) : grad_theta, staged ? ab.st_out : out, bst);
+  };
+  return run_step(ctx, key, noise_is_native(noise), ab, x, y, M * B, noise, o, body, st);
 }
 
 int brl_hnn_step(brl_ctx* ctx, const float* x, const float* y, int64_t B, const float* theta, float p_dropout,
