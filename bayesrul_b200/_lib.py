@@ -75,6 +75,10 @@ SIGNATURES = {
                                     _vp, _vp, _sz, _vp]),
     "brl_hnn_step": (_i, [_vp, _vp, _vp, _i64, _vp, _f, _np, _i, _vp, _vp, _vp, _vp, _sz, _vp]),
     "brl_hnn_step_ensemble": (_i, [_vp, _vp, _vp, _i64, _i64, _vp, _f, _np, _i, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "brl_elbo_train_steps": (_i, [_vp, _vp, _vp, _i64, _vp, _i64, _i64, _i64] + [_vp] * 7 + [_i64] + [_f] * 7 + [_i, _i, _i, _f, _f, _i64,
+                                 C.c_uint64, _i64, _i64, _vp, _vp, _vp, _sz, _vp]),
+    "brl_hnn_train_steps": (_i, [_vp, _vp, _vp, _i64, _vp, _i64, _i64, _i64] + [_vp] * 3 + [_i64] + [_f] * 8 + [C.c_uint64, _i64, _i64,
+                                _vp, _vp, _vp, _sz, _vp]),
     "brl_mixture_moments": (_i, [_vp, _vp, _i64, _i64, _vp, _vp, _vp]),
     "brl_step_metrics": (_i, [_vp, _vp, _vp, _i64, _vp, _vp, _sz, _vp]),
     "brl_step_metrics_ensemble": (_i, [_vp, _vp, _vp, _i64, _i64, _vp, _vp, _sz, _vp]),

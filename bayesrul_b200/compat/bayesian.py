@@ -114,8 +114,8 @@ class BNN(_Base):
         # bnn.predict(aggregate = n > 1) (bayesian.py:149-153): precision-weighted aggregate when n > 1
         return self.bnn.engine.aggregate_predictions(out) if n > 1 else out[0]
 
-    def training_step(self, batch, batch_idx):  # bayesian.py:134-166
-        (x, y) = batch[0], batch[1]
+    def _train_batch(self, x, y):
+        """svi.step on one batch; the values training_step logs (bayesian.py:134-166)."""
         with self.fit_ctxt():
             elbo = self.svi.step(x, y.unsqueeze(-1))
             output = self._agg(self.svi.last["out"], self.hparams.mc_samples_train)
@@ -123,12 +123,72 @@ class BNN(_Base):
             kl = float(self.svi.last["scalars"][2].item())
         m = self.bnn.engine.step_metrics(loc, scale, y)  # mse, sharpness, rmsce (+ nll, mace) in one fused pass (N3)
         mse, sharp, rmsce = m[1].item(), m[2].float(), m[3].float()
-        self.log("mse/train", mse, on_step=False, on_epoch=True)
-        self.log("elbo/train", elbo, on_step=False, on_epoch=True)
-        self.log("kl/train", kl, on_step=False, on_epoch=True)
-        self.log("likelihood/train", elbo - kl, on_step=False, on_epoch=True)
-        self.log("rmsce/train", rmsce, on_step=False, on_epoch=True)
-        self.log("sharp/train", sharp, on_step=False, on_epoch=True)
+        return {"mse/train": mse, "elbo/train": elbo, "kl/train": kl, "likelihood/train": elbo - kl, "rmsce/train": rmsce,
+                "sharp/train": sharp}
+
+    def training_step(self, batch, batch_idx):  # bayesian.py:134-166
+        for k, v in self._train_batch(batch[0], batch[1]).items():
+            self.log(k, v, on_step=False, on_epoch=True)
+
+    def fit_epoch(self, x, y, batch_size: int, generator=None):
+        """One training epoch over the DEVICE-resident split x [N,30,18], y [N]: what Lightning's fit does with training_step
+        over the shuffled batches of a DataLoader, without a host round trip per batch.  The permutation is
+        torch.randperm(N, generator=generator, device=x.device); its floor(N / batch_size) full batches run as ONE
+        Engine.elbo_train_steps call, which continues the seed sequence of the BNN's steps and ClippedAdam's step count and
+        advances both; the remainder batch goes through training_step.  Logs the epoch means of the keys training_step logs,
+        each batch weighted by its size as Lightning's epoch mean weighs it, and returns dict(scalars [K,1,4], metrics [K,1,5],
+        perm) of the K full batches (Engine.elbo_train_steps)."""
+        N, bs = int(x.shape[0]), int(batch_size)
+        if bs <= 0 or y.numel() != N:
+            raise RuntimeError("bayesrul_b200: fit_epoch needs batch_size > 0 and one target per window")
+        bnn, svi = self.bnn, self.svi
+        opt, g = svi.optim, bnn.net_guide
+        grad_factor = svi.model_scale / (1.0 / (bnn.likelihood.dataset_size * 30 * 18))  # what SVI.step multiplies the gradients by
+        if svi.no_obs or grad_factor != 1.0 or not (hasattr(opt, "step_vi") and g.loc.is_contiguous() and g.log_scale.is_contiguous()):
+            raise RuntimeError("bayesrul_b200: fit_epoch runs the ClippedAdam step of a mean-field guide at the ELBO's own scale")
+        perm = torch.randperm(N, generator=generator, device=x.device)
+        K = N // bs
+        x, y = x.contiguous(), y.reshape(-1).contiguous()
+        res = None
+        sums, weight = {}, 0
+        if K > 0:
+            with self.fit_ctxt():
+                ctx = tyxe.active_context()
+            mode = ctx if (ctx and g.family == "normal") else "ws"
+            be = bnn.train_backend
+            if be == "auto":
+                be = "fused" if getattr(self.net, "kind", "") == "inception" else "simt"
+            eng = bnn.engine
+            eng.set_gemm_backend(be)
+            sts = [opt._slot(name, p) for name, p in (("loc", g.loc), ("log_scale", g.log_scale))]
+            a = opt.args
+            res = eng.elbo_train_steps(x, y, perm[: K * bs].view(K, bs), g.loc, g.log_scale, g.scale,
+                                       (sts[0]["m"], sts[0]["v"], sts[1]["m"], sts[1]["v"]), step0=sts[0]["step"], lr=a["lr"],
+                                       betas=tuple(a["betas"]), eps=a["eps"], clip_norm=a["clip_norm"], lrd=a["lrd"],
+                                       weight_decay=a["weight_decay"], mode=mode, guide=g.family,
+                                       particles=self.hparams.mc_samples_train, prior_loc=bnn.prior.loc, prior_scale=bnn.prior.scale,
+                                       dataset_size=bnn.likelihood.dataset_size,
+                                       seed=(bnn.seed + 0x9E3779B97F4A7C15 * bnn._step) & 0xFFFFFFFFFFFFFFFF)
+            bnn._step += K
+            for st in sts:
+                st["step"] += K
+            bnn._last_kl = res["scalars"][K - 1, 0, 2]
+            sc, mt = res["scalars"][:, 0], res["metrics"][:, 0]
+            elbo, kl = sc[:, 0].sum(), sc[:, 2].sum()
+            sums = {"mse/train": mt[:, 1].sum(), "elbo/train": elbo, "kl/train": kl, "likelihood/train": elbo - kl,
+                    "rmsce/train": mt[:, 3].float().double().sum(), "sharp/train": mt[:, 2].float().double().sum()}  # logged as float32
+            sums = {k: v * bs for k, v in sums.items()}
+            weight = K * bs
+        if K * bs < N:
+            rest = perm[K * bs:]
+            vals = self._train_batch(x[rest], y[rest])
+            for k, v in vals.items():
+                sums[k] = sums.get(k, 0.0) + v * rest.numel()
+            weight += rest.numel()
+        means = torch.stack([torch.as_tensor(v, dtype=torch.float64, device=x.device) for v in sums.values()]).div(weight).tolist()
+        for k, v in zip(sums, means):
+            self.log(k, v, on_step=False, on_epoch=True)
+        return dict(scalars=res["scalars"] if res else None, metrics=res["metrics"] if res else None, perm=perm)
 
     def validation_step(self, batch, batch_idx):  # bayesian.py:168-197 (no fit context: weight sampling)
         (x, y) = batch[0], batch[1]

@@ -2,6 +2,8 @@
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
+#include <cstddef>
+#include <cstdint>
 #include <cstring>
 #include <stdexcept>
 #include <list>
@@ -94,11 +96,16 @@ struct brl_ctx {
     float prior_loc, prior_scale;
     const void *mu, *sigma, *ws;
     size_t ws_bytes;
+    // brl_elbo_train_steps / brl_hnn_train_steps (train = 5 / 6; 0: a single step): the step's optimizer hyper-parameters
+    // {beta1, beta2, eps, clip_norm, weight_decay} and its other state buffers, baked into the captured optimizer launch
+    int train;
+    float opt[5];
+    const void* state[5];
     bool operator==(const StepKey& o) const {
       return B == o.B && dataset_size == o.dataset_size && mode == o.mode && guide == o.guide && particles == o.particles &&
              compute_grads == o.compute_grads && backend == o.backend && has_log_sigma == o.has_log_sigma && members == o.members &&
              prior_loc == o.prior_loc && prior_scale == o.prior_scale && mu == o.mu && sigma == o.sigma && ws == o.ws &&
-             ws_bytes == o.ws_bytes;
+             ws_bytes == o.ws_bytes && train == o.train && !memcmp(opt, o.opt, sizeof(opt)) && !memcmp(state, o.state, sizeof(state));
     }
   };
   struct StepGraph { StepKey key; cudaGraphExec_t exec = nullptr; int seen = 0, launches = 0; bool bad = false; };
@@ -252,6 +259,30 @@ static void carve_members(const NetSpec& n, Carve& c, long long B, long long M, 
     ab.acc = e.acc;
     ab.st_gsig = e.st_gsig; ab.st_glog = e.st_glog;
   }
+}
+
+// brl_elbo_train_steps / brl_hnn_train_steps: the call's descriptor, the gathered batch and one step's gradients, outputs, logged
+// predictions, scalars and metrics, in front of the workspace of the step itself (brl_workspace_bytes codes 3 / 4, or 1 for M = 1)
+struct TrainBufs {
+  TrainDesc* d;
+  float *xb, *yb, *g0, *g1, *g2, *out, *agg, *pred, *std;
+  double *scal, *met;
+  unsigned int* hist;
+};
+static void carve_train_steps(const NetSpec& n, Carve& c, long long M, long long B, bool elbo, TrainBufs& t) {
+  t.d = c.take<TrainDesc>(1);
+  t.xb = c.take<float>(M * B * 540);
+  t.yb = c.take<float>(M * B);
+  t.g0 = c.take<float>(M * n.P);
+  t.g1 = elbo ? c.take<float>(M * n.P) : nullptr;
+  t.g2 = elbo ? c.take<float>(M * n.P) : nullptr;
+  t.out = c.take<float>((elbo ? GRAPH_MAX_PARTICLES : 1) * M * B * 2);
+  t.agg = elbo ? c.take<float>(M * B * 2) : nullptr;
+  t.pred = c.take<float>(M * B);
+  t.std = c.take<float>(M * B);
+  t.scal = c.take<double>((elbo ? 4 : 2) * M);
+  t.met = c.take<double>(5 * M);
+  t.hist = c.take<unsigned int>(256 * M);  // the step metrics' scratch, 1024 bytes per member
 }
 
 // device {seed, sample0, window0} of the step being captured (nullptr outside a capture): every Philox stream built by
@@ -602,6 +633,50 @@ static int zero_grads(const NetSpec& n, const ActBufs& ab, long long B, cudaStre
   return BRL_OK;
 }
 
+// the caller is capturing `st` itself (e.g. torch.cuda.graph): stay on the eager, capturable path
+static bool stream_capturing(cudaStream_t st) {
+  cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+  if (cudaStreamIsCapturing(st, &cs) != cudaSuccess) { cudaGetLastError(); return true; }
+  return cs != cudaStreamCaptureStatusNone;
+}
+
+// the context's captured step for `key` (most recently used first, at most 16), a new empty one on first sight
+static brl_ctx::StepGraph* graph_slot(brl_ctx* ctx, const brl_ctx::StepKey& key) {
+  for (auto it = ctx->graphs.begin(); it != ctx->graphs.end(); ++it)
+    if (it->key == key) { ctx->graphs.splice(ctx->graphs.begin(), ctx->graphs, it); return &ctx->graphs.front(); }
+  if (ctx->graphs.size() >= 16) {
+    if (ctx->graphs.back().exec) cudaGraphExecDestroy(ctx->graphs.back().exec);
+    ctx->graphs.pop_back();
+  }
+  ctx->graphs.emplace_front();
+  ctx->graphs.front().key = key;
+  return &ctx->graphs.front();
+}
+
+// captures issue(stream) into sg (on `cap`, since the caller's stream may be the legacy default stream), every Philox stream
+// reading the per-step part of its key from `dyn`; a failed capture marks sg bad, and the caller stays eager
+template <class Issue>
+static void capture_step(brl_ctx* ctx, brl_ctx::StepGraph* sg, const unsigned long long* dyn, Issue issue) {
+  cudaGraph_t graph = nullptr;
+  if (cudaStreamBeginCapture(ctx->cap, cudaStreamCaptureModeThreadLocal) == cudaSuccess) {
+    g_dyn = dyn;
+    const long long l0 = launch_count();
+    const int rc = issue(ctx->cap);
+    g_dyn = nullptr;
+    sg->launches = (int)(launch_count() - l0);
+    count_launch(-sg->launches);  // captured, not executed
+    const cudaError_t e = cudaStreamEndCapture(ctx->cap, &graph);
+    if (rc != BRL_OK || e != cudaSuccess || !graph || cudaGraphInstantiate(&sg->exec, graph, 0) != cudaSuccess) {
+      sg->exec = nullptr;
+      sg->bad = true;
+    }
+    if (graph) cudaGraphDestroy(graph);
+  } else {
+    sg->bad = true;
+  }
+  cudaGetLastError();  // a failed capture must not poison the eager path
+}
+
 // Graph replay of a training step whose configuration is `key`, where `graphable` (native Philox noise): eager on first sight of
 // the key, captured on the second, replayed after.  body(x, y, noise, staged, stream) issues the step's launches; `staged` selects
 // the outputs among ab's staging buffers instead of the caller's.  The capture runs it over the staging inputs with the Philox key
@@ -610,48 +685,15 @@ template <class Body>
 static int run_step(brl_ctx* ctx, const brl_ctx::StepKey& key, bool graphable, const ActBufs& ab, const float* x, const float* y,
                     long long MB, const brl_noise* noise, CopyJobs out, Body body, cudaStream_t st) {
   brl_ctx::StepGraph* sg = nullptr;
-  bool caller_captures = false;  // the caller is capturing `st` itself (e.g. torch.cuda.graph): stay on the eager, capturable path
-  {
-    cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
-    if (cudaStreamIsCapturing(st, &cs) != cudaSuccess) { cudaGetLastError(); caller_captures = true; }
-    else caller_captures = cs != cudaStreamCaptureStatusNone;
-  }
-  if (ctx->graph_enabled && !caller_captures && graphable) {
-    for (auto it = ctx->graphs.begin(); it != ctx->graphs.end(); ++it)
-      if (it->key == key) { ctx->graphs.splice(ctx->graphs.begin(), ctx->graphs, it); sg = &ctx->graphs.front(); break; }
-    if (!sg) {
-      if (ctx->graphs.size() >= 16) {
-        if (ctx->graphs.back().exec) cudaGraphExecDestroy(ctx->graphs.back().exec);
-        ctx->graphs.pop_back();
-      }
-      ctx->graphs.emplace_front();
-      ctx->graphs.front().key = key;
-      sg = &ctx->graphs.front();
-    }
+  if (ctx->graph_enabled && graphable && !stream_capturing(st)) {
+    sg = graph_slot(ctx, key);
     ++sg->seen;
-    if (sg->seen >= 2 && !sg->exec && !sg->bad) {
-      cudaGraph_t graph = nullptr;
-      // on `cap`, since the caller's stream may be the legacy default stream
-      if (cudaStreamBeginCapture(ctx->cap, cudaStreamCaptureModeThreadLocal) == cudaSuccess) {
-        g_dyn = ab.dyn;
-        const long long l0 = launch_count();
+    if (sg->seen >= 2 && !sg->exec && !sg->bad)
+      capture_step(ctx, sg, ab.dyn, [&](cudaStream_t cs) {
         brl_noise zero;
         memset(&zero, 0, sizeof(zero));
-        const int rc = body(ab.st_x, ab.st_y, &zero, true, ctx->cap);
-        g_dyn = nullptr;
-        sg->launches = (int)(launch_count() - l0);
-        count_launch(-sg->launches);  // captured, not executed
-        const cudaError_t e = cudaStreamEndCapture(ctx->cap, &graph);
-        if (rc != BRL_OK || e != cudaSuccess || !graph || cudaGraphInstantiate(&sg->exec, graph, 0) != cudaSuccess) {
-          sg->exec = nullptr;
-          sg->bad = true;
-        }
-        if (graph) cudaGraphDestroy(graph);
-      } else {
-        sg->bad = true;
-      }
-      cudaGetLastError();  // a failed capture must not poison the eager path below
-    }
+        return body(ab.st_x, ab.st_y, &zero, true, cs);
+      });
   }
   if (!sg || !sg->exec) return body(x, y, noise, false, st);
   count_launch(sg->launches);
@@ -668,6 +710,13 @@ static int run_step(brl_ctx* ctx, const brl_ctx::StepKey& key, bool graphable, c
   launch_copy_jobs(out, st);
   BRL_CUDA(cudaGetLastError());
   return BRL_OK;
+}
+
+// the step size of ClippedAdam step `step` (>= 1): lr lrd^step sqrt(1 - beta2^step) / (1 - beta1^step), in double, rounded once
+static float adam_step_size(float lr, float lrd, float beta1, float beta2, long long step) {
+  const double lr_t = (double)lr * std::pow((double)lrd, (double)step);
+  const double bc1 = 1.0 - std::pow((double)beta1, (double)step), bc2 = 1.0 - std::pow((double)beta2, (double)step);
+  return (float)(lr_t * std::sqrt(bc2) / bc1);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -882,6 +931,13 @@ int64_t brl_workspace_bytes(const brl_ctx* ctx, int64_t B, int64_t S, int train,
   const NetSpec& n = *ctx->net;
   Carve c(nullptr, 0);
   ActBufs ab;
+  if (train == 5 || train == 6) {  // brl_elbo_train_steps / brl_hnn_train_steps: their buffers, then the step's workspace
+    TrainBufs t;
+    carve_train_steps(n, c, S, B, train == 5, t);
+    const int64_t step = train == 5 ? (S == 1 ? brl_workspace_bytes(ctx, B, 2, 1, 0) : brl_workspace_bytes(ctx, B, S, 4, 0))
+                                    : (S == 1 ? brl_workspace_bytes(ctx, B, 1, 1, 0) : brl_workspace_bytes(ctx, B, S, 3, 0));
+    return (int64_t)c.used + step;
+  }
   if (train == 3 || train == 4) {  // brl_hnn_step_ensemble / brl_elbo_step_ensemble over S members: the layout of their steps
     carve_forward(n, c, B, 1, ab);
     carve_train(n, c, B, ab);
@@ -1536,7 +1592,8 @@ int brl_set_step_graph(brl_ctx* ctx, int enable) {
 static int elbo_step(brl_ctx* ctx, const float* x, const float* y, int64_t M, int64_t B, const float* mu, const float* sigma,
                      int mode, int guide, int particles, float prior_loc, float prior_scale, int64_t dataset_size,
                      const brl_noise* noise, int compute_grads, double* scalars, float* grad_mu, float* grad_sigma,
-                     float* grad_log_sigma, float* out, void* workspace, size_t workspace_bytes, cudaStream_t st) {
+                     float* grad_log_sigma, float* out, void* workspace, size_t workspace_bytes, cudaStream_t st,
+                     bool graphs = true) {
   const NetSpec& n = *ctx->net;
   Carve c(workspace, workspace_bytes);
   ActBufs ab;
@@ -1559,7 +1616,7 @@ static int elbo_step(brl_ctx* ctx, const float* x, const float* y, int64_t M, in
                                  prior_loc, prior_scale, dataset_size, &nm, compute_grads, scalars + 4 * m,
                                  compute_grads ? grad_mu + m * n.P : nullptr, compute_grads ? grad_sigma + m * n.P : nullptr,
                                  (compute_grads && grad_log_sigma) ? grad_log_sigma + m * n.P : nullptr,
-                                 out + m * particles * B * 2, workspace, workspace_bytes, st);
+                                 out + m * particles * B * 2, workspace, workspace_bytes, st, graphs);
         if (rc != BRL_OK) return rc;
       }
       return BRL_OK;
@@ -1603,7 +1660,7 @@ static int elbo_step(brl_ctx* ctx, const float* x, const float* y, int64_t M, in
                      staged ? ((compute_grads && grad_log_sigma) ? ab.st_glog : nullptr) : grad_log_sigma,
                      staged ? ab.st_out : out, bst);
   };
-  return run_step(ctx, key, noise_is_native(noise) && particles <= GRAPH_MAX_PARTICLES, ab, x, y, M * B, noise, o, body, st);
+  return run_step(ctx, key, graphs && noise_is_native(noise) && particles <= GRAPH_MAX_PARTICLES, ab, x, y, M * B, noise, o, body, st);
 }
 
 int brl_elbo_step(brl_ctx* ctx, const float* x, const float* y, int64_t B, const float* mu, const float* sigma, int mode,
@@ -1680,7 +1737,7 @@ static int hnn_body(brl_ctx* ctx, const ActBufs& ab, const float* x, const float
 // after another on the single-member step
 static int hnn_step(brl_ctx* ctx, const float* x, const float* y, int64_t M, int64_t B, const float* theta, float p_dropout,
                     const brl_noise* noise, int compute_grads, double* scalars, float* grad_theta, float* out,
-                    void* workspace, size_t workspace_bytes, cudaStream_t st) {
+                    void* workspace, size_t workspace_bytes, cudaStream_t st, bool graphs = true) {
   const NetSpec& n = *ctx->net;
   Carve c(workspace, workspace_bytes);
   ActBufs ab;
@@ -1696,7 +1753,7 @@ static int hnn_step(brl_ctx* ctx, const float* x, const float* y, int64_t M, int
     for (int64_t m = 0; m < M; ++m) {
       const brl_noise nm = noise_at_sample(n, &base, m, B);  // MC-sample index sample0 + m, injected masks of member m
       const int rc = hnn_step(ctx, x + m * B * 540, y + m * B, 1, B, theta + m * n.P, p_dropout, &nm, compute_grads, scalars + 2 * m,
-                              compute_grads ? grad_theta + m * n.P : nullptr, out + m * B * 2, workspace, workspace_bytes, st);
+                              compute_grads ? grad_theta + m * n.P : nullptr, out + m * B * 2, workspace, workspace_bytes, st, graphs);
       if (rc != BRL_OK) return rc;
     }
     return BRL_OK;
@@ -1716,7 +1773,7 @@ static int hnn_step(brl_ctx* ctx, const float* x, const float* y, int64_t M, int
     return hnn_body(ctx, ab, bx, by, M, B, theta, p_dropout, bnoise, compute_grads, staged ? ab.st_scal : scalars,
                     staged ? (compute_grads ? ab.st_gmu : nullptr) : grad_theta, staged ? ab.st_out : out, bst);
   };
-  return run_step(ctx, key, noise_is_native(noise), ab, x, y, M * B, noise, o, body, st);
+  return run_step(ctx, key, graphs && noise_is_native(noise), ab, x, y, M * B, noise, o, body, st);
 }
 
 int brl_hnn_step(brl_ctx* ctx, const float* x, const float* y, int64_t B, const float* theta, float p_dropout,
@@ -1739,6 +1796,172 @@ int brl_hnn_step_ensemble(brl_ctx* ctx, const float* x, const float* y, int64_t 
   BRL_REQUIRE(!compute_grads || grad_theta, "brl_hnn_step_ensemble: grad_theta is NULL");
   return hnn_step(ctx, x, y, M, B, theta, p_dropout, noise, compute_grads, scalars, grad_theta, out, workspace, workspace_bytes,
                   (cudaStream_t)stream);
+}
+
+}  // extern "C"
+
+// ---- K training steps per call ----------------------------------------------------------------------------------------------
+struct TrainArgs {
+  const float *X, *Y;
+  long long N;
+  const int64_t* idx;
+  long long K, M, B, step0;
+  float lr, beta1, beta2, eps, clip_norm, lrd, weight_decay;
+  uint64_t seed;
+  long long sample0, window0;
+  double *scalars, *metrics;
+};
+
+static int train_args_ok(const char* fn, const TrainArgs& a) {
+  BRL_REQUIRE(a.X && a.Y && a.idx && a.scalars && a.metrics, std::string(fn) + ": NULL argument");
+  BRL_REQUIRE(a.N > 0 && a.K > 0 && a.M > 0 && a.M < (1 << 16) && a.B > 0 && a.step0 >= 0, std::string(fn) + ": bad N, K, M, B or step0");
+  BRL_REQUIRE(((uintptr_t)a.X & 15) == 0, std::string(fn) + ": X must be 16-byte aligned");
+  return BRL_OK;
+}
+
+// Step k of the call is body(noise, stream): gather -> step -> optimizer -> metrics -> row k.  With graphs on and nobody capturing
+// `st`, the first step of a configuration runs eagerly, the second is captured (the Philox key read from the descriptor) and every
+// later step, in this call or a later one, is one graph launch.  Every TRAIN_TABLE steps one setup launch writes the descriptor
+// and the next table of Adam step sizes, computed here as brl_clipped_adam{,_vi} computes them.  Nothing synchronises the host.
+template <class Body>
+static int train_steps(brl_ctx* ctx, const TrainArgs& a, const brl_ctx::StepKey& key, const TrainBufs& t, Body body, cudaStream_t st) {
+  brl_ctx::StepGraph* sg = ctx->graph_enabled && !stream_capturing(st) ? graph_slot(ctx, key) : nullptr;
+  const unsigned long long* dyn = reinterpret_cast<const unsigned long long*>(reinterpret_cast<const char*>(t.d) + offsetof(TrainDesc, dyn));
+  TrainSetup su;
+  su.d = t.d; su.X = a.X; su.Y = a.Y; su.idx = reinterpret_cast<const long long*>(a.idx); su.scalars = a.scalars; su.metrics = a.metrics;
+  su.N = a.N; su.seed = a.seed; su.sample0 = (unsigned long long)a.sample0; su.window0 = (unsigned long long)a.window0;
+  for (long long k = 0; k < a.K; ++k) {
+    if (k % TRAIN_TABLE == 0) {
+      su.k0 = k;
+      su.n = (int)std::min<long long>(TRAIN_TABLE, a.K - k);
+      for (int i = 0; i < su.n; ++i) su.steps[i] = adam_step_size(a.lr, a.lrd, a.beta1, a.beta2, a.step0 + k + i + 1);
+      launch_train_setup(su, st);
+    }
+    if (sg && !sg->exec && !sg->bad && sg->seen >= 1)
+      capture_step(ctx, sg, dyn, [&](cudaStream_t cs) {
+        brl_noise zero;
+        memset(&zero, 0, sizeof(zero));
+        return body(&zero, cs);
+      });
+    if (sg && sg->exec) {
+      count_launch(sg->launches);
+      BRL_CUDA(cudaGraphLaunch(sg->exec, st));
+    } else {
+      brl_noise nz;
+      memset(&nz, 0, sizeof(nz));
+      nz.seed = a.seed + 0x9E3779B97F4A7C15ull * (uint64_t)(k + 1);
+      nz.sample0 = a.sample0;
+      nz.window0 = a.window0;
+      const int rc = body(&nz, st);
+      if (rc != BRL_OK) return rc;
+    }
+    if (sg) ++sg->seen;
+  }
+  BRL_CUDA(cudaGetLastError());
+  return BRL_OK;
+}
+
+// the logged step metrics of M members from their (loc, scale) pairs at src + m mstride, then row k of the results
+static void train_metrics_tail(const TrainBufs& t, const float* src, long long mstride, long long M, long long B, int nscal,
+                               cudaStream_t st) {
+  launch_split_pred(src, mstride, (int)M, B, t.pred, t.std, st);
+  launch_test_metrics(t.pred, t.std, t.yb, B, t.met, t.hist, st, 5, (int)M);
+  launch_train_tail(t.d, t.scal, nscal, t.met, (int)M, st);
+}
+
+extern "C" {
+
+int brl_elbo_train_steps(brl_ctx* ctx, const float* X, const float* Y, int64_t N, const int64_t* idx, int64_t K, int64_t M, int64_t B,
+                         float* loc, float* log_scale, float* scale, float* m_loc, float* v_loc, float* m_log_scale,
+                         float* v_log_scale, int64_t step0, float lr, float beta1, float beta2, float eps, float clip_norm, float lrd,
+                         float weight_decay, int mode, int guide, int particles, float prior_loc, float prior_scale,
+                         int64_t dataset_size, uint64_t seed, int64_t sample0, int64_t window0, double* scalars, double* metrics,
+                         void* workspace, size_t workspace_bytes, void* stream) {
+  BRL_REQUIRE(ctx && loc && log_scale && scale && m_loc && v_loc && m_log_scale && v_log_scale && workspace,
+              "brl_elbo_train_steps: NULL argument");
+  DeviceGuard dg(ctx->device);
+  const TrainArgs a{X, Y, N, idx, K, M, B, step0, lr, beta1, beta2, eps, clip_norm, lrd, weight_decay, seed, sample0, window0,
+                    scalars, metrics};
+  if (int rc = train_args_ok("brl_elbo_train_steps", a)) return rc;
+  BRL_REQUIRE(particles > 0 && particles <= GRAPH_MAX_PARTICLES && dataset_size > 0 && prior_scale > 0.f,
+              "brl_elbo_train_steps: bad particles (1 to 8), dataset size or prior scale");
+  BRL_REQUIRE(guide == BRL_GUIDE_NORMAL || guide == BRL_GUIDE_RADIAL, "Guide unknown. Choose from 'normal', 'radial'.");
+  BRL_REQUIRE(mode == BRL_MODE_WS || mode == BRL_MODE_LRT || mode == BRL_MODE_FLIPOUT, "brl_elbo_train_steps: mode must be WS, LRT or FLIPOUT");
+  if (guide == BRL_GUIDE_RADIAL) mode = BRL_MODE_WS;  // bayesian.py:81-83: radial forces nullcontext
+  const int64_t need = brl_workspace_bytes(ctx, B, M, 5, 0);
+  if ((int64_t)workspace_bytes < need)
+    return fail(BRL_ERR_WORKSPACE, "brl_elbo_train_steps: workspace too small; need " + std::to_string(need) + " bytes");
+  const NetSpec& n = *ctx->net;
+  Carve c(workspace, workspace_bytes);
+  TrainBufs t;
+  carve_train_steps(n, c, M, B, true, t);
+  char* sws = (char*)workspace + c.used;
+  const size_t sws_bytes = workspace_bytes - c.used;
+  brl_ctx::StepKey key;
+  memset(&key, 0, sizeof(key));
+  key.B = B; key.dataset_size = dataset_size; key.mode = mode; key.guide = guide; key.particles = particles;
+  key.compute_grads = 1; key.backend = ctx->gemm_backend; key.has_log_sigma = 1; key.members = (int)M;
+  key.prior_loc = prior_loc; key.prior_scale = prior_scale; key.mu = loc; key.sigma = scale; key.ws = workspace;
+  key.ws_bytes = workspace_bytes; key.train = 5;
+  const float opt[5] = {beta1, beta2, eps, clip_norm, weight_decay};
+  memcpy(key.opt, opt, sizeof(opt));
+  const void* state[5] = {log_scale, m_loc, v_loc, m_log_scale, v_log_scale};
+  memcpy(key.state, state, sizeof(state));
+  auto body = [&](const brl_noise* nz, cudaStream_t s) {
+    launch_train_gather(t.d, t.xb, t.yb, M * B, s);
+    const int rc = elbo_step(ctx, t.xb, t.yb, M, B, loc, scale, mode, guide, particles, prior_loc, prior_scale, dataset_size, nz, 1,
+                             t.scal, t.g0, t.g1, t.g2, t.out, sws, sws_bytes, s, false);
+    if (rc != BRL_OK) return rc;
+    launch_clipped_adam_vi(loc, log_scale, scale, t.g0, t.g2, m_loc, v_loc, m_log_scale, v_log_scale, M * n.P, t.d, beta1, beta2,
+                           eps, clip_norm, weight_decay, s);
+    if (particles == 1) {
+      train_metrics_tail(t, t.out, B * 2, M, B, 4, s);
+    } else {  // BNN._agg: the precision-weighted aggregate of each member's particles
+      for (int64_t m = 0; m < M; ++m) launch_aggregate(t.out + m * particles * B * 2, particles, B, t.agg + m * B * 2, s);
+      train_metrics_tail(t, t.agg, B * 2, M, B, 4, s);
+    }
+    BRL_CUDA(cudaGetLastError());
+    return BRL_OK;
+  };
+  return train_steps(ctx, a, key, t, body, (cudaStream_t)stream);
+}
+
+int brl_hnn_train_steps(brl_ctx* ctx, const float* X, const float* Y, int64_t N, const int64_t* idx, int64_t K, int64_t M, int64_t B,
+                        float* theta, float* exp_avg, float* exp_avg_sq, int64_t step0, float lr, float beta1, float beta2, float eps,
+                        float clip_norm, float lrd, float weight_decay, float p_dropout, uint64_t seed, int64_t sample0,
+                        int64_t window0, double* scalars, double* metrics, void* workspace, size_t workspace_bytes, void* stream) {
+  BRL_REQUIRE(ctx && theta && exp_avg && exp_avg_sq && workspace, "brl_hnn_train_steps: NULL argument");
+  DeviceGuard dg(ctx->device);
+  const TrainArgs a{X, Y, N, idx, K, M, B, step0, lr, beta1, beta2, eps, clip_norm, lrd, weight_decay, seed, sample0, window0,
+                    scalars, metrics};
+  if (int rc = train_args_ok("brl_hnn_train_steps", a)) return rc;
+  BRL_REQUIRE(p_dropout >= 0.f && p_dropout < 1.f, "brl_hnn_train_steps: bad p_dropout");
+  const int64_t need = brl_workspace_bytes(ctx, B, M, 6, 0);
+  if ((int64_t)workspace_bytes < need)
+    return fail(BRL_ERR_WORKSPACE, "brl_hnn_train_steps: workspace too small; need " + std::to_string(need) + " bytes");
+  const NetSpec& n = *ctx->net;
+  Carve c(workspace, workspace_bytes);
+  TrainBufs t;
+  carve_train_steps(n, c, M, B, false, t);
+  char* sws = (char*)workspace + c.used;
+  const size_t sws_bytes = workspace_bytes - c.used;
+  brl_ctx::StepKey key;
+  memset(&key, 0, sizeof(key));
+  key.B = B; key.mode = -1 /* HNN */; key.particles = 1; key.compute_grads = 1; key.backend = ctx->gemm_backend;
+  key.members = (int)M; key.prior_loc = p_dropout; key.mu = theta; key.ws = workspace; key.ws_bytes = workspace_bytes; key.train = 6;
+  const float opt[5] = {beta1, beta2, eps, clip_norm, weight_decay};
+  memcpy(key.opt, opt, sizeof(opt));
+  key.state[0] = exp_avg; key.state[1] = exp_avg_sq;
+  auto body = [&](const brl_noise* nz, cudaStream_t s) {
+    launch_train_gather(t.d, t.xb, t.yb, M * B, s);
+    const int rc = hnn_step(ctx, t.xb, t.yb, M, B, theta, p_dropout, nz, 1, t.scal, t.g0, t.out, sws, sws_bytes, s, false);
+    if (rc != BRL_OK) return rc;
+    launch_clipped_adam(theta, t.g0, exp_avg, exp_avg_sq, M * n.P, t.d, beta1, beta2, eps, clip_norm, weight_decay, s);
+    train_metrics_tail(t, t.out, B * 2, M, B, 2, s);
+    BRL_CUDA(cudaGetLastError());
+    return BRL_OK;
+  };
+  return train_steps(ctx, a, key, t, body, (cudaStream_t)stream);
 }
 
 int brl_mixture_moments(const float* mu_m, const float* sigma_m, int64_t M, int64_t nn, float* mu, float* sigma, void* stream) {
@@ -1779,9 +2002,7 @@ int brl_step_metrics_ensemble(const float* pred, const float* std, const float* 
 int brl_clipped_adam(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, int64_t nn, int64_t step, float lr,
                      float beta1, float beta2, float eps, float clip_norm, float lrd, float weight_decay, void* stream) {
   BRL_REQUIRE(param && grad && exp_avg && exp_avg_sq && nn > 0 && step >= 1, "brl_clipped_adam: bad argument");
-  const double lr_t = (double)lr * std::pow((double)lrd, (double)step);
-  const double bc1 = 1.0 - std::pow((double)beta1, (double)step), bc2 = 1.0 - std::pow((double)beta2, (double)step);
-  launch_clipped_adam(param, grad, exp_avg, exp_avg_sq, nn, (float)(lr_t * std::sqrt(bc2) / bc1), beta1, beta2, eps,
+  launch_clipped_adam(param, grad, exp_avg, exp_avg_sq, nn, adam_step_size(lr, lrd, beta1, beta2, step), beta1, beta2, eps,
                       clip_norm, weight_decay, (cudaStream_t)stream);
   BRL_CUDA(cudaGetLastError());
   return BRL_OK;
@@ -1793,10 +2014,9 @@ int brl_clipped_adam_vi_scaled(float* loc, float* log_scale, float* scale, const
                                void* stream) {
   BRL_REQUIRE(loc && log_scale && scale && grad_loc && grad_log_scale && m_loc && v_loc && m_log_scale && v_log_scale && nn > 0 && step >= 1,
               "brl_clipped_adam_vi_scaled: bad argument");
-  const double lr_t = (double)lr * std::pow((double)lrd, (double)step);
-  const double bc1 = 1.0 - std::pow((double)beta1, (double)step), bc2 = 1.0 - std::pow((double)beta2, (double)step);
   launch_clipped_adam_vi(loc, log_scale, scale, grad_loc, grad_log_scale, m_loc, v_loc, m_log_scale, v_log_scale, nn,
-                         (float)(lr_t * std::sqrt(bc2) / bc1), beta1, beta2, eps, clip_norm, weight_decay, (cudaStream_t)stream, grad_scale);
+                         adam_step_size(lr, lrd, beta1, beta2, step), beta1, beta2, eps, clip_norm, weight_decay, (cudaStream_t)stream,
+                         grad_scale);
   BRL_CUDA(cudaGetLastError());
   return BRL_OK;
 }
@@ -1806,10 +2026,8 @@ int brl_clipped_adam_vi(float* loc, float* log_scale, float* scale, const float*
                         float beta1, float beta2, float eps, float clip_norm, float lrd, float weight_decay, void* stream) {
   BRL_REQUIRE(loc && log_scale && scale && grad_loc && grad_log_scale && m_loc && v_loc && m_log_scale && v_log_scale && nn > 0 && step >= 1,
               "brl_clipped_adam_vi: bad argument");
-  const double lr_t = (double)lr * std::pow((double)lrd, (double)step);
-  const double bc1 = 1.0 - std::pow((double)beta1, (double)step), bc2 = 1.0 - std::pow((double)beta2, (double)step);
   launch_clipped_adam_vi(loc, log_scale, scale, grad_loc, grad_log_scale, m_loc, v_loc, m_log_scale, v_log_scale, nn,
-                         (float)(lr_t * std::sqrt(bc2) / bc1), beta1, beta2, eps, clip_norm, weight_decay, (cudaStream_t)stream);
+                         adam_step_size(lr, lrd, beta1, beta2, step), beta1, beta2, eps, clip_norm, weight_decay, (cudaStream_t)stream);
   BRL_CUDA(cudaGetLastError());
   return BRL_OK;
 }

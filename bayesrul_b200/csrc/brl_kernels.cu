@@ -2,6 +2,7 @@
 // gather prologue and the epilogue, plus the small reductions of the ELBO / predictive path.
 // This is the parity engine (rtol 1e-3 vs the oracle); the tcgen05 engine lives in brl_tc.cu.
 #include <atomic>
+#include <cstddef>
 
 #include "brl_kernels.cuh"
 #include "brl_philox.cuh"
@@ -711,9 +712,22 @@ void launch_test_metrics(const float* pred, const float* std, const float* y, lo
 // ------------------------------------------------------------------------------------------------
 // ClippedAdam
 // ------------------------------------------------------------------------------------------------
+// The step size comes from the host (HostStep: brl_clipped_adam{,_vi}) or from a device table at a device index (DevStep: step k
+// of brl_{elbo,hnn}_train_steps, whose launches are replayed from one graph)
+struct HostStep {
+  float v;
+  __device__ __forceinline__ float get() const { return v; }
+};
+struct DevStep {
+  const float* tab;
+  const int* at;
+  __device__ __forceinline__ float get() const { return tab[*at]; }
+};
+template <class Step>
 __global__ void clipped_adam_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m,
-                                    float* __restrict__ v, long long n, float step_size, float b1, float b2, float eps,
+                                    float* __restrict__ v, long long n, Step ss, float b1, float b2, float eps,
                                     float clip, float wd) {
+  const float step_size = ss.get();
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
     float gr = fminf(fmaxf(g[i], -clip), clip);
     const float pi = p[i];
@@ -727,10 +741,12 @@ __global__ void clipped_adam_kernel(float* __restrict__ p, const float* __restri
 }
 // the optimiser step of a mean-field guide in one launch: ClippedAdam on loc and on log scale (the unconstrained parameter of
 // Pyro's positive constraint), then scale = exp(log scale) for the next forward pass
+template <class Step>
 __global__ void clipped_adam_vi_kernel(float* __restrict__ loc, float* __restrict__ ls, float* __restrict__ scale,
                                        const float* __restrict__ g_loc, const float* __restrict__ g_ls, float* __restrict__ m_loc,
                                        float* __restrict__ v_loc, float* __restrict__ m_ls, float* __restrict__ v_ls, long long n,
-                                       float step_size, float b1, float b2, float eps, float clip, float wd, float gscale) {
+                                       Step ss, float b1, float b2, float eps, float clip, float wd, float gscale) {
+  const float step_size = ss.get();
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
     {
       float gr = fminf(fmaxf(g_loc[i] * gscale, -clip), clip);
@@ -754,19 +770,124 @@ __global__ void clipped_adam_vi_kernel(float* __restrict__ loc, float* __restric
     }
   }
 }
+static DevStep dev_step(const TrainDesc* d) {  // device addresses of the descriptor's table and index
+  const char* base = reinterpret_cast<const char*>(d);
+  return DevStep{reinterpret_cast<const float*>(base + offsetof(TrainDesc, steps)), reinterpret_cast<const int*>(base + offsetof(TrainDesc, kt))};
+}
+template <class Step>
+static void clipped_adam_vi_on(float* loc, float* ls, float* scale, const float* g_loc, const float* g_ls, float* m_loc, float* v_loc,
+                               float* m_ls, float* v_ls, long long n, Step ss, float b1, float b2, float eps, float clip, float wd,
+                               cudaStream_t st, float gscale) {
+  ++g_launch_count;
+  clipped_adam_vi_kernel<<<(unsigned)min((n + 255) / 256, (long long)148 * 8), 256, 0, st>>>(loc, ls, scale, g_loc, g_ls, m_loc, v_loc,
+                                                                                            m_ls, v_ls, n, ss, b1, b2, eps, clip, wd,
+                                                                                            gscale);
+}
+template <class Step>
+static void clipped_adam_on(float* p, const float* g, float* m, float* v, long long n, Step ss, float b1, float b2, float eps,
+                            float clip, float wd, cudaStream_t st) {
+  ++g_launch_count;
+  clipped_adam_kernel<<<(unsigned)min((n + 255) / 256, (long long)148 * 8), 256, 0, st>>>(p, g, m, v, n, ss, b1, b2, eps, clip, wd);
+}
 void launch_clipped_adam_vi(float* loc, float* ls, float* scale, const float* g_loc, const float* g_ls, float* m_loc, float* v_loc,
                             float* m_ls, float* v_ls, long long n, float step_size, float b1, float b2, float eps, float clip, float wd,
                             cudaStream_t st, float gscale) {
-  ++g_launch_count;
-  clipped_adam_vi_kernel<<<(unsigned)min((n + 255) / 256, (long long)148 * 8), 256, 0, st>>>(loc, ls, scale, g_loc, g_ls, m_loc, v_loc,
-                                                                                            m_ls, v_ls, n, step_size, b1, b2, eps, clip, wd,
-                                                                                            gscale);
+  clipped_adam_vi_on(loc, ls, scale, g_loc, g_ls, m_loc, v_loc, m_ls, v_ls, n, HostStep{step_size}, b1, b2, eps, clip, wd, st, gscale);
 }
 void launch_clipped_adam(float* p, const float* g, float* m, float* v, long long n, float step_size, float b1,
                          float b2, float eps, float clip, float wd, cudaStream_t st) {
+  clipped_adam_on(p, g, m, v, n, HostStep{step_size}, b1, b2, eps, clip, wd, st);
+}
+void launch_clipped_adam_vi(float* loc, float* ls, float* scale, const float* g_loc, const float* g_ls, float* m_loc, float* v_loc,
+                            float* m_ls, float* v_ls, long long n, const TrainDesc* d, float b1, float b2, float eps, float clip,
+                            float wd, cudaStream_t st) {
+  clipped_adam_vi_on(loc, ls, scale, g_loc, g_ls, m_loc, v_loc, m_ls, v_ls, n, dev_step(d), b1, b2, eps, clip, wd, st, 1.0f);
+}
+void launch_clipped_adam(float* p, const float* g, float* m, float* v, long long n, const TrainDesc* d, float b1, float b2, float eps,
+                         float clip, float wd, cudaStream_t st) {
+  clipped_adam_on(p, g, m, v, n, dev_step(d), b1, b2, eps, clip, wd, st);
+}
+
+// ------------------------------------------------------------------------------------------------
+// K training steps per call (brl_elbo_train_steps / brl_hnn_train_steps): every per-step quantity is read from the call's
+// descriptor in device memory, so one captured step serves every step of every later call with the same configuration
+// ------------------------------------------------------------------------------------------------
+__global__ void train_setup_kernel(const TrainSetup s) {
+  TrainDesc* d = s.d;
+  for (int i = threadIdx.x; i < s.n; i += blockDim.x) d->steps[i] = s.steps[i];
+  if (threadIdx.x == 0) {
+    d->X = s.X; d->Y = s.Y; d->idx = s.idx; d->scalars = s.scalars; d->metrics = s.metrics;
+    d->N = s.N; d->k = s.k0; d->kt = 0; d->bad = 0;
+    d->seed = s.seed; d->sample0 = s.sample0; d->window0 = s.window0;
+  }
+}
+void launch_train_setup(const TrainSetup& s, cudaStream_t st) {
   ++g_launch_count;
-  clipped_adam_kernel<<<(unsigned)min((n + 255) / 256, (long long)148 * 8), 256, 0, st>>>(p, g, m, v, n, step_size, b1, b2,
-                                                                                         eps, clip, wd);
+  train_setup_kernel<<<1, 256, 0, st>>>(s);
+}
+
+// windows X[idx[k, w]] -> xb [MB,30,18] as float4 (a window is 135 of them), labels -> yb [MB]; an index outside [0, N) reads
+// nothing (zeros) and marks the step; thread 0 writes step k's Philox key {seed + 0x9E3779B97F4A7C15 (k + 1), sample0, window0}
+__global__ void train_gather_kernel(TrainDesc* d, float* __restrict__ xb, float* __restrict__ yb, long long MB) {
+  const long long k = d->k, N = d->N;
+  const long long* row = d->idx + k * MB;
+  const float4* X = reinterpret_cast<const float4*>(d->X);
+  const float* Y = d->Y;
+  const long long stride = (long long)gridDim.x * blockDim.x;
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < MB * 135; i += stride) {
+    const long long w = i / 135, e = i - w * 135, j = row[w];
+    float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (j >= 0 && j < N) v = __ldg(X + j * 135 + e);
+    else if (e == 0) d->bad = 1;
+    reinterpret_cast<float4*>(xb)[i] = v;
+  }
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < MB; i += stride) {
+    const long long j = row[i];
+    yb[i] = (j >= 0 && j < N) ? __ldg(Y + j) : 0.f;
+  }
+  if (blockIdx.x == 0 && threadIdx.x == 0) {
+    d->dyn[0] = d->seed + 0x9E3779B97F4A7C15ull * (unsigned long long)(k + 1);
+    d->dyn[1] = d->sample0;
+    d->dyn[2] = d->window0;
+  }
+}
+void launch_train_gather(TrainDesc* d, float* xb, float* yb, long long MB, cudaStream_t st) {
+  ++g_launch_count;
+  train_gather_kernel<<<(unsigned)min((MB * 135 + 255) / 256, (long long)148 * 8), 256, 0, st>>>(d, xb, yb, MB);
+}
+
+// member m's (loc, scale) pairs at src + m mstride -> the [M,B] planes of the step metrics
+__global__ void split_pred_kernel(const float* __restrict__ src, long long mstride, long long B, float* pred, float* std) {
+  const long long m = blockIdx.y;
+  for (long long b = blockIdx.x * (long long)blockDim.x + threadIdx.x; b < B; b += (long long)gridDim.x * blockDim.x) {
+    const float2 o = *reinterpret_cast<const float2*>(src + m * mstride + 2 * b);
+    pred[m * B + b] = o.x;
+    std[m * B + b] = o.y;
+  }
+}
+void launch_split_pred(const float* src, long long mstride, int M, long long B, float* pred, float* std, cudaStream_t st) {
+  ++g_launch_count;
+  split_pred_kernel<<<dim3((unsigned)min((B + 255) / 256, (long long)148), (unsigned)M), 256, 0, st>>>(src, mstride, B, pred, std);
+}
+
+// the step's scalars [M,nscal] and metrics [M,5] -> row k of the caller's [K,M,.] buffers (NaN where the gather met a bad index);
+// then the next step
+__global__ void train_tail_kernel(TrainDesc* d, const double* __restrict__ scal, int nscal, const double* __restrict__ met, int M) {
+  const long long k = d->k;
+  const bool bad = d->bad != 0;
+  const double nan = __longlong_as_double(0x7ff8000000000000ll);
+  for (int i = threadIdx.x; i < M * nscal; i += blockDim.x) d->scalars[k * M * nscal + i] = bad ? nan : scal[i];
+  for (int i = threadIdx.x; i < M * 5; i += blockDim.x) d->metrics[k * M * 5 + i] = bad ? nan : met[i];
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    d->k = k + 1;
+    d->kt += 1;
+    d->bad = 0;
+  }
+}
+void launch_train_tail(TrainDesc* d, const double* scal, int nscal, const double* met, int M, cudaStream_t st) {
+  ++g_launch_count;
+  train_tail_kernel<<<1, 128, 0, st>>>(d, scal, nscal, met, M);
 }
 
 }  // namespace brl

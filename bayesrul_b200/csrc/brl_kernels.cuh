@@ -214,4 +214,41 @@ void launch_clipped_adam_vi(float* loc, float* ls, float* scale, const float* g_
                             float* m_ls, float* v_ls, long long n, float step_size, float b1, float b2, float eps, float clip, float wd,
                             cudaStream_t st, float gscale = 1.0f);  // gscale: multiplies the gradients first (1 / world after a SUM all-reduce)
 
+
+// ---- K training steps per call (brl_elbo_train_steps / brl_hnn_train_steps) ----
+constexpr int TRAIN_TABLE = 896;  // Adam step sizes one setup launch brings (its arguments stay below 4 KB)
+// the call's descriptor in device memory: everything a replayed step reads that changes from step to step or call to call
+struct TrainDesc {
+  const float* X;  // [N,30,18]
+  const float* Y;  // [N]
+  const long long* idx;  // [K,M,B]
+  double* scalars;  // [K,M,nscal]
+  double* metrics;  // [K,M,5]
+  long long N, k;   // k: the step being run
+  int kt, bad;      // kt: step k's entry of `steps`; bad: step k's gather met an index outside [0, N)
+  unsigned long long seed, sample0, window0;
+  unsigned long long dyn[4];  // step k's Philox key {seed + 0x9E3779B97F4A7C15 (k + 1), sample0, window0} (NoiseRef::dyn)
+  float steps[TRAIN_TABLE];   // Adam step sizes of steps k - kt ...
+};
+struct TrainSetup {
+  TrainDesc* d;
+  const float *X, *Y;
+  const long long* idx;
+  double *scalars, *metrics;
+  long long N, k0;  // k0: first step of this table
+  unsigned long long seed, sample0, window0;
+  int n;
+  float steps[TRAIN_TABLE];
+};
+void launch_train_setup(const TrainSetup& s, cudaStream_t st);
+void launch_train_gather(TrainDesc* d, float* xb, float* yb, long long MB, cudaStream_t st);
+void launch_split_pred(const float* src, long long mstride, int M, long long B, float* pred, float* std, cudaStream_t st);
+void launch_train_tail(TrainDesc* d, const double* scal, int nscal, const double* met, int M, cudaStream_t st);
+// ClippedAdam with the step size d->steps[d->kt] read on the device
+void launch_clipped_adam(float* p, const float* g, float* m, float* v, long long n, const TrainDesc* d, float b1, float b2, float eps,
+                         float clip, float wd, cudaStream_t st);
+void launch_clipped_adam_vi(float* loc, float* ls, float* scale, const float* g_loc, const float* g_ls, float* m_loc, float* v_loc,
+                            float* m_ls, float* v_ls, long long n, const TrainDesc* d, float b1, float b2, float eps, float clip,
+                            float wd, cudaStream_t st);
+
 }  // namespace brl

@@ -454,6 +454,92 @@ class Engine:
                                                   ws.numel(), self._stream()))
         return dict(scalars=scalars, grad=grad, out=out)
 
+    # -- K training steps per call over a device-resident dataset ---------------------------------------
+    def _train_inputs(self, X, Y, idx, params):
+        """Checks the dataset, the index tensor and the [M,P] (or [P] for M = 1) parameter / optimiser-state tensors; returns
+        (X, Y, idx [K,M,B], M).  The index range check is one device reduction and one host read: the only synchronisation of
+        a K-step call."""
+        X = _chk(X, self.device, "X")
+        if X.dim() != 3 or X.shape[1] != WIN_LENGTH or X.shape[2] != N_FEATURES or X.shape[0] == 0:
+            raise RuntimeError(f"bayesrul_b200: X must be [N,{WIN_LENGTH},{N_FEATURES}] with N > 0, got {tuple(X.shape)}")
+        N = X.shape[0]
+        if X.data_ptr() % 16:
+            raise RuntimeError("bayesrul_b200: X must be 16-byte aligned")
+        Y = _chk(Y, self.device, "Y")
+        if Y.numel() != N:
+            raise RuntimeError(f"bayesrul_b200: Y must have {N} elements, got {Y.numel()}")
+        lead = tuple(params[0][0].shape[:-1]) if isinstance(params[0][0], torch.Tensor) else ()
+        if len(lead) > 1:
+            raise RuntimeError(f"bayesrul_b200: parameters must be [M,{self.P}] or [{self.P}]")
+        M = lead[0] if lead else 1
+        for t, what in params:
+            self._theta(t, what, lead)
+        idx = _chk(idx, self.device, "idx", dtype=torch.int64)
+        if idx.dim() == 2 and not lead:
+            idx = idx.view(idx.shape[0], 1, idx.shape[1])
+        if idx.dim() != 3 or idx.shape[1] != M or idx.shape[0] == 0 or idx.shape[2] == 0:
+            raise RuntimeError(f"bayesrul_b200: idx must be [K,{M},B] (or [K,B] for one member) with K, B > 0, got {tuple(idx.shape)}")
+        lo, hi = torch.stack(torch.aminmax(idx)).tolist()
+        if lo < 0 or hi >= N:
+            raise RuntimeError(f"bayesrul_b200: idx holds windows outside [0, {N}): min {lo}, max {hi}")
+        return X, Y, idx, M
+
+    def elbo_train_steps(self, X, Y, idx, loc, log_scale, scale, opt_state, *, step0: int, lr: float, betas=(0.95, 0.999),
+                         eps: float = 1e-8, clip_norm: float = 15.0, lrd: float = 1.0, weight_decay: float = 0.0, mode: str = "lrt",
+                         guide: str = "normal", particles: int = 1, prior_loc: float = 0.0, prior_scale: float = 1.0,
+                         dataset_size: int, seed: int, sample0: int = 0, window0: int = 0):
+        """K ELBO training steps in one call over the device-resident split X [N,30,18], Y [N].  idx [K,M,B] (int64; [K,B] with
+        [P] parameters) names the windows of member m's minibatch at step k.  Step k is elbo_step_ensemble (elbo_step at M = 1)
+        on X[idx[k]], Y[idx[k]] with Noise(seed + 0x9E3779B97F4A7C15 (k + 1) mod 2**64, sample0, window0), then
+        clipped_adam_vi at step step0 + k + 1, then step_metrics_ensemble of the logged predictions (particle 0, or the aggregate
+        of several particles).  loc / log_scale / scale [M,P] and opt_state = (m_loc, v_loc, m_log_scale, v_log_scale) [M,P] are
+        updated in place.  Returns dict(scalars [K,M,4] = (loss, nll_sum, kl, mse), metrics [K,M,5] = (nll, mse, sharpness,
+        rmsce, mace)), float64 device tensors.  The index range check before the launches is the call's only synchronisation;
+        from the third step of a configuration on, each step is one CUDA-graph launch."""
+        if len(opt_state) != 4:
+            raise RuntimeError("bayesrul_b200: opt_state must be (m_loc, v_loc, m_log_scale, v_log_scale)")
+        ts = (loc, log_scale, scale) + tuple(opt_state)
+        names = ("loc", "log_scale", "scale", "m_loc", "v_loc", "m_log_scale", "v_log_scale")
+        X, Y, idx, M = self._train_inputs(X, Y, idx, list(zip(ts, names)))
+        if guide not in GUIDE_IDS:
+            raise RuntimeError("Guide unknown. Choose from 'normal', 'radial'.")
+        if mode is None:
+            mode = "ws"
+        K, B = idx.shape[0], idx.shape[2]
+        scalars = torch.empty(K, M, 4, dtype=torch.float64, device=self.device)
+        metrics = torch.empty(K, M, 5, dtype=torch.float64, device=self.device)
+        ws = self._ws_for(B, M, 5, "simt")
+        _lib.check(self.lib.brl_elbo_train_steps(self.ctx, X.data_ptr(), Y.data_ptr(), X.shape[0], idx.data_ptr(), K, M, B,
+                                                 *[t.data_ptr() for t in ts], int(step0), float(lr), float(betas[0]), float(betas[1]),
+                                                 float(eps), float(clip_norm), float(lrd), float(weight_decay), MODE_IDS[mode],
+                                                 GUIDE_IDS[guide], int(particles), float(prior_loc), float(prior_scale),
+                                                 int(dataset_size), int(seed) & 0xFFFFFFFFFFFFFFFF, int(sample0), int(window0),
+                                                 scalars.data_ptr(), metrics.data_ptr(), ws.data_ptr(), ws.numel(), self._stream()))
+        return dict(scalars=scalars, metrics=metrics)
+
+    def hnn_train_steps(self, X, Y, idx, theta, opt_state, *, step0: int, lr: float, betas=(0.9, 0.999), eps: float = 1e-8,
+                        clip_norm: float = 1e30, lrd: float = 1.0, weight_decay: float = 0.0, p_dropout: float = 0.0, seed: int,
+                        sample0: int = 0, window0: int = 0):
+        """K heteroscedastic-NN training steps in one call (the members of a deep ensemble): step k is hnn_step_ensemble
+        (hnn_step at M = 1) on X[idx[k]], Y[idx[k]] with Noise(seed + 0x9E3779B97F4A7C15 (k + 1) mod 2**64, sample0, window0),
+        then clipped_adam over theta [M,P] with opt_state = (exp_avg, exp_avg_sq) at step step0 + k + 1 (the default clip_norm
+        disables the clip: plain Adam), then step_metrics_ensemble of the step's (loc, scale).  Returns dict(scalars [K,M,2] =
+        (loss, mse), metrics [K,M,5]); synchronises only for the index range check, as elbo_train_steps."""
+        if len(opt_state) != 2:
+            raise RuntimeError("bayesrul_b200: opt_state must be (exp_avg, exp_avg_sq)")
+        ts = (theta,) + tuple(opt_state)
+        X, Y, idx, M = self._train_inputs(X, Y, idx, list(zip(ts, ("theta", "exp_avg", "exp_avg_sq"))))
+        K, B = idx.shape[0], idx.shape[2]
+        scalars = torch.empty(K, M, 2, dtype=torch.float64, device=self.device)
+        metrics = torch.empty(K, M, 5, dtype=torch.float64, device=self.device)
+        ws = self._ws_for(B, M, 6, "simt")
+        _lib.check(self.lib.brl_hnn_train_steps(self.ctx, X.data_ptr(), Y.data_ptr(), X.shape[0], idx.data_ptr(), K, M, B,
+                                                *[t.data_ptr() for t in ts], int(step0), float(lr), float(betas[0]), float(betas[1]),
+                                                float(eps), float(clip_norm), float(lrd), float(weight_decay), float(p_dropout),
+                                                int(seed) & 0xFFFFFFFFFFFFFFFF, int(sample0), int(window0), scalars.data_ptr(),
+                                                metrics.data_ptr(), ws.data_ptr(), ws.numel(), self._stream()))
+        return dict(scalars=scalars, metrics=metrics)
+
     # -- A14 / A15 / N1 ------------------------------------------------------------------------------------
     def mixture_moments(self, mu_m: torch.Tensor, sigma_m: torch.Tensor):
         mu_m, sigma_m = _chk(mu_m, self.device, "mu_m"), _chk(sigma_m, self.device, "sigma_m")

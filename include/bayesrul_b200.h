@@ -115,7 +115,9 @@ int brl_destroy(brl_ctx* ctx);
  * that brl_elbo_step runs two particles side by side on two stream lanes),
  * train == 2 the sign tensors brl_forward generates in BRL_MODE_FLIPOUT when none are injected,
  * train == 3 the buffers of brl_hnn_step_ensemble over S = M members (all of them in one chain of launches where it can),
- * train == 4 the buffers of brl_elbo_step_ensemble over S = M members (the same, one particle lane of M members) */
+ * train == 4 the buffers of brl_elbo_step_ensemble over S = M members (the same, one particle lane of M members),
+ * train == 5 the buffers of brl_elbo_train_steps over S = M members (its own, then those of code 4, or of code 1 with S = 2 at M = 1),
+ * train == 6 the buffers of brl_hnn_train_steps over S = M members (its own, then those of code 3, or of code 1 at M = 1) */
 /* 1 when `engine` can run this net's forward on this build, else 0 */
 int brl_engine_available(const brl_ctx* ctx, int engine);
 int64_t brl_workspace_bytes(const brl_ctx* ctx, int64_t B, int64_t S, int train, int engine);
@@ -265,6 +267,39 @@ int brl_hnn_step_ensemble(brl_ctx* ctx, const float* x /*[M,B,30,18]*/, const fl
                           const float* theta /*[M,P]*/, float p_dropout, const brl_noise* noise, int compute_grads,
                           double* scalars /*[M,2] = {loss, mse}*/, float* grad_theta /*[M,P]*/, float* out /*[M,B,2]*/,
                           void* workspace, size_t workspace_bytes, void* stream);
+
+/* ---- K consecutive training steps in ONE call, over a device-resident dataset (replaces the epoch loop of Lightning's fit:
+ *      DataLoader collate + copy, svi.step / HNN.step, the optimiser, the logged step metrics and their .item() reads, per batch).
+ *      X [N,30,18] (16-byte aligned) and Y [N] are the training split; idx [K,M,B] (int64, device) holds the windows of member m's
+ *      minibatch at step k.  Step k does exactly:
+ *        1. brl_elbo_step_ensemble (brl_elbo_step at M = 1) on X[idx[k]], Y[idx[k]] with the Philox key
+ *           {seed + 0x9E3779B97F4A7C15 (k + 1) mod 2^64, sample0, window0} (the key sequence of the reference's per-step seeds);
+ *           brl_hnn_train_steps: brl_hnn_step_ensemble (brl_hnn_step at M = 1);
+ *        2. brl_clipped_adam_vi (ELBO: loc / log_scale / scale with their moments) or brl_clipped_adam (HNN: theta) over M*P
+ *           elements at Adam step step0 + k + 1, with the step size brl_clipped_adam computes;
+ *        3. brl_step_metrics_ensemble of particle 0's (loc, scale), or with several particles of each member's
+ *           brl_aggregate_predictions, into metrics[k] [M,5] = {nll, mse, sharpness, rmsce, mace};
+ *      and scalars[k] [M,4] = {loss, nll_sum, kl, mse} (ELBO) or [M,2] = {loss, mse} (HNN).  Parameters and optimiser state are
+ *      updated in place; no gradient is returned.  Every net, back-end and member count of the single steps runs, the same way.
+ *      With step graphs on (brl_set_step_graph) and `stream` not being captured by the caller, the first step of a configuration
+ *      runs eagerly, the second is captured, and every later step (this call's and a later call's with the same sizes, parameter,
+ *      optimiser-state and workspace pointers and optimiser hyper-parameters beta1, beta2, eps, clip_norm, weight_decay) is one
+ *      graph launch: the step reads k, the windows, the Philox key and the Adam step size from a descriptor in the workspace,
+ *      which one small launch per 896 steps rewrites.  Otherwise the same launches run eagerly.  The host is never synchronised.
+ *      An index outside [0, N) reads no memory: that step's rows of scalars and metrics are NaN.
+ *      Workspace: brl_workspace_bytes(B, M, 5) / brl_workspace_bytes(B, M, 6); less returns BRL_ERR_WORKSPACE. */
+int brl_elbo_train_steps(brl_ctx* ctx, const float* X /*[N,30,18]*/, const float* Y /*[N]*/, int64_t N, const int64_t* idx /*[K,M,B]*/,
+                         int64_t K, int64_t M, int64_t B, float* loc /*[M,P]*/, float* log_scale, float* scale, float* m_loc,
+                         float* v_loc, float* m_log_scale, float* v_log_scale, int64_t step0, float lr, float beta1, float beta2,
+                         float eps, float clip_norm, float lrd, float weight_decay, int mode, int guide, int particles,
+                         float prior_loc, float prior_scale, int64_t dataset_size, uint64_t seed, int64_t sample0, int64_t window0,
+                         double* scalars /*[K,M,4]*/, double* metrics /*[K,M,5]*/, void* workspace, size_t workspace_bytes,
+                         void* stream);
+int brl_hnn_train_steps(brl_ctx* ctx, const float* X /*[N,30,18]*/, const float* Y /*[N]*/, int64_t N, const int64_t* idx /*[K,M,B]*/,
+                        int64_t K, int64_t M, int64_t B, float* theta /*[M,P]*/, float* exp_avg, float* exp_avg_sq, int64_t step0,
+                        float lr, float beta1, float beta2, float eps, float clip_norm, float lrd, float weight_decay,
+                        float p_dropout, uint64_t seed, int64_t sample0, int64_t window0, double* scalars /*[K,M,2]*/,
+                        double* metrics /*[K,M,5]*/, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- deep-ensemble mixture moments (models/deepens.py:21-24), [M,n] -> [n] ------------- */
 int brl_mixture_moments(const float* mu_m, const float* sigma_m, int64_t M, int64_t n, float* mu,
