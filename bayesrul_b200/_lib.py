@@ -37,7 +37,7 @@ class BrlNoise(C.Structure):
 
 
 # name -> (restype, argtypes); the single source of truth for tests/test_cabi.py too
-_vp, _i, _i64, _f, _sz = C.c_void_p, C.c_int, C.c_int64, C.c_float, C.c_size_t
+_vp, _i, _i64, _f, _d, _sz = C.c_void_p, C.c_int, C.c_int64, C.c_float, C.c_double, C.c_size_t
 _np = C.POINTER(BrlNoise)
 SIGNATURES = {
     "brl_version": (_i, []),
@@ -79,6 +79,8 @@ SIGNATURES = {
                                  C.c_uint64, _i64, _i64, _vp, _vp, _vp, _sz, _vp]),
     "brl_hnn_train_steps": (_i, [_vp, _vp, _vp, _i64, _vp, _i64, _i64, _i64] + [_vp] * 3 + [_i64] + [_f] * 8 + [C.c_uint64, _i64, _i64,
                                 _vp, _vp, _vp, _sz, _vp]),
+    "brl_hnn_train_steps_adam": (_i, [_vp, _vp, _vp, _i64, _vp, _i64, _i64, _i64] + [_vp] * 3 + [_i64] + [_d] * 5 + [_f, C.c_uint64, _i64,
+                                     _i64, _vp, _vp, _vp, _sz, _vp]),
     "brl_mixture_moments": (_i, [_vp, _vp, _i64, _i64, _vp, _vp, _vp]),
     "brl_step_metrics": (_i, [_vp, _vp, _vp, _i64, _vp, _vp, _sz, _vp]),
     "brl_step_metrics_ensemble": (_i, [_vp, _vp, _vp, _i64, _i64, _vp, _vp, _sz, _vp]),
@@ -86,6 +88,7 @@ SIGNATURES = {
     "brl_test_metrics": (_i, [_vp, _vp, _vp, _i64, _vp, _vp, _sz, _vp]),
     "brl_clipped_adam": (_i, [_vp, _vp, _vp, _vp, _i64, _i64, _f, _f, _f, _f, _f, _f, _f, _vp]),
     "brl_clipped_adam_vi": (_i, [_vp] * 9 + [_i64, _i64, _f, _f, _f, _f, _f, _f, _f, _vp]),
+    "brl_adam": (_i, [_vp, _vp, _vp, _vp, _i64, _i64, _d, _d, _d, _d, _d, _vp]),
 }
 
 _lib = None

@@ -62,31 +62,143 @@ class HNN(_Base):
         self._it += 1
         return Noise(seed=(torch.initial_seed() + 0x9E3779B97F4A7C15 * self._it) & 0xFFFFFFFFFFFFFFFF)
 
+    def _train_backend_of_net(self):
+        """the back-end of the training step: "auto" is the level-fused kernels for the Inception net, the fp32 ones otherwise"""
+        be = self._train_backend
+        if be == "auto":
+            be = "fused" if getattr(self.net, "kind", "") == "inception" else "simt"
+        return be
+
+    def _step(self, x, y, phase):
+        """HNN.step without its log: (loss, loc, scale)"""
+        train = phase == "train"
+        p = float(self.net.dropout) if (train or getattr(self.net, "mc_dropout", False)) else 0.0
+        self.net.engine().set_gemm_backend(self._train_backend_of_net())
+        res = self.net.engine().hnn_step(x.contiguous(), y.contiguous(), self.net.flat(), p, self._noise(), compute_grads=train)
+        loss = res["scalars"][0].float()
+        if train:  # the returned loss carries a grad_fn whose backward writes the fused step's gradient into param.grad
+            loss = _FusedStepLoss.apply(loss, res["grad"], tuple(self.net._sites), *self.net._params)
+        return loss, res["out"][:, 0], res["out"][:, 1]
+
     def step(self, batch, phase):  # frequentist.py:39-48
         (x, y) = batch
         if phase == "predict":
             output = self.net(x)
             return output[:, 0], output[:, 1]
-        train = phase == "train"
-        p = float(self.net.dropout) if (train or getattr(self.net, "mc_dropout", False)) else 0.0
-        be = self._train_backend
-        if be == "auto":
-            be = "fused" if getattr(self.net, "kind", "") == "inception" else "simt"
-        self.net.engine().set_gemm_backend(be)
-        res = self.net.engine().hnn_step(x.contiguous(), y.contiguous(), self.net.flat(), p, self._noise(), compute_grads=train)
-        loss = res["scalars"][0].float()
-        if train:  # the returned loss carries a grad_fn whose backward writes the fused step's gradient into param.grad
-            loss = _FusedStepLoss.apply(loss, res["grad"], tuple(self.net._sites), *self.net._params)
+        loss, loc, scale = self._step(x, y, phase)
         self.log(f"nll/{phase}", loss, on_step=False, on_epoch=True)
-        return loss, res["out"][:, 0], res["out"][:, 1]
+        return loss, loc, scale
+
+    def _train_batch(self, x, y):
+        """the training step on one batch: (loss, the values training_step logs, in its order)"""
+        loss, loc, scale = self._step(x, y, "train")
+        m = self.net.engine().step_metrics(loc, scale, y)  # mse, sharpness, rmsce in one fused pass (N3)
+        return loss, {"nll/train": loss, "mse/train": m[1].float(), "rmsce/train": m[3].float(), "sharp/train": m[2].float()}
 
     def training_step(self, batch, batch_idx):
-        loss, loc, scale = self.step(batch, "train")
-        m = self.net.engine().step_metrics(loc, scale, batch[1])  # mse, sharpness, rmsce in one fused pass (N3)
-        self.log("mse/train", m[1].float(), on_step=False, on_epoch=True)
-        self.log("rmsce/train", m[3].float(), on_step=False, on_epoch=True)
-        self.log("sharp/train", m[2].float(), on_step=False, on_epoch=True)
+        loss, vals = self._train_batch(batch[0], batch[1])
+        for k, v in vals.items():
+            self.log(k, v, on_step=False, on_epoch=True)
         return loss
+
+    def _adam_group(self, optimizer):
+        """the one param group of `optimizer` if it is a torch.optim.Adam over exactly the net's site parameters whose update
+        Engine.adam computes (amsgrad, maximize, differentiable, capturable, fused and decoupled weight decay off); else raises"""
+        why = None
+        if type(optimizer) is not torch.optim.Adam:
+            why = f"runs torch.optim.Adam, got {type(optimizer).__name__}"
+        elif len(optimizer.param_groups) != 1:
+            why = f"needs one param group, got {len(optimizer.param_groups)}"
+        else:
+            g = optimizer.param_groups[0]
+            sites = self.net._params
+            theta = self.net.flat()
+            if len(g["params"]) != len(sites) or {id(p) for p in g["params"]} != {id(p) for p in sites}:
+                why = "needs the param group to hold exactly the net's site parameters"
+            elif any(p.data_ptr() != theta.data_ptr() + 4 * off for p, (off, _) in zip(sites, self.net._sites)):
+                why = "needs the site parameters to be the views of net.flat()"
+            else:
+                on = [k for k in ("amsgrad", "maximize", "differentiable", "capturable", "fused", "decoupled_weight_decay") if g.get(k)]
+                if on:
+                    why = f"runs Adam without {', '.join(on)}"
+        if why:
+            raise RuntimeError(f"bayesrul_b200: HNN.fit_epoch {why}")
+        return optimizer.param_groups[0]
+
+    def fit_epoch(self, x, y, batch_size: int, optimizer, generator=None):
+        """One training epoch over the DEVICE-resident split x [N,30,18], y [N]: what Lightning's fit does with training_step and
+        the torch.optim.Adam `optimizer` that configure_optimizers() returned, over the shuffled batches of a DataLoader, without
+        a host round trip per batch.  The permutation is torch.randperm(N, generator=generator, device=x.device); its
+        floor(N / batch_size) full batches run as ONE Engine.hnn_train_steps(optimizer="adam") call with the dropout rate and
+        back-end of training_step, continuing the seed sequence of the HNN's steps and the optimizer's step count.  The
+        optimizer's per-site exp_avg / exp_avg_sq go in as flat [P] buffers and come back, and each state["step"] advances by
+        the number of full batches.  The remainder batch goes through training_step, zero_grad, backward and optimizer.step, as
+        Lightning's automatic optimisation runs it.  Logs the epoch means of the keys training_step logs, each batch weighted by
+        its size as Lightning's epoch mean weighs it, and returns dict(scalars [K,1,2], metrics [K,1,5], perm) of the K full
+        batches (Engine.hnn_train_steps)."""
+        N, bs = int(x.shape[0]), int(batch_size)
+        if bs <= 0 or y.numel() != N:
+            raise RuntimeError("bayesrul_b200: fit_epoch needs batch_size > 0 and one target per window")
+        group = self._adam_group(optimizer)
+        net, theta = self.net, self.net.flat()
+        perm = torch.randperm(N, generator=generator, device=x.device)
+        K = N // bs
+        x, y = x.contiguous(), y.reshape(-1).contiguous()
+        res = None
+        sums, weight = {}, 0
+        if K > 0:
+            states = [optimizer.state.get(p) for p in net._params]
+            steps = {float(st["step"]) if st else 0.0 for st in states}
+            if len(steps) != 1:
+                raise RuntimeError("bayesrul_b200: HNN.fit_epoch needs every site parameter at the same Adam step")
+            # exp_avg / exp_avg_sq in net.flat() order, in buffers kept from epoch to epoch: stable addresses let a later epoch
+            # replay the step graph the first one captured
+            if getattr(self, "_flat_moments", None) is None or self._flat_moments[0].shape != theta.shape or \
+                    self._flat_moments[0].device != theta.device:
+                self._flat_moments = (torch.empty_like(theta), torch.empty_like(theta))
+            m, v = self._flat_moments
+            m.zero_()
+            v.zero_()
+            for st, (off, _) in zip(states, net._sites):
+                if st:
+                    n = st["exp_avg"].numel()
+                    m[off: off + n].copy_(st["exp_avg"].reshape(-1))
+                    v[off: off + n].copy_(st["exp_avg_sq"].reshape(-1))
+            eng = net.engine()
+            eng.set_gemm_backend(self._train_backend_of_net())
+            res = eng.hnn_train_steps(x, y, perm[: K * bs].view(K, bs), theta, (m, v), step0=int(steps.pop()), lr=float(group["lr"]),
+                                      betas=tuple(float(b) for b in group["betas"]), eps=float(group["eps"]),
+                                      weight_decay=float(group["weight_decay"]), p_dropout=float(net.dropout),
+                                      seed=(torch.initial_seed() + 0x9E3779B97F4A7C15 * self._it) & 0xFFFFFFFFFFFFFFFF,
+                                      optimizer="adam")
+            self._it += K
+            for p, st, (off, _) in zip(net._params, states, net._sites):
+                if not st:  # Adam's lazy state: a CPU step counter of the default scalar dtype, moments shaped as the parameter
+                    st = optimizer.state[p]
+                    st["step"] = torch.tensor(0.0, dtype=torch.float64 if torch.get_default_dtype() == torch.float64 else torch.float32)
+                    st["exp_avg"] = torch.zeros_like(p, memory_format=torch.preserve_format)
+                    st["exp_avg_sq"] = torch.zeros_like(p, memory_format=torch.preserve_format)
+                n = p.numel()
+                st["exp_avg"].copy_(m[off: off + n].view_as(st["exp_avg"]))
+                st["exp_avg_sq"].copy_(v[off: off + n].view_as(st["exp_avg_sq"]))
+                st["step"] += K
+            sc, mt = res["scalars"][:, 0], res["metrics"][:, 0]
+            sums = {"nll/train": sc[:, 0], "mse/train": mt[:, 1], "rmsce/train": mt[:, 3], "sharp/train": mt[:, 2]}
+            sums = {k: t.float().double().sum() * bs for k, t in sums.items()}  # each logged as float32
+            weight = K * bs
+        if K * bs < N:
+            rest = perm[K * bs:]
+            loss, vals = self._train_batch(x[rest], y[rest])
+            optimizer.zero_grad()
+            loss.backward()
+            optimizer.step()
+            for k, val in vals.items():
+                sums[k] = sums.get(k, 0.0) + val.detach().double() * rest.numel()
+            weight += rest.numel()
+        means = torch.stack([torch.as_tensor(val, dtype=torch.float64, device=x.device) for val in sums.values()]).div(weight).tolist()
+        for k, val in zip(sums, means):
+            self.log(k, val, on_step=False, on_epoch=True)
+        return dict(scalars=res["scalars"] if res else None, metrics=res["metrics"] if res else None, perm=perm)
 
     def mc_sampling(self, batch, mc_samples: int, phase: str, agg: bool = True):  # frequentist.py:60-81
         (x, y) = batch

@@ -96,8 +96,9 @@ struct brl_ctx {
     float prior_loc, prior_scale;
     const void *mu, *sigma, *ws;
     size_t ws_bytes;
-    // brl_elbo_train_steps / brl_hnn_train_steps (train = 5 / 6; 0: a single step): the step's optimizer hyper-parameters
-    // {beta1, beta2, eps, clip_norm, weight_decay} and its other state buffers, baked into the captured optimizer launch
+    // brl_elbo_train_steps / brl_hnn_train_steps / brl_hnn_train_steps_adam (train = 5 / 6 / 7; 0: a single step): the step's
+    // optimizer operands ({beta1, beta2, eps, clip_norm, weight_decay}; torch's Adam: AdamArgs) and its other state buffers, baked
+    // into the captured optimizer launch
     int train;
     float opt[5];
     const void* state[5];
@@ -717,6 +718,18 @@ static float adam_step_size(float lr, float lrd, float beta1, float beta2, long 
   const double lr_t = (double)lr * std::pow((double)lrd, (double)step);
   const double bc1 = 1.0 - std::pow((double)beta1, (double)step), bc2 = 1.0 - std::pow((double)beta2, (double)step);
   return (float)(lr_t * std::sqrt(bc2) / bc1);
+}
+
+// torch.optim.Adam's per-step scalars of step `step` (>= 1), as Python computes them in double from the hyper-parameters the
+// optimizer holds: step_size = lr / (1 - beta1^step) and bc2_sqrt = sqrt(1 - beta2^step), each rounded once to the float its
+// kernel receives
+static void torch_adam_step(double lr, double beta1, double beta2, long long step, float* step_size, float* bc2_sqrt) {
+  *step_size = (float)(lr / (1.0 - std::pow(beta1, (double)step)));
+  *bc2_sqrt = (float)std::sqrt(1.0 - std::pow(beta2, (double)step));
+}
+// and its step-independent float operands (1 - beta1 and 1 - beta2 are taken in double first, as in Python)
+static AdamArgs torch_adam_args(double beta1, double beta2, double eps, double weight_decay) {
+  return AdamArgs{(float)(1.0 - beta1), (float)beta2, (float)(1.0 - beta2), (float)eps, (float)weight_decay};
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1806,7 +1819,6 @@ struct TrainArgs {
   long long N;
   const int64_t* idx;
   long long K, M, B, step0;
-  float lr, beta1, beta2, eps, clip_norm, lrd, weight_decay;
   uint64_t seed;
   long long sample0, window0;
   double *scalars, *metrics;
@@ -1821,10 +1833,12 @@ static int train_args_ok(const char* fn, const TrainArgs& a) {
 
 // Step k of the call is body(noise, stream): gather -> step -> optimizer -> metrics -> row k.  With graphs on and nobody capturing
 // `st`, the first step of a configuration runs eagerly, the second is captured (the Philox key read from the descriptor) and every
-// later step, in this call or a later one, is one graph launch.  Every TRAIN_TABLE steps one setup launch writes the descriptor
-// and the next table of Adam step sizes, computed here as brl_clipped_adam{,_vi} computes them.  Nothing synchronises the host.
-template <class Body>
-static int train_steps(brl_ctx* ctx, const TrainArgs& a, const brl_ctx::StepKey& key, const TrainBufs& t, Body body, cudaStream_t st) {
+// later step, in this call or a later one, is one graph launch.  Every TRAIN_TABLE steps setup(su, stream) fills the table of the
+// optimizer's per-step scalars for steps step0 + su.k0 + 1 ... (as the single-step optimizer entry point computes them) and makes
+// the one launch that writes the descriptor and that table.  Nothing synchronises the host.
+template <class Setup, class Body>
+static int train_steps(brl_ctx* ctx, const TrainArgs& a, const brl_ctx::StepKey& key, const TrainBufs& t, Setup setup, Body body,
+                       cudaStream_t st) {
   brl_ctx::StepGraph* sg = ctx->graph_enabled && !stream_capturing(st) ? graph_slot(ctx, key) : nullptr;
   const unsigned long long* dyn = reinterpret_cast<const unsigned long long*>(reinterpret_cast<const char*>(t.d) + offsetof(TrainDesc, dyn));
   TrainSetup su;
@@ -1834,8 +1848,7 @@ static int train_steps(brl_ctx* ctx, const TrainArgs& a, const brl_ctx::StepKey&
     if (k % TRAIN_TABLE == 0) {
       su.k0 = k;
       su.n = (int)std::min<long long>(TRAIN_TABLE, a.K - k);
-      for (int i = 0; i < su.n; ++i) su.steps[i] = adam_step_size(a.lr, a.lrd, a.beta1, a.beta2, a.step0 + k + i + 1);
-      launch_train_setup(su, st);
+      setup(su, st);
     }
     if (sg && !sg->exec && !sg->bad && sg->seen >= 1)
       capture_step(ctx, sg, dyn, [&](cudaStream_t cs) {
@@ -1861,12 +1874,74 @@ static int train_steps(brl_ctx* ctx, const TrainArgs& a, const brl_ctx::StepKey&
   return BRL_OK;
 }
 
+// ClippedAdam's table: the step sizes brl_clipped_adam{,_vi} computes
+static auto clipped_adam_setup(float lr, float lrd, float beta1, float beta2, long long step0) {
+  return [=](TrainSetup& su, cudaStream_t st) {
+    for (int i = 0; i < su.n; ++i) su.steps[i] = adam_step_size(lr, lrd, beta1, beta2, step0 + su.k0 + i + 1);
+    launch_train_setup(su, st);
+  };
+}
+
 // the logged step metrics of M members from their (loc, scale) pairs at src + m mstride, then row k of the results
 static void train_metrics_tail(const TrainBufs& t, const float* src, long long mstride, long long M, long long B, int nscal,
                                cudaStream_t st) {
   launch_split_pred(src, mstride, (int)M, B, t.pred, t.std, st);
   launch_test_metrics(t.pred, t.std, t.yb, B, t.met, t.hist, st, 5, (int)M);
   launch_train_tail(t.d, t.scal, nscal, t.met, (int)M, st);
+}
+
+// the most hnn_step carves from its workspace for M members of B windows (every optional image included)
+static size_t hnn_step_bytes(const NetSpec& n, long long M, long long B) {
+  Carve c(nullptr, 0);
+  ActBufs ab;
+  carve_forward(n, c, B, 1, ab);
+  carve_train(n, c, B, ab);
+  carve_tl(n, c, B, ab);
+  carve_members(n, c, B, M, false, ab);
+  return c.used;
+}
+
+// brl_hnn_train_steps (kind 6: ClippedAdam) and brl_hnn_train_steps_adam (kind 7: torch's Adam), which differ in the optimizer
+// alone.  `opt` holds the float operands the optimizer launch bakes into a captured step; with `kind` they join the graph key, so
+// neither call replays the other's graph.  setup(su, col2, stream) writes the descriptor and its table (an Adam call also the second
+// column col2), optim(bufs, col2, stream) is step 2 of step k.  Torch's Adam keeps its sqrt(1 - beta2^t) column of TRAIN_TABLE floats
+// in front of the step's workspace: brl_workspace_bytes(B, M, 6) leaves the HNN step more than that beyond what it carves (code 3
+// adds 4 KB, code 1 at M = 1 a [P] weight sample and the moment state the step does not use).
+template <class Setup, class Optim>
+static int hnn_train_steps(brl_ctx* ctx, const char* fn, const TrainArgs& a, float* theta, const float* exp_avg, const float* exp_avg_sq,
+                           float p_dropout, int kind, const float opt[5], void* workspace, size_t workspace_bytes, Setup setup,
+                           Optim optim, cudaStream_t st) {
+  if (int rc = train_args_ok(fn, a)) return rc;
+  BRL_REQUIRE(p_dropout >= 0.f && p_dropout < 1.f, std::string(fn) + ": bad p_dropout");
+  const long long M = a.M, B = a.B;
+  const int64_t need = brl_workspace_bytes(ctx, B, M, 6, 0);
+  if ((int64_t)workspace_bytes < need)
+    return fail(BRL_ERR_WORKSPACE, std::string(fn) + ": workspace too small; need " + std::to_string(need) + " bytes");
+  const NetSpec& n = *ctx->net;
+  Carve c(workspace, workspace_bytes);
+  TrainBufs t;
+  carve_train_steps(n, c, M, B, false, t);
+  float* col2 = kind == 7 ? c.take<float>(TRAIN_TABLE) : nullptr;
+  char* sws = (char*)workspace + c.used;
+  const size_t sws_bytes = workspace_bytes - c.used;
+  if (col2 && (!c.ok || hnn_step_bytes(n, M, B) > sws_bytes))
+    return fail(BRL_ERR_WORKSPACE, std::string(fn) + ": workspace too small for the optimizer's table");
+  brl_ctx::StepKey key;
+  memset(&key, 0, sizeof(key));
+  key.B = B; key.mode = -1 /* HNN */; key.particles = 1; key.compute_grads = 1; key.backend = ctx->gemm_backend;
+  key.members = (int)M; key.prior_loc = p_dropout; key.mu = theta; key.ws = workspace; key.ws_bytes = workspace_bytes; key.train = kind;
+  memcpy(key.opt, opt, sizeof(key.opt));
+  key.state[0] = exp_avg; key.state[1] = exp_avg_sq;
+  auto body = [&](const brl_noise* nz, cudaStream_t s) {
+    launch_train_gather(t.d, t.xb, t.yb, M * B, s);
+    const int rc = hnn_step(ctx, t.xb, t.yb, M, B, theta, p_dropout, nz, 1, t.scal, t.g0, t.out, sws, sws_bytes, s, false);
+    if (rc != BRL_OK) return rc;
+    optim(t, col2, s);
+    train_metrics_tail(t, t.out, B * 2, M, B, 2, s);
+    BRL_CUDA(cudaGetLastError());
+    return BRL_OK;
+  };
+  return train_steps(ctx, a, key, t, [&](TrainSetup& su, cudaStream_t s) { setup(su, col2, s); }, body, st);
 }
 
 extern "C" {
@@ -1880,8 +1955,7 @@ int brl_elbo_train_steps(brl_ctx* ctx, const float* X, const float* Y, int64_t N
   BRL_REQUIRE(ctx && loc && log_scale && scale && m_loc && v_loc && m_log_scale && v_log_scale && workspace,
               "brl_elbo_train_steps: NULL argument");
   DeviceGuard dg(ctx->device);
-  const TrainArgs a{X, Y, N, idx, K, M, B, step0, lr, beta1, beta2, eps, clip_norm, lrd, weight_decay, seed, sample0, window0,
-                    scalars, metrics};
+  const TrainArgs a{X, Y, N, idx, K, M, B, step0, seed, sample0, window0, scalars, metrics};
   if (int rc = train_args_ok("brl_elbo_train_steps", a)) return rc;
   BRL_REQUIRE(particles > 0 && particles <= GRAPH_MAX_PARTICLES && dataset_size > 0 && prior_scale > 0.f,
               "brl_elbo_train_steps: bad particles (1 to 8), dataset size or prior scale");
@@ -1923,7 +1997,7 @@ int brl_elbo_train_steps(brl_ctx* ctx, const float* X, const float* Y, int64_t N
     BRL_CUDA(cudaGetLastError());
     return BRL_OK;
   };
-  return train_steps(ctx, a, key, t, body, (cudaStream_t)stream);
+  return train_steps(ctx, a, key, t, clipped_adam_setup(lr, lrd, beta1, beta2, step0), body, (cudaStream_t)stream);
 }
 
 int brl_hnn_train_steps(brl_ctx* ctx, const float* X, const float* Y, int64_t N, const int64_t* idx, int64_t K, int64_t M, int64_t B,
@@ -1932,36 +2006,42 @@ int brl_hnn_train_steps(brl_ctx* ctx, const float* X, const float* Y, int64_t N,
                         int64_t window0, double* scalars, double* metrics, void* workspace, size_t workspace_bytes, void* stream) {
   BRL_REQUIRE(ctx && theta && exp_avg && exp_avg_sq && workspace, "brl_hnn_train_steps: NULL argument");
   DeviceGuard dg(ctx->device);
-  const TrainArgs a{X, Y, N, idx, K, M, B, step0, lr, beta1, beta2, eps, clip_norm, lrd, weight_decay, seed, sample0, window0,
-                    scalars, metrics};
-  if (int rc = train_args_ok("brl_hnn_train_steps", a)) return rc;
-  BRL_REQUIRE(p_dropout >= 0.f && p_dropout < 1.f, "brl_hnn_train_steps: bad p_dropout");
-  const int64_t need = brl_workspace_bytes(ctx, B, M, 6, 0);
-  if ((int64_t)workspace_bytes < need)
-    return fail(BRL_ERR_WORKSPACE, "brl_hnn_train_steps: workspace too small; need " + std::to_string(need) + " bytes");
-  const NetSpec& n = *ctx->net;
-  Carve c(workspace, workspace_bytes);
-  TrainBufs t;
-  carve_train_steps(n, c, M, B, false, t);
-  char* sws = (char*)workspace + c.used;
-  const size_t sws_bytes = workspace_bytes - c.used;
-  brl_ctx::StepKey key;
-  memset(&key, 0, sizeof(key));
-  key.B = B; key.mode = -1 /* HNN */; key.particles = 1; key.compute_grads = 1; key.backend = ctx->gemm_backend;
-  key.members = (int)M; key.prior_loc = p_dropout; key.mu = theta; key.ws = workspace; key.ws_bytes = workspace_bytes; key.train = 6;
+  const TrainArgs a{X, Y, N, idx, K, M, B, step0, seed, sample0, window0, scalars, metrics};
   const float opt[5] = {beta1, beta2, eps, clip_norm, weight_decay};
-  memcpy(key.opt, opt, sizeof(opt));
-  key.state[0] = exp_avg; key.state[1] = exp_avg_sq;
-  auto body = [&](const brl_noise* nz, cudaStream_t s) {
-    launch_train_gather(t.d, t.xb, t.yb, M * B, s);
-    const int rc = hnn_step(ctx, t.xb, t.yb, M, B, theta, p_dropout, nz, 1, t.scal, t.g0, t.out, sws, sws_bytes, s, false);
-    if (rc != BRL_OK) return rc;
-    launch_clipped_adam(theta, t.g0, exp_avg, exp_avg_sq, M * n.P, t.d, beta1, beta2, eps, clip_norm, weight_decay, s);
-    train_metrics_tail(t, t.out, B * 2, M, B, 2, s);
-    BRL_CUDA(cudaGetLastError());
-    return BRL_OK;
-  };
-  return train_steps(ctx, a, key, t, body, (cudaStream_t)stream);
+  const long long MP = M * ctx->net->P;
+  return hnn_train_steps(ctx, "brl_hnn_train_steps", a, theta, exp_avg, exp_avg_sq, p_dropout, 6, opt, workspace, workspace_bytes,
+                         [su0 = clipped_adam_setup(lr, lrd, beta1, beta2, step0)](TrainSetup& su, float*, cudaStream_t s) { su0(su, s); },
+                         [=](const TrainBufs& t, const float*, cudaStream_t s) {
+                           launch_clipped_adam(theta, t.g0, exp_avg, exp_avg_sq, MP, t.d, beta1, beta2, eps, clip_norm, weight_decay, s);
+                         },
+                         (cudaStream_t)stream);
+}
+
+int brl_hnn_train_steps_adam(brl_ctx* ctx, const float* X, const float* Y, int64_t N, const int64_t* idx, int64_t K, int64_t M,
+                             int64_t B, float* theta, float* exp_avg, float* exp_avg_sq, int64_t step0, double lr, double beta1,
+                             double beta2, double eps, double weight_decay, float p_dropout, uint64_t seed, int64_t sample0,
+                             int64_t window0, double* scalars, double* metrics, void* workspace, size_t workspace_bytes, void* stream) {
+  BRL_REQUIRE(ctx && theta && exp_avg && exp_avg_sq && workspace, "brl_hnn_train_steps_adam: NULL argument");
+  DeviceGuard dg(ctx->device);
+  BRL_REQUIRE(lr >= 0.0 && beta1 >= 0.0 && beta1 < 1.0 && beta2 >= 0.0 && beta2 < 1.0 && eps >= 0.0,
+              "brl_hnn_train_steps_adam: bad lr, betas or eps");
+  const TrainArgs a{X, Y, N, idx, K, M, B, step0, seed, sample0, window0, scalars, metrics};
+  const AdamArgs aa = torch_adam_args(beta1, beta2, eps, weight_decay);
+  const float opt[5] = {aa.w1, aa.b2, aa.w2, aa.eps, aa.wd};
+  const long long MP = M * ctx->net->P;
+  return hnn_train_steps(ctx, "brl_hnn_train_steps_adam", a, theta, exp_avg, exp_avg_sq, p_dropout, 7, opt, workspace, workspace_bytes,
+                         [=](TrainSetup& su, float* bc2, cudaStream_t s) {
+                           TrainSetupAdam sa;
+                           sa.s = su;
+                           sa.bc2 = bc2;
+                           for (int i = 0; i < su.n; ++i)
+                             torch_adam_step(lr, beta1, beta2, step0 + su.k0 + i + 1, &sa.s.steps[i], &sa.bc2_tab[i]);
+                           launch_train_setup(sa, s);
+                         },
+                         [=](const TrainBufs& t, const float* bc2, cudaStream_t s) {
+                           launch_adam(theta, t.g0, exp_avg, exp_avg_sq, MP, t.d, bc2, aa, s);
+                         },
+                         (cudaStream_t)stream);
 }
 
 int brl_mixture_moments(const float* mu_m, const float* sigma_m, int64_t M, int64_t nn, float* mu, float* sigma, void* stream) {
@@ -2004,6 +2084,17 @@ int brl_clipped_adam(float* param, const float* grad, float* exp_avg, float* exp
   BRL_REQUIRE(param && grad && exp_avg && exp_avg_sq && nn > 0 && step >= 1, "brl_clipped_adam: bad argument");
   launch_clipped_adam(param, grad, exp_avg, exp_avg_sq, nn, adam_step_size(lr, lrd, beta1, beta2, step), beta1, beta2, eps,
                       clip_norm, weight_decay, (cudaStream_t)stream);
+  BRL_CUDA(cudaGetLastError());
+  return BRL_OK;
+}
+
+int brl_adam(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, int64_t nn, int64_t step, double lr, double beta1,
+             double beta2, double eps, double weight_decay, void* stream) {
+  BRL_REQUIRE(param && grad && exp_avg && exp_avg_sq && nn > 0 && step >= 1, "brl_adam: bad argument");
+  BRL_REQUIRE(lr >= 0.0 && beta1 >= 0.0 && beta1 < 1.0 && beta2 >= 0.0 && beta2 < 1.0 && eps >= 0.0, "brl_adam: bad lr, betas or eps");
+  float ss, bc2;
+  torch_adam_step(lr, beta1, beta2, step, &ss, &bc2);
+  launch_adam(param, grad, exp_avg, exp_avg_sq, nn, ss, bc2, torch_adam_args(beta1, beta2, eps, weight_decay), (cudaStream_t)stream);
   BRL_CUDA(cudaGetLastError());
   return BRL_OK;
 }

@@ -809,10 +809,71 @@ void launch_clipped_adam(float* p, const float* g, float* m, float* v, long long
 }
 
 // ------------------------------------------------------------------------------------------------
+// torch.optim.Adam
+// ------------------------------------------------------------------------------------------------
+// Per element, what torch.optim.Adam's single-tensor path (fp32, amsgrad = maximize = False) computes, one torch op per line, each
+// written with round-to-nearest intrinsics so that no contraction spans two torch ops (measured against torch on a B200: moments
+// bit-identical without weight decay, parameters within 5.3e-8 of their largest magnitude, as far as torch's foreach path lies):
+//   grad.add(param, alpha=wd)              g = fma(wd, p, g)                       (L2 weight decay, only when wd != 0)
+//   exp_avg.lerp_(grad, w1)                m = fma(w1, g - m, m)  (w1 < 0.5; else fma(-(g - m), 1 - w1, g), torch's lerp)
+//   exp_avg_sq.mul_(b2).addcmul_(g, g, w2) v = fma(w2, g g, v b2)
+//   exp_avg_sq.sqrt() / bc2_sqrt + eps     d = sqrt(v) (1 / bc2_sqrt) + eps        (a tensor over a host scalar multiplies by its
+//                                                                                   reciprocal, rounded in float)
+//   param.addcdiv_(m, d, -step_size)       p = fma(-step_size, m / d, p)
+// The (step_size, bc2_sqrt) pair comes from the host (HostAdam: brl_adam) or from the K-step call's table at a device index
+// (DevAdam: brl_hnn_train_steps_adam).
+struct HostAdam {
+  float ss, bc2;
+  __device__ __forceinline__ float2 get() const { return make_float2(ss, bc2); }
+};
+struct DevAdam {
+  const float *ss, *bc2;
+  const int* at;
+  __device__ __forceinline__ float2 get() const {
+    const int k = *at;
+    return make_float2(ss[k], bc2[k]);
+  }
+};
+template <class Step>
+__global__ void adam_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v,
+                            long long n, Step sp, AdamArgs a) {
+  const float2 s = sp.get();
+  const float neg_ss = -s.x, inv_bc2 = __fdiv_rn(1.f, s.y);
+  const bool small = fabsf(a.w1) < 0.5f;
+  const float omw1 = __fsub_rn(1.f, a.w1);
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+    const float pi = p[i], mo = m[i], vo = v[i];
+    float gr = g[i];
+    if (a.wd != 0.f) gr = __fmaf_rn(a.wd, pi, gr);
+    const float diff = __fsub_rn(gr, mo);
+    const float mi = small ? __fmaf_rn(a.w1, diff, mo) : __fmaf_rn(-diff, omw1, gr);
+    const float vi = __fmaf_rn(a.w2, __fmul_rn(gr, gr), __fmul_rn(vo, a.b2));
+    const float den = __fadd_rn(__fmul_rn(__fsqrt_rn(vi), inv_bc2), a.eps);
+    m[i] = mi;
+    v[i] = vi;
+    p[i] = __fmaf_rn(neg_ss, __fdiv_rn(mi, den), pi);
+  }
+}
+template <class Step>
+static void adam_on(float* p, const float* g, float* m, float* v, long long n, Step sp, const AdamArgs& a, cudaStream_t st) {
+  ++g_launch_count;
+  adam_kernel<<<(unsigned)min((n + 255) / 256, (long long)148 * 8), 256, 0, st>>>(p, g, m, v, n, sp, a);
+}
+void launch_adam(float* p, const float* g, float* m, float* v, long long n, float step_size, float bc2_sqrt, const AdamArgs& a,
+                 cudaStream_t st) {
+  adam_on(p, g, m, v, n, HostAdam{step_size, bc2_sqrt}, a, st);
+}
+void launch_adam(float* p, const float* g, float* m, float* v, long long n, const TrainDesc* d, const float* bc2, const AdamArgs& a,
+                 cudaStream_t st) {
+  const DevStep s = dev_step(d);
+  adam_on(p, g, m, v, n, DevAdam{s.tab, bc2, s.at}, a, st);
+}
+
+// ------------------------------------------------------------------------------------------------
 // K training steps per call (brl_elbo_train_steps / brl_hnn_train_steps): every per-step quantity is read from the call's
 // descriptor in device memory, so one captured step serves every step of every later call with the same configuration
 // ------------------------------------------------------------------------------------------------
-__global__ void train_setup_kernel(const TrainSetup s) {
+__device__ __forceinline__ void train_setup(const TrainSetup& s) {
   TrainDesc* d = s.d;
   for (int i = threadIdx.x; i < s.n; i += blockDim.x) d->steps[i] = s.steps[i];
   if (threadIdx.x == 0) {
@@ -821,9 +882,19 @@ __global__ void train_setup_kernel(const TrainSetup s) {
     d->seed = s.seed; d->sample0 = s.sample0; d->window0 = s.window0;
   }
 }
+__global__ void train_setup_kernel(const TrainSetup s) { train_setup(s); }
 void launch_train_setup(const TrainSetup& s, cudaStream_t st) {
   ++g_launch_count;
   train_setup_kernel<<<1, 256, 0, st>>>(s);
+}
+// the same, plus torch Adam's sqrt(1 - beta2^t) column of this table
+__global__ void train_setup_adam_kernel(const TrainSetupAdam s) {
+  train_setup(s.s);
+  for (int i = threadIdx.x; i < s.s.n; i += blockDim.x) s.bc2[i] = s.bc2_tab[i];
+}
+void launch_train_setup(const TrainSetupAdam& s, cudaStream_t st) {
+  ++g_launch_count;
+  train_setup_adam_kernel<<<1, 256, 0, st>>>(s);
 }
 
 // windows X[idx[k, w]] -> xb [MB,30,18] as float4 (a window is 135 of them), labels -> yb [MB]; an index outside [0, N) reads

@@ -251,4 +251,27 @@ void launch_clipped_adam_vi(float* loc, float* ls, float* scale, const float* g_
                             float* m_ls, float* v_ls, long long n, const TrainDesc* d, float b1, float b2, float eps, float clip,
                             float wd, cudaStream_t st);
 
+// ---- torch.optim.Adam (brl_adam / brl_hnn_train_steps_adam) ----
+// its float operands, each the float torch rounds its Python double to: w1 = 1 - beta1 (the lerp weight), b2 = beta2,
+// w2 = 1 - beta2 (the addcmul value), eps, wd = weight_decay
+struct AdamArgs {
+  float w1, b2, w2, eps, wd;
+};
+// one step with step_size = lr / (1 - beta1^t) and bc2_sqrt = sqrt(1 - beta2^t) from the host ...
+void launch_adam(float* p, const float* g, float* m, float* v, long long n, float step_size, float bc2_sqrt, const AdamArgs& a,
+                 cudaStream_t st);
+// ... or step k's pair d->steps[d->kt], bc2[d->kt] read on the device
+void launch_adam(float* p, const float* g, float* m, float* v, long long n, const TrainDesc* d, const float* bc2, const AdamArgs& a,
+                 cudaStream_t st);
+// the setup launch of brl_hnn_train_steps_adam: TrainSetup (step sizes in `steps`) plus the sqrt(1 - beta2^t) column, which goes to
+// `bc2` [TRAIN_TABLE] in the workspace.  Its arguments take 7.3 KB: above the 4 KB of old toolkits, within the 32 764 bytes that
+// CUDA 12.1+ allows a kernel on Volta and newer.
+struct TrainSetupAdam {
+  TrainSetup s;
+  float* bc2;
+  float bc2_tab[TRAIN_TABLE];
+};
+static_assert(sizeof(TrainSetupAdam) <= 32764, "train_setup_adam_kernel's arguments exceed the kernel parameter limit");
+void launch_train_setup(const TrainSetupAdam& s, cudaStream_t st);
+
 }  // namespace brl

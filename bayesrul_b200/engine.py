@@ -518,13 +518,19 @@ class Engine:
         return dict(scalars=scalars, metrics=metrics)
 
     def hnn_train_steps(self, X, Y, idx, theta, opt_state, *, step0: int, lr: float, betas=(0.9, 0.999), eps: float = 1e-8,
-                        clip_norm: float = 1e30, lrd: float = 1.0, weight_decay: float = 0.0, p_dropout: float = 0.0, seed: int,
-                        sample0: int = 0, window0: int = 0):
+                        clip_norm: Optional[float] = None, lrd: Optional[float] = None, weight_decay: float = 0.0,
+                        p_dropout: float = 0.0, seed: int, sample0: int = 0, window0: int = 0, optimizer: str = "clipped_adam"):
         """K heteroscedastic-NN training steps in one call (the members of a deep ensemble): step k is hnn_step_ensemble
         (hnn_step at M = 1) on X[idx[k]], Y[idx[k]] with Noise(seed + 0x9E3779B97F4A7C15 (k + 1) mod 2**64, sample0, window0),
-        then clipped_adam over theta [M,P] with opt_state = (exp_avg, exp_avg_sq) at step step0 + k + 1 (the default clip_norm
-        disables the clip: plain Adam), then step_metrics_ensemble of the step's (loc, scale).  Returns dict(scalars [K,M,2] =
-        (loss, mse), metrics [K,M,5]); synchronises only for the index range check, as elbo_train_steps."""
+        then the optimizer over theta [M,P] with opt_state = (exp_avg, exp_avg_sq) at step step0 + k + 1, then
+        step_metrics_ensemble of the step's (loc, scale).  optimizer="clipped_adam" is clipped_adam (clip_norm defaults to 1e30,
+        which disables the clip, and lrd to 1.0); optimizer="adam" is Engine.adam, torch.optim.Adam's update, and takes no
+        clip_norm or lrd.  Returns dict(scalars [K,M,2] = (loss, mse), metrics [K,M,5]); synchronises only for the index range
+        check, as elbo_train_steps."""
+        if optimizer not in ("clipped_adam", "adam"):
+            raise RuntimeError(f"bayesrul_b200: optimizer must be 'clipped_adam' or 'adam', got {optimizer!r}")
+        if optimizer == "adam" and (clip_norm is not None or lrd is not None):
+            raise RuntimeError("bayesrul_b200: optimizer='adam' (torch.optim.Adam) has no clip_norm or lrd")
         if len(opt_state) != 2:
             raise RuntimeError("bayesrul_b200: opt_state must be (exp_avg, exp_avg_sq)")
         ts = (theta,) + tuple(opt_state)
@@ -533,11 +539,16 @@ class Engine:
         scalars = torch.empty(K, M, 2, dtype=torch.float64, device=self.device)
         metrics = torch.empty(K, M, 5, dtype=torch.float64, device=self.device)
         ws = self._ws_for(B, M, 6, "simt")
-        _lib.check(self.lib.brl_hnn_train_steps(self.ctx, X.data_ptr(), Y.data_ptr(), X.shape[0], idx.data_ptr(), K, M, B,
-                                                *[t.data_ptr() for t in ts], int(step0), float(lr), float(betas[0]), float(betas[1]),
-                                                float(eps), float(clip_norm), float(lrd), float(weight_decay), float(p_dropout),
-                                                int(seed) & 0xFFFFFFFFFFFFFFFF, int(sample0), int(window0), scalars.data_ptr(),
-                                                metrics.data_ptr(), ws.data_ptr(), ws.numel(), self._stream()))
+        head = (self.ctx, X.data_ptr(), Y.data_ptr(), X.shape[0], idx.data_ptr(), K, M, B, *[t.data_ptr() for t in ts], int(step0))
+        tail = (float(p_dropout), int(seed) & 0xFFFFFFFFFFFFFFFF, int(sample0), int(window0), scalars.data_ptr(), metrics.data_ptr(),
+                ws.data_ptr(), ws.numel(), self._stream())
+        if optimizer == "adam":
+            _lib.check(self.lib.brl_hnn_train_steps_adam(*head, float(lr), float(betas[0]), float(betas[1]), float(eps),
+                                                         float(weight_decay), *tail))
+        else:
+            _lib.check(self.lib.brl_hnn_train_steps(*head, float(lr), float(betas[0]), float(betas[1]), float(eps),
+                                                    float(1e30 if clip_norm is None else clip_norm), float(1.0 if lrd is None else lrd),
+                                                    float(weight_decay), *tail))
         return dict(scalars=scalars, metrics=metrics)
 
     # -- A14 / A15 / N1 ------------------------------------------------------------------------------------
@@ -601,6 +612,20 @@ class Engine:
             _lib.check(self.lib.brl_clipped_adam(param.data_ptr(), grad.data_ptr(), exp_avg.data_ptr(),
                                                  exp_avg_sq.data_ptr(), param.numel(), int(step), lr, betas[0], betas[1],
                                                  eps, clip_norm, lrd, weight_decay, self._stream()))
+
+    def adam(self, param, grad, exp_avg, exp_avg_sq, step: int, lr: float, betas=(0.9, 0.999), eps: float = 1e-8,
+             weight_decay: float = 0.0) -> None:
+        """One torch.optim.Adam step (amsgrad=False, maximize=False; L2 weight decay) over flat fp32 tensors, in place:
+        step `step` >= 1 of the optimizer, with the hyper-parameters it holds.  The update is torch's single-tensor formula, one
+        rounding per torch op (DESIGN §4.8.1)."""
+        ts = (param, grad, exp_avg, exp_avg_sq)
+        for t, n in zip(ts, ("param", "grad", "exp_avg", "exp_avg_sq")):
+            _chk(t, self.device, n)
+            if t.numel() != param.numel():
+                raise RuntimeError("bayesrul_b200: adam tensors must have the same number of elements")
+        with self._on_device():
+            _lib.check(self.lib.brl_adam(*[t.data_ptr() for t in ts], param.numel(), int(step), float(lr), float(betas[0]),
+                                         float(betas[1]), float(eps), float(weight_decay), self._stream()))
 
     def clipped_adam_vi(self, loc, log_scale, scale, grad_loc, grad_log_scale, m_loc, v_loc, m_ls, v_ls, step: int, lr: float,
                         betas=(0.95, 0.999), eps=1e-8, clip_norm=15.0, lrd=1.0, weight_decay=0.0, grad_scale: float = 1.0) -> None:

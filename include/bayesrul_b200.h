@@ -300,6 +300,14 @@ int brl_hnn_train_steps(brl_ctx* ctx, const float* X /*[N,30,18]*/, const float*
                         float lr, float beta1, float beta2, float eps, float clip_norm, float lrd, float weight_decay,
                         float p_dropout, uint64_t seed, int64_t sample0, int64_t window0, double* scalars /*[K,M,2]*/,
                         double* metrics /*[K,M,5]*/, void* workspace, size_t workspace_bytes, void* stream);
+/* brl_hnn_train_steps with step 2 replaced by brl_adam (torch.optim.Adam) at Adam step step0 + k + 1: no clip, no lr decay.  The
+ * data, index, seed, member, metrics and graph contract and the workspace (brl_workspace_bytes(B, M, 6)) are those of
+ * brl_hnn_train_steps; a step graph captured by one of the two calls is never replayed by the other. */
+int brl_hnn_train_steps_adam(brl_ctx* ctx, const float* X /*[N,30,18]*/, const float* Y /*[N]*/, int64_t N,
+                             const int64_t* idx /*[K,M,B]*/, int64_t K, int64_t M, int64_t B, float* theta /*[M,P]*/, float* exp_avg,
+                             float* exp_avg_sq, int64_t step0, double lr, double beta1, double beta2, double eps, double weight_decay,
+                             float p_dropout, uint64_t seed, int64_t sample0, int64_t window0, double* scalars /*[K,M,2]*/,
+                             double* metrics /*[K,M,5]*/, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- deep-ensemble mixture moments (models/deepens.py:21-24), [M,n] -> [n] ------------- */
 int brl_mixture_moments(const float* mu_m, const float* sigma_m, int64_t M, int64_t n, float* mu,
@@ -339,6 +347,15 @@ int brl_clipped_adam_vi_scaled(float* loc, float* log_scale, float* scale, const
                                float* m_loc, float* v_loc, float* m_log_scale, float* v_log_scale, int64_t n, int64_t step, float lr,
                                float beta1, float beta2, float eps, float clip_norm, float lrd, float weight_decay, float grad_scale,
                                void* stream);
+
+/* ---- torch.optim.Adam over a flat buffer (single-tensor fp32 path, amsgrad = maximize = False: the optimizer the HNN
+ *      and deep-ensemble members are configured with), one step t = `step` >= 1, per element:
+ *        g += weight_decay p (L2, when weight_decay != 0);  m = lerp(m, g, 1 - beta1);  v = beta2 v + (1 - beta2) g g;
+ *        p -= step_size m / (sqrt(v) / bc2_sqrt + eps),  step_size = lr / (1 - beta1^t),  bc2_sqrt = sqrt(1 - beta2^t).
+ *      The hyper-parameters are doubles, as the optimizer holds them: the step scalars are computed in double and every operand
+ *      is rounded to float where torch rounds it; each of torch's ops is rounded on its own (no contraction across them). */
+int brl_adam(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, int64_t n, int64_t step, double lr, double beta1,
+             double beta2, double eps, double weight_decay, void* stream);
 
 #ifdef __cplusplus
 }
