@@ -81,6 +81,8 @@ SIGNATURES = {
                                 _vp, _vp, _vp, _sz, _vp]),
     "brl_hnn_train_steps_adam": (_i, [_vp, _vp, _vp, _i64, _vp, _i64, _i64, _i64] + [_vp] * 3 + [_i64] + [_d] * 5 + [_f, C.c_uint64, _i64,
                                      _i64, _vp, _vp, _vp, _sz, _vp]),
+    "brl_elbo_val_steps": (_i, [_vp, _vp, _vp, _i64, _vp, _i64, _i64, _vp, _vp, _i, _i, _i64, _i, _f, _f, _i64, C.c_uint64, _i64, _i64,
+                               _vp, _vp, _vp, _sz, _vp]),
     "brl_mixture_moments": (_i, [_vp, _vp, _i64, _i64, _vp, _vp, _vp]),
     "brl_step_metrics": (_i, [_vp, _vp, _vp, _i64, _vp, _vp, _sz, _vp]),
     "brl_step_metrics_ensemble": (_i, [_vp, _vp, _vp, _i64, _i64, _vp, _vp, _sz, _vp]),

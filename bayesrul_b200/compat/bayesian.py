@@ -190,8 +190,8 @@ class BNN(_Base):
             self.log(k, v, on_step=False, on_epoch=True)
         return dict(scalars=res["scalars"] if res else None, metrics=res["metrics"] if res else None, perm=perm)
 
-    def validation_step(self, batch, batch_idx):  # bayesian.py:168-197 (no fit context: weight sampling)
-        (x, y) = batch[0], batch[1]
+    def _val_batch(self, x, y):
+        """svi.evaluate_loss, the predictive and the metrics of one batch; the values validation_step logs (bayesian.py:168-197)"""
         elbo = self.svi.evaluate_loss(x, y.unsqueeze(-1))
         kl = float(self.svi.last["scalars"][2].item())
         output = self.bnn.predict(x, num_predictions=self.hparams.mc_samples_eval,
@@ -200,12 +200,62 @@ class BNN(_Base):
             output = output[0]
         loc, scale = output[:, 0], output[:, 1]
         m = self.bnn.engine.step_metrics(loc, scale, y)
-        self.log("elbo/val", elbo)
-        self.log("mse/val", m[1].float())
-        self.log("kl/val", kl)
-        self.log("likelihood/val", elbo - kl)
-        self.log("rmsce/val", m[3].float())
-        self.log("sharp/val", m[2].float())
+        return {"elbo/val": elbo, "mse/val": m[1].float(), "kl/val": kl, "likelihood/val": elbo - kl, "rmsce/val": m[3].float(),
+                "sharp/val": m[2].float()}
+
+    def validation_step(self, batch, batch_idx):  # bayesian.py:168-197 (no fit context: weight sampling)
+        for k, v in self._val_batch(batch[0], batch[1]).items():
+            self.log(k, v)
+
+    def validate_epoch(self, x, y, batch_size: int):
+        """One validation epoch over the DEVICE-resident split x [N,30,18], y [N]: what Lightning does with validation_step over
+        the batches of an unshuffled DataLoader, without two host reads per batch.  The floor(N / batch_size) full batches of
+        arange(N), in order, run as ONE Engine.elbo_val_steps call with the BNN's guide, mc_samples_train particles,
+        mc_samples_eval predictive samples, engine and ELBO back-end; it continues the BNN's seed sequence (two keys per batch, as
+        validation_step draws them) and advances it.  The remainder batch goes through validation_step's own path.  Logs the epoch
+        means of the keys validation_step logs, each batch weighted by its size as Lightning's epoch mean weighs it, each with the
+        type validation_step logs it with; returns dict(scalars [K,4], metrics [K,5]) of the K full batches."""
+        N, bs = int(x.shape[0]), int(batch_size)
+        if bs <= 0 or y.numel() != N:
+            raise RuntimeError("bayesrul_b200: validate_epoch needs batch_size > 0 and one target per window")
+        bnn, svi = self.bnn, self.svi
+        loss_factor = svi.model_scale / (1.0 / (bnn.likelihood.dataset_size * 30 * 18))  # what evaluate_loss multiplies the loss by
+        if svi.no_obs or loss_factor != 1.0:
+            raise RuntimeError("bayesrul_b200: validate_epoch evaluates the ELBO at its own scale (a scaled or KL-only loss is not supported)")
+        K = N // bs
+        x, y = x.contiguous(), y.reshape(-1).contiguous()
+        res = None
+        sums, weight = {}, 0
+        if K > 0:
+            g, eng = bnn.net_guide, bnn.engine
+            be = bnn.train_backend
+            if be == "auto":
+                be = "fused" if getattr(self.net, "kind", "") == "inception" else "simt"
+            eng.set_gemm_backend(be)
+            idx = torch.arange(K * bs, device=x.device).view(K, bs)
+            res = eng.elbo_val_steps(x, y, idx, g.loc, g.scale, guide=g.family, particles=self.hparams.mc_samples_train,
+                                     S=self.hparams.mc_samples_eval, prior_loc=bnn.prior.loc, prior_scale=bnn.prior.scale,
+                                     dataset_size=bnn.likelihood.dataset_size,
+                                     seed=(bnn.seed + 0x9E3779B97F4A7C15 * bnn._step) & 0xFFFFFFFFFFFFFFFF, engine=bnn.engine_kind)
+            bnn._step += 2 * K
+            bnn._last_kl = res["scalars"][K - 1, 2]
+            sc, mt = res["scalars"], res["metrics"]
+            elbo, kl = sc[:, 0].sum(), sc[:, 2].sum()
+            f32 = lambda t: t.float().double().sum()  # logged as float32 by validation_step
+            sums = {"elbo/val": elbo, "mse/val": f32(mt[:, 1]), "kl/val": kl, "likelihood/val": elbo - kl, "rmsce/val": f32(mt[:, 3]),
+                    "sharp/val": f32(mt[:, 2])}
+            sums = {k: v * bs for k, v in sums.items()}
+            weight = K * bs
+        if K * bs < N:
+            vals = self._val_batch(x[K * bs:], y[K * bs:])
+            for k, v in vals.items():
+                sums[k] = sums.get(k, 0.0) + (v.double() if isinstance(v, torch.Tensor) else v) * (N - K * bs)
+            weight += N - K * bs
+        tensor_keys = ("mse/val", "rmsce/val", "sharp/val")
+        means = torch.stack([torch.as_tensor(v, dtype=torch.float64, device=x.device) for v in sums.values()]).div(weight).tolist()
+        for k, v in zip(sums, means):
+            self.log(k, torch.tensor(v, dtype=torch.float32, device=x.device) if k in tensor_keys else v)
+        return dict(scalars=res["scalars"] if res else None, metrics=res["metrics"] if res else None)
 
     def on_test_start(self) -> None:
         self.define_bnn()

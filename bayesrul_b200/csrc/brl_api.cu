@@ -102,11 +102,15 @@ struct brl_ctx {
     int train;
     float opt[5];
     const void* state[5];
+    // brl_elbo_val_steps (train = 8; mode WS, no gradients): the predictive's MC samples and engine
+    long long S;
+    int engine;
     bool operator==(const StepKey& o) const {
       return B == o.B && dataset_size == o.dataset_size && mode == o.mode && guide == o.guide && particles == o.particles &&
              compute_grads == o.compute_grads && backend == o.backend && has_log_sigma == o.has_log_sigma && members == o.members &&
              prior_loc == o.prior_loc && prior_scale == o.prior_scale && mu == o.mu && sigma == o.sigma && ws == o.ws &&
-             ws_bytes == o.ws_bytes && train == o.train && !memcmp(opt, o.opt, sizeof(opt)) && !memcmp(state, o.state, sizeof(state));
+             ws_bytes == o.ws_bytes && train == o.train && !memcmp(opt, o.opt, sizeof(opt)) && !memcmp(state, o.state, sizeof(state)) &&
+             S == o.S && engine == o.engine;
     }
   };
   struct StepGraph { StepKey key; cudaGraphExec_t exec = nullptr; int seen = 0, launches = 0; bool bad = false; };
@@ -284,6 +288,48 @@ static void carve_train_steps(const NetSpec& n, Carve& c, long long M, long long
   t.scal = c.take<double>((elbo ? 4 : 2) * M);
   t.met = c.take<double>(5 * M);
   t.hist = c.take<unsigned int>(256 * M);  // the step metrics' scratch, 1024 bytes per member
+}
+
+// brl_elbo_val_steps: the call's descriptor, the predictive draw's Philox key, the gathered batch and one batch's outputs ([S,B,2] of
+// the predictive, or [particles,B,2] of the ELBO step before it), aggregate, logged predictions, scalars and metrics (TrainBufs
+// without gradients), in front of the region that the ELBO step and then the predictive use in turn
+static void carve_val_steps(Carve& c, long long B, long long S, TrainBufs& t, unsigned long long*& key2) {
+  t.d = c.take<TrainDesc>(1);
+  key2 = c.take<unsigned long long>(4);
+  t.xb = c.take<float>(B * 540);
+  t.yb = c.take<float>(B);
+  t.g0 = t.g1 = t.g2 = nullptr;
+  t.out = c.take<float>(std::max<long long>(GRAPH_MAX_PARTICLES, S) * B * 2);
+  t.agg = c.take<float>(B * 2);
+  t.pred = c.take<float>(B);
+  t.std = c.take<float>(B);
+  t.scal = c.take<double>(4);
+  t.met = c.take<double>(5);
+  t.hist = c.take<unsigned int>(256);  // the step metrics' scratch
+}
+// the predictive's part of that region: S weight draws [S,P], their radial norms [S,n_sites], then brl_forward's workspace
+struct ValPredict {
+  float *wsamp, *norms;
+  size_t norms_bytes;
+  char* fws;
+  size_t fws_bytes;
+};
+static size_t carve_val_predict(const brl_ctx* ctx, Carve& c, long long B, long long S, int engine, ValPredict& v) {
+  const NetSpec& n = *ctx->net;
+  v.wsamp = c.take<float>(S * n.P);
+  const size_t at = c.used;
+  v.norms = c.take<float>(S * 2 * (long long)n.layers.size());
+  v.norms_bytes = c.used - at;
+  size_t fwd = tc_workspace_bytes(ctx->tc, B, S);
+  if (engine != BRL_ENGINE_TC_FP16) {
+    Carve f(nullptr, 0);
+    ActBufs ab;
+    carve_forward(n, f, B, S, ab);
+    fwd = f.used;
+  }
+  v.fws = c.take<char>((long long)fwd);
+  v.fws_bytes = fwd;
+  return c.used;
 }
 
 // device {seed, sample0, window0} of the step being captured (nullptr outside a capture): every Philox stream built by
@@ -950,6 +996,16 @@ int64_t brl_workspace_bytes(const brl_ctx* ctx, int64_t B, int64_t S, int train,
     const int64_t step = train == 5 ? (S == 1 ? brl_workspace_bytes(ctx, B, 2, 1, 0) : brl_workspace_bytes(ctx, B, S, 4, 0))
                                     : (S == 1 ? brl_workspace_bytes(ctx, B, 1, 1, 0) : brl_workspace_bytes(ctx, B, S, 3, 0));
     return (int64_t)c.used + step;
+  }
+  if (train == 7) {  // brl_elbo_val_steps: its buffers, then the larger of the ELBO step's workspace and the predictive's
+    TrainBufs t;
+    unsigned long long* key2;
+    carve_val_steps(c, B, S, t, key2);
+    Carve p(nullptr, 0);
+    ValPredict v;
+    const int64_t predict = (int64_t)carve_val_predict(ctx, p, B, S, engine, v);
+    const int64_t elbo = brl_workspace_bytes(ctx, B, 2, 1, 0);  // two particle lanes: Engine.elbo_step's workspace for particles > 1
+    return (int64_t)c.used + std::max(elbo, predict);
   }
   if (train == 3 || train == 4) {  // brl_hnn_step_ensemble / brl_elbo_step_ensemble over S members: the layout of their steps
     carve_forward(n, c, B, 1, ab);
@@ -1836,10 +1892,13 @@ static int train_args_ok(const char* fn, const TrainArgs& a) {
 // later step, in this call or a later one, is one graph launch.  Every TRAIN_TABLE steps setup(su, stream) fills the table of the
 // optimizer's per-step scalars for steps step0 + su.k0 + 1 ... (as the single-step optimizer entry point computes them) and makes
 // the one launch that writes the descriptor and that table.  Nothing synchronises the host.
+// A step that draws `keys` Philox keys takes keys k + 1 ... keys k + keys of the sequence seed + 0x9E3779B97F4A7C15 i; its body gets
+// the first (and derives the others: their captured launches read them from where the step's gather writes them).  graphable =
+// false keeps every step eager.
 template <class Setup, class Body>
 static int train_steps(brl_ctx* ctx, const TrainArgs& a, const brl_ctx::StepKey& key, const TrainBufs& t, Setup setup, Body body,
-                       cudaStream_t st) {
-  brl_ctx::StepGraph* sg = ctx->graph_enabled && !stream_capturing(st) ? graph_slot(ctx, key) : nullptr;
+                       cudaStream_t st, bool graphable = true, int keys = 1) {
+  brl_ctx::StepGraph* sg = graphable && ctx->graph_enabled && !stream_capturing(st) ? graph_slot(ctx, key) : nullptr;
   const unsigned long long* dyn = reinterpret_cast<const unsigned long long*>(reinterpret_cast<const char*>(t.d) + offsetof(TrainDesc, dyn));
   TrainSetup su;
   su.d = t.d; su.X = a.X; su.Y = a.Y; su.idx = reinterpret_cast<const long long*>(a.idx); su.scalars = a.scalars; su.metrics = a.metrics;
@@ -1862,7 +1921,7 @@ static int train_steps(brl_ctx* ctx, const TrainArgs& a, const brl_ctx::StepKey&
     } else {
       brl_noise nz;
       memset(&nz, 0, sizeof(nz));
-      nz.seed = a.seed + 0x9E3779B97F4A7C15ull * (uint64_t)(k + 1);
+      nz.seed = a.seed + 0x9E3779B97F4A7C15ull * (uint64_t)(keys * k + 1);
       nz.sample0 = a.sample0;
       nz.window0 = a.window0;
       const int rc = body(&nz, st);
@@ -2042,6 +2101,65 @@ int brl_hnn_train_steps_adam(brl_ctx* ctx, const float* X, const float* Y, int64
                            launch_adam(theta, t.g0, exp_avg, exp_avg_sq, MP, t.d, bc2, aa, s);
                          },
                          (cudaStream_t)stream);
+}
+
+// Batch k: gather -> brl_elbo_step (weight sampling, no gradients) with key 2k + 1 -> brl_sample_weights, brl_forward and (S > 1)
+// brl_aggregate_predictions with key 2k + 2 -> step metrics -> row k.  The ELBO step and the predictive share one region of the
+// workspace, one after the other.  A captured batch reads its ELBO key from the descriptor (g_dyn of the capture) and its predictive
+// key from key2: the sampler is captured with g_dyn pointing there.
+int brl_elbo_val_steps(brl_ctx* ctx, const float* X, const float* Y, int64_t N, const int64_t* idx, int64_t K, int64_t B, const float* loc,
+                       const float* scale, int guide, int particles, int64_t S, int engine, float prior_loc, float prior_scale,
+                       int64_t dataset_size, uint64_t seed, int64_t sample0, int64_t window0, double* scalars, double* metrics,
+                       void* workspace, size_t workspace_bytes, void* stream) {
+  BRL_REQUIRE(ctx && loc && scale && workspace, "brl_elbo_val_steps: NULL argument");
+  DeviceGuard dg(ctx->device);
+  const TrainArgs a{X, Y, N, idx, K, 1, B, 0, seed, sample0, window0, scalars, metrics};
+  if (int rc = train_args_ok("brl_elbo_val_steps", a)) return rc;
+  BRL_REQUIRE(particles > 0 && particles <= GRAPH_MAX_PARTICLES && dataset_size > 0 && prior_scale > 0.f,
+              "brl_elbo_val_steps: bad particles (1 to 8), dataset size or prior scale");
+  BRL_REQUIRE(S > 0 && S < (1 << 16) && B * 30 < (1ll << 31) / 512, "brl_elbo_val_steps: bad S or B");
+  BRL_REQUIRE(guide == BRL_GUIDE_NORMAL || guide == BRL_GUIDE_RADIAL, "Guide unknown. Choose from 'normal', 'radial'.");
+  BRL_REQUIRE(engine == BRL_ENGINE_SIMT_FP32 || engine == BRL_ENGINE_TC_FP16, "brl_elbo_val_steps: unknown engine");
+  const int64_t need = brl_workspace_bytes(ctx, B, S, 7, engine);
+  if ((int64_t)workspace_bytes < need)
+    return fail(BRL_ERR_WORKSPACE, "brl_elbo_val_steps: workspace too small; need " + std::to_string(need) + " bytes");
+  Carve c(workspace, workspace_bytes);
+  TrainBufs t;
+  unsigned long long* key2;
+  carve_val_steps(c, B, S, t, key2);
+  char* rws = (char*)workspace + c.used;
+  const size_t rbytes = workspace_bytes - c.used;
+  Carve pc(rws, rbytes);
+  ValPredict v;
+  carve_val_predict(ctx, pc, B, S, engine, v);
+  brl_ctx::StepKey key;
+  memset(&key, 0, sizeof(key));
+  key.B = B; key.dataset_size = dataset_size; key.mode = BRL_MODE_WS; key.guide = guide; key.particles = particles;
+  key.compute_grads = 0; key.backend = ctx->gemm_backend; key.members = 1;
+  key.prior_loc = prior_loc; key.prior_scale = prior_scale; key.mu = loc; key.sigma = scale; key.ws = workspace;
+  key.ws_bytes = workspace_bytes; key.train = 8; key.S = S; key.engine = engine;
+  auto body = [&](const brl_noise* nz, cudaStream_t s) {
+    launch_val_gather(t.d, t.xb, t.yb, B, key2, s);
+    int rc = elbo_step(ctx, t.xb, t.yb, 1, B, loc, scale, BRL_MODE_WS, guide, particles, prior_loc, prior_scale, dataset_size, nz, 0,
+                       t.scal, nullptr, nullptr, nullptr, t.out, rws, rbytes, s, false);
+    if (rc != BRL_OK) return rc;
+    brl_noise nz2 = *nz;
+    nz2.seed += 0x9E3779B97F4A7C15ull;
+    const unsigned long long* dyn = g_dyn;
+    if (dyn) g_dyn = key2;
+    rc = brl_sample_weights(ctx, loc, scale, guide, S, &nz2, v.wsamp, nullptr, v.norms, v.norms_bytes, s);
+    if (rc == BRL_OK)
+      rc = brl_forward(ctx, t.xb, B, S, BRL_MODE_WS, nullptr, nullptr, v.wsamp, 0.f, &nz2, t.out, engine, v.fws, v.fws_bytes, s);
+    g_dyn = dyn;
+    if (rc != BRL_OK) return rc;
+    if (S > 1) launch_aggregate(t.out, S, B, t.agg, s);  // validation_step uses sample 0 as it is for S = 1
+    train_metrics_tail(t, S > 1 ? t.agg : t.out, B * 2, 1, B, 4, s);
+    BRL_CUDA(cudaGetLastError());
+    return BRL_OK;
+  };
+  const bool graphable = engine != BRL_ENGINE_TC_FP16 || tc_capturable(ctx->tc);
+  return train_steps(ctx, a, key, t, [](TrainSetup& su, cudaStream_t s) { su.n = 0; launch_train_setup(su, s); }, body,
+                     (cudaStream_t)stream, graphable, 2);
 }
 
 int brl_mixture_moments(const float* mu_m, const float* sigma_m, int64_t M, int64_t nn, float* mu, float* sigma, void* stream) {

@@ -898,9 +898,9 @@ void launch_train_setup(const TrainSetupAdam& s, cudaStream_t st) {
 }
 
 // windows X[idx[k, w]] -> xb [MB,30,18] as float4 (a window is 135 of them), labels -> yb [MB]; an index outside [0, N) reads
-// nothing (zeros) and marks the step; thread 0 writes step k's Philox key {seed + 0x9E3779B97F4A7C15 (k + 1), sample0, window0}
-__global__ void train_gather_kernel(TrainDesc* d, float* __restrict__ xb, float* __restrict__ yb, long long MB) {
-  const long long k = d->k, N = d->N;
+// nothing (zeros) and marks the step
+__device__ __forceinline__ void gather_batch(TrainDesc* d, long long k, float* __restrict__ xb, float* __restrict__ yb, long long MB) {
+  const long long N = d->N;
   const long long* row = d->idx + k * MB;
   const float4* X = reinterpret_cast<const float4*>(d->X);
   const float* Y = d->Y;
@@ -916,6 +916,11 @@ __global__ void train_gather_kernel(TrainDesc* d, float* __restrict__ xb, float*
     const long long j = row[i];
     yb[i] = (j >= 0 && j < N) ? __ldg(Y + j) : 0.f;
   }
+}
+// the batch of step k; thread 0 writes step k's Philox key {seed + 0x9E3779B97F4A7C15 (k + 1), sample0, window0}
+__global__ void train_gather_kernel(TrainDesc* d, float* __restrict__ xb, float* __restrict__ yb, long long MB) {
+  const long long k = d->k;
+  gather_batch(d, k, xb, yb, MB);
   if (blockIdx.x == 0 && threadIdx.x == 0) {
     d->dyn[0] = d->seed + 0x9E3779B97F4A7C15ull * (unsigned long long)(k + 1);
     d->dyn[1] = d->sample0;
@@ -925,6 +930,26 @@ __global__ void train_gather_kernel(TrainDesc* d, float* __restrict__ xb, float*
 void launch_train_gather(TrainDesc* d, float* xb, float* yb, long long MB, cudaStream_t st) {
   ++g_launch_count;
   train_gather_kernel<<<(unsigned)min((MB * 135 + 255) / 256, (long long)148 * 8), 256, 0, st>>>(d, xb, yb, MB);
+}
+
+// brl_elbo_val_steps: the batch of step k and its two Philox keys, {seed + 0x9E3779B97F4A7C15 (2k + 1), sample0, window0} of the
+// ELBO into d->dyn and {seed + 0x9E3779B97F4A7C15 (2k + 2), sample0, window0} of the predictive draw into key2
+__global__ void val_gather_kernel(TrainDesc* d, float* __restrict__ xb, float* __restrict__ yb, long long B, unsigned long long* key2) {
+  const long long k = d->k;
+  gather_batch(d, k, xb, yb, B);
+  if (blockIdx.x == 0 && threadIdx.x == 0) {
+    const unsigned long long s1 = d->seed + 0x9E3779B97F4A7C15ull * (unsigned long long)(2 * k + 1);
+    d->dyn[0] = s1;
+    d->dyn[1] = d->sample0;
+    d->dyn[2] = d->window0;
+    key2[0] = s1 + 0x9E3779B97F4A7C15ull;
+    key2[1] = d->sample0;
+    key2[2] = d->window0;
+  }
+}
+void launch_val_gather(TrainDesc* d, float* xb, float* yb, long long B, unsigned long long* key2, cudaStream_t st) {
+  ++g_launch_count;
+  val_gather_kernel<<<(unsigned)min((B * 135 + 255) / 256, (long long)148 * 8), 256, 0, st>>>(d, xb, yb, B, key2);
 }
 
 // member m's (loc, scale) pairs at src + m mstride -> the [M,B] planes of the step metrics

@@ -242,6 +242,9 @@ struct TrainSetup {
 };
 void launch_train_setup(const TrainSetup& s, cudaStream_t st);
 void launch_train_gather(TrainDesc* d, float* xb, float* yb, long long MB, cudaStream_t st);
+// brl_elbo_val_steps (M = 1): the gather of step k, which writes the ELBO's Philox key {seed + 0x9E3779B97F4A7C15 (2k + 1), sample0,
+// window0} to d->dyn and the predictive draw's {seed + 0x9E3779B97F4A7C15 (2k + 2), sample0, window0} to key2 [4]
+void launch_val_gather(TrainDesc* d, float* xb, float* yb, long long B, unsigned long long* key2, cudaStream_t st);
 void launch_split_pred(const float* src, long long mstride, int M, long long B, float* pred, float* std, cudaStream_t st);
 void launch_train_tail(TrainDesc* d, const double* scal, int nscal, const double* met, int M, cudaStream_t st);
 // ClippedAdam with the step size d->steps[d->kt] read on the device

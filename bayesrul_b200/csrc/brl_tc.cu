@@ -408,6 +408,7 @@ static void tc_time_end(TcState* st, int k, cudaStream_t stream) {
   if (st->timing) cudaEventRecord(st->evs[k][st->ev_used[k]++].second, stream);
 }
 void tc_trace(TcState* s, long long* buf) { s->trace = buf; }
+bool tc_capturable(const TcState* s) { return !s || (!s->timing && !s->trace); }
 bool tc_available(const TcState* s) { return s && s->status != nullptr; }  // all three nets (the status word exists: sm_100 context)
 bool tc_host_pipeline(const TcState* s) { return tc_available(s) && s->net == BRL_NET_INCEPTION; }
 int tc_status(const TcState* s) {

@@ -15,6 +15,9 @@ int tc_status(const TcState*);  // 0 ok; else the code of the first mbarrier wai
 void tc_timing(TcState*, bool enable);
 void tc_timing_read(TcState*, double ms[2], long long launches[2]);  // [conv, fc]; synchronises the recorded events
 void tc_trace(TcState*, long long* device_buf);
+// false while brl_tc_timing brackets launches with events or brl_tc_trace names a buffer: those host-side hooks act at enqueue
+// time, so a captured forward would replay without them (and with a trace pointer that may be gone); run such forwards eagerly
+bool tc_capturable(const TcState*);
 size_t tc_workspace_bytes(const TcState*, long long B, long long S);
 // returns nullptr on success, else a static error string.  pack_x = false re-uses the fp16 window images a previous
 // call built in the same workspace for the same x (later chunks of MC samples of one batch).

@@ -517,6 +517,36 @@ class Engine:
                                                  scalars.data_ptr(), metrics.data_ptr(), ws.data_ptr(), ws.numel(), self._stream()))
         return dict(scalars=scalars, metrics=metrics)
 
+    def elbo_val_steps(self, X, Y, idx, loc, scale, *, guide: str = "normal", particles: int = 1, S: int = 1, prior_loc: float = 0.0,
+                       prior_scale: float = 1.0, dataset_size: int, seed: int, sample0: int = 0, window0: int = 0,
+                       engine: str = "simt"):
+        """K validation batches of one variational BNN in one call over the device-resident split X [N,30,18], Y [N]; idx [K,B]
+        (int64) names the windows of batch k.  Batch k is elbo_step(X[idx[k]], Y[idx[k]], loc, scale, mode="ws", compute_grads=False)
+        with Noise(seed + 0x9E3779B97F4A7C15 (2k + 1) mod 2**64, sample0, window0) on the current gemm back-end, then
+        sample_weights(S) with Noise(seed + 0x9E3779B97F4A7C15 (2k + 2) mod 2**64, sample0, window0), forward("ws", engine) and,
+        for S > 1, aggregate_predictions, then step_metrics of that (loc, scale).  loc / scale [P] are not changed.  Returns
+        dict(scalars [K,4] = (loss, nll_sum, kl, mse), metrics [K,5] = (nll, mse, sharpness, rmsce, mace)), float64 device tensors.
+        The index range check is the call's only synchronisation; from the third batch of a configuration on, each batch is one
+        CUDA-graph launch."""
+        X, Y, idx, _ = self._train_inputs(X, Y, idx, [(loc, "loc"), (scale, "scale")])
+        if guide not in GUIDE_IDS:
+            raise RuntimeError("Guide unknown. Choose from 'normal', 'radial'.")
+        if engine not in ENGINE_IDS:
+            raise RuntimeError(f"bayesrul_b200: unknown engine {engine!r}")
+        K, B = idx.shape[0], idx.shape[2]
+        scalars = torch.empty(K, 4, dtype=torch.float64, device=self.device)
+        metrics = torch.empty(K, 5, dtype=torch.float64, device=self.device)
+        n = self.lib.brl_workspace_bytes(self.ctx, B, int(S), 7, ENGINE_IDS[engine])
+        if n < 0:
+            raise RuntimeError(f"bayesrul_b200: bad workspace query (B = {B}, S = {S})")
+        ws = self.workspace(n)
+        _lib.check(self.lib.brl_elbo_val_steps(self.ctx, X.data_ptr(), Y.data_ptr(), X.shape[0], idx.data_ptr(), K, B, loc.data_ptr(),
+                                               scale.data_ptr(), GUIDE_IDS[guide], int(particles), int(S), ENGINE_IDS[engine],
+                                               float(prior_loc), float(prior_scale), int(dataset_size), int(seed) & 0xFFFFFFFFFFFFFFFF,
+                                               int(sample0), int(window0), scalars.data_ptr(), metrics.data_ptr(), ws.data_ptr(),
+                                               ws.numel(), self._stream()))
+        return dict(scalars=scalars, metrics=metrics)
+
     def hnn_train_steps(self, X, Y, idx, theta, opt_state, *, step0: int, lr: float, betas=(0.9, 0.999), eps: float = 1e-8,
                         clip_norm: Optional[float] = None, lrd: Optional[float] = None, weight_decay: float = 0.0,
                         p_dropout: float = 0.0, seed: int, sample0: int = 0, window0: int = 0, optimizer: str = "clipped_adam"):

@@ -117,7 +117,9 @@ int brl_destroy(brl_ctx* ctx);
  * train == 3 the buffers of brl_hnn_step_ensemble over S = M members (all of them in one chain of launches where it can),
  * train == 4 the buffers of brl_elbo_step_ensemble over S = M members (the same, one particle lane of M members),
  * train == 5 the buffers of brl_elbo_train_steps over S = M members (its own, then those of code 4, or of code 1 with S = 2 at M = 1),
- * train == 6 the buffers of brl_hnn_train_steps over S = M members (its own, then those of code 3, or of code 1 at M = 1) */
+ * train == 6 the buffers of brl_hnn_train_steps over S = M members (its own, then those of code 3, or of code 1 at M = 1),
+ * train == 7 the buffers of brl_elbo_val_steps with S predictive samples on `engine` (its own for up to 8 particles, then the larger
+ *            of code 1 at S = 2 with engine 0 and the predictive's [S,P] draws and forward workspace) */
 /* 1 when `engine` can run this net's forward on this build, else 0 */
 int brl_engine_available(const brl_ctx* ctx, int engine);
 int64_t brl_workspace_bytes(const brl_ctx* ctx, int64_t B, int64_t S, int train, int engine);
@@ -308,6 +310,29 @@ int brl_hnn_train_steps_adam(brl_ctx* ctx, const float* X /*[N,30,18]*/, const f
                              float* exp_avg_sq, int64_t step0, double lr, double beta1, double beta2, double eps, double weight_decay,
                              float p_dropout, uint64_t seed, int64_t sample0, int64_t window0, double* scalars /*[K,M,2]*/,
                              double* metrics /*[K,M,5]*/, void* workspace, size_t workspace_bytes, void* stream);
+
+/* ---- K validation batches of ONE variational BNN in one call, over a device-resident split (replaces Lightning's validation loop
+ *      of validation_step, bayesian.py:168-197: svi.evaluate_loss, the kl read, bnn.predict(x, S, aggregate = S > 1) and the logged
+ *      metrics, with two .item() reads per batch).  X [N,30,18] (16-byte aligned), Y [N]; idx [K,B] (int64, device).  Batch k does
+ *      exactly, with phi = 0x9E3779B97F4A7C15 and keys mod 2^64:
+ *        1. brl_elbo_step(X[idx[k]], Y[idx[k]], mode BRL_MODE_WS, compute_grads = 0, key {seed + phi (2k + 1), sample0, window0}) on the
+ *           context's gemm back-end -- validation has no fit context, so it samples weights also in LRT / Flipout experiments;
+ *        2. brl_sample_weights(S, key {seed + phi (2k + 2), sample0, window0}), brl_forward(BRL_MODE_WS, engine) of the S draws and,
+ *           for S > 1, brl_aggregate_predictions (S = 1: sample 0 as it is);
+ *        3. brl_step_metrics of that (loc, scale) against Y[idx[k]];
+ *      into scalars[k] = {loss, nll_sum, kl, mse} (brl_elbo_step) and metrics[k] = {nll, mse, sharpness, rmsce, mace}.  The two keys
+ *      per batch continue the reference's per-call key sequence: validation_step draws twice per batch.  loc, scale and any optimiser
+ *      state are left untouched; the host is never synchronised.  Graphs as brl_elbo_train_steps: with step graphs on, the first batch
+ *      of a configuration (sizes, guide, particles, S, engine, back-end, parameter and workspace pointers) runs eagerly, the second is
+ *      captured and every later batch is one graph launch (a captured graph of one kind of call is never replayed by another); with
+ *      brl_tc_timing or brl_tc_trace on, the tensor-core engine's batches run eagerly, with the same results.  An index outside
+ *      [0, N) reads no memory: that batch's rows are NaN.  particles 1..8, S >= 1.  Workspace: brl_workspace_bytes(B, S, 7, engine);
+ *      less returns BRL_ERR_WORKSPACE. */
+int brl_elbo_val_steps(brl_ctx* ctx, const float* X /*[N,30,18]*/, const float* Y /*[N]*/, int64_t N, const int64_t* idx /*[K,B]*/,
+                       int64_t K, int64_t B, const float* loc /*[P]*/, const float* scale /*[P]*/, int guide, int particles, int64_t S,
+                       int engine, float prior_loc, float prior_scale, int64_t dataset_size, uint64_t seed, int64_t sample0,
+                       int64_t window0, double* scalars /*[K,4]*/, double* metrics /*[K,5]*/, void* workspace, size_t workspace_bytes,
+                       void* stream);
 
 /* ---- deep-ensemble mixture moments (models/deepens.py:21-24), [M,n] -> [n] ------------- */
 int brl_mixture_moments(const float* mu_m, const float* sigma_m, int64_t M, int64_t n, float* mu,
