@@ -61,6 +61,7 @@ SIGNATURES = {
     "brl_tc_trace": (_i, [_vp, _vp]),
     "brl_tt_trace": (_i, [_vp, _vp]),
     "brl_workspace_bytes": (_i64, [_vp, _i64, _i64, _i, _i]),
+    "brl_workspace_bytes_val": (_i64, [_vp, _i64, _i64, _i64, _i]),
     "brl_sample_weights": (_i, [_vp, _vp, _vp, _i, _i64, _np, _vp, _vp, _vp, _sz, _vp]),
     "brl_forward": (_i, [_vp, _vp, _i64, _i64, _i, _vp, _vp, _vp, _f, _np, _vp, _i, _vp, _sz, _vp]),
     "brl_predict_moments": (_i, [_vp, _vp, _i64, _i64, _i, _vp, _vp, _f, _np, _vp, _vp, _vp, _vp, _i, _vp, _sz, _vp]),
@@ -83,6 +84,8 @@ SIGNATURES = {
                                      _i64, _vp, _vp, _vp, _sz, _vp]),
     "brl_elbo_val_steps": (_i, [_vp, _vp, _vp, _i64, _vp, _i64, _i64, _vp, _vp, _i, _i, _i64, _i, _f, _f, _i64, C.c_uint64, _i64, _i64,
                                _vp, _vp, _vp, _sz, _vp]),
+    "brl_elbo_val_steps_ensemble": (_i, [_vp, _vp, _vp, _i64, _vp, _i64, _i64, _i64, _vp, _vp, _i, _i, _i64, _i, _f, _f, _i64, C.c_uint64,
+                                        _i64, _i64, _vp, _vp, _vp, _sz, _vp]),
     "brl_mixture_moments": (_i, [_vp, _vp, _i64, _i64, _vp, _vp, _vp]),
     "brl_step_metrics": (_i, [_vp, _vp, _vp, _i64, _vp, _vp, _sz, _vp]),
     "brl_step_metrics_ensemble": (_i, [_vp, _vp, _vp, _i64, _i64, _vp, _vp, _sz, _vp]),

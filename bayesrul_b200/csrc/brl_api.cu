@@ -102,7 +102,8 @@ struct brl_ctx {
     int train;
     float opt[5];
     const void* state[5];
-    // brl_elbo_val_steps (train = 8; mode WS, no gradients): the predictive's MC samples and engine
+    // brl_elbo_val_steps / brl_elbo_val_steps_ensemble (train = 8 / 9; mode WS, no gradients): the predictive's MC samples per
+    // member and engine
     long long S;
     int engine;
     bool operator==(const StepKey& o) const {
@@ -290,24 +291,26 @@ static void carve_train_steps(const NetSpec& n, Carve& c, long long M, long long
   t.hist = c.take<unsigned int>(256 * M);  // the step metrics' scratch, 1024 bytes per member
 }
 
-// brl_elbo_val_steps: the call's descriptor, the predictive draw's Philox key, the gathered batch and one batch's outputs ([S,B,2] of
-// the predictive, or [particles,B,2] of the ELBO step before it), aggregate, logged predictions, scalars and metrics (TrainBufs
-// without gradients), in front of the region that the ELBO step and then the predictive use in turn
-static void carve_val_steps(Carve& c, long long B, long long S, TrainBufs& t, unsigned long long*& key2) {
+// brl_elbo_val_steps{,_ensemble} over M members: the call's descriptor, the predictive draw's Philox key, the batch gathered into M
+// member slots and one batch's outputs ([M S,B,2] of the predictive, or [M particles,B,2] of the ELBO step before it), aggregates,
+// logged predictions, scalars and metrics (TrainBufs without gradients), in front of the region that the ELBO step and then the
+// predictive use in turn
+static void carve_val_steps(Carve& c, long long B, long long M, long long S, TrainBufs& t, unsigned long long*& key2) {
   t.d = c.take<TrainDesc>(1);
   key2 = c.take<unsigned long long>(4);
-  t.xb = c.take<float>(B * 540);
-  t.yb = c.take<float>(B);
+  t.xb = c.take<float>(M * B * 540);
+  t.yb = c.take<float>(M * B);
   t.g0 = t.g1 = t.g2 = nullptr;
-  t.out = c.take<float>(std::max<long long>(GRAPH_MAX_PARTICLES, S) * B * 2);
-  t.agg = c.take<float>(B * 2);
-  t.pred = c.take<float>(B);
-  t.std = c.take<float>(B);
-  t.scal = c.take<double>(4);
-  t.met = c.take<double>(5);
-  t.hist = c.take<unsigned int>(256);  // the step metrics' scratch
+  t.out = c.take<float>(M * std::max<long long>(GRAPH_MAX_PARTICLES, S) * B * 2);
+  t.agg = c.take<float>(M * B * 2);
+  t.pred = c.take<float>(M * B);
+  t.std = c.take<float>(M * B);
+  t.scal = c.take<double>(4 * M);
+  t.met = c.take<double>(5 * M);
+  t.hist = c.take<unsigned int>(256 * M);  // the step metrics' scratch, 1024 bytes per member
 }
-// the predictive's part of that region: S weight draws [S,P], their radial norms [S,n_sites], then brl_forward's workspace
+// the predictive's part of that region: S weight draws [S,P] (S = M S' of the ensemble call: all of them at once), their radial
+// norms [S,n_sites], then brl_forward's workspace
 struct ValPredict {
   float *wsamp, *norms;
   size_t norms_bytes;
@@ -985,6 +988,26 @@ int brl_engine_available(const brl_ctx* ctx, int engine) {
   return 0;
 }
 
+// brl_elbo_val_steps{,_ensemble} over M members: their buffers, then the larger of the ELBO step's workspace (that of
+// brl_elbo_step_ensemble; at M = 1 two particle lanes, Engine.elbo_step's workspace for particles > 1) and the predictive's
+static int64_t val_steps_bytes(const brl_ctx* ctx, long long B, long long M, long long S, int engine) {
+  Carve c(nullptr, 0);
+  TrainBufs t;
+  unsigned long long* key2;
+  carve_val_steps(c, B, M, S, t, key2);
+  Carve p(nullptr, 0);
+  ValPredict v;
+  const int64_t predict = (int64_t)carve_val_predict(ctx, p, B, M * S, engine, v);
+  const int64_t elbo = M == 1 ? brl_workspace_bytes(ctx, B, 2, 1, 0) : brl_workspace_bytes(ctx, B, M, 4, 0);
+  return (int64_t)c.used + std::max(elbo, predict);
+}
+
+int64_t brl_workspace_bytes_val(const brl_ctx* ctx, int64_t B, int64_t M, int64_t S, int engine) {
+  if (!ctx || B <= 0 || M <= 0 || M >= (1 << 16) || S <= 0 || S >= (1 << 16) || M * S >= (1 << 16)) return BRL_ERR_INVALID;
+  if (engine != BRL_ENGINE_SIMT_FP32 && engine != BRL_ENGINE_TC_FP16) return BRL_ERR_INVALID;
+  return val_steps_bytes(ctx, B, M, S, engine);
+}
+
 int64_t brl_workspace_bytes(const brl_ctx* ctx, int64_t B, int64_t S, int train, int engine) {
   if (!ctx || B <= 0 || S <= 0) return BRL_ERR_INVALID;
   const NetSpec& n = *ctx->net;
@@ -997,16 +1020,7 @@ int64_t brl_workspace_bytes(const brl_ctx* ctx, int64_t B, int64_t S, int train,
                                     : (S == 1 ? brl_workspace_bytes(ctx, B, 1, 1, 0) : brl_workspace_bytes(ctx, B, S, 3, 0));
     return (int64_t)c.used + step;
   }
-  if (train == 7) {  // brl_elbo_val_steps: its buffers, then the larger of the ELBO step's workspace and the predictive's
-    TrainBufs t;
-    unsigned long long* key2;
-    carve_val_steps(c, B, S, t, key2);
-    Carve p(nullptr, 0);
-    ValPredict v;
-    const int64_t predict = (int64_t)carve_val_predict(ctx, p, B, S, engine, v);
-    const int64_t elbo = brl_workspace_bytes(ctx, B, 2, 1, 0);  // two particle lanes: Engine.elbo_step's workspace for particles > 1
-    return (int64_t)c.used + std::max(elbo, predict);
-  }
+  if (train == 7) return val_steps_bytes(ctx, B, 1, S, engine);  // brl_elbo_val_steps
   if (train == 3 || train == 4) {  // brl_hnn_step_ensemble / brl_elbo_step_ensemble over S members: the layout of their steps
     carve_forward(n, c, B, 1, ab);
     carve_train(n, c, B, ab);
@@ -2003,6 +2017,71 @@ static int hnn_train_steps(brl_ctx* ctx, const char* fn, const TrainArgs& a, flo
   return train_steps(ctx, a, key, t, [&](TrainSetup& su, cudaStream_t s) { setup(su, col2, s); }, body, st);
 }
 
+// Batch k of M members, all on the windows idx[k]: gather into M member slots -> brl_elbo_step_ensemble (weight sampling, no
+// gradients; brl_elbo_step at M = 1) with key 2k + 1 -> M S weight draws, draw j = m S + s from member m at MC-sample index
+// sample0 + j (brl_predict_moments_ensemble's sample axis), ONE brl_forward of them on `engine` and (S > 1) each member's aggregate,
+// with key 2k + 2 -> the members' step metrics -> row k.  At M = 1 these are the launches of brl_sample_weights(S),
+// brl_forward(S) and brl_aggregate_predictions.  The ELBO step and the predictive share one region of the workspace, one after the
+// other.  A captured batch reads its ELBO key from the descriptor (g_dyn of the capture) and its predictive key from key2: the
+// sampler is captured with g_dyn pointing there.  kind (8: brl_elbo_val_steps, 9: brl_elbo_val_steps_ensemble) keeps the two
+// calls' graphs apart.
+static int elbo_val_steps(brl_ctx* ctx, const char* fn, int kind, const TrainArgs& a, const float* loc, const float* scale, int guide,
+                          int particles, long long S, int engine, float prior_loc, float prior_scale, int64_t dataset_size,
+                          void* workspace, size_t workspace_bytes, cudaStream_t st) {
+  if (int rc = train_args_ok(fn, a)) return rc;
+  const long long M = a.M, B = a.B;
+  BRL_REQUIRE(particles > 0 && particles <= GRAPH_MAX_PARTICLES && dataset_size > 0 && prior_scale > 0.f,
+              std::string(fn) + ": bad particles (1 to 8), dataset size or prior scale");
+  BRL_REQUIRE(S > 0 && S < (1 << 16) && M * S < (1 << 16) && B * 30 < (1ll << 31) / 512, std::string(fn) + ": bad S or B");
+  BRL_REQUIRE(guide == BRL_GUIDE_NORMAL || guide == BRL_GUIDE_RADIAL, "Guide unknown. Choose from 'normal', 'radial'.");
+  BRL_REQUIRE(engine == BRL_ENGINE_SIMT_FP32 || engine == BRL_ENGINE_TC_FP16, std::string(fn) + ": unknown engine");
+  const int64_t need = val_steps_bytes(ctx, B, M, S, engine);
+  if ((int64_t)workspace_bytes < need)
+    return fail(BRL_ERR_WORKSPACE, std::string(fn) + ": workspace too small; need " + std::to_string(need) + " bytes");
+  const NetSpec& n = *ctx->net;
+  const int nsites = 2 * (int)n.layers.size();
+  Carve c(workspace, workspace_bytes);
+  TrainBufs t;
+  unsigned long long* key2;
+  carve_val_steps(c, B, M, S, t, key2);
+  char* rws = (char*)workspace + c.used;
+  const size_t rbytes = workspace_bytes - c.used;
+  Carve pc(rws, rbytes);
+  ValPredict v;
+  carve_val_predict(ctx, pc, B, M * S, engine, v);
+  brl_ctx::StepKey key;
+  memset(&key, 0, sizeof(key));
+  key.B = B; key.dataset_size = dataset_size; key.mode = BRL_MODE_WS; key.guide = guide; key.particles = particles;
+  key.compute_grads = 0; key.backend = ctx->gemm_backend; key.members = (int)M;
+  key.prior_loc = prior_loc; key.prior_scale = prior_scale; key.mu = loc; key.sigma = scale; key.ws = workspace;
+  key.ws_bytes = workspace_bytes; key.train = kind; key.S = S; key.engine = engine;
+  auto body = [&](const brl_noise* nz, cudaStream_t s) {
+    launch_val_gather(t.d, t.xb, t.yb, B, (int)M, key2, s);
+    int rc = elbo_step(ctx, t.xb, t.yb, M, B, loc, scale, BRL_MODE_WS, guide, particles, prior_loc, prior_scale, dataset_size, nz, 0,
+                       t.scal, nullptr, nullptr, nullptr, t.out, rws, rbytes, s, false);
+    if (rc != BRL_OK) return rc;
+    brl_noise nz2 = *nz;
+    nz2.seed += 0x9E3779B97F4A7C15ull;
+    const unsigned long long* dyn = g_dyn;
+    if (dyn) g_dyn = key2;
+    const NoiseRef eps = nref(&nz2, nullptr, KIND_WEIGHT_EPS, 0);
+    if (guide == BRL_GUIDE_NORMAL)
+      launch_sample_normal(loc, scale, n.P, M * S, eps, v.wsamp, nullptr, s, n.P, 1, (int)S);
+    else
+      launch_sample_radial(loc, scale, n.P, M * S, ctx->site_off_dev, nsites, ctx->max_site, eps, nref(&nz2, nullptr, KIND_RADIAL_R, 0),
+                           v.norms, v.wsamp, nullptr, s, n.P, 1, (int)S);
+    rc = brl_forward(ctx, t.xb, B, M * S, BRL_MODE_WS, nullptr, nullptr, v.wsamp, 0.f, &nz2, t.out, engine, v.fws, v.fws_bytes, s);
+    g_dyn = dyn;
+    if (rc != BRL_OK) return rc;
+    if (S > 1) launch_aggregate(t.out, S, B, t.agg, s, (int)M);  // validation_step uses sample 0 as it is for S = 1
+    train_metrics_tail(t, S > 1 ? t.agg : t.out, B * 2, M, B, 4, s);
+    BRL_CUDA(cudaGetLastError());
+    return BRL_OK;
+  };
+  const bool graphable = engine != BRL_ENGINE_TC_FP16 || tc_capturable(ctx->tc);
+  return train_steps(ctx, a, key, t, [](TrainSetup& su, cudaStream_t s) { su.n = 0; launch_train_setup(su, s); }, body, st, graphable, 2);
+}
+
 extern "C" {
 
 int brl_elbo_train_steps(brl_ctx* ctx, const float* X, const float* Y, int64_t N, const int64_t* idx, int64_t K, int64_t M, int64_t B,
@@ -2103,10 +2182,6 @@ int brl_hnn_train_steps_adam(brl_ctx* ctx, const float* X, const float* Y, int64
                          (cudaStream_t)stream);
 }
 
-// Batch k: gather -> brl_elbo_step (weight sampling, no gradients) with key 2k + 1 -> brl_sample_weights, brl_forward and (S > 1)
-// brl_aggregate_predictions with key 2k + 2 -> step metrics -> row k.  The ELBO step and the predictive share one region of the
-// workspace, one after the other.  A captured batch reads its ELBO key from the descriptor (g_dyn of the capture) and its predictive
-// key from key2: the sampler is captured with g_dyn pointing there.
 int brl_elbo_val_steps(brl_ctx* ctx, const float* X, const float* Y, int64_t N, const int64_t* idx, int64_t K, int64_t B, const float* loc,
                        const float* scale, int guide, int particles, int64_t S, int engine, float prior_loc, float prior_scale,
                        int64_t dataset_size, uint64_t seed, int64_t sample0, int64_t window0, double* scalars, double* metrics,
@@ -2114,52 +2189,19 @@ int brl_elbo_val_steps(brl_ctx* ctx, const float* X, const float* Y, int64_t N, 
   BRL_REQUIRE(ctx && loc && scale && workspace, "brl_elbo_val_steps: NULL argument");
   DeviceGuard dg(ctx->device);
   const TrainArgs a{X, Y, N, idx, K, 1, B, 0, seed, sample0, window0, scalars, metrics};
-  if (int rc = train_args_ok("brl_elbo_val_steps", a)) return rc;
-  BRL_REQUIRE(particles > 0 && particles <= GRAPH_MAX_PARTICLES && dataset_size > 0 && prior_scale > 0.f,
-              "brl_elbo_val_steps: bad particles (1 to 8), dataset size or prior scale");
-  BRL_REQUIRE(S > 0 && S < (1 << 16) && B * 30 < (1ll << 31) / 512, "brl_elbo_val_steps: bad S or B");
-  BRL_REQUIRE(guide == BRL_GUIDE_NORMAL || guide == BRL_GUIDE_RADIAL, "Guide unknown. Choose from 'normal', 'radial'.");
-  BRL_REQUIRE(engine == BRL_ENGINE_SIMT_FP32 || engine == BRL_ENGINE_TC_FP16, "brl_elbo_val_steps: unknown engine");
-  const int64_t need = brl_workspace_bytes(ctx, B, S, 7, engine);
-  if ((int64_t)workspace_bytes < need)
-    return fail(BRL_ERR_WORKSPACE, "brl_elbo_val_steps: workspace too small; need " + std::to_string(need) + " bytes");
-  Carve c(workspace, workspace_bytes);
-  TrainBufs t;
-  unsigned long long* key2;
-  carve_val_steps(c, B, S, t, key2);
-  char* rws = (char*)workspace + c.used;
-  const size_t rbytes = workspace_bytes - c.used;
-  Carve pc(rws, rbytes);
-  ValPredict v;
-  carve_val_predict(ctx, pc, B, S, engine, v);
-  brl_ctx::StepKey key;
-  memset(&key, 0, sizeof(key));
-  key.B = B; key.dataset_size = dataset_size; key.mode = BRL_MODE_WS; key.guide = guide; key.particles = particles;
-  key.compute_grads = 0; key.backend = ctx->gemm_backend; key.members = 1;
-  key.prior_loc = prior_loc; key.prior_scale = prior_scale; key.mu = loc; key.sigma = scale; key.ws = workspace;
-  key.ws_bytes = workspace_bytes; key.train = 8; key.S = S; key.engine = engine;
-  auto body = [&](const brl_noise* nz, cudaStream_t s) {
-    launch_val_gather(t.d, t.xb, t.yb, B, key2, s);
-    int rc = elbo_step(ctx, t.xb, t.yb, 1, B, loc, scale, BRL_MODE_WS, guide, particles, prior_loc, prior_scale, dataset_size, nz, 0,
-                       t.scal, nullptr, nullptr, nullptr, t.out, rws, rbytes, s, false);
-    if (rc != BRL_OK) return rc;
-    brl_noise nz2 = *nz;
-    nz2.seed += 0x9E3779B97F4A7C15ull;
-    const unsigned long long* dyn = g_dyn;
-    if (dyn) g_dyn = key2;
-    rc = brl_sample_weights(ctx, loc, scale, guide, S, &nz2, v.wsamp, nullptr, v.norms, v.norms_bytes, s);
-    if (rc == BRL_OK)
-      rc = brl_forward(ctx, t.xb, B, S, BRL_MODE_WS, nullptr, nullptr, v.wsamp, 0.f, &nz2, t.out, engine, v.fws, v.fws_bytes, s);
-    g_dyn = dyn;
-    if (rc != BRL_OK) return rc;
-    if (S > 1) launch_aggregate(t.out, S, B, t.agg, s);  // validation_step uses sample 0 as it is for S = 1
-    train_metrics_tail(t, S > 1 ? t.agg : t.out, B * 2, 1, B, 4, s);
-    BRL_CUDA(cudaGetLastError());
-    return BRL_OK;
-  };
-  const bool graphable = engine != BRL_ENGINE_TC_FP16 || tc_capturable(ctx->tc);
-  return train_steps(ctx, a, key, t, [](TrainSetup& su, cudaStream_t s) { su.n = 0; launch_train_setup(su, s); }, body,
-                     (cudaStream_t)stream, graphable, 2);
+  return elbo_val_steps(ctx, "brl_elbo_val_steps", 8, a, loc, scale, guide, particles, S, engine, prior_loc, prior_scale, dataset_size,
+                        workspace, workspace_bytes, (cudaStream_t)stream);
+}
+
+int brl_elbo_val_steps_ensemble(brl_ctx* ctx, const float* X, const float* Y, int64_t N, const int64_t* idx, int64_t K, int64_t M,
+                                int64_t B, const float* loc, const float* scale, int guide, int particles, int64_t S, int engine,
+                                float prior_loc, float prior_scale, int64_t dataset_size, uint64_t seed, int64_t sample0, int64_t window0,
+                                double* scalars, double* metrics, void* workspace, size_t workspace_bytes, void* stream) {
+  BRL_REQUIRE(ctx && loc && scale && workspace, "brl_elbo_val_steps_ensemble: NULL argument");
+  DeviceGuard dg(ctx->device);
+  const TrainArgs a{X, Y, N, idx, K, M, B, 0, seed, sample0, window0, scalars, metrics};
+  return elbo_val_steps(ctx, "brl_elbo_val_steps_ensemble", 9, a, loc, scale, guide, particles, S, engine, prior_loc, prior_scale,
+                        dataset_size, workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
 int brl_mixture_moments(const float* mu_m, const float* sigma_m, int64_t M, int64_t nn, float* mu, float* sigma, void* stream) {

@@ -600,7 +600,10 @@ void launch_moments_direct(const float* out, long long S, long long B, float* pr
   moments_direct_kernel<<<(unsigned)min((B + 127) / 128, (long long)148 * 8), 128, 0, st>>>(out, S, B, pred, std, ep, al);
 }
 
+// member blockIdx.y: its S outputs at out + m S B 2 (out [M S,B,2], member-major) -> agg + m B 2
 __global__ void aggregate_kernel(const float* __restrict__ out, long long S, long long B, float* agg) {
+  out += blockIdx.y * S * B * 2;
+  agg += blockIdx.y * B * 2;
   for (long long b = blockIdx.x * (long long)blockDim.x + threadIdx.x; b < B; b += (long long)gridDim.x * blockDim.x) {
     float n = 0.f, mean = 0.f, m2 = 0.f, s2 = 0.f, wl = 0.f, wp = 0.f;
     for (long long s = 0; s < S; ++s) {
@@ -619,10 +622,11 @@ __global__ void aggregate_kernel(const float* __restrict__ out, long long S, lon
     agg[2 * b + 1] = sc + logf(-expm1f(-sc));  // inverse softplus (positive_scale=False)
   }
 }
-void launch_aggregate(const float* out, long long S, long long B, float* agg, cudaStream_t st) {
+void launch_aggregate(const float* out, long long S, long long B, float* agg, cudaStream_t st, int members) {
   ++g_launch_count;
-  aggregate_kernel<<<(unsigned)min((B + 127) / 128, (long long)148 * 8), 128, 0, st>>>(out, S, B, agg);
+  aggregate_kernel<<<dim3((unsigned)min((B + 127) / 128, (long long)148 * 8), (unsigned)members), 128, 0, st>>>(out, S, B, agg);
 }
+void launch_aggregate(const float* out, long long S, long long B, float* agg, cudaStream_t st) { launch_aggregate(out, S, B, agg, st, 1); }
 
 __global__ void mixture_kernel(const float* __restrict__ mu_m, const float* __restrict__ sd_m, long long M, long long n,
                                float* mu, float* sd) {
@@ -932,12 +936,13 @@ void launch_train_gather(TrainDesc* d, float* xb, float* yb, long long MB, cudaS
   train_gather_kernel<<<(unsigned)min((MB * 135 + 255) / 256, (long long)148 * 8), 256, 0, st>>>(d, xb, yb, MB);
 }
 
-// brl_elbo_val_steps: the batch of step k and its two Philox keys, {seed + 0x9E3779B97F4A7C15 (2k + 1), sample0, window0} of the
-// ELBO into d->dyn and {seed + 0x9E3779B97F4A7C15 (2k + 2), sample0, window0} of the predictive draw into key2
+// brl_elbo_val_steps{,_ensemble}: the batch of step k into member slot blockIdx.y of xb [M,B,30,18] / yb [M,B] (every member
+// validates the same windows), and its two Philox keys, {seed + 0x9E3779B97F4A7C15 (2k + 1), sample0, window0} of the ELBO into
+// d->dyn and {seed + 0x9E3779B97F4A7C15 (2k + 2), sample0, window0} of the predictive draw into key2
 __global__ void val_gather_kernel(TrainDesc* d, float* __restrict__ xb, float* __restrict__ yb, long long B, unsigned long long* key2) {
   const long long k = d->k;
-  gather_batch(d, k, xb, yb, B);
-  if (blockIdx.x == 0 && threadIdx.x == 0) {
+  gather_batch(d, k, xb + blockIdx.y * B * 540, yb + blockIdx.y * B, B);
+  if (blockIdx.x == 0 && blockIdx.y == 0 && threadIdx.x == 0) {
     const unsigned long long s1 = d->seed + 0x9E3779B97F4A7C15ull * (unsigned long long)(2 * k + 1);
     d->dyn[0] = s1;
     d->dyn[1] = d->sample0;
@@ -947,9 +952,9 @@ __global__ void val_gather_kernel(TrainDesc* d, float* __restrict__ xb, float* _
     key2[2] = d->window0;
   }
 }
-void launch_val_gather(TrainDesc* d, float* xb, float* yb, long long B, unsigned long long* key2, cudaStream_t st) {
+void launch_val_gather(TrainDesc* d, float* xb, float* yb, long long B, int M, unsigned long long* key2, cudaStream_t st) {
   ++g_launch_count;
-  val_gather_kernel<<<(unsigned)min((B * 135 + 255) / 256, (long long)148 * 8), 256, 0, st>>>(d, xb, yb, B, key2);
+  val_gather_kernel<<<dim3((unsigned)min((B * 135 + 255) / 256, (long long)148 * 8), (unsigned)M), 256, 0, st>>>(d, xb, yb, B, key2);
 }
 
 // member m's (loc, scale) pairs at src + m mstride -> the [M,B] planes of the step metrics

@@ -203,6 +203,8 @@ void launch_moments_final_members(const float* state, long long M, long long B, 
 void launch_moments_direct(const float* out, long long S, long long B, float* pred, float* std, float* ep, float* al,
                            cudaStream_t st);
 void launch_aggregate(const float* out, long long S, long long B, float* agg, cudaStream_t st);
+// the aggregates of `members` members in one launch: member m's S outputs at out + m S B 2 (out [members S,B,2]) -> agg [members,B,2]
+void launch_aggregate(const float* out, long long S, long long B, float* agg, cudaStream_t st, int members);
 void launch_mixture(const float* mu_m, const float* sd_m, long long M, long long n, float* mu, float* sd,
                     cudaStream_t st);
 // members > 1: row m of pred / std / y [members,n] -> scalars + m nscal, with the m-th 1024 bytes of the scratch at `hist`
@@ -242,9 +244,10 @@ struct TrainSetup {
 };
 void launch_train_setup(const TrainSetup& s, cudaStream_t st);
 void launch_train_gather(TrainDesc* d, float* xb, float* yb, long long MB, cudaStream_t st);
-// brl_elbo_val_steps (M = 1): the gather of step k, which writes the ELBO's Philox key {seed + 0x9E3779B97F4A7C15 (2k + 1), sample0,
-// window0} to d->dyn and the predictive draw's {seed + 0x9E3779B97F4A7C15 (2k + 2), sample0, window0} to key2 [4]
-void launch_val_gather(TrainDesc* d, float* xb, float* yb, long long B, unsigned long long* key2, cudaStream_t st);
+// brl_elbo_val_steps{,_ensemble}: the gather of step k (idx [K,B]) into each of M member slots, xb [M,B,30,18] and yb [M,B]; it writes
+// the ELBO's Philox key {seed + 0x9E3779B97F4A7C15 (2k + 1), sample0, window0} to d->dyn and the predictive draw's
+// {seed + 0x9E3779B97F4A7C15 (2k + 2), sample0, window0} to key2 [4]
+void launch_val_gather(TrainDesc* d, float* xb, float* yb, long long B, int M, unsigned long long* key2, cudaStream_t st);
 void launch_split_pred(const float* src, long long mstride, int M, long long B, float* pred, float* std, cudaStream_t st);
 void launch_train_tail(TrainDesc* d, const double* scal, int nscal, const double* met, int M, cudaStream_t st);
 // ClippedAdam with the step size d->steps[d->kt] read on the device

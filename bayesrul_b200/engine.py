@@ -455,10 +455,10 @@ class Engine:
         return dict(scalars=scalars, grad=grad, out=out)
 
     # -- K training steps per call over a device-resident dataset ---------------------------------------
-    def _train_inputs(self, X, Y, idx, params):
+    def _train_inputs(self, X, Y, idx, params, shared_idx=False):
         """Checks the dataset, the index tensor and the [M,P] (or [P] for M = 1) parameter / optimiser-state tensors; returns
-        (X, Y, idx [K,M,B], M).  The index range check is one device reduction and one host read: the only synchronisation of
-        a K-step call."""
+        (X, Y, idx [K,M,B], M).  shared_idx: idx must be [K,B], the windows of every member (returned as [K,1,B]).  The index range
+        check is one device reduction and one host read: the only synchronisation of a K-step call."""
         X = _chk(X, self.device, "X")
         if X.dim() != 3 or X.shape[1] != WIN_LENGTH or X.shape[2] != N_FEATURES or X.shape[0] == 0:
             raise RuntimeError(f"bayesrul_b200: X must be [N,{WIN_LENGTH},{N_FEATURES}] with N > 0, got {tuple(X.shape)}")
@@ -475,9 +475,11 @@ class Engine:
         for t, what in params:
             self._theta(t, what, lead)
         idx = _chk(idx, self.device, "idx", dtype=torch.int64)
-        if idx.dim() == 2 and not lead:
+        if shared_idx and idx.dim() != 2:
+            raise RuntimeError(f"bayesrul_b200: idx must be [K,B] (every member sees the same windows), got {tuple(idx.shape)}")
+        if idx.dim() == 2 and (shared_idx or not lead):
             idx = idx.view(idx.shape[0], 1, idx.shape[1])
-        if idx.dim() != 3 or idx.shape[1] != M or idx.shape[0] == 0 or idx.shape[2] == 0:
+        if idx.dim() != 3 or idx.shape[1] != (1 if shared_idx else M) or idx.shape[0] == 0 or idx.shape[2] == 0:
             raise RuntimeError(f"bayesrul_b200: idx must be [K,{M},B] (or [K,B] for one member) with K, B > 0, got {tuple(idx.shape)}")
         lo, hi = torch.stack(torch.aminmax(idx)).tolist()
         if lo < 0 or hi >= N:
@@ -527,13 +529,34 @@ class Engine:
         for S > 1, aggregate_predictions, then step_metrics of that (loc, scale).  loc / scale [P] are not changed.  Returns
         dict(scalars [K,4] = (loss, nll_sum, kl, mse), metrics [K,5] = (nll, mse, sharpness, rmsce, mace)), float64 device tensors.
         The index range check is the call's only synchronisation; from the third batch of a configuration on, each batch is one
-        CUDA-graph launch."""
-        X, Y, idx, _ = self._train_inputs(X, Y, idx, [(loc, "loc"), (scale, "scale")])
+        CUDA-graph launch.
+
+        loc / scale [M,P]: the M seeds of an experiment, validated together on the same batches idx [K,B].  Member m of batch k is
+        the batch above with its elbo_step's particles at sample0 + m particles and its S weight draws at sample0 + m S
+        (elbo_step_ensemble's and predict_moments_ensemble's conventions); the members share every launch they can.  Returns
+        dict(scalars [K,M,4], metrics [K,M,5])."""
+        ens = isinstance(loc, torch.Tensor) and loc.dim() == 2
+        X, Y, idx, M = self._train_inputs(X, Y, idx, [(loc, "loc"), (scale, "scale")], shared_idx=ens)
+        if M == 0:
+            raise RuntimeError("bayesrul_b200: empty ensemble (loc / scale have M = 0 rows)")
         if guide not in GUIDE_IDS:
             raise RuntimeError("Guide unknown. Choose from 'normal', 'radial'.")
         if engine not in ENGINE_IDS:
             raise RuntimeError(f"bayesrul_b200: unknown engine {engine!r}")
         K, B = idx.shape[0], idx.shape[2]
+        if ens:
+            scalars = torch.empty(K, M, 4, dtype=torch.float64, device=self.device)
+            metrics = torch.empty(K, M, 5, dtype=torch.float64, device=self.device)
+            n = self.lib.brl_workspace_bytes_val(self.ctx, B, M, int(S), ENGINE_IDS[engine])
+            if n < 0:
+                raise RuntimeError(f"bayesrul_b200: bad workspace query (B = {B}, M = {M}, S = {S})")
+            ws = self.workspace(n)
+            _lib.check(self.lib.brl_elbo_val_steps_ensemble(
+                self.ctx, X.data_ptr(), Y.data_ptr(), X.shape[0], idx.data_ptr(), K, M, B, loc.data_ptr(), scale.data_ptr(),
+                GUIDE_IDS[guide], int(particles), int(S), ENGINE_IDS[engine], float(prior_loc), float(prior_scale), int(dataset_size),
+                int(seed) & 0xFFFFFFFFFFFFFFFF, int(sample0), int(window0), scalars.data_ptr(), metrics.data_ptr(), ws.data_ptr(),
+                ws.numel(), self._stream()))
+            return dict(scalars=scalars, metrics=metrics)
         scalars = torch.empty(K, 4, dtype=torch.float64, device=self.device)
         metrics = torch.empty(K, 5, dtype=torch.float64, device=self.device)
         n = self.lib.brl_workspace_bytes(self.ctx, B, int(S), 7, ENGINE_IDS[engine])

@@ -123,6 +123,11 @@ int brl_destroy(brl_ctx* ctx);
 /* 1 when `engine` can run this net's forward on this build, else 0 */
 int brl_engine_available(const brl_ctx* ctx, int engine);
 int64_t brl_workspace_bytes(const brl_ctx* ctx, int64_t B, int64_t S, int train, int engine);
+/* the buffers of brl_elbo_val_steps_ensemble over M members with S predictive samples each on `engine` (its own for up to 8
+ * particles, then the larger of code 4 over M members -- code 1 at S = 2 for M = 1 -- and the predictive's [M S,P] draws and
+ * forward workspace: all M S draws are resident at once).  brl_workspace_bytes_val(B, 1, S, e) == brl_workspace_bytes(B, S, 7, e).
+ * BRL_ERR_INVALID for B, M, S <= 0, M S >= 65536 or an unknown engine. */
+int64_t brl_workspace_bytes_val(const brl_ctx* ctx, int64_t B, int64_t M, int64_t S, int engine);
 /* tensor-core engine health: 0 = ok, > 0 = code of the first mbarrier wait that timed out inside a
  * tcgen05 kernel (waits are bounded so a protocol bug ends the kernel instead of hanging the GPU),
  * < 0 = engine unavailable.  Synchronises the device. */
@@ -333,6 +338,26 @@ int brl_elbo_val_steps(brl_ctx* ctx, const float* X /*[N,30,18]*/, const float* 
                        int engine, float prior_loc, float prior_scale, int64_t dataset_size, uint64_t seed, int64_t sample0,
                        int64_t window0, double* scalars /*[K,4]*/, double* metrics /*[K,5]*/, void* workspace, size_t workspace_bytes,
                        void* stream);
+
+/* ---- K validation batches of the M seeds of a BNN experiment in one call (brl_elbo_val_steps for M members that share every launch
+ *      it can).  Every member validates the same windows idx[k] (validation loaders are unshuffled); loc / scale [M,P].  Batch k
+ *      does exactly, with phi = 0x9E3779B97F4A7C15 and keys mod 2^64:
+ *        1. brl_elbo_step_ensemble on M copies of X[idx[k]], Y[idx[k]] (mode BRL_MODE_WS, compute_grads = 0, key {seed + phi (2k + 1),
+ *           sample0, window0}, the context's gemm back-end): member m's particle pt draws at MC-sample index sample0 + m particles + pt;
+ *        2. with key {seed + phi (2k + 2), sample0, window0}: M S weight draws, draw j = m S + s being member m's draw s at MC-sample
+ *           index sample0 + j (brl_predict_moments_ensemble's sample axis), ONE brl_forward(BRL_MODE_WS, engine) of all M S draws over
+ *           the shared batch and, for S > 1, each member's precision-weighted aggregate of its S outputs (S = 1: draw m S as it is);
+ *        3. the step metrics of each member's (loc, scale) against Y[idx[k]];
+ *      into scalars[k] [M,4] = {loss, nll_sum, kl, mse} and metrics[k] [M,5] = {nll, mse, sharpness, rmsce, mace}.  At M = 1 this is
+ *      brl_elbo_val_steps, launch for launch.  Everything else as brl_elbo_val_steps: loc / scale are never written, the host is
+ *      never synchronised, an index outside [0, N) gives NaN rows for every member of that batch, particles 1..8, S >= 1 (M S <
+ *      65536), graphs as there (the two calls never replay each other's graphs, nor graphs of another M).  Workspace:
+ *      brl_workspace_bytes_val(B, M, S, engine); less returns BRL_ERR_WORKSPACE. */
+int brl_elbo_val_steps_ensemble(brl_ctx* ctx, const float* X /*[N,30,18]*/, const float* Y /*[N]*/, int64_t N, const int64_t* idx /*[K,B]*/,
+                                int64_t K, int64_t M, int64_t B, const float* loc /*[M,P]*/, const float* scale /*[M,P]*/, int guide,
+                                int particles, int64_t S, int engine, float prior_loc, float prior_scale, int64_t dataset_size,
+                                uint64_t seed, int64_t sample0, int64_t window0, double* scalars /*[K,M,4]*/, double* metrics /*[K,M,5]*/,
+                                void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- deep-ensemble mixture moments (models/deepens.py:21-24), [M,n] -> [n] ------------- */
 int brl_mixture_moments(const float* mu_m, const float* sigma_m, int64_t M, int64_t n, float* mu,
