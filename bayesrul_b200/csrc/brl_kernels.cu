@@ -138,7 +138,7 @@ __global__ void bwd_act_kernel(const BwdAct p) {
     const long long oidx = img * p.img_stride + (long long)(p.co_off + n) * p.out_P + pp;
     const float g = p.gout[oidx], o = p.outv[oidx];
     float d;
-    if (p.head) d = o > 1e-9f ? g * (1.0f - expf(-o)) : 0.f;
+    if (p.head) d = o > 1e-9f ? g * -expm1f(-o) : 0.f;  // softplus' = 1 - exp(-out), without the cancellation at small out
     else if (p.relu) d = o > 0.f ? g * p.inv_keep : 0.f;
     else d = g * p.inv_keep;
     p.dpre[i] = d;
@@ -355,13 +355,14 @@ __global__ void nll_hnn_kernel(const float* __restrict__ out, const float* __res
   const float invB = 1.0f / (float)B;
   for (long long b = blockIdx.x * (long long)blockDim.x + threadIdx.x; b < B; b += (long long)gridDim.x * blockDim.x) {
     const float loc = out[2 * b], sc = out[2 * b + 1];
-    const float var0 = sc * sc, var = fmaxf(var0, 1e-6f);  // F.gaussian_nll_loss eps clamp
+    // F.gaussian_nll_loss eps clamp: it clamps a copy of var under no_grad, so the gradient flows through with the clamped value
+    const float var = fmaxf(sc * sc, 1e-6f);
     const float d = loc - y[b];
     loss += 0.5 * ((double)logf(var) + (double)d * d / var);
     se += (double)d * d;
     if (gout) {
       gout[2 * b] = d / var * invB;
-      gout[2 * b + 1] = var0 > 1e-6f ? 0.5f * (1.0f / var - d * d / (var * var)) * 2.0f * sc * invB : 0.f;
+      gout[2 * b + 1] = 0.5f * (1.0f / var - d * d / (var * var)) * 2.0f * sc * invB;
     }
   }
   loss = block_sum(loss);

@@ -1282,14 +1282,15 @@ __global__ void __launch_bounds__(256) tt_tail_kernel(const TtTailArgs a_) {
     // ---- likelihood (SURVEY A.6) and its gradient w.r.t. the two outputs
     const float loc = outv[0], sc = outv[1];
     float go[2];
-    if (MODE == TT_PLAIN && a.loss_kind == 1) {  // F.gaussian_nll_loss(loc, y, scale^2): eps clamp 1e-6 on the variance, mean reduction
-      const float var0 = sc * sc, var = fmaxf(var0, 1e-6f), dl = loc - a.y[m], invB = 1.0f / (float)a.B;
+    if (MODE == TT_PLAIN && a.loss_kind == 1) {  // F.gaussian_nll_loss(loc, y, scale^2): eps clamp 1e-6 on the variance (gradient
+                                                 // through the clamped value, as nll_hnn_kernel), mean reduction
+      const float var = fmaxf(sc * sc, 1e-6f), dl = loc - a.y[m], invB = 1.0f / (float)a.B;
       if (lane == 0) {
         nll += 0.5 * ((double)logf(var) + (double)dl * dl / var);
         se += (double)dl * dl;
       }
       go[0] = dl / var * invB;
-      go[1] = var0 > 1e-6f ? 0.5f * (1.0f / var - dl * dl / (var * var)) * 2.0f * sc * invB : 0.f;
+      go[1] = 0.5f * (1.0f / var - dl * dl / (var * var)) * 2.0f * sc * invB;
     } else {
       const float s = sc > 20.0f ? sc : log1pf(expf(sc));
       const float dy = a.y[m] - loc, r = dy / s;
@@ -1306,7 +1307,7 @@ __global__ void __launch_bounds__(256) tt_tail_kernel(const TtTailArgs a_) {
     float d[2], d1[2];
 #pragma unroll
     for (int o = 0; o < 2; ++o) {
-      d[o] = outv[o] > 1e-9f ? go[o] * (1.0f - expf(-outv[o])) : 0.f;
+      d[o] = outv[o] > 1e-9f ? go[o] * -expm1f(-outv[o]) : 0.f;
       d1[o] = MODE == TT_PLAIN ? 0.f : MODE == BRL_MODE_LRT ? (sdo[o] > 0.f ? d[o] * eo[o] / (2.0f * sdo[o]) : 0.f) : d[o] * eo[o];
       gb0[o] += d[o];
       gb1[o] += MODE == BRL_MODE_LRT ? d1[o] : d[o];
